@@ -2,6 +2,7 @@
 """bench.py — CoreSLAM scan-to-map hot path on B200: scan-point map lookups/s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|cfg1|cfg3|cfg4|cfg5]
+                    [--dump-outputs DIR]
 
 A *step* is one CoreSLAMProcessor.Update of the replay: Monte-Carlo pose search over C+1 candidate
 poses x P scan points (the lookups) followed by the HoleMap integration of the same scan.  The N=1
@@ -20,6 +21,11 @@ workload is BASELINE.json configs[1]: synthetic replay, 4096 candidates x 1024-p
 
 N > 1 (torchrun, one rank per GPU): independent replays (sessions) sharded one per GPU, no data-path
 collective, weak scaling; value = lookups of all ranks / max-over-ranks time.
+
+--dump-outputs DIR (cfg1 / cfg2 line): after the K timed steps, rank 0 writes what a caller of the timed Update holds
+after the last of them, as float32: DIR/pose.npy (x, y, theta) and DIR/hole_map.npy (the HoleMap, size x size; the u16
+cells are exact in float32).  The inputs are generated from --seed, so two builds run with the same arguments can be
+compared array for array.
 """
 from __future__ import annotations
 
@@ -789,7 +795,11 @@ def main():
                          "a torch.distributed all_reduce between two kernels (nccl)")
     ap.add_argument("--no-sharded", action="store_true",
                     help="default (cfg2) line: skip the `sharded` block (cfg5 session batches and the cfg4 candidate split over the ranks)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="cfg1 / cfg2 line: write the pose and HoleMap after the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in ("cfg1", "cfg2") or args.streaming):
+        ap.error("--dump-outputs covers the timed replay of the cfg1 / cfg2 line (--impl ours, no --streaming)")
 
     rank, world, local = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     K, W = args.steps, max(args.warmup, 3)
@@ -952,6 +962,11 @@ def main():
         cur += K
         pose_after_timed = proc.get_pose()
         plan = proc.search_plan(P)
+        if args.dump_outputs and rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "pose.npy"), pose_after_timed.astype(np.float32))
+            np.save(os.path.join(args.dump_outputs, "hole_map.npy"),
+                    proc.map_download().reshape(wl["size"], wl["size"]).astype(np.float32))
 
         # ---- per-kernel pass (roofline numerator): same replay continues, events around every kernel
         proc.set_flags(N.FLAG_TIMING)
