@@ -228,9 +228,10 @@ cs_status cs_get_rays(cs_processor* h, int32_t* rays, int32_t n_points);        
 cs_status cs_get_visits(cs_processor* h, int64_t* visits);   /* cells written by the last integration (waits for it) */
 /* Diagnostics (timeline of the last step; the first call enables the recording and returns nothing, later calls
  * copy `count` values).  Records of 8 int64 each:
- *   record b < Size             block b of the rings kernel: [0] cycles start->end, [1] SM id, then %globaltimer
- *                               (ns) at [2] start, [3] dependency wait over, [4] ray preparation seen, [5] rays in
- *                               shared memory, [6] end
+ *   record b < Size             sub-task b of the draw kernel (cs_wedge_kernel): %globaltimer (ns) at [0] task start,
+ *                               [1] candidates of its first piece found, [2] task end; [3] most candidates of a piece
+ *                               | general path used << 16 | pieces << 20 | first ring << 32; %globaltimer of its block
+ *                               at [4] block start, [5] rays ready, [6] task table ready; [7] SM id | block << 16
  *   record Size + b, b < 8192   block b of the search kernel: [0] SM id, %globaltimer at [1] start, [2] dependency
  *                               wait over, [3] scan staged, [4] warp 0 done, [5] block done, [6] pose published
  *                               (last block only), [7] 1 for the block that published */

@@ -420,7 +420,8 @@ class Processor:
         return int(v.value)
 
     def ring_cycles(self, count: Optional[int] = None) -> np.ndarray:
-        """Diagnostics (first call enables recording): (rings, 8) cycle stamps of the last rings kernel."""
+        """Diagnostics (first call enables recording): (count, 8) timeline records of the last step; record b < size
+        is sub-task b of the draw kernel (cs_wedge_kernel), see cs_get_ring_cycles in include/coreslam_b200.h."""
         count = self.size if count is None else count
         out = np.zeros(count * 8, dtype=np.int64)
         self._ck(N.lib().cs_get_ring_cycles(self._h, out.ctypes.data_as(C.POINTER(C.c_int64)), count * 8))

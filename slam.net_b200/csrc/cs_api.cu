@@ -265,18 +265,6 @@ StagePlan plan_stage(int n_points, int n_cand_floats3, bool with_cs) {
   return p;
 }
 
-// Upper bound on the ring count of a scan: |rotated, scaled point| + half the hole width, plus rounding slack.
-// The 512-thread instances of the rings kernel use more dynamic shared memory than the default limit.
-cudaError_t rings_allow_shared_memory() {
-  const int one = (int)CS_RING_SMEM(CS_RING_MAX_THREADS, CS_RING_MAX_SLOT_BITS, 0);
-  const int two = (int)CS_RING_SMEM(CS_RING_MAX_THREADS, CS_RING_MAX_SLOT_BITS, 1);
-  cudaError_t e = cudaFuncSetAttribute(cs_rings_kernel<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, one);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(cs_rings_kernel<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, one);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(cs_rings_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, two);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(cs_rings_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, two);
-  return e;
-}
-
 // Wedge integration (cs_wedge.cuh): levels a ray of a size x size map can reach, the words of one half of CsSession::w_top,
 // and the dynamic shared memory of the kernel (one 16-bit count per level and key sector).
 int wedge_levels(int size) {
@@ -289,6 +277,7 @@ size_t wedge_top_words(int size) { return (size_t)wedge_levels(size) * (CS_W_SEC
 size_t wedge_smem(int) { return 0; }
 cudaError_t wedge_allow_shared_memory();
 
+// Upper bound on the ring count of a scan: |rotated, scaled point| + half the hole width, plus rounding slack.
 int rings_hint_of(int size, float scale, float hole_width, double max_range) {
   if (!(max_range == max_range) || max_range > 1e30) return size;
   double cells = max_range * (double)scale * 1.00001 + 0.5 * (double)hole_width * (double)scale + 4.0;
@@ -326,12 +315,12 @@ double max_range_of(const float* points, int n) {
 
 // What a step is launched on: one processor (n_sessions = 1) or a batch of independent sessions
 // (grid.y = n_sessions; every kernel indexes its session by blockIdx.y).
-// Experiment knobs (environment, read once): CS_TUNE_SEARCH_WARPS (2/4/8), CS_TUNE_RING_SPAN, CS_TUNE_RING_THREADS.
+// Experiment knobs (environment, read once; tools/README.md lists them), e.g. CS_TUNE_SEARCH_WARPS (2/4/8).
 // Unset = the built-in choice.  They change launch shapes only, never results.
 struct Tune {
-  int search_warps = 0, ring_span = 0, ring_threads = 0, ring_slot_bits = 0, ring_blocks_per_sm = 0, ring_small = 0;
+  int search_warps = 0;
   int search2 = 0, s2_points = 0, s2_threads = 0, s2_min_cand = 0, s2_sort_one_block = 0, copy_stream = 0;
-  int integrate = 0, w_general = 0, w_blocks = 0, w_prefetch = 0, w_sub = 0, w_prev = 0, w_carveout = 0, s2_carveout = 0;
+  int w_general = 0, w_blocks = 0, w_prefetch = 0, w_sub = 0, w_prev = 0, w_carveout = 0, s2_carveout = 0;
   int spin_ms = 0, fault = 0, w_resident = 0, spec = 0, presort = 0;
   Tune() {
     auto geti = [](const char* name) { const char* v = getenv(name); return v ? atoi(v) : 0; };
@@ -342,7 +331,6 @@ struct Tune {
     s2_sort_one_block = geti("CS_TUNE_S2_SORT_ONE_BLOCK");  // 1: sort generated candidates with one block whenever they fit
     copy_stream = geti("CS_TUNE_COPY_STREAM");  // -1: cs_update stages its inputs on the main stream
     s2_min_cand = geti("CS_TUNE_S2_MIN_CAND");  // fewest candidates the slab search is used for
-    integrate = geti("CS_TUNE_INTEGRATE");      // 1: the rings kernel draws the scan instead of the wedge kernel (A/B runs)
     w_general = geti("CS_TUNE_W_GENERAL");      // 1: every task of the wedge kernel takes its general path (tests)
     w_blocks = geti("CS_TUNE_W_BLOCKS");        // blocks of the wedge kernel per session
     w_prefetch = geti("CS_TUNE_W_PREFETCH");    // -1: no L2 prefetch of the map around the pose
@@ -355,11 +343,6 @@ struct Tune {
     w_sub = geti("CS_TUNE_W_SUB");              // most warps a task's rings are split over (1, 2, 4, 8)
     spin_ms = geti("CS_TUNE_SPIN_MS");          // CS_FLAG_DEBUG_BOUNDED_SPIN: milliseconds a device-side poll lasts (default 2000)
     fault = geti("CS_TUNE_FAULT");              // tests of the bounded polls: 1 = the draw kernel waits for a pose tag nobody publishes
-    ring_span = geti("CS_TUNE_RING_SPAN");
-    ring_threads = geti("CS_TUNE_RING_THREADS");
-    ring_slot_bits = geti("CS_TUNE_RING_SLOT_BITS");
-    ring_small = geti("CS_TUNE_RING_SMALL");  // -1: batches use the 512-thread instance of the rings kernel too
-    ring_blocks_per_sm = geti("CS_TUNE_RING_BLOCKS_PER_SM");  // resident blocks per SM the one-session rings grid is capped at
   }
 };
 const Tune& tune() { static Tune t; return t; }
@@ -505,16 +488,16 @@ struct LaunchCtx {
   volatile unsigned* stuck_dev = nullptr;  // CS_FLAG_DEBUG_BOUNDED_SPIN: device address of the mapped-host word (CsSpin)
   unsigned long long* spec = nullptr;      // glue table of the handle (one session alone)
   cudaEvent_t ev_pose;   // optional: recorded once the pose is out
-  cudaEvent_t ev_done;   // optional: recorded after the rings kernel
+  cudaEvent_t ev_done;   // optional: recorded after the draw kernel
 };
 
 enum { CS_PHASE_SEARCH = 1, CS_PHASE_FINISH = 2, CS_PHASE_ALL = 3 };
 
-// One step on the stream: [search kernel, whose last block publishes the pose and prepares the rays] or
-// [set-up kernel] -> (big scans: multi-block ray preparation) -> rings kernel.  Split phases (multi-GPU
-// candidate split): SEARCH launches only the search over this GPU's candidate slice and leaves the packed
-// arg-min in CsSession::key[parity]; FINISH — after the caller's 8-byte min exchange — launches the set-up
-// kernel (which decodes the reduced key) and the rings kernel.
+// One step on the stream: [search kernel, whose last block publishes the pose] or [set-up kernel] -> draw
+// kernel (cs_wedge_kernel, whose first blocks prepare the rays).  Split phases (multi-GPU candidate split):
+// SEARCH launches only the search over this GPU's candidate slice and leaves the packed arg-min in
+// CsSession::key[parity]; FINISH — after the caller's 8-byte min exchange — launches the set-up kernel
+// (which decodes the reduced key) and the draw kernel.
 // Launch with the programmatic-stream-serialization attribute: the kernel may become resident while its
 // predecessor in the stream drains; every kernel here calls cs_pdl_wait() before it reads anything the
 // predecessor wrote.
@@ -653,7 +636,7 @@ cudaError_t launch_step_ctx(const LaunchCtx& c, CsStepArgs a, int n_points, int 
   }
   // the pose is out once this kernel has finished
   if (c.ev_pose) cudaEventRecord(c.ev_pose, c.stream);
-  if (draws && tune().integrate != 1 && c.w_slot) {
+  if (draws) {
     // The wedge kernel: (ring range x angular wedge) tasks, one warp each (cs_wedge.cuh).  The first blocks prepare the rays,
     // 128 each (big scans: bigger groups, so that at most 64 blocks prepare); every warp of the grid then takes tasks (small
     // scans: by block tickets; otherwise round-robin).  One session alone gets a resident wave — three blocks per SM of the
@@ -696,50 +679,6 @@ cudaError_t launch_step_ctx(const LaunchCtx& c, CsStepArgs a, int n_points, int 
     });
     if (e != cudaSuccess) return e;
     (*c.launches)++;
-  } else if (draws) {
-    int threads = ((n_points + CS_RING_RPT - 1) / CS_RING_RPT + 31) / 32 * 32;
-    if (tune().ring_threads >= 32) threads = tune().ring_threads / 32 * 32;
-    if (threads < 32) threads = 32;
-    if (threads > CS_RING_MAX_THREADS) threads = CS_RING_MAX_THREADS;
-    if (rings < 1) rings = 1;
-    // One session alone: a grid of at most one resident wave (2 blocks per SM) whose blocks draw work units of
-    // `span` rings from a ticket counter.  A batch of sessions: one unit of 64 rings per block, grid.y = sessions (measured on cfg5: 8 -> 64 rings per unit, a 2048-entry slot table and the small-block instance of the kernel take the rings from 4.8 to 2.8 ms per step).
-    const bool dynamic = c.n_sessions == 1;
-    // scans of several rounds (more rays than 2 x threads): two rings per unit, so that a round's rays serve two rings and
-    // the second ring's evaluation hides the first one's map loads (cfg3: 208 -> 183 us; 4 and more rings per unit lose to imbalance)
-    const bool multi_round = n_points > threads * CS_RING_RPT;
-    // Batches: 64 rings per block; 32 for batches of at most 256 sessions, where the grid is only a wave or two of blocks and
-    // shorter blocks leave a shorter tail (128 sessions, the per-GPU share of cfg5 on eight GPUs: 0.49 -> 0.455 ms per step).
-    int span = dynamic ? (multi_round ? 2 : 1) : (c.n_sessions <= 256 ? 32 : 64);
-    if (tune().ring_span > 0) span = tune().ring_span;
-    if (span < 1) span = 1;
-    if (span > CS_RING_MAX_SPAN) span = CS_RING_MAX_SPAN;
-    a.ring_span = span;
-    a.ring_dynamic = dynamic ? 1 : 0;
-    // slot table: a session alone keeps every ring up to k = 1024 in one window; a batch trades windows on its outer
-    // rings for resident blocks (shared memory per block is what limits them)
-    a.ring_slot_bits = dynamic ? CS_RING_MAX_SLOT_BITS : 11;
-    if (tune().ring_slot_bits >= 8 && tune().ring_slot_bits <= CS_RING_MAX_SLOT_BITS) a.ring_slot_bits = tune().ring_slot_bits;
-    int blocks = (rings + span - 1) / span;
-    const int per_sm = tune().ring_blocks_per_sm > 0 ? tune().ring_blocks_per_sm : 2;
-    if (dynamic && blocks > per_sm * c.num_sms) blocks = per_sm * c.num_sms;
-    // the first blocks also prepare the rays, 128 each (one warp per SM sub-partition: the preparation is a
-    // latency chain, not throughput); big scans use bigger groups so that at most 64 blocks prepare
-    int group = (((n_points + 63) / 64) + 31) / 32 * 32;
-    if (group < 128) group = 128;
-    a.prep_group = group;
-    const int nprep = (n_points + group - 1) / group;
-    if (blocks < nprep) blocks = nprep;
-    const bool small_rings = !dynamic && !multi_round && threads <= CS_RING_SMALL_THREADS && tune().ring_small >= 0;
-    dispatch_layout(c.tiled, [&](auto T) {
-      constexpr bool tiled = decltype(T)::value;
-      e = launch_pdl(small_rings ? cs_rings_kernel<tiled, true, false>
-                                 : (multi_round ? cs_rings_kernel<tiled, false, true> : cs_rings_kernel<tiled, false, false>),
-                     dim3((unsigned)blocks, (unsigned)c.n_sessions), dim3(threads),
-                     CS_RING_SMEM(threads, a.ring_slot_bits, multi_round), c.stream, c.d_sess, a);
-    });
-    if (e != cudaSuccess) return e;
-    (*c.launches)++;
   }
   // ---- production mode: the next scan's candidate sort, queued in the shadow of this scan's draw kernel (see Presort).  Not
   // under CS_FLAG_TIMING (the events around the stages would count it to the wrong one).
@@ -768,7 +707,7 @@ cudaError_t launch_step_ctx(const LaunchCtx& c, CsStepArgs a, int n_points, int 
 }
 
 // UpdateObstacleMap (CoreSLAMProcessor.cs:540-593) for n_sessions sessions: the ray kernel (hits + no-hit marks), then the
-// sweep over the marked tiles.  Plain stream order: both follow the rings kernel of the same step.
+// sweep over the marked tiles.  Plain stream order: both follow the draw kernel of the same step.
 cudaError_t launch_obstacle_update(cudaStream_t stream, const CsSession* d_sess, const CsObstacle* d_obst, const CsObstacle& ho,
                                    const CsStepArgs& a, int n_points, int n_sessions, int num_sms, uint64_t* launches) {
   const int warps = CS_OBST_RAY_THREADS / 32;
@@ -877,7 +816,7 @@ cs_status collect_timing(cs_processor* h, bool had_h2d) {
   cs_timing& t = h->last_timing;
   if (had_h2d) { cudaEventElapsedTime(&ms, h->tm.ev[0], h->tm.ev[1]); t.h2d_ms = ms; } else t.h2d_ms = 0;
   cudaEventElapsedTime(&ms, h->tm.ev[1], h->tm.ev[2]); t.search_ms = ms;
-  cudaEventElapsedTime(&ms, h->tm.ev[2], h->tm.ev[3]); t.integrate_ms = ms;  // rings kernel (+ set-up kernels of big scans)
+  cudaEventElapsedTime(&ms, h->tm.ev[2], h->tm.ev[3]); t.integrate_ms = ms;  // the draw kernel
   t.finalize_ms = 0.f;
   cudaEventElapsedTime(&ms, h->tm.ev[0], h->tm.ev[4]); t.total_device_ms = ms;
   t.obstacle_ms = 0.f;
@@ -971,7 +910,6 @@ cs_status cs_create(const cs_config* cfg, cs_processor** out) {
   CS_CREATE_CUDA(cudaMalloc(&h->d_batch_max, (size_t)kRayCopies * h->batch_stride * sizeof(int)));
   CS_CREATE_CUDA(cudaMalloc(&h->d_prep_words, (size_t)2 * kRayCopies * 16 * sizeof(unsigned long long)));
   CS_CREATE_CUDA(cudaMemset(h->d_prep_words, 0, (size_t)2 * kRayCopies * 16 * sizeof(unsigned long long)));
-  CS_CREATE_CUDA(rings_allow_shared_memory());
   CS_CREATE_CUDA(cudaMalloc(&h->d_w_rk, (size_t)h->ray_stride * sizeof(int2)));
   CS_CREATE_CUDA(cudaMalloc(&h->d_w_bkey, (size_t)(h->ray_stride / 32 + 1) * sizeof(float2)));
   CS_CREATE_CUDA(cudaMalloc(&h->d_w_top, (size_t)3 * wedge_top_words(h->size) * sizeof(int)));
@@ -2463,7 +2401,6 @@ cs_status cs_batch_create(const cs_config* cfgs, int32_t n_sessions, cs_batch** 
     ok = ok && cudaHostGetDevicePointer((void**)&b->d_stuck, b->h_stuck, 0) == cudaSuccess;
     if (ok) memset(b->h_stuck, 0, 64);
   }
-  ok = ok && rings_allow_shared_memory() == cudaSuccess;
   if (!ok) {
     cudaError_t e = cudaGetLastError();
     bfail(nullptr, e == cudaErrorMemoryAllocation ? CS_ERR_OUT_OF_MEMORY : CS_ERR_CUDA, "cs_batch_create: %s", cudaGetErrorString(e));

@@ -3,12 +3,14 @@
 //   cs_search_kernel     CalculateDistanceSISD + MonteCarloSearch + ParallelMonteCarloSearch arg-min
 //                        (CoreSLAM/CoreSLAMProcessor.cs:226-259, 624-653, 674-710)
 //                        The last block to finish also runs the Update glue (:717-752: gate, searchPose,
-//                        NormalizeAngle, state), publishes the pose and prepares the rays, so the pose
-//                        leaves the device at the end of the search kernel itself.
-//   cs_setup_kernel      the same glue + per-ray part of UpdateHoleMap / DrawLaserRayOnHoleMap / ClipRay
-//                        (:496-534, 359-402, 320-345) on its own, for scans without a search and big scans
-//   cs_rings_kernel      the draw loop (:404-442) re-organised by rings (see below) so the ordered
-//                        read-modify-write is exact without atomics or sorting
+//                        NormalizeAngle, state) and publishes the pose, so the pose leaves the device at
+//                        the end of the search kernel itself.
+//   cs_sort_kernel,      the slab search: the same arg-min over candidates sorted by heading (many candidates)
+//   cs_search2_kernel
+//   cs_setup_kernel      the same glue on its own, for steps without a search kernel that publishes
+//
+// The draw kernel that follows (UpdateHoleMap / ClipRay / DrawLaserRayOnHoleMap, :496-534, 320-345,
+// 359-443) is cs_wedge_kernel in cs_wedge.cuh; the closed-form ray set-up it calls (cs_ray_from_point) is here.
 //
 // No tensor cores: nothing here is a contraction.  The search is a 2-byte gather per (candidate, point)
 // out of an L2-resident map; the integration is an ordered 2-byte read-modify-write per visited cell.
@@ -97,23 +99,24 @@ struct CsSession {  // one CoreSLAMProcessor, device resident
   int* batch_max;              // per 32 consecutive rays: largest dxc of a valid ray, -1 if none; ray_copies copies of
                                // batch_stride entries
   int ray_copies, ray_stride, batch_stride, pad1;
-  unsigned long long* prep_words;  // [2 slots][ray_copies] words, 128 B apart: preparing blocks of the rings kernel that are
+  unsigned long long* prep_words;  // [2 slots][ray_copies] words, 128 B apart: preparing blocks of the draw kernel that are
                                    // done; slot = step id & 1, re-armed for the next step by this step's publishing thread
   int* ray_dbg;                // optional 6 ints per ray (x1,y1,x2,y2,xp,yp), CS_FLAG_DEBUG_RAYS
   int* distances;              // optional n_cand+1
-  long long* ring_cycles;      // optional diagnostics: cycles each ring's block spent in the rings kernel
+  long long* ring_cycles;      // set by cs_get_ring_cycles but read by no kernel (they record through CsStepArgs::diag);
+                               // kept so that the polled words below stay where they are relative to 128-byte lines
   float cur_pose[3];           // pose the current integration draws from (Pose after :745-747)
   float cur_cs[2];             // its (cos, sin), unscaled
   unsigned search_done;        // blocks of the running search kernel that have finished
   unsigned pad0;
   // The pose the current integration draws from, published without a fence: five 8-byte words {float bits, step id},
-  // each single-copy atomic — x, y, theta (Pose after :745-747), cos, sin (unscaled).  The rings kernel's blocks are
+  // each single-copy atomic — x, y, theta (Pose after :745-747), cos, sin (unscaled).  The draw kernel's blocks are
   // resident before the search ends and poll the words for their step id.
   unsigned long long ll_pose[5];
   unsigned long long pad2;
   long long visits_slot[2];    // cells written by the integration of step id & 1 = sum over valid rays of dxc+1
-  unsigned ring_ticket[2];     // work-unit tickets of the rings kernel; slot = step id & 1, re-armed for the next step by
-                               // the publishing thread of this step
+  unsigned ring_ticket[2];     // block tickets of the draw kernel (small scans); slot = step id & 1, re-armed for the next
+                               // step by the publishing thread of this step
   // ---- scratch of the slab search (cs_sort_kernel + cs_search2_kernel; one session alone, many candidates)
   float4* s2_sorted;            // [2][s2_cap]: this step's candidates in ascending order of heading offset, as
                                 // (x, y, theta [offsets or absolute pose], flat index bits); slot = CsStepArgs::s2_slot
@@ -148,18 +151,15 @@ struct CsStepArgs {  // by-value kernel argument; session j uses element j of ev
   int cand_count;  // number of flat indices evaluated by this GPU, normally n_cand+1
   int fuse_publish;  // search kernel: its last block runs the Update glue and publishes the pose
   int max_ring_hint; // rings the host launched blocks for, minus one
-  int ring_span;     // rings per work unit of the rings kernel
-  int prep_group;    // rays prepared by each of the first blocks of the rings kernel (multiple of 32)
-  int ring_dynamic;  // 1: blocks draw further units from CsSession::ring_ticket (one session, grid <= one wave)
-  int ring_slot_bits; // log2 of the rings kernel's slot table (<= CS_RING_MAX_SLOT_BITS)
+  int prep_group;    // rays prepared by each of the first blocks of the draw kernel (multiple of 32)
   int search_chunk;  // points staged in shared memory per pass of the search kernel (<= CS_SEARCH_CHUNK)
   unsigned step_id;  // nonzero, different for consecutive steps on the same session(s): tags ll_pose, selects the counter slots
   long long* visits_out;  // optional device slot that receives the visit count
   volatile unsigned* stuck_flag;  // CS_FLAG_DEBUG_BOUNDED_SPIN: mapped-host word that receives the CsStuckSite of a poll
   long long spin_ns;              // that gave up after spin_ns nanoseconds (0: polls are unbounded, the normal build of a step)
-  long long* diag;        // optional diagnostics buffer (8 values per block of the rings kernel, then 8 per block of
+  long long* diag;        // optional diagnostics buffer (8 values per task of the draw kernel, then 8 per block of
                           // the search kernel), see cs_get_ring_cycles
-  int diag_rings;         // records reserved for the rings kernel in diag
+  int diag_rings;         // records reserved for the draw kernel in diag
   // slab search (cs_search2_kernel): block (c, s) evaluates points [c*s2_points, ...) for sorted candidates [s*s2_slab, ...)
   int s2_points;          // points per cluster (<= CS_S2_MAX_POINTS)
   int s2_slab;            // candidates per slab (multiple of 32, = threads per block)
@@ -427,7 +427,7 @@ __device__ __forceinline__ int cs_ray_minor(const CsRay& r, int x) {
 // ---------------------------------------------------------------------------------------------------
 // Update glue (:717-752) — run by ONE thread.  cs_glue_pose decodes the arg-min, applies the search gate
 // and normalises the angle; cs_glue_publish stores state / result / flag and leaves the pose and its
-// (cos, sin) in the session's cur_pose / cur_cs for the ray preparation and the rings kernel.
+// (cos, sin) in the session's cur_pose / cur_cs for the kernels that follow.
 // ---------------------------------------------------------------------------------------------------
 struct CsGlue {
   float pose[3];
@@ -486,7 +486,7 @@ __device__ __forceinline__ void cs_glue_publish(CsSession& S, const CsStepHeader
   }
   S.cur_pose[0] = g.pose[0]; S.cur_pose[1] = g.pose[1]; S.cur_pose[2] = g.pose[2];
   S.cur_cs[0] = g.cs[0]; S.cur_cs[1] = g.cs[1];
-  // re-arm the NEXT step's counters (kernel boundaries order this before that step's rings kernel; this step's
+  // re-arm the NEXT step's counters (kernel boundaries order this before that step's draw kernel; this step's
   // were re-armed by the previous step's publisher, or are zero from the start)
   {
     const unsigned nslot = (a.step_id + 1u) & 1u;
@@ -551,29 +551,6 @@ __device__ __forceinline__ CsRay cs_ray_from_point(const CsRayFrame& f, const fl
   return r;
 }
 
-// Per-ray part of UpdateHoleMap (:517-530) + ClipRay + the prologue of DrawLaserRayOnHoleMap for rays
-// first, first+stride, ... < n.  Returns this thread's (max dxc, visits) contribution.
-__device__ __forceinline__ void cs_prepare_rays(CsSession& S, const float2* __restrict__ points, float2 p_first, int n, int first,
-                                                int stride, const float pose[3], const float cs[2], bool write_dbg,
-                                                long long& visits) {
-  const CsRayFrame f = cs_ray_frame(S, pose, cs);
-  for (int i = first; i < n; i += stride) {
-    const float2 p = (i == first) ? p_first : points[i];  // the first one was loaded while the pose was awaited
-    const CsRay r = cs_ray_from_point(f, p, (write_dbg && S.ray_dbg) ? S.ray_dbg + 6 * (size_t)i : nullptr);
-    if (r.flags & 1) visits += (long long)r.dxc + 1;
-    {
-      const int4 q = cs_pack_ray(r);
-      for (int c = 0; c < S.ray_copies; c++) S.rays[(size_t)c * S.ray_stride + i] = q;
-    }
-    {  // the 32 lanes of a warp hold 32 consecutive rays (first and stride are multiples of 32 apart)
-      int bm = (r.flags & 1) ? r.dxc : -1;
-      bm = __reduce_max_sync(__activemask(), bm);
-      if ((i & 31) == 0)
-        for (int c = 0; c < S.ray_copies; c++) S.batch_max[(size_t)c * S.batch_stride + (i >> 5)] = bm;
-    }
-  }
-}
-
 // The one exchange step of the candidate split (SURVEY 8e), run by the publishing thread: this rank's packed arg-min goes
 // into every rank's table (8-byte stores over NVLink / peer-mapped memory, key first, then the tag behind a system fence),
 // then the thread waits until its own table holds the world's keys of this exchange and takes their minimum — the same
@@ -603,7 +580,7 @@ __device__ __forceinline__ unsigned long long cs_exchange_min(const CsStepArgs& 
   return best;
 }
 
-// Glue + publish by one thread (the rays are prepared by the first blocks of the rings kernel).
+// Glue + publish by one thread (the rays are prepared by the first blocks of the draw kernel).
 __device__ __forceinline__ void cs_publish(CsSession& S, const CsStepHeader& hdr, const CsStepArgs& a, const float* cand,
                                            CsDevResult* result, bool have_guess = false, unsigned long long guess = 0ull) {
   long long* d = a.diag ? a.diag + ((size_t)a.diag_rings + CS_DIAG_SEARCH_BLOCKS - 1) * 8 : nullptr;  // (diagnostics: one session)
@@ -673,7 +650,7 @@ cs_search_kernel(CsSession* __restrict__ sessions, CsStepArgs a) {
   const int nwarps = blockDim.x >> 5;
   const int chunk = a.search_chunk;
 
-  // This grid depends on the previous step's rings kernel (cs_pdl_wait below); the next kernel of this step may
+  // This grid depends on the previous step's draw kernel (cs_pdl_wait below); the next kernel of this step may
   // become resident once every block here is past that wait.
   long long* tl = nullptr;  // timeline record of this block (diagnostics)
   if (a.diag && blockIdx.y == 0 && blockIdx.x < CS_DIAG_SEARCH_BLOCKS && threadIdx.x == 0) {
@@ -694,7 +671,7 @@ cs_search_kernel(CsSession* __restrict__ sessions, CsStepArgs a) {
   // ---- everything that does not depend on the previous step goes first: the step's inputs (scan, header,
   // candidate table) were uploaded before the kernels in front, and size / scale / seed / sigmas are host-owned
   // constants.  When this grid becomes resident early (programmatic dependent launch) all of it overlaps the tail
-  // of the previous step's rings kernel.
+  // of the previous step's draw kernel.
   const int P = hdr.n_points;
   const int size = S.size, pitch_tiles = S.pitch_tiles;
   const uint16_t* __restrict__ map = S.map;
@@ -726,8 +703,8 @@ cs_search_kernel(CsSession* __restrict__ sessions, CsStepArgs a) {
     }
   }
 
-  cs_pdl_wait();  // the previous step (its rings kernel: map, and through it the search kernel: state) is complete
-  // Only now may this step's rings kernel become resident: it does not wait for this grid as a whole but polls
+  cs_pdl_wait();  // the previous step (its draw kernel: map, and through it the search kernel: state) is complete
+  // Only now may this step's draw kernel become resident: it does not wait for this grid as a whole but polls
   // counters that the previous step's publishing thread re-armed, so it must not run ahead of that step's end.
   cs_pdl_launch_dependents();
   if (tl) tl[2] = cs_globaltimer();
@@ -1231,512 +1208,6 @@ cs_setup_kernel(CsSession* __restrict__ sessions, CsStepArgs a) {
   const float* cand = a.cand ? a.cand + (size_t)sj * a.cand_stride : nullptr;
   CsDevResult* result = a.result ? a.result + (size_t)sj * a.result_stride : nullptr;
   cs_publish(S, hdr, a, cand, result);
-}
-
-// ---------------------------------------------------------------------------------------------------
-// rings kernel: the draw loop (:404-442).
-//
-// Every ray starts in the same cell (x1,y1) and advances exactly one cell along its major axis per step,
-// so the cell written at step k lies on the square ring of Chebyshev radius k around the start.  Rings
-// are independent of each other, and inside a ring the only ordering that matters is the reference's
-// ray order (foreach over cloud.Points, :517) among rays that hit the same cell WITH DIFFERENT pixvals:
-// blends of one pixval commute with themselves, so a cell visited n times with one pixval just needs n.
-//
-// One block owns a span of rings; one lane evaluates one (ray, ring) visit in closed form.  Per ring:
-//   1. every live lane stores (ray, pixval) into a shared slot indexed by the cell's position on the ring
-//      (plain store; one writer survives and becomes the cell's owner);
-//   2. the others — the cell is contested — add 1 to the slot's counter, plus a "mixed" mark if their
-//      pixval differs from the owner's;
-//   3. owners of uncontested cells do the read-modify-write directly (the overwhelming majority of
-//      visits outside the dense disc around the robot); owners of contested uniform cells apply the blend
-//      count+1 times (with the exact fixed-point early-out); for mixed cells the 32-ray batches that visit
-//      the cell are chained in ascending order through the slot (mask of batches + a hand-off word), each
-//      batch applying its lanes in lane order.
-// Rings with more positions (8k) than the slot table has entries go through the table in windows of positions; the
-// table size is chosen per launch (CsStepArgs::ring_slot_bits): 8192 entries for a session alone, fewer for batches of
-// sessions, where more resident blocks are worth more than single-pass outer rings.
-// No global atomics, no sort, bit-exact for any ray order; shared-memory atomics only on contested visits.
-// Scans with more rays than one round (threads x CS_RING_RPT) are processed in consecutive rounds; a
-// round starts after the previous round's stores, which keeps the ray order across rounds.
-// ---------------------------------------------------------------------------------------------------
-#define CS_RING_MAX_THREADS 512
-#define CS_RING_RPT 2                  // rays per lane and round
-#define CS_RING_MAX_SLOT_BITS 13        // largest slot table: 8192 entries, rings up to k = 1024 in one window
-#define CS_RING_MAX_SPAN 256
-// dynamic shared memory for a block of `threads` threads
-// (prefetch = 1: scans of more than one round keep a second ray buffer, filled by cp.async while the current round is drawn)
-#define CS_RING_SMEM(threads, slot_bits, prefetch) \
-  (((size_t)8 << (slot_bits)) + (size_t)(threads) * CS_RING_RPT * (16 + 4 + ((prefetch) ? 16 : 0)))
-#define CS_RING_MAX_ROUNDS 64           // rounds with their own "largest ring" entry; later rounds share the last entry
-
-__device__ __forceinline__ void cs_cp_async16(void* smem_dst, const void* gmem_src) {
-  const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gmem_src) : "memory");
-}
-__device__ __forceinline__ void cs_cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
-
-__device__ __forceinline__ int cs_blend(int old, int pixval, int alpha) {
-  return (int)(uint16_t)(((256 - alpha) * old + alpha * pixval) >> 8);  // :431
-}
-
-struct CsBlendState {
-  int val, last_pv;
-  bool fixed;  // val is a fixed point of blending with last_pv: more of the same changes nothing (exact)
-  __device__ __forceinline__ void apply(int pv, int alpha) {
-    if (fixed && pv == last_pv) return;
-    const int nv = cs_blend(val, pv, alpha);
-    fixed = (nv == val);
-    last_pv = pv;
-    val = nv;
-  }
-  __device__ __forceinline__ void apply_n(int pv, int cnt, int alpha) {
-    while (cnt-- > 0) {
-      const int nv = cs_blend(val, pv, alpha);
-      if (nv == val) break;  // fixed point of this pixval
-      val = nv;
-    }
-  }
-};
-
-// One visit: ray r at ring k.  pos = the cell's index along the ring (0 .. 8k-1, one value per cell:
-// side s of the square contributes (2s+1)k +- minor, the corner 8k wraps to 0).
-template <bool TILED>
-__device__ __forceinline__ bool cs_ring_visit(const CsRay& r, int k, int x1, int y1, int size, int pitch_tiles, int& pos,
-                                              uint32_t& cell, int& pv) {
-  if (!(r.flags & 1) || k > r.dxc) return false;
-  const int m = cs_ray_minor(r, k);
-  const int dmaj = (r.flags & 4) ? -k : k;
-  const int dmin = (r.flags & 8) ? -m : m;
-  const bool steep = (r.flags & 2) != 0;
-  const int ox = steep ? dmin : dmaj;
-  const int oy = steep ? dmaj : dmin;
-  const int x = x1 + ox, y = y1 + oy;
-  if ((unsigned)x >= (unsigned)size || (unsigned)y >= (unsigned)size) return false;  // cannot happen for a clipped ray
-  int p;
-  if (!steep) p = (r.flags & 4) ? 5 * k - oy : k + oy;
-  else p = (r.flags & 4) ? 7 * k + ox : 3 * k - ox;
-  pos = (p == 8 * k) ? 0 : p;
-  cell = cs_cell_offset<TILED>(x, y, size, pitch_tiles);
-  pv = cs_ray_pixval(r, k);
-  return true;
-}
-
-// SMALL = true: the instance for blocks of at most CS_RING_SMALL_THREADS threads (the sessions of a batch, short scans):
-// compiled for more resident blocks per SM (fewer registers per thread) than the 512-thread instance of a session alone.
-#define CS_RING_SMALL_THREADS 256
-// MULTI = true: the instance for scans of more rays than one round holds (2 x threads): rounds that do not reach a ring are
-// skipped and the next round's rays are prefetched; the other instances are compiled without any of it (n <= one round).
-template <bool TILED, bool SMALL, bool MULTI>
-__global__ void __launch_bounds__(SMALL ? CS_RING_SMALL_THREADS : CS_RING_MAX_THREADS, SMALL ? 5 : 2)
-cs_rings_kernel(CsSession* __restrict__ sessions, CsStepArgs a) {
-  extern __shared__ int4 cs_ring_smem[];
-
-  const long long t_begin = a.diag ? clock64() : 0;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  long long* tl = (a.diag && blockIdx.y == 0 && (int)blockIdx.x < a.diag_rings && tid == 0) ? a.diag + (size_t)blockIdx.x * 8 : nullptr;
-  if (tl) { tl[1] = cs_smid(); tl[2] = cs_globaltimer(); tl[4] = 0; tl[5] = 0; tl[6] = 0; }
-  const int nthreads = blockDim.x;
-  const int round_cap = nthreads * CS_RING_RPT;
-  const unsigned lt_mask = (1u << lane) - 1u;
-  unsigned* s_w = reinterpret_cast<unsigned*>(cs_ring_smem);            // slot -> local ray << 18 | pixval (0 .. 2*65500 + carries: 18 bits); later: batch mask
-  const int slot_bits = a.ring_slot_bits, n_slots = 1 << slot_bits;
-  unsigned* s_c = s_w + n_slots;                                         // slot -> contested visits | mixed marks << 16; later: hand-off word
-  int4* s_rays = reinterpret_cast<int4*>(s_c + n_slots);                 // this round's packed rays
-  int* s_lpv = reinterpret_cast<int*>(s_rays + round_cap);               // pixvals of the visits of mixed cells
-  int4* s_rays2 = reinterpret_cast<int4*>(s_lpv + round_cap);            // second ray buffer (scans of several rounds only)
-  {  // the counters start at zero; done before the dependency wait, so it overlaps the previous kernel's tail
-    uint4* c4 = reinterpret_cast<uint4*>(s_c);
-    for (int i = tid; i < n_slots / 4; i += nthreads) c4[i] = make_uint4(0u, 0u, 0u, 0u);
-  }
-  cs_pdl_launch_dependents();  // the next step's search may become resident once every block here has started
-  // No griddepcontrol.wait here: the kernel in front (search / set-up) is not awaited as a whole.  Its publishing
-  // thread writes CsSession::ll_pose as soon as the pose is final; this kernel's preparing blocks poll that, the
-  // others poll the preparing blocks' count.  (The wait is executed at the very end, to keep completion
-  // transitive for the next kernel in the stream.)  Nothing the search kernel writes is read before the polls.
-
-  const int sj = blockIdx.y;
-  CsSession& S = sessions[sj];
-  const int span = a.ring_span;
-  const CsStepHeader& hdr = a.hdr[(size_t)sj * a.hdr_stride];
-  const int n = hdr.n_points;                      // input of the step: uploaded before the kernels in front
-  const int size = S.size, pitch_tiles = S.pitch_tiles;  // host-owned constants
-  const float scale = S.scale;
-  const int alpha = S.quality;
-  uint16_t* __restrict__ map = S.map;
-  const int copies = S.ray_copies;
-  const int copy = cs_smid() % copies;  // the blocks of one SM share a copy (and its L1 lines)
-  const int4* rays = S.rays + (size_t)copy * S.ray_stride;
-  const int* batch_max = S.batch_max + (size_t)copy * S.batch_stride;
-  const unsigned slot = a.step_id & 1u;
-  unsigned long long* prep_words = S.prep_words + (size_t)slot * copies * 16;
-  const unsigned long long ll_tag = (unsigned long long)a.step_id << 32;
-
-  // ---- ray preparation (UpdateHoleMap :517-530, ClipRay, the prologue of DrawLaserRayOnHoleMap): the first nprep
-  // blocks of the grid each take a group of `a.prep_group` rays (a multiple of 32, one ray per lane and pass), write
-  // them to every copy and raise the copies' counts; every block waits for the count of its copy.  Blocks are
-  // dispatched in index order, so the preparing blocks are resident before any block can wait on them.
-  const int group = a.prep_group;
-  const int nprep = (n + group - 1) / group;
-  if ((int)blockIdx.x < nprep) {
-    __shared__ long long sh_vis[CS_RING_MAX_THREADS / 32];
-    __shared__ float sh_pose[5];
-    const float2* __restrict__ points = a.points + (size_t)sj * a.points_stride;
-    const int g_begin = blockIdx.x * group, g_end = min(n, g_begin + group);
-    const int i0 = g_begin + tid;
-    const float2 p0 = (i0 < g_end) ? __ldg(points + i0) : make_float2(1.f, 0.f);  // in flight while the pose is awaited
-    bool stuck = false;
-    if (tid < 5) {
-      volatile unsigned long long* ll = S.ll_pose + tid;
-      unsigned long long w;
-      CsSpin spin;
-      while (((w = *ll) & 0xffffffff00000000ull) != ll_tag)
-        if (spin.expired(a, CS_STUCK_POSE)) { stuck = true; break; }
-      sh_pose[tid] = __uint_as_float((unsigned)w);
-      if (tl) tl[3] = cs_globaltimer();
-    }
-    if (__syncthreads_or(stuck)) return;  // (bounded polls only: the pose never came)
-    const float pose[3] = {sh_pose[0], sh_pose[1], sh_pose[2]};
-    const float cs[2] = {sh_pose[3], sh_pose[4]};
-    long long vis = 0;
-    long long* pd = (tl && blockIdx.x == 0) ? a.diag + ((size_t)a.diag_rings + CS_DIAG_SEARCH_BLOCKS - 2) * 8 : nullptr;
-    if (pd) { pd[0] = tl[3]; pd[1] = cs_globaltimer(); }
-    if (tid < group) cs_prepare_rays(S, points, p0, g_end, i0, nthreads, pose, cs, true, vis);
-    if (pd) pd[2] = cs_globaltimer();
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) vis += __shfl_xor_sync(0xffffffffu, vis, o);
-    if (lane == 0) sh_vis[warp] = vis;
-    __threadfence();  // this thread's ray stores are visible device-wide before the block's arrival is counted
-    if (pd) pd[3] = cs_globaltimer();
-    __syncthreads();
-    if (tid < copies) atomicAdd(S.prep_words + ((size_t)slot * copies + tid) * 16, 1ull);
-    if (tid == 0) {
-      if (pd) pd[4] = cs_globaltimer();
-      for (int w = 1; w < (nthreads >> 5); w++) vis += sh_vis[w];
-      if (vis) {
-        atomicAdd((unsigned long long*)&S.visits_slot[slot], (unsigned long long)vis);
-        if (a.visits_out) atomicAdd((unsigned long long*)a.visits_out, (unsigned long long)vis);
-      }
-    }
-  }
-  __shared__ int sh_max_ring;
-  __shared__ int sh_round_max[CS_RING_MAX_ROUNDS];  // largest dxc of the rays of round r: later rings skip the round
-  if (MULTI && tid < CS_RING_MAX_ROUNDS) sh_round_max[tid] = -1;
-  bool rays_stuck = false;
-  if (tid == 0) {
-    sh_max_ring = -1;
-    volatile unsigned long long* pw = prep_words + (size_t)copy * 16;
-    CsSpin spin;
-    while (*pw != (unsigned long long)nprep)
-      if (spin.expired(a, CS_STUCK_RAYS)) { rays_stuck = true; break; }
-    __threadfence();
-    if (tl) tl[4] = cs_globaltimer();
-  }
-  if (__syncthreads_or(rays_stuck)) return;  // (bounded polls only: the rays never came)
-  // the pose words are final: the preparing blocks saw them before they counted themselves
-  const float pose_x = __uint_as_float((unsigned)__ldcg(&S.ll_pose[0]));
-  const float pose_y = __uint_as_float((unsigned)__ldcg(&S.ll_pose[1]));
-  const int x1 = cs_cvt_i32(__fadd_rn(__fmul_rn(pose_x, scale), 0.5f));  // :499, :505
-  const int y1 = cs_cvt_i32(__fadd_rn(__fmul_rn(pose_y, scale), 0.5f));  // :500, :506
-  const int nrounds = MULTI ? (n + round_cap - 1) / round_cap : 1;
-  bool rays_resident = false;
-  int bmax[CS_RING_RPT];
-#pragma unroll
-  for (int j = 0; j < CS_RING_RPT; j++) bmax[j] = -1;
-  if (nrounds == 1) {
-    // The whole scan fits one round: its rays go to shared memory now, in the same L2 round trip as the per-batch maxima
-    // below instead of one trip later.  (Written during this kernel by the preparing blocks and not read by anybody
-    // before their count was seen — L1 is invalidated at kernel start — so the default L1-allocating load is coherent,
-    // and the blocks of one SM share one L2 fetch of lines that every block of the grid wants at the same moment.)
-    for (int i = tid; i < n; i += nthreads) s_rays[i] = rays[i];
-#pragma unroll
-    for (int j = 0; j < CS_RING_RPT; j++) {
-      const int bu = warp * CS_RING_RPT + j;
-      bmax[j] = (bu * 32 < n) ? batch_max[bu] : -1;
-    }
-    rays_resident = true;
-  }
-  {  // max_ring = largest dxc of a valid ray (-1: nothing to draw), from the per-batch maxima
-    int m = -1;
-    for (int i = tid; i < (n + 31) / 32; i += nthreads) {
-      const int bm = batch_max[i];
-      m = max(m, bm);
-      if (MULTI && nrounds > 1 && bm >= 0) atomicMax(&sh_round_max[min((i * 32) / round_cap, CS_RING_MAX_ROUNDS - 1)], bm);
-    }
-    m = __reduce_max_sync(0xffffffffu, m);
-    if (lane == 0 && m >= 0) atomicMax(&sh_max_ring, m);
-  }
-  __syncthreads();
-  const int max_ring = sh_max_ring;
-  // ---- work units: unit u = rings [u*span, (u+1)*span).  Block b starts on unit b; when the rings kernel runs one
-  // session alone (a.ring_dynamic) the grid is at most one resident wave and every further unit is drawn from a
-  // ticket counter in ascending ring order, so the dense inner rings start first and the blocks stay busy until the
-  // rings run out.  In a batch of sessions every block owns exactly one unit.
-  unsigned* ticket = &S.ring_ticket[a.step_id & 1u];
-  __shared__ int sh_next_unit;
-  int pf_round0 = -1;   // round whose rays are in flight into the other ray buffer
-  int cur_round0 = -1;  // round whose rays the current buffer holds (scans of several rounds)
-  for (int unit = blockIdx.x;;) {
-  const int k_begin = unit * span;
-  if (k_begin > max_ring) break;
-  const int k_end = min(k_begin + span - 1, max_ring);
-  unsigned next_ticket = 0u;  // requested now, consumed after the unit: the L2 round trip hides behind the rings
-  if (a.ring_dynamic && tid == 0) next_ticket = atomicAdd(ticket, 1u);
-
-  for (int round0 = 0; round0 < n; round0 += round_cap) {
-    const int round_n = min(round_cap, n - round0);
-    if (MULTI && nrounds > 1) {
-      // Scans of several rounds.  A round none of whose rays reaches this unit's first ring is skipped (block-uniform).
-      // The rays of the next round to be drawn are fetched with cp.async into the second buffer while this round is
-      // drawn, so that only the unit's first round waits for its rays.  (The rays were written during this kernel by the
-      // preparing blocks and are not read by anybody before their count was seen — L1 is invalidated at kernel start —
-      // so L1-allocating loads are coherent, and the blocks of one SM share one L2 fetch.)
-      if (sh_round_max[min(round0 / round_cap, CS_RING_MAX_ROUNDS - 1)] < k_begin) continue;
-      if (cur_round0 != round0) {  // (a unit of one live round often follows another one of the same round)
-        if (pf_round0 == round0) {
-          cs_cp_async_wait_all();
-          int4* t = s_rays; s_rays = s_rays2; s_rays2 = t;
-        } else {
-          if (rays_resident) __syncthreads();  // previous round: the current buffer is free
-          for (int i = tid; i < round_n; i += nthreads) s_rays[i] = rays[round0 + i];
-        }
-#pragma unroll
-        for (int j = 0; j < CS_RING_RPT; j++) {
-          const int bu = warp * CS_RING_RPT + j;
-          bmax[j] = (bu * 32 < round_n) ? batch_max[(round0 >> 5) + bu] : -1;
-        }
-        cur_round0 = round0;
-      }
-      pf_round0 = -1;  // whatever was fetched is either current now or was not wanted
-      rays_resident = true;
-      __syncthreads();  // everybody's part of the buffer has landed; the previous round's reads of the other one are over
-      int next0 = round0 + round_cap;
-      while (next0 < n && sh_round_max[min(next0 / round_cap, CS_RING_MAX_ROUNDS - 1)] < k_begin) next0 += round_cap;
-      if (next0 < n) {
-        const int next_n = min(round_cap, n - next0);
-        for (int i = tid; i < next_n; i += nthreads) cs_cp_async16(s_rays2 + i, rays + next0 + i);
-        pf_round0 = next0;
-      }
-    } else {
-      if (!rays_resident) {
-        for (int i = tid; i < round_n; i += nthreads) s_rays[i] = rays[round0 + i];
-#pragma unroll
-        for (int j = 0; j < CS_RING_RPT; j++) {
-          const int bu = warp * CS_RING_RPT + j;
-          bmax[j] = (bu * 32 < round_n) ? batch_max[(round0 >> 5) + bu] : -1;
-        }
-        rays_resident = true;
-      }
-      __syncthreads();
-    }
-    if (tl && round0 == 0 && unit == (int)blockIdx.x) tl[5] = cs_globaltimer();
-
-    // read-modify-writes whose load is in flight (see 3a)
-    bool pend[CS_RING_RPT];
-    uint32_t pend_cell[CS_RING_RPT];
-    int pend_v[CS_RING_RPT], pend_pv[CS_RING_RPT];
-#pragma unroll
-    for (int j = 0; j < CS_RING_RPT; j++) { pend[j] = false; pend_cell[j] = 0; pend_v[j] = 0; pend_pv[j] = 0; }
-
-    for (int k = k_begin; k <= k_end; k++) {
-      int pos[CS_RING_RPT], pv[CS_RING_RPT];
-      uint32_t cell[CS_RING_RPT];
-      bool live[CS_RING_RPT];
-      // ---- evaluate this lane's visits of ring k ------------------------------------------------------------
-#pragma unroll
-      for (int j = 0; j < CS_RING_RPT; j++) {
-        live[j] = false;
-        const int li = (warp * CS_RING_RPT + j) * 32 + lane;
-        if (bmax[j] >= k && li < round_n) {  // bmax: warp-uniform skip of batches that do not reach this ring
-          const CsRay r = cs_unpack_ray(s_rays[li]);
-          live[j] = cs_ring_visit<TILED>(r, k, x1, y1, size, pitch_tiles, pos[j], cell[j], pv[j]);
-        }
-      }
-      // rings longer than the slot table are handled in windows of n_slots positions
-      const int nwin = max((8 * k + n_slots - 1) >> slot_bits, 1);
-      bool warp_dead = true;
-#pragma unroll
-      for (int j = 0; j < CS_RING_RPT; j++) warp_dead = warp_dead && (bmax[j] < k);
-      if (warp_dead) {
-        // none of this warp's rays reaches ring k (nor any later ring): it only keeps the block's barrier
-        // sequence — A, B(or), then C(or) on contested rings, then D, E, F on rings with mixed cells
-#pragma unroll
-        for (int j = 0; j < CS_RING_RPT; j++) {
-          if (pend[j]) __stcg(map + pend_cell[j], (uint16_t)cs_blend(pend_v[j], pend_pv[j], alpha));
-          pend[j] = false;
-        }
-        for (int win = 0; win < nwin; win++) {
-          __syncthreads();
-          if (!__syncthreads_or(0)) continue;
-          if (!__syncthreads_or(0)) continue;
-          __syncthreads();
-          __syncthreads();
-          __syncthreads();
-        }
-        continue;
-      }
-      for (int win = 0; win < nwin; win++) {
-        bool act[CS_RING_RPT], owner[CS_RING_RPT];
-        unsigned word[CS_RING_RPT];
-        int h[CS_RING_RPT];
-        // ---- 1. claim the slots ------------------------------------------------------------------------------
-#pragma unroll
-        for (int j = 0; j < CS_RING_RPT; j++) {
-          act[j] = live[j] && (pos[j] >> slot_bits) == win;
-          h[j] = pos[j] & (n_slots - 1);
-          if (act[j]) {
-            const int li = (warp * CS_RING_RPT + j) * 32 + lane;
-            word[j] = ((unsigned)li << 18) | ((unsigned)pv[j] & 0x3ffffu);
-            s_w[h[j]] = word[j];
-          }
-        }
-        // the previous fast ring's loads have had this ring's evaluation to arrive: blend and store them
-#pragma unroll
-        for (int j = 0; j < CS_RING_RPT; j++) {
-          if (pend[j]) __stcg(map + pend_cell[j], (uint16_t)cs_blend(pend_v[j], pend_pv[j], alpha));
-          pend[j] = false;
-        }
-        __syncthreads();
-        // ---- 2. owners are the lanes that read their own word back; the others mark the slot ---------------
-        bool contested = false;
-#pragma unroll
-        for (int j = 0; j < CS_RING_RPT; j++) {
-          owner[j] = false;
-          if (act[j]) {
-            const unsigned w = s_w[h[j]];
-            owner[j] = (w == word[j]);
-            if (!owner[j]) {
-              atomicAdd(&s_c[h[j]], 1u + ((((w ^ word[j]) & 0x3ffffu) != 0u) ? 0x10000u : 0u));
-              contested = true;
-            }
-          }
-        }
-        if (!__syncthreads_or(contested)) {
-          // ---- 3a. no cell is visited twice in this round: plain read-modify-write.  The loads are issued
-          // now; the blend and the store follow after the next ring's evaluation (different rings never
-          // share a cell), so the L2 / HBM latency overlaps it.
-#pragma unroll
-          for (int j = 0; j < CS_RING_RPT; j++) {
-            pend[j] = act[j];
-            if (act[j]) {
-              pend_v[j] = (int)__ldcg(map + cell[j]);
-              pend_cell[j] = cell[j];
-              pend_pv[j] = pv[j];
-            }
-          }
-          continue;
-        }
-        // ---- 3b. contested cells with one pixval: the owner applies it count+1 times -------------------------
-        unsigned cnt[CS_RING_RPT];
-        bool slow[CS_RING_RPT];
-        bool any_slow_l = false;
-        int v[CS_RING_RPT];
-#pragma unroll
-        for (int j = 0; j < CS_RING_RPT; j++) {
-          cnt[j] = 0u; slow[j] = false; v[j] = 0;
-          if (act[j]) {
-            cnt[j] = s_c[h[j]];
-            slow[j] = (cnt[j] >> 16) != 0u;
-            any_slow_l = any_slow_l || slow[j];
-            if (owner[j] && !slow[j]) v[j] = (int)__ldcg(map + cell[j]);
-          }
-        }
-        const int any_slow = __syncthreads_or(any_slow_l);
-#pragma unroll
-        for (int j = 0; j < CS_RING_RPT; j++) {
-          if (act[j] && owner[j]) {
-            if (cnt[j]) s_c[h[j]] = 0u;  // everybody has read it (barrier above): re-arm / hand-off word "empty"
-            if (!slow[j]) {
-              CsBlendState st;
-              st.val = v[j]; st.last_pv = -1; st.fixed = false;
-              st.apply_n(pv[j], (int)(cnt[j] & 0xffffu) + 1, alpha);
-              __stcg(map + cell[j], (uint16_t)st.val);
-            } else {
-              s_w[h[j]] = 0u;  // becomes the mask of the 32-ray batches that visit this cell
-            }
-          }
-        }
-        if (!any_slow) continue;
-        // ---- 3c. cells visited with different pixvals: per cell, the batches that visit it are applied in
-        // ascending (= ray) order.  Lanes of a batch on the same cell form a group; its first lane sets the
-        // batch's bit in the cell's mask, then — in mask order — loads the cell or takes it from the
-        // previous batch through the slot's hand-off word, applies the group's pixvals in lane order and
-        // stores the cell or hands it on.  A batch only waits for lower batches: lower warps, or this
-        // warp's earlier j.
-#pragma unroll
-        for (int j = 0; j < CS_RING_RPT; j++)
-          if (act[j] && slow[j]) s_lpv[(warp * CS_RING_RPT + j) * 32 + lane] = pv[j];
-        __syncthreads();
-        unsigned peers[CS_RING_RPT];
-#pragma unroll
-        for (int j = 0; j < CS_RING_RPT; j++) {
-          peers[j] = 0u;
-          const bool sl = act[j] && slow[j];
-          const unsigned bal = __ballot_sync(0xffffffffu, sl);
-          if (sl) {
-            peers[j] = __match_any_sync(bal, pos[j]);
-            if ((peers[j] & lt_mask) == 0u) atomicOr(&s_w[h[j]], 1u << (warp * CS_RING_RPT + j));
-          }
-        }
-        __syncthreads();
-        int pred[CS_RING_RPT];
-        bool lead[CS_RING_RPT], last[CS_RING_RPT];
-#pragma unroll
-        for (int j = 0; j < CS_RING_RPT; j++) {
-          const int unit = warp * CS_RING_RPT + j;
-          lead[j] = peers[j] != 0u && (peers[j] & lt_mask) == 0u;
-          pred[j] = -1; last[j] = true;
-          if (lead[j]) {
-            const unsigned m = s_w[h[j]];
-            const unsigned below = m & ((1u << unit) - 1u);
-            if (below) pred[j] = 31 - __clz(below);
-            last[j] = unit == 31 || (m >> (unit + 1)) == 0u;
-            if (pred[j] < 0) v[j] = (int)__ldcg(map + cell[j]);  // all opening loads are in flight before anything waits
-          }
-        }
-        __syncthreads();  // every mask has been read: s_w may be claimed again by the lanes that run ahead
-#pragma unroll
-        for (int j = 0; j < CS_RING_RPT; j++) {
-          if (lead[j]) {
-            const int unit = warp * CS_RING_RPT + j;
-            volatile unsigned* hand = s_c + h[j];
-            CsBlendState st;
-            st.last_pv = -1; st.fixed = false;
-            if (pred[j] >= 0) {
-              unsigned w;
-              CsSpin spin;  // (a give-up leaves the cell wrong; the handle is failed by the host, see CsSpin)
-              do { w = *hand; } while ((w >> 16) != (unsigned)(pred[j] + 1) && !spin.expired(a, CS_STUCK_HANDOFF));
-              st.val = (int)(w & 0xffffu);
-            } else {
-              st.val = v[j];
-            }
-            unsigned pm = peers[j];
-            while (pm) {
-              const int l = __ffs(pm) - 1;
-              pm &= pm - 1;
-              st.apply(s_lpv[unit * 32 + l], alpha);
-            }
-            if (last[j]) {
-              __stcg(map + cell[j], (uint16_t)st.val);
-              if (pred[j] >= 0) *hand = 0u;  // re-arm the slot's counter
-            } else {
-              *hand = ((unsigned)(unit + 1) << 16) | (unsigned)st.val;
-            }
-          }
-        }
-      }
-    }
-    // complete the deferred read-modify-writes before the next round may touch the same cells
-#pragma unroll
-    for (int j = 0; j < CS_RING_RPT; j++)
-      if (pend[j]) __stcg(map + pend_cell[j], (uint16_t)cs_blend(pend_v[j], pend_pv[j], alpha));
-  }
-  if (!a.ring_dynamic) break;
-  if (tid == 0) sh_next_unit = (int)(gridDim.x + next_ticket);
-  __syncthreads();
-  unit = sh_next_unit;
-  }
-  if (tl) { tl[0] = clock64() - t_begin; tl[6] = cs_globaltimer(); }
-  cs_pdl_wait();  // the kernel in front has long finished; this only makes "this grid done" imply "that grid done"
 }
 
 // ---------------------------------------------------------------------------------------------------

@@ -23,9 +23,10 @@
 //            candidates are walked in ray order with the next batch's rays in flight, same-cell groups fold into the
 //            staged values (uniform groups as a count with the exact fixed-point early-out), then the touched cells go back.
 // Rings 0 .. CS_W_CENTER - 1, which every ray crosses, are drawn by one block as shared-memory counts (cs_w_center).
-// The first blocks prepare the rays exactly as the rings kernel's do (cs_ray_from_point), plus each ray's key, the key
-// range of every 32 rays, and per level and key sector the number of rays that reach it (which sizes the wedges: ~26
-// candidates each, cut at the quantiles of the level's rays).  DESIGN.md section 4 has the scheduling and the measurements.
+// The first blocks prepare the rays (cs_ray_from_point: UpdateHoleMap, ClipRay, the prologue of the draw loop), plus each
+// ray's key, the key range of every 32 rays, and per level and key sector the number of rays that reach it (which sizes
+// the wedges: ~26 candidates each, cut at the quantiles of the level's rays).  DESIGN.md section 4 has the scheduling and
+// the measurements.
 #pragma once
 #include "cs_kernels.cuh"
 
@@ -202,6 +203,53 @@ __device__ __forceinline__ int cs_w_next_batch(const unsigned* s_bmap, int nw, i
 __device__ __forceinline__ bool cs_w_is_candidate(const CsWTask& t, const int2 rk) {
   const float key = __int_as_float(rk.x);
   return rk.y >= t.k0 && ((key >= t.flo && key < t.fhi) || key >= t.wrap_lo);
+}
+
+// one blend of the draw loop; CsBlendState applies a run of them with the exact fixed-point early-out
+__device__ __forceinline__ int cs_blend(int old, int pixval, int alpha) {
+  return (int)(uint16_t)(((256 - alpha) * old + alpha * pixval) >> 8);  // :431
+}
+
+struct CsBlendState {
+  int val, last_pv;
+  bool fixed;  // val is a fixed point of blending with last_pv: more of the same changes nothing (exact)
+  __device__ __forceinline__ void apply(int pv, int alpha) {
+    if (fixed && pv == last_pv) return;
+    const int nv = cs_blend(val, pv, alpha);
+    fixed = (nv == val);
+    last_pv = pv;
+    val = nv;
+  }
+  __device__ __forceinline__ void apply_n(int pv, int cnt, int alpha) {
+    while (cnt-- > 0) {
+      const int nv = cs_blend(val, pv, alpha);
+      if (nv == val) break;  // fixed point of this pixval
+      val = nv;
+    }
+  }
+};
+
+// One visit: ray r at ring k.  pos = the cell's index along the ring (0 .. 8k-1, one value per cell:
+// side s of the square contributes (2s+1)k +- minor, the corner 8k wraps to 0).
+template <bool TILED>
+__device__ __forceinline__ bool cs_ring_visit(const CsRay& r, int k, int x1, int y1, int size, int pitch_tiles, int& pos,
+                                              uint32_t& cell, int& pv) {
+  if (!(r.flags & 1) || k > r.dxc) return false;
+  const int m = cs_ray_minor(r, k);
+  const int dmaj = (r.flags & 4) ? -k : k;
+  const int dmin = (r.flags & 8) ? -m : m;
+  const bool steep = (r.flags & 2) != 0;
+  const int ox = steep ? dmin : dmaj;
+  const int oy = steep ? dmaj : dmin;
+  const int x = x1 + ox, y = y1 + oy;
+  if ((unsigned)x >= (unsigned)size || (unsigned)y >= (unsigned)size) return false;  // cannot happen for a clipped ray
+  int p;
+  if (!steep) p = (r.flags & 4) ? 5 * k - oy : k + oy;
+  else p = (r.flags & 4) ? 7 * k + ox : 3 * k - ox;
+  pos = (p == 8 * k) ? 0 : p;
+  cell = cs_cell_offset<TILED>(x, y, size, pitch_tiles);
+  pv = cs_ray_pixval(r, k);
+  return true;
 }
 
 // cell of position p on ring k around (x1, y1) (inverse of cs_ring_visit's position)
@@ -675,8 +723,8 @@ cs_wedge_kernel(CsSession* __restrict__ sessions, CsStepArgs a) {
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const long long t_start = a.diag ? cs_globaltimer() : 0;  // diagnostics (cs_get_ring_cycles): block start, rays ready, table ready
   cs_pdl_launch_dependents();  // the next step's search may become resident once every block here has started
-  // No griddepcontrol.wait in front: like the rings kernel, this one is resident before the search in front has ended; its
-  // preparing blocks poll the pose words, everybody else the preparing blocks' count (see cs_rings_kernel).
+  // No griddepcontrol.wait in front: this kernel is resident before the search in front has ended; its preparing blocks
+  // poll the pose words (CsSession::ll_pose), everybody else the preparing blocks' count (CsSession::prep_words).
 
   const int sj = blockIdx.y;
   CsSession& S = sessions[sj];

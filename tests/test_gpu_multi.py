@@ -161,24 +161,6 @@ def test_candidate_split_two_processes_nccl():
     assert "SPLIT_OK" in out.stdout
 
 
-@pytest.mark.parametrize("span", ["64", "8"])
-def test_batch_parity_with_other_rings_per_block(span):
-    """Batches of at most 256 sessions draw 32 rings per block, larger ones 64 (launch_step): the partition of the rings
-    into blocks must not change a result.  The library reads its tuning knobs once per process, so the batch parity tests
-    are run again in a child process with CS_TUNE_RING_SPAN forced."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, CS_TUNE_RING_SPAN=span)
-    r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-x", "-m", "gpu",
-                        "tests/test_gpu_search2.py::test_slab_batch_update_matches_oracle_per_session",
-                        "tests/test_gpu_search2.py::test_batch_with_scans_of_several_rounds",
-                        "tests/test_gpu_multi.py::test_batch_replay_shared_log_philox_equals_single_handles"],
-                       cwd=root, env=env, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-1000:]
-
-
 def test_batch_submit_collect_pipeline_equals_blocking_updates():
     """cs_batch_submit / cs_batch_collect (two steps in flight, host staging overlapped with the previous step) must give the
     records and maps of the blocking cs_batch_update, and refuse a third step in flight / a collect with nothing submitted."""

@@ -377,10 +377,10 @@ def test_cfg3_integration_stress_8192_rays_4096_map():
 
 @pytest.mark.parametrize("n_rays", [2500, 4096])
 def test_integrate_large_map_several_rounds_sorted_and_unsorted(n_rays):
-    """Scans of several rounds (more rays than 2 x 512) on a map whose outer rings are longer than the slot table (k > 1024):
-    the several-rounds instance of the rings kernel claims all windows of such a ring in one pass when the rays come in
-    angular order, and must fall back to window-by-window claims when an unsorted scan aliases two cells onto one slot.
-    Sorted, permuted, reversed and wall-hugging scans, all bit-exact against the cell-by-cell oracle."""
+    """Big scans (more than 2048 rays) on a 4096 x 4096 map, rays up to 3000 cells long: the draw kernel's big-scan path
+    (the 64-register instance, the task table built from the scan's own counts).  A permuted scan puts candidates of every
+    wedge into every batch of 32 rays, and short rays among the long ones crowd the inner levels.  Sorted, permuted,
+    reversed and border-clipped scans, all bit-exact against the cell-by-cell oracle."""
     size, phys = 4096, 40.96
     rng = np.random.default_rng(n_rays)
     p = _mk(size, phys, 1, 1, max_points=n_rays)

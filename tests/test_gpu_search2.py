@@ -131,7 +131,7 @@ def test_slab_update_replay_bit_exact(philox, layout):
 
 @pytest.mark.parametrize("philox", [False, True])
 def test_slab_scanlog_replay_back_to_back(philox):
-    """cs_replay queues every scan's sort / search / rings kernels back to back (programmatic dependent launches, no host
+    """cs_replay queues every scan's sort / search / draw kernels back to back (programmatic dependent launches, no host
     round trip): the chain must give the oracle's poses and map, and the same as the warp-per-candidate kernel."""
     n_scans, n_points, size, phys, iters, threads = 60, 512, 640, 40.0, 320, 4
     rp = synth.make_replay(n_scans, n_points, phys, seed=77)
@@ -246,9 +246,9 @@ def test_slab_batch_update_matches_oracle_per_session(flags):
 
 
 def test_batch_with_scans_of_several_rounds():
-    """A batch whose sessions carry more rays than one round of the rings kernel holds (2 x 512), with ragged point counts —
-    one session stays below a round: the batch runs the several-rounds instance (grid.y = session, fixed units), every
-    session must still equal the oracle (poses, winners, maps)."""
+    """A batch whose largest scan has more than 2048 rays, with ragged point counts (2600, 1500 and 700 rays in one launch
+    sized for the largest): the draw kernel's big-scan path for a batch (grid.y = session, each session's task table built
+    from its own counts, its tasks dealt over its blocks).  Every session must still equal the oracle (poses, winners, maps)."""
     n_sess, n_scans, P, size, phys, iters, threads = 3, 8, 2600, 512, 40.0, 40, 2
     rps = [synth.make_replay(n_scans, P, phys, seed=150 + j) for j in range(n_sess)]
     sxy, sth = [0.05, 0.07, 0.09], [0.10, 0.11, 0.12]

@@ -16,9 +16,6 @@ timeout 600 python bench.py --streaming --no-cpu-baseline --no-sharded > $O/${TA
 for wl in cfg1 cfg3 cfg4 cfg5; do
   timeout 900 python bench.py --workload $wl --steps 100 --warmup 10 > $O/${TAG}_bench_$wl.json 2> $O/${TAG}_bench_$wl.err; echo "$wl rc=$?"
 done
-CS_TUNE_INTEGRATE=1 timeout 600 python bench.py --no-cpu-baseline --no-sharded --steps 200 --warmup 10 > $O/${TAG}_bench_cfg2_rings.json 2>/dev/null; echo "cfg2 with round 1's rings kernel rc=$?"
-CS_TUNE_INTEGRATE=1 timeout 600 python bench.py --workload cfg3 --no-cpu-baseline --steps 100 --warmup 10 > $O/${TAG}_bench_cfg3_rings.json 2>/dev/null; echo "cfg3 rings rc=$?"
-CS_TUNE_INTEGRATE=1 timeout 600 python bench.py --workload cfg5 --no-cpu-baseline --steps 50 --warmup 5 > $O/${TAG}_bench_cfg5_rings.json 2>/dev/null; echo "cfg5 rings rc=$?"
 timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file $O/${TAG}_launches_cfg2.csv python bench.py --steps 20 --warmup 3 --no-cpu-baseline --no-sharded > $O/${TAG}_ncu_launch.log 2>&1; echo "ncu launches cfg2 rc=$?"
 timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -c 60 --csv --log-file $O/${TAG}_launches_cfg3.csv python bench.py --workload cfg3 --steps 5 --warmup 3 --no-cpu-baseline > /dev/null 2>&1; echo "ncu launches cfg3 rc=$?"
 timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -c 60 --csv --log-file $O/${TAG}_launches_cfg5.csv python bench.py --workload cfg5 --steps 3 --warmup 3 --no-cpu-baseline --no-sharded > /dev/null 2>&1; echo "ncu launches cfg5 rc=$?"

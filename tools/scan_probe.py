@@ -1,4 +1,4 @@
-"""Diagnostics: per-scan device times of the search and rings kernels over a long cfg2 replay."""
+"""Diagnostics: per-scan device times of the search and draw kernels over a long cfg2 replay."""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -20,6 +20,6 @@ for k in range(n):
 s, g, v = np.array(s), np.array(g), np.array(v)
 for a in range(0, n, 50):
     b = min(n, a + 50)
-    print("scans %4d-%4d: search mean %.1f max %.1f | rings mean %.1f max %.1f | visits %.0f | min wall dist %.2f m" % (
+    print("scans %4d-%4d: search mean %.1f max %.1f | draw mean %.1f max %.1f | visits %.0f | min wall dist %.2f m" % (
         a, b, s[a:b].mean(), s[a:b].max(), g[a:b].mean(), g[a:b].max(), v[a:b].mean(),
         min(np.hypot(rp.points[k][:, 0], rp.points[k][:, 1]).min() for k in range(a, b))))
