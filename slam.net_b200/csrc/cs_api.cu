@@ -66,20 +66,55 @@ struct Presort {
   uint64_t tag = 0;             // ... and the upload of the log it belongs to
 };
 
-struct cs_processor {
-  cs_config cfg{};
+// Host mirror of the deterministic parts of the state machine.  A batch steps all its sessions together, so one mirror
+// serves one processor or a whole batch.
+struct StepState {
+  int parity = 0;      // which CsSession::state / key slot is current
+  int scan_count = 0;  // CoreSLAMProcessor.cs:34 (saturates at PositionSearchBeginning)
+  int search_begin = 5;
+  unsigned update_count = 0;  // Philox scan index
+  unsigned step_counter = 0;  // source of CsStepArgs::step_id
+  int w_slot = 0;             // which third of CsSession::w_top the next drawn step counts into
+  int s2_toggle = 0;          // which half of CsSession::s2_sorted the next sort writes
+
+  bool searches() const { return scan_count >= search_begin; }  // :726
+  // after an Update has been enqueued
+  void advance(bool searched) {
+    parity ^= 1;
+    update_count++;
+    if (!searched) scan_count++;  // :741
+  }
+};
+
+// What a processor (one session) and a batch (n sessions of the same shape) both have and mean alike.
+struct CsHost {
   int device = 0;
   cudaStream_t stream = nullptr;
   bool own_stream = false;
   bool tiled = true;
-  int size = 0, pitch_tiles = 0, max_points = 0, n_cand = 0;
+  int size = 0, pitch_tiles = 0, n_cand = 0;
   float scale = 0.f;
-  size_t map_cells = 0;  // allocated cells (tiled: pitch_tiles^2 * 64)
+  size_t map_cells = 0;  // allocated cells of one map (tiled: pitch_tiles^2 * 64)
+  CsSession* d_sess = nullptr;
+  uint16_t* d_linear = nullptr;  // lazily allocated row-major scratch for upload/download
+  unsigned long long* d_checksum = nullptr;
+  int s2_cap = 0;                // slab-search capacity of one session (0: no slab-search scratch)
+  StepState step;
+  // stuck-poll word (CsSpin) in pinned+mapped memory, and its device address: a processor's lies in its result slot, a
+  // batch allocates its own under CS_FLAG_DEBUG_BOUNDED_SPIN (NULL otherwise)
+  uint8_t* h_stuck = nullptr;
+  uint8_t* d_stuck = nullptr;
+  uint64_t launches = 0;
+  std::string error;
+  bool poisoned = false;
+};
+
+struct cs_processor : CsHost {
+  cs_config cfg{};
+  int max_points = 0;
 
   CsSession hs{};            // host mirror of the session descriptor
-  CsSession* d_sess = nullptr;
   uint16_t* d_map = nullptr;
-  uint16_t* d_linear = nullptr;  // lazily allocated row-major scratch for upload/download
   uint8_t* d_packed = nullptr;
   int4* d_rays = nullptr;       // kRayCopies copies of ray_stride entries
   int* d_batch_max = nullptr;   // kRayCopies copies of batch_stride entries
@@ -92,9 +127,7 @@ struct cs_processor {
   float2* d_w_bkey = nullptr;
   int* d_w_top = nullptr;
   unsigned long long* d_spec = nullptr;  // glue table (CsStepArgs::spec): 8 words per flat candidate
-  int w_slot = 0;
   long long* d_ring_cycles = nullptr;
-  unsigned long long* d_checksum = nullptr;
 
   // slab search scratch (CsSession::s2_*), allocated when the handle has enough candidates for it to pay
   float4* d_s2_sorted = nullptr;
@@ -102,7 +135,6 @@ struct cs_processor {
   unsigned long long* d_s2_meta = nullptr;
   unsigned long long* d_s2_acc = nullptr;
   unsigned* d_s2_ghist = nullptr;
-  int s2_cap = 0, s2_toggle = 0;
   Presort presort;
 
   // ObstacleMap (cfg.obstacle_map_size > 0): CoreSLAM/ObstacleMap.cs, CoreSLAMProcessor.cs:53, :132-133
@@ -135,12 +167,6 @@ struct cs_processor {
   uint8_t* d_slot = nullptr;
   unsigned seq = 0;
 
-  // host mirrors of the deterministic parts of the state machine
-  int parity = 0;      // which CsSession::state / key slot is current
-  int scan_count = 0;  // CoreSLAMProcessor.cs:34 (saturates at PositionSearchBeginning)
-  int search_begin = 5;
-  unsigned update_count = 0;  // Philox scan index
-
   // split-phase update in flight (cs_update_begin ... cs_update_finish)
   bool pending = false;
   CsStepArgs pending_args{};
@@ -154,12 +180,8 @@ struct cs_processor {
   unsigned long long* xchg_peer[CS_GROUP_MAX] = {};
   bool xchg_ipc[CS_GROUP_MAX] = {};  // opened with cudaIpcOpenMemHandle (to be closed on detach)
 
-  uint64_t launches = 0;
-  unsigned step_counter = 0;
   Timing tm;
   cs_timing last_timing{};
-  std::string error;
-  bool poisoned = false;
 };
 
 struct cs_scanlog {
@@ -178,7 +200,7 @@ struct cs_scanlog {
 
 namespace {
 
-cs_status fail(cs_processor* h, cs_status code, const char* fmt, ...) {
+cs_status fail(CsHost* h, cs_status code, const char* fmt, ...) {
   char buf[512];
   va_list ap;
   va_start(ap, fmt);
@@ -209,21 +231,33 @@ const char* stuck_site_name(unsigned w) {
     default: return "an unknown word";
   }
 }
-#define CS_CHECK_STUCK(h, slot, failfn)                                                                         \
-  do {                                                                                                          \
-    const unsigned _w = (slot) ? *reinterpret_cast<volatile unsigned*>(slot) : 0u;                              \
-    if (_w)                                                                                                     \
-      return failfn((h), CS_ERR_CUDA, "bounded polls: block %u of the draw kernel gave up waiting for %s", _w >> 8, \
-                    stuck_site_name(_w));                                                                       \
+#define CS_CHECK_STUCK(h)                                                                                        \
+  do {                                                                                                           \
+    const unsigned _w = (h)->h_stuck ? *reinterpret_cast<volatile unsigned*>((h)->h_stuck) : 0u;                \
+    if (_w)                                                                                                      \
+      return fail((h), CS_ERR_CUDA, "bounded polls: block %u of the draw kernel gave up waiting for %s", _w >> 8, \
+                  stuck_site_name(_w));                                                                          \
   } while (0)
 
 #define CS_CHECK_HANDLE(h)                                                          \
   do {                                                                              \
     if (!(h)) return CS_ERR_INVALID_ARGUMENT;                                       \
     if ((h)->poisoned) return CS_ERR_CUDA;                                          \
-    CS_CHECK_STUCK(h, (h)->h_slot ? (h)->h_slot + 96 : nullptr, fail);              \
+    CS_CHECK_STUCK(h);                                                              \
     cudaError_t _e = cudaSetDevice((h)->device);                                    \
     if (_e != cudaSuccess) return fail((h), CS_ERR_CUDA, "cudaSetDevice: %s", cudaGetErrorString(_e)); \
+  } while (0)
+
+// In cs_create / cs_batch_create: a failed call records its message and returns through the function's `bail`, which
+// destroys the half-built handle.
+#define CS_CREATE_CUDA(h, expr)                                                                              \
+  do {                                                                                                       \
+    cudaError_t _e = (expr);                                                                                 \
+    if (_e != cudaSuccess) {                                                                                 \
+      const cs_status _st = _e == cudaErrorMemoryAllocation ? CS_ERR_OUT_OF_MEMORY : CS_ERR_CUDA;            \
+      fail((h), _st, "%s failed: %s", #expr, cudaGetErrorString(_e));                                        \
+      return bail(_st);                                                                                      \
+    }                                                                                                        \
   } while (0)
 
 cs_status push_session(cs_processor* h) {
@@ -265,8 +299,7 @@ StagePlan plan_stage(int n_points, int n_cand_floats3, bool with_cs) {
   return p;
 }
 
-// Wedge integration (cs_wedge.cuh): levels a ray of a size x size map can reach, the words of one half of CsSession::w_top,
-// and the dynamic shared memory of the kernel (one 16-bit count per level and key sector).
+// Wedge integration (cs_wedge.cuh): levels a ray of a size x size map can reach, and the words of one half of CsSession::w_top.
 int wedge_levels(int size) {
   const int k = size > 1 ? size - 1 : 1;
   int L = 0;
@@ -274,8 +307,37 @@ int wedge_levels(int size) {
   return L + 1;
 }
 size_t wedge_top_words(int size) { return (size_t)wedge_levels(size) * (CS_W_SECTORS + 1); }
-size_t wedge_smem(int) { return 0; }
-cudaError_t wedge_allow_shared_memory();
+
+// The host-owned constants of a session (the defaults of CoreSLAMProcessor.cs:82-92); the caller adds its scratch pointers.
+void init_session(CsSession& s, const CsHost& h, const cs_config& cfg, uint16_t* map) {
+  memset(&s, 0, sizeof(s));
+  s.map = map;
+  s.size = h.size;
+  s.pitch_tiles = h.pitch_tiles;
+  s.scale = h.scale;
+  s.sigma_xy = cfg.sigma_xy;
+  s.sigma_theta = cfg.sigma_theta;
+  s.iters = cfg.iterations_per_thread;
+  s.threads = cfg.num_search_threads;
+  s.n_cand = h.n_cand;
+  s.quality = 50;        // :82
+  s.hole_width = 0.6f;   // :87
+  s.search_begin = 5;    // :92
+  s.seed = cfg.seed;
+  s.w_levels = wedge_levels(h.size);
+}
+
+// The device-owned state of a session after Reset (CoreSLAMProcessor.cs:167-175): the start pose, scan count 0
+// (lastOdometryPose = 0, :173-174), no search or integration in flight.
+void reset_session(CsSession& s, const float start_pose[3]) {
+  memset(s.state, 0, sizeof(s.state));
+  for (int k = 0; k < 3; k++) s.state[0].pose[k] = start_pose[k];  // :172
+  s.key[0] = s.key[1] = ~0ull;
+  s.search_done = 0;
+  s.visits_slot[0] = s.visits_slot[1] = 0;
+  s.ring_ticket[0] = s.ring_ticket[1] = 0;
+  memset(s.ll_pose, 0, sizeof(s.ll_pose));
+}
 
 // Upper bound on the ring count of a scan: |rotated, scaled point| + half the hole width, plus rounding slack.
 int rings_hint_of(int size, float scale, float hole_width, double max_range) {
@@ -470,25 +532,30 @@ bool cs_plan_search2(int n_sessions, int s2_cap, int min_cand, long long cand_co
 struct LaunchCtx {
   int s2_cap = 0;            // capacity of the slab-search scratch (0: none)
   int s2_min_cand = 0;       // cs_s2_min_cand of the handle
-  int* s2_toggle = nullptr;  // which half of CsSession::s2_sorted the next sort writes
   Presort* presort = nullptr;  // one session alone: the sort queued ahead for the next scan, if any
   const float* next_cand = nullptr;  // cs_replay with tables: the next scan's table (nullptr: none) and the log's upload number
   uint64_t log_tag = 0;
-  const CsSession* hs = nullptr;  // host mirror of the session (host-owned constants for the slab kernels)
-  int num_sms;
-  cudaStream_t stream;
-  CsSession* d_sess;
-  bool tiled;
-  int n_sessions;
-  uint64_t* launches;
-  unsigned* step_counter;  // source of CsStepArgs::step_id
-  int* w_slot = nullptr;   // which half of CsSession::w_top the next drawn step counts into
-  long long* diag;
-  int diag_rings;
+  const CsSession* hs = nullptr;  // host mirror of the (first) session (host-owned constants for the slab kernels)
+  int num_sms = 0;
+  cudaStream_t stream = nullptr;
+  CsSession* d_sess = nullptr;
+  bool tiled = true;
+  int n_sessions = 1;
+  uint64_t* launches = nullptr;
+  StepState* step = nullptr;  // step_counter, w_slot and s2_toggle advance with every launch
+  long long* diag = nullptr;
+  int diag_rings = 0;
   volatile unsigned* stuck_dev = nullptr;  // CS_FLAG_DEBUG_BOUNDED_SPIN: device address of the mapped-host word (CsSpin)
   unsigned long long* spec = nullptr;      // glue table of the handle (one session alone)
-  cudaEvent_t ev_pose;   // optional: recorded once the pose is out
-  cudaEvent_t ev_done;   // optional: recorded after the draw kernel
+  cudaEvent_t ev_pose = nullptr;  // optional: recorded once the pose is out
+  cudaEvent_t ev_done = nullptr;  // optional: recorded after the draw kernel
+
+  // what a step of either handle is launched on; launch_step adds what only a processor has
+  LaunchCtx(CsHost* h, uint32_t flags, int sessions, const CsSession* host_sessions)
+      : s2_cap(h->s2_cap), s2_min_cand(cs_s2_min_cand(flags, sessions)), hs(host_sessions), num_sms(device_sm_count(h->device)),
+        stream(h->stream), d_sess(h->d_sess), tiled(h->tiled), n_sessions(sessions), launches(&h->launches), step(&h->step) {
+    if (flags & CS_FLAG_DEBUG_BOUNDED_SPIN) stuck_dev = reinterpret_cast<volatile unsigned*>(h->d_stuck);
+  }
 };
 
 enum { CS_PHASE_SEARCH = 1, CS_PHASE_FINISH = 2, CS_PHASE_ALL = 3 };
@@ -569,8 +636,8 @@ cudaError_t launch_step_ctx(const LaunchCtx& c, CsStepArgs a, int n_points, int 
   a.stuck_flag = c.stuck_dev;
   a.spin_ns = c.stuck_dev ? (long long)(tune().spin_ms > 0 ? tune().spin_ms : 2000) * 1000000ll : 0;
   if (phases & CS_PHASE_FINISH) {  // a call that publishes a pose takes the next step id: never 0, alternating parity
-    if (++(*c.step_counter) == 0) *c.step_counter = 2;
-    a.step_id = *c.step_counter;
+    if (++c.step->step_counter == 0) c.step->step_counter = 2;
+    a.step_id = c.step->step_counter;
   }
   cudaError_t e = cudaSuccess;
   S2Plan s2;
@@ -581,7 +648,7 @@ cudaError_t launch_step_ctx(const LaunchCtx& c, CsStepArgs a, int n_points, int 
     used_s2 = true;
     a.s2_points = s2.points;
     a.s2_slab = s2.threads;
-    a.s2_slot = (*c.s2_toggle ^= 1);
+    a.s2_slot = (c.step->s2_toggle ^= 1);
     a.s2_batch = c.n_sessions > 1 ? 1 : 0;
     // (Measured and dropped: letting the candidate sort — the first kernel of the step, one block — prefetch the map around
     // the search pose: 65 k prefetches from one SM take 40 us.  CS_TUNE_W_PREFETCH=1 still selects it for experiments.)
@@ -656,14 +723,14 @@ cudaError_t launch_step_ctx(const LaunchCtx& c, CsStepArgs a, int n_points, int 
     // would starve each other: its draw kernel starts after the search.  Ranks on devices of their own overlap as usual.
     if (a.xchg_world > 1 && a.xchg_serial_draw) g_next_launch_plain = true;
     {  // the counters rotate through three thirds: counted into now / counted into by the previous drawn step / zeroed now
-      const int d = (*c.w_slot)++;
+      const int d = c.step->w_slot++;
       a.w_slot = d % 3;
       // The previous scan's counts size this scan's wedges (the table is then ready before the pose) where a scan is a latency
       // chain; a big scan is throughput, its wedges are narrow (a few degrees of heading change between scans would
       // overfill some) and it builds the table from its own counts.
       a.w_prev = (d > 0 && tune().w_prev >= 0 && n_points <= 2048) ? (d + 2) % 3 : -1;
       a.w_zero = (d + 1) % 3;
-      if (*c.w_slot >= 3000) *c.w_slot -= 2997;  // (keeps d > 0 and d mod 3)
+      if (c.step->w_slot >= 3000) c.step->w_slot -= 2997;  // (keeps d > 0 and d mod 3)
     }
     a.w_general = tune().w_general > 0 ? 1 : 0;
     if (a.w_prefetch == 0 && c.n_sessions == 1 && c.tiled && tune().w_prefetch >= 0) a.w_prefetch = 2;
@@ -675,7 +742,7 @@ cudaError_t launch_step_ctx(const LaunchCtx& c, CsStepArgs a, int n_points, int 
     if (tune().fault == 1 && c.stuck_dev) draw_args.step_id ^= 0x40000000u;  // (fault injection: a pose tag nobody publishes)
     dispatch_layout(c.tiled, [&](auto T) {
       e = launch_pdl(latency ? cs_wedge_kernel<decltype(T)::value, 3> : cs_wedge_kernel<decltype(T)::value, 4>,
-                     dim3((unsigned)blocks, (unsigned)c.n_sessions), dim3(CS_W_THREADS), wedge_smem(c.hs->size), c.stream, c.d_sess, draw_args);
+                     dim3((unsigned)blocks, (unsigned)c.n_sessions), dim3(CS_W_THREADS), 0, c.stream, c.d_sess, draw_args);
     });
     if (e != cudaSuccess) return e;
     (*c.launches)++;
@@ -726,26 +793,13 @@ cudaError_t launch_obstacle_update(cudaStream_t stream, const CsSession* d_sess,
 
 cs_status launch_step(cs_processor* h, CsStepArgs a, int n_points, int rings, bool timing, int ev_base, int phases = CS_PHASE_ALL,
                       const float* next_cand = nullptr, uint64_t log_tag = 0) {
-  LaunchCtx c{};
-  c.num_sms = device_sm_count(h->device);
-  c.stream = h->stream;
-  c.d_sess = h->d_sess;
-  c.tiled = h->tiled;
-  c.n_sessions = 1;
-  c.launches = &h->launches;
-  c.step_counter = &h->step_counter;
-  c.w_slot = &h->w_slot;
-  c.diag = h->d_ring_cycles;
-  c.diag_rings = h->size;
-  c.s2_cap = h->s2_cap;
-  c.s2_min_cand = cs_s2_min_cand(h->cfg.flags);
-  c.s2_toggle = &h->s2_toggle;
+  LaunchCtx c(h, h->cfg.flags, 1, &h->hs);
   c.presort = &h->presort;
   c.next_cand = next_cand;
   c.log_tag = log_tag;
-  c.hs = &h->hs;
   c.spec = h->d_spec;
-  if (h->cfg.flags & CS_FLAG_DEBUG_BOUNDED_SPIN) c.stuck_dev = reinterpret_cast<volatile unsigned*>(h->d_slot + 96);
+  c.diag = h->d_ring_cycles;
+  c.diag_rings = h->size;
   a.hdr_stride = 1;
   const bool want_pose_event = timing || (a.seq_flag && (h->cfg.flags & CS_FLAG_NO_HOST_SPIN));
   c.ev_pose = (want_pose_event && (phases & CS_PHASE_FINISH)) ? h->tm.ev[ev_base + 0] : nullptr;
@@ -808,6 +862,56 @@ void copy_result(cs_result* out, const CsDevResult* r) {
   out->index = r->index;
   out->searched = r->searched;
   out->visits = r->visits;
+}
+
+// The result records of an Update, for the caller: the visits are counted on the device while the integration runs
+// (cs_get_visits after cs_sync), so they read -1 here.
+void copy_update_results(cs_result* out, const CsDevResult* r, int n) {
+  for (int j = 0; j < n; j++) {
+    copy_result(out + j, r + j);
+    out[j].visits = -1;
+  }
+}
+
+// The arguments of an Update step (CoreSLAMProcessor.Update, :717-752) that follow from the handle's step state; the caller
+// adds its inputs, outputs and strides.
+CsStepArgs update_args(const CsHost& h, bool with_offsets, int n_points) {
+  CsStepArgs a{};
+  a.scan_index = h.step.update_count;
+  a.cand_mode = with_offsets ? CS_CAND_OFFSETS : CS_CAND_PHILOX;
+  a.step_mode = CS_STEP_UPDATE;
+  a.parity = h.step.parity;
+  a.do_search = h.step.searches() ? 1 : 0;
+  a.n_cand = h.n_cand;
+  a.cand_first = 0;
+  a.cand_count = h.n_cand + 1;
+  a.s2_host_points = n_points;
+  return a;
+}
+
+cs_status ensure_linear(CsHost* h) {
+  if (!h->d_linear) CS_CUDA(h, cudaMalloc(&h->d_linear, (size_t)h->size * h->size * sizeof(uint16_t)));
+  return CS_OK;
+}
+
+// A row-major copy of `map` in d_linear, queued on the handle's stream.
+cs_status relayout_to_linear(CsHost* h, uint16_t* map) {
+  cs_status st = ensure_linear(h);
+  if (st != CS_OK) return st;
+  dispatch_layout(h->tiled, [&](auto T) {
+    cs_relayout_kernel<decltype(T)::value><<<148 * 8, 256, 0, h->stream>>>(map, h->d_linear, h->size, h->pitch_tiles, 0);
+  });
+  h->launches++;
+  return CS_OK;
+}
+
+// ... and copied out to `pixels` (size * size, row-major); returns once the copy is complete.
+cs_status download_map(CsHost* h, uint16_t* map, uint16_t* pixels) {
+  cs_status st = relayout_to_linear(h, map);
+  if (st != CS_OK) return st;
+  CS_CUDA(h, cudaMemcpyAsync(pixels, h->d_linear, (size_t)h->size * h->size * 2, cudaMemcpyDeviceToHost, h->stream));
+  CS_CUDA(h, cudaStreamSynchronize(h->stream));
+  return CS_OK;
 }
 
 cs_status collect_timing(cs_processor* h, bool had_h2d) {
@@ -884,65 +988,57 @@ cs_status cs_create(const cs_config* cfg, cs_processor** out) {
     cs_destroy(h);
     return st;
   };
-#define CS_CREATE_CUDA(expr)                                                                           \
-  do {                                                                                                 \
-    cudaError_t _e = (expr);                                                                           \
-    if (_e != cudaSuccess) {                                                                           \
-      fail(h, _e == cudaErrorMemoryAllocation ? CS_ERR_OUT_OF_MEMORY : CS_ERR_CUDA, "%s failed: %s", #expr, \
-           cudaGetErrorString(_e));                                                                    \
-      return bail(_e == cudaErrorMemoryAllocation ? CS_ERR_OUT_OF_MEMORY : CS_ERR_CUDA);               \
-    }                                                                                                  \
-  } while (0)
-
-  CS_CREATE_CUDA(cudaSetDevice(h->device));
+  CS_CREATE_CUDA(h, cudaSetDevice(h->device));
   if (cfg->stream) {
     h->stream = (cudaStream_t)cfg->stream;
   } else {
-    CS_CREATE_CUDA(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
+    CS_CREATE_CUDA(h, cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
     h->own_stream = true;
   }
-  CS_CREATE_CUDA(cudaMalloc(&h->d_map, h->map_cells * sizeof(uint16_t)));
-  CS_CREATE_CUDA(cudaMalloc(&h->d_sess, sizeof(CsSession)));
-  if (cfg->flags & CS_FLAG_DEBUG_RAYS) CS_CREATE_CUDA(cudaMalloc(&h->d_ray_dbg, (size_t)max_points * 6 * sizeof(int)));
+  CS_CREATE_CUDA(h, cudaMalloc(&h->d_map, h->map_cells * sizeof(uint16_t)));
+  CS_CREATE_CUDA(h, cudaMalloc(&h->d_sess, sizeof(CsSession)));
+  if (cfg->flags & CS_FLAG_DEBUG_RAYS) CS_CREATE_CUDA(h, cudaMalloc(&h->d_ray_dbg, (size_t)max_points * 6 * sizeof(int)));
   h->ray_stride = (max_points + 31) / 32 * 32;
   h->batch_stride = (h->ray_stride / 32 + 31) / 32 * 32;  // whole 128-byte lines per copy
-  CS_CREATE_CUDA(cudaMalloc(&h->d_rays, (size_t)kRayCopies * h->ray_stride * sizeof(int4)));
-  CS_CREATE_CUDA(cudaMalloc(&h->d_batch_max, (size_t)kRayCopies * h->batch_stride * sizeof(int)));
-  CS_CREATE_CUDA(cudaMalloc(&h->d_prep_words, (size_t)2 * kRayCopies * 16 * sizeof(unsigned long long)));
-  CS_CREATE_CUDA(cudaMemset(h->d_prep_words, 0, (size_t)2 * kRayCopies * 16 * sizeof(unsigned long long)));
-  CS_CREATE_CUDA(cudaMalloc(&h->d_w_rk, (size_t)h->ray_stride * sizeof(int2)));
-  CS_CREATE_CUDA(cudaMalloc(&h->d_w_bkey, (size_t)(h->ray_stride / 32 + 1) * sizeof(float2)));
-  CS_CREATE_CUDA(cudaMalloc(&h->d_w_top, (size_t)3 * wedge_top_words(h->size) * sizeof(int)));
-  CS_CREATE_CUDA(cudaMemset(h->d_w_top, 0, (size_t)3 * wedge_top_words(h->size) * sizeof(int)));
-  CS_CREATE_CUDA(wedge_allow_shared_memory());
-  CS_CREATE_CUDA(cudaMalloc(&h->d_spec, ((size_t)n_cand + 1) * 8 * sizeof(unsigned long long)));
-  CS_CREATE_CUDA(cudaMemset(h->d_spec, 0, ((size_t)n_cand + 1) * 8 * sizeof(unsigned long long)));  // (tag 0 is never a step's)
-  CS_CREATE_CUDA(cudaMalloc(&h->d_distances, ((size_t)n_cand + 1) * sizeof(int)));
-  CS_CREATE_CUDA(cudaMalloc(&h->d_checksum, sizeof(unsigned long long)));
+  CS_CREATE_CUDA(h, cudaMalloc(&h->d_rays, (size_t)kRayCopies * h->ray_stride * sizeof(int4)));
+  CS_CREATE_CUDA(h, cudaMalloc(&h->d_batch_max, (size_t)kRayCopies * h->batch_stride * sizeof(int)));
+  CS_CREATE_CUDA(h, cudaMalloc(&h->d_prep_words, (size_t)2 * kRayCopies * 16 * sizeof(unsigned long long)));
+  CS_CREATE_CUDA(h, cudaMemset(h->d_prep_words, 0, (size_t)2 * kRayCopies * 16 * sizeof(unsigned long long)));
+  CS_CREATE_CUDA(h, cudaMalloc(&h->d_w_rk, (size_t)h->ray_stride * sizeof(int2)));
+  CS_CREATE_CUDA(h, cudaMalloc(&h->d_w_bkey, (size_t)(h->ray_stride / 32 + 1) * sizeof(float2)));
+  CS_CREATE_CUDA(h, cudaMalloc(&h->d_w_top, (size_t)3 * wedge_top_words(h->size) * sizeof(int)));
+  CS_CREATE_CUDA(h, cudaMemset(h->d_w_top, 0, (size_t)3 * wedge_top_words(h->size) * sizeof(int)));
+  CS_CREATE_CUDA(h, wedge_allow_shared_memory());
+  CS_CREATE_CUDA(h, cudaMalloc(&h->d_spec, ((size_t)n_cand + 1) * 8 * sizeof(unsigned long long)));
+  CS_CREATE_CUDA(h, cudaMemset(h->d_spec, 0, ((size_t)n_cand + 1) * 8 * sizeof(unsigned long long)));  // (tag 0 is never a step's)
+  CS_CREATE_CUDA(h, cudaMalloc(&h->d_distances, ((size_t)n_cand + 1) * sizeof(int)));
+  CS_CREATE_CUDA(h, cudaMalloc(&h->d_checksum, sizeof(unsigned long long)));
   if (cs_s2_min_cand(cfg->flags) > 0 && n_cand + 1 >= cs_s2_min_cand(cfg->flags)) {
     h->s2_cap = (int)n_cand + 1;
-    CS_CREATE_CUDA(cudaMalloc(&h->d_s2_sorted, (size_t)2 * h->s2_cap * sizeof(float4)));
-    CS_CREATE_CUDA(cudaMalloc(&h->d_s2_tmp, (size_t)h->s2_cap * sizeof(float4)));
-    CS_CREATE_CUDA(cudaMalloc(&h->d_s2_meta, (size_t)h->s2_cap * sizeof(unsigned long long)));
-    CS_CREATE_CUDA(cudaMalloc(&h->d_s2_acc, (size_t)h->s2_cap * sizeof(unsigned long long)));
-    CS_CREATE_CUDA(cudaMemsetAsync(h->d_s2_acc, 0, (size_t)h->s2_cap * sizeof(unsigned long long), h->stream));
-    CS_CREATE_CUDA(cudaMalloc(&h->d_s2_ghist, (size_t)(CS_SORT_BINS + 1) * sizeof(unsigned)));
-    CS_CREATE_CUDA(cudaMemsetAsync(h->d_s2_ghist, 0, (size_t)(CS_SORT_BINS + 1) * sizeof(unsigned), h->stream));
+    CS_CREATE_CUDA(h, cudaMalloc(&h->d_s2_sorted, (size_t)2 * h->s2_cap * sizeof(float4)));
+    CS_CREATE_CUDA(h, cudaMalloc(&h->d_s2_tmp, (size_t)h->s2_cap * sizeof(float4)));
+    CS_CREATE_CUDA(h, cudaMalloc(&h->d_s2_meta, (size_t)h->s2_cap * sizeof(unsigned long long)));
+    CS_CREATE_CUDA(h, cudaMalloc(&h->d_s2_acc, (size_t)h->s2_cap * sizeof(unsigned long long)));
+    CS_CREATE_CUDA(h, cudaMemsetAsync(h->d_s2_acc, 0, (size_t)h->s2_cap * sizeof(unsigned long long), h->stream));
+    CS_CREATE_CUDA(h, cudaMalloc(&h->d_s2_ghist, (size_t)(CS_SORT_BINS + 1) * sizeof(unsigned)));
+    CS_CREATE_CUDA(h, cudaMemsetAsync(h->d_s2_ghist, 0, (size_t)(CS_SORT_BINS + 1) * sizeof(unsigned), h->stream));
   }
   h->stage_bytes = plan_stage(max_points, (int)n_cand, true).total + 16 * ((size_t)max_points + 1) + 64;  // + segment tables
-  CS_CREATE_CUDA(cudaMalloc(&h->d_cloud, (size_t)max_points * sizeof(float2)));
-  CS_CREATE_CUDA(cudaHostAlloc(&h->h_stage, h->stage_bytes, cudaHostAllocDefault));
-  CS_CREATE_CUDA(cudaMalloc(&h->d_stage, h->stage_bytes));
+  CS_CREATE_CUDA(h, cudaMalloc(&h->d_cloud, (size_t)max_points * sizeof(float2)));
+  CS_CREATE_CUDA(h, cudaHostAlloc(&h->h_stage, h->stage_bytes, cudaHostAllocDefault));
+  CS_CREATE_CUDA(h, cudaMalloc(&h->d_stage, h->stage_bytes));
   if (tune().copy_stream >= 0) {
-    CS_CREATE_CUDA(cudaMalloc(&h->d_stage_b, h->stage_bytes));
-    CS_CREATE_CUDA(cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
-    CS_CREATE_CUDA(cudaEventCreateWithFlags(&h->ev_copy, cudaEventDisableTiming));
-    for (auto& e : h->ev_stage_free) CS_CREATE_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    CS_CREATE_CUDA(h, cudaMalloc(&h->d_stage_b, h->stage_bytes));
+    CS_CREATE_CUDA(h, cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
+    CS_CREATE_CUDA(h, cudaEventCreateWithFlags(&h->ev_copy, cudaEventDisableTiming));
+    for (auto& e : h->ev_stage_free) CS_CREATE_CUDA(h, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
   }
-  CS_CREATE_CUDA(cudaHostAlloc(&h->h_slot, 128, cudaHostAllocMapped));
-  CS_CREATE_CUDA(cudaHostGetDevicePointer((void**)&h->d_slot, h->h_slot, 0));
+  CS_CREATE_CUDA(h, cudaHostAlloc(&h->h_slot, 128, cudaHostAllocMapped));
+  CS_CREATE_CUDA(h, cudaHostGetDevicePointer((void**)&h->d_slot, h->h_slot, 0));
   memset(h->h_slot, 0, 128);
-  for (auto& e : h->tm.ev) CS_CREATE_CUDA(cudaEventCreate(&e));
+  h->h_stuck = h->h_slot + 96;
+  h->d_stuck = h->d_slot + 96;
+  for (auto& e : h->tm.ev) CS_CREATE_CUDA(h, cudaEventCreate(&e));
   if (cfg->obstacle_map_size > 0) {  // :132-133
     CsObstacle& o = h->ho;
     o.size = cfg->obstacle_map_size;
@@ -951,11 +1047,11 @@ cs_status cs_create(const cs_config* cfg, cs_processor** out) {
     o.words_per_row = o.pitch / 8;
     o.scale = (float)cfg->obstacle_map_size / cfg->physical_map_size;  // ObstacleMap.cs:20
     o.max_hits = 10;                                                   // :103
-    CS_CREATE_CUDA(cudaMalloc(&o.pixels, (size_t)o.pitch * o.rows));
-    CS_CREATE_CUDA(cudaMalloc(&o.no_hit, (size_t)o.words_per_row * (o.rows / 4) * sizeof(uint32_t)));
-    CS_CREATE_CUDA(cudaMalloc(&o.touched, sizeof(long long)));
-    CS_CREATE_CUDA(cudaMalloc(&h->d_obst, sizeof(CsObstacle)));
-    CS_CREATE_CUDA(cudaMemcpy(h->d_obst, &o, sizeof(CsObstacle), cudaMemcpyHostToDevice));
+    CS_CREATE_CUDA(h, cudaMalloc(&o.pixels, (size_t)o.pitch * o.rows));
+    CS_CREATE_CUDA(h, cudaMalloc(&o.no_hit, (size_t)o.words_per_row * (o.rows / 4) * sizeof(uint32_t)));
+    CS_CREATE_CUDA(h, cudaMalloc(&o.touched, sizeof(long long)));
+    CS_CREATE_CUDA(h, cudaMalloc(&h->d_obst, sizeof(CsObstacle)));
+    CS_CREATE_CUDA(h, cudaMemcpy(h->d_obst, &o, sizeof(CsObstacle), cudaMemcpyHostToDevice));
   }
 
   // Optional L2 persistence window over the map (the gathers are served from L2 either way when the
@@ -981,20 +1077,7 @@ cs_status cs_create(const cs_config* cfg, cs_processor** out) {
   }
 
   CsSession& s = h->hs;
-  memset(&s, 0, sizeof(s));
-  s.map = h->d_map;
-  s.size = h->size;
-  s.pitch_tiles = h->pitch_tiles;
-  s.scale = h->scale;
-  s.sigma_xy = cfg->sigma_xy;
-  s.sigma_theta = cfg->sigma_theta;
-  s.iters = cfg->iterations_per_thread;
-  s.threads = cfg->num_search_threads;
-  s.n_cand = h->n_cand;
-  s.quality = 50;        // :82
-  s.hole_width = 0.6f;   // :87
-  s.search_begin = 5;    // :92
-  s.seed = cfg->seed;
+  init_session(s, *h, *cfg, h->d_map);
   s.rays = h->d_rays;
   s.batch_max = h->d_batch_max;
   s.ray_copies = kRayCopies;
@@ -1004,7 +1087,6 @@ cs_status cs_create(const cs_config* cfg, cs_processor** out) {
   s.w_rk = h->d_w_rk;
   s.w_bkey = h->d_w_bkey;
   s.w_top = h->d_w_top;
-  s.w_levels = wedge_levels(h->size);
   s.s2_sorted = h->d_s2_sorted;
   s.s2_tmp = h->d_s2_tmp;
   s.s2_meta = h->d_s2_meta;
@@ -1017,7 +1099,6 @@ cs_status cs_create(const cs_config* cfg, cs_processor** out) {
   if (st != CS_OK) return bail(st);
   *out = h;
   return CS_OK;
-#undef CS_CREATE_CUDA
 }
 
 cs_status cs_destroy(cs_processor* h) {
@@ -1075,19 +1156,11 @@ cs_status cs_destroy(cs_processor* h) {
 
 cs_status cs_reset(cs_processor* h) {  // CoreSLAMProcessor.cs:167-175
   CS_CHECK_HANDLE(h);
-  CsSession& s = h->hs;
-  memset(s.state, 0, sizeof(s.state));
-  for (int k = 0; k < 3; k++) s.state[0].pose[k] = h->cfg.start_pose[k];  // :172
-  s.state[0].scan_count = 0;                                               // :174 (lastOdometryPose = 0, :173)
-  s.key[0] = s.key[1] = ~0ull;
-  s.search_done = 0;
-  s.visits_slot[0] = s.visits_slot[1] = 0;
-  s.ring_ticket[0] = s.ring_ticket[1] = 0;
-  memset(s.ll_pose, 0, sizeof(s.ll_pose));
-  h->parity = 0;
-  h->scan_count = 0;
-  h->update_count = 0;
-  h->search_begin = s.search_begin;
+  reset_session(h->hs, h->cfg.start_pose);
+  h->step.parity = 0;
+  h->step.scan_count = 0;
+  h->step.update_count = 0;
+  h->step.search_begin = h->hs.search_begin;
   cs_status st = push_session(h);
   if (st != CS_OK) return st;
   st = launch_fill(h, (uint16_t)((CS_TS_OBSTACLE + CS_TS_NO_OBSTACLE) / 2));  // :169
@@ -1193,7 +1266,7 @@ cs_status cs_set_hole_width(cs_processor* h, float metres) {
 cs_status cs_set_position_search_beginning(cs_processor* h, int32_t scans) {
   CS_CHECK_HANDLE(h);
   h->hs.search_begin = scans;
-  h->search_begin = scans;
+  h->step.search_begin = scans;
   return patch_session(h, offsetof(CsSession, search_begin), &h->hs.search_begin, sizeof(int));
 }
 
@@ -1201,7 +1274,7 @@ cs_status cs_get_pose(cs_processor* h, float pose[3]) {
   CS_CHECK_HANDLE(h);
   if (!pose) return fail(h, CS_ERR_INVALID_ARGUMENT, "null pose");
   CsState st;
-  CS_CUDA(h, cudaMemcpyAsync(&st, reinterpret_cast<uint8_t*>(h->d_sess) + offsetof(CsSession, state) + h->parity * sizeof(CsState),
+  CS_CUDA(h, cudaMemcpyAsync(&st, reinterpret_cast<uint8_t*>(h->d_sess) + offsetof(CsSession, state) + h->step.parity * sizeof(CsState),
                              sizeof(CsState), cudaMemcpyDeviceToHost, h->stream));
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
   pose[0] = st.pose[0]; pose[1] = st.pose[1]; pose[2] = st.pose[2];
@@ -1214,8 +1287,8 @@ cs_status cs_set_pose(cs_processor* h, const float pose[3], const float last_odo
   CsState st{};
   for (int k = 0; k < 3; k++) { st.pose[k] = pose[k]; st.last_odo[k] = last_odometry[k]; }
   st.scan_count = scan_count;
-  h->scan_count = scan_count;
-  return patch_session(h, offsetof(CsSession, state) + h->parity * sizeof(CsState), &st, sizeof(CsState));
+  h->step.scan_count = scan_count;
+  return patch_session(h, offsetof(CsSession, state) + h->step.parity * sizeof(CsState), &st, sizeof(CsState));
 }
 
 cs_status cs_get_map_info(const cs_processor* h, int32_t* size, float* scale) {
@@ -1265,7 +1338,7 @@ cs_status cs_search(cs_processor* h, const float* points, int32_t n_points, cons
   a.scan_index = scan_index;
   a.cand_mode = cand_poses ? CS_CAND_ABSOLUTE : CS_CAND_PHILOX;
   a.step_mode = CS_STEP_SEARCH_ONLY;
-  a.parity = h->parity;
+  a.parity = h->step.parity;
   a.do_search = 1;
   a.n_cand = n_cand;
   a.cand_first = 0;
@@ -1309,12 +1382,12 @@ cs_status cs_integrate(cs_processor* h, const float* points, int32_t n_points, c
   a.points = reinterpret_cast<const float2*>(h->d_stage + sp.off_points);
   a.result = reinterpret_cast<CsDevResult*>(h->d_slot);
   a.step_mode = CS_STEP_INTEGRATE_ONLY;
-  a.parity = h->parity;
+  a.parity = h->step.parity;
   cs_status st = launch_step(h, a, n_points, rings_hint(h, max_range_of(points, n_points)), false, 0);
   if (st != CS_OK) return st;
   if (visits) {
     long long v = 0;
-    CS_CUDA(h, cudaMemcpyAsync(&v, reinterpret_cast<uint8_t*>(h->d_sess) + offsetof(CsSession, visits_slot) + (h->step_counter & 1u) * sizeof(long long), sizeof(v),
+    CS_CUDA(h, cudaMemcpyAsync(&v, reinterpret_cast<uint8_t*>(h->d_sess) + offsetof(CsSession, visits_slot) + (h->step.step_counter & 1u) * sizeof(long long), sizeof(v),
                                cudaMemcpyDeviceToHost, h->stream));
     CS_CUDA(h, cudaStreamSynchronize(h->stream));
     *visits = v;
@@ -1381,7 +1454,7 @@ static cs_status stage_update(cs_processor* h, const float* points, int32_t n_po
 
   // The previous call's integration may still be running: the pinned block is free again (its H2D copy
   // finished before that call's pose flag), the device block is protected by stream order.
-  const bool do_search = h->scan_count >= h->search_begin;  // :726
+  const bool do_search = h->step.searches();
   const bool with_offsets = cand_offsets != nullptr && do_search;
   StagePlan sp = plan_stage(n_points, with_offsets ? h->n_cand : 0, false);
   CsStepHeader* hdr = reinterpret_cast<CsStepHeader*>(h->h_stage);
@@ -1424,22 +1497,13 @@ static cs_status stage_update(cs_processor* h, const float* points, int32_t n_po
   }
   if (timing) cudaEventRecord(h->tm.ev[1], h->stream);
 
-  CsStepArgs a{};
+  CsStepArgs a = update_args(*h, with_offsets, n_points);
   a.hdr = reinterpret_cast<const CsStepHeader*>(d_base);
   a.points = seg ? h->d_cloud : reinterpret_cast<const float2*>(d_base + sp.off_points);
   a.cand = with_offsets ? reinterpret_cast<const float*>(d_base + sp.off_cand) : nullptr;
   a.result = reinterpret_cast<CsDevResult*>(h->d_slot);
   a.seq_flag = reinterpret_cast<volatile unsigned*>(h->d_slot + 64);
   a.seq_value = ++h->seq;
-  a.scan_index = h->update_count;
-  a.cand_mode = with_offsets ? CS_CAND_OFFSETS : CS_CAND_PHILOX;
-  a.step_mode = CS_STEP_UPDATE;
-  a.parity = h->parity;
-  a.do_search = do_search ? 1 : 0;
-  a.n_cand = h->n_cand;
-  a.cand_first = 0;
-  a.cand_count = h->n_cand + 1;
-  a.s2_host_points = n_points;
   a.empty_cloud = (do_search && n_points == 0) ? 1 : 0;
   if (!split_phase) apply_group(h, a);  // (cs_update_begin / _finish: the caller exchanges the key between the phases)
   *out_args = a;
@@ -1448,25 +1512,22 @@ static cs_status stage_update(cs_processor* h, const float* points, int32_t n_po
 
 // Host-side bookkeeping after an Update has been enqueued, the wait for the pose, and the result copy.
 static cs_status complete_update(cs_processor* h, const CsStepArgs& a, bool timing, cs_result* out) {
-  h->parity ^= 1;
-  h->update_count++;
-  if (!a.do_search) h->scan_count++;  // :741
+  h->step.advance(a.do_search);
   cs_status st = wait_for_pose(h, a.seq_value, h->tm.ev[2]);
   if (st != CS_OK) return st;
   if (timing) {
     st = collect_timing(h, true);
     if (st != CS_OK) return st;
   }
-  CS_CHECK_STUCK(h, h->h_slot + 96, fail);
+  CS_CHECK_STUCK(h);
   if (reinterpret_cast<const CsDevResult*>(h->h_slot)->searched < 0)
     return fail(h, CS_ERR_NCCL, "candidate-split group: a rank never delivered its arg-min (exchange timed out after %.1f s)",
                 (double)CS_XCHG_TIMEOUT_NS * 1e-9);
   if (out) {
-    copy_result(out, reinterpret_cast<const CsDevResult*>(h->h_slot));
-    out->visits = -1;  // counted on the device while the integration runs; cs_get_visits() after cs_sync()
+    copy_update_results(out, reinterpret_cast<const CsDevResult*>(h->h_slot), 1);
     if (timing) {
       long long v = 0;
-      CS_CUDA(h, cudaMemcpyAsync(&v, reinterpret_cast<uint8_t*>(h->d_sess) + offsetof(CsSession, visits_slot) + (h->step_counter & 1u) * sizeof(long long), sizeof(v),
+      CS_CUDA(h, cudaMemcpyAsync(&v, reinterpret_cast<uint8_t*>(h->d_sess) + offsetof(CsSession, visits_slot) + (h->step.step_counter & 1u) * sizeof(long long), sizeof(v),
                                  cudaMemcpyDeviceToHost, h->stream));
       CS_CUDA(h, cudaStreamSynchronize(h->stream));
       out->visits = v;
@@ -1696,33 +1757,21 @@ static cs_status export_wait(cs_processor* h) {
   return CS_OK;
 }
 
-static cs_status ensure_linear(cs_processor* h) {
-  cs_status st = export_wait(h);  // the staging buffers below may still be read by an export's D2H copy
-  if (st != CS_OK) return st;
-  if (!h->d_linear) CS_CUDA(h, cudaMalloc(&h->d_linear, (size_t)h->size * h->size * sizeof(uint16_t)));
-  return CS_OK;
-}
-
 cs_status cs_map_download(cs_processor* h, uint16_t* pixels) {
   NvtxRange nvtx_range("cs_map_download");
   CS_CHECK_HANDLE(h);
   if (!pixels) return fail(h, CS_ERR_INVALID_ARGUMENT, "null pixels");
-  cs_status st = ensure_linear(h);
+  cs_status st = export_wait(h);  // d_linear may still be read by an export's D2H copy
   if (st != CS_OK) return st;
-  dispatch_layout(h->tiled, [&](auto T) {
-    cs_relayout_kernel<decltype(T)::value><<<148 * 8, 256, 0, h->stream>>>(h->d_map, h->d_linear, h->size, h->pitch_tiles, 0);
-  });
-  h->launches++;
-  CS_CUDA(h, cudaMemcpyAsync(pixels, h->d_linear, (size_t)h->size * h->size * 2, cudaMemcpyDeviceToHost, h->stream));
-  CS_CUDA(h, cudaStreamSynchronize(h->stream));
-  return CS_OK;
+  return download_map(h, h->d_map, pixels);
 }
 
 cs_status cs_map_upload(cs_processor* h, const uint16_t* pixels) {
   NvtxRange nvtx_range("cs_map_upload");
   CS_CHECK_HANDLE(h);
   if (!pixels) return fail(h, CS_ERR_INVALID_ARGUMENT, "null pixels");
-  cs_status st = ensure_linear(h);
+  cs_status st = export_wait(h);  // d_linear may still be read by an export's D2H copy
+  if (st == CS_OK) st = ensure_linear(h);
   if (st != CS_OK) return st;
   CS_CUDA(h, cudaMemcpyAsync(h->d_linear, pixels, (size_t)h->size * h->size * 2, cudaMemcpyHostToDevice, h->stream));
   dispatch_layout(h->tiled, [&](auto T) {
@@ -1780,11 +1829,8 @@ cs_status cs_map_export_begin(cs_processor* h, int32_t format, void* dst) {
   const void* src = nullptr;
   size_t bytes = 0;
   if (format == CS_EXPORT_GRAY16) {
-    if (!h->d_linear) CS_CUDA(h, cudaMalloc(&h->d_linear, cells * sizeof(uint16_t)));
-    dispatch_layout(h->tiled, [&](auto T) {
-      cs_relayout_kernel<decltype(T)::value><<<148 * 8, 256, 0, h->stream>>>(h->d_map, h->d_linear, h->size, h->pitch_tiles, 0);
-    });
-    h->launches++;
+    cs_status st = relayout_to_linear(h, h->d_map);
+    if (st != CS_OK) return st;
     src = h->d_linear; bytes = cells * 2;
   } else if (format == CS_EXPORT_PACKED4) {
     if (!h->d_packed) CS_CUDA(h, cudaMalloc(&h->d_packed, cells / 2));
@@ -1815,18 +1861,23 @@ cs_status cs_map_export_wait(cs_processor* h) {
   return export_wait(h);
 }
 
+// Queues the checksum of `map` (cs_host_map_checksum of its row-major pixels) into *out; the caller synchronises.
+static cs_status queue_map_checksum(CsHost* h, const uint16_t* map, int blocks, uint64_t* out) {
+  CS_CUDA(h, cudaMemsetAsync(h->d_checksum, 0, sizeof(unsigned long long), h->stream));
+  dispatch_layout(h->tiled, [&](auto T) {
+    cs_checksum_kernel<decltype(T)::value><<<blocks, 256, 0, h->stream>>>(map, h->size, h->pitch_tiles, h->d_checksum);
+  });
+  h->launches++;
+  CS_CUDA(h, cudaMemcpyAsync(out, h->d_checksum, sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+  return CS_OK;
+}
+
 cs_status cs_map_checksum(cs_processor* h, uint64_t* checksum) {
   CS_CHECK_HANDLE(h);
   if (!checksum) return fail(h, CS_ERR_INVALID_ARGUMENT, "null checksum");
-  CS_CUDA(h, cudaMemsetAsync(h->d_checksum, 0, sizeof(unsigned long long), h->stream));
-  dispatch_layout(h->tiled, [&](auto T) {
-    cs_checksum_kernel<decltype(T)::value><<<148 * 8, 256, 0, h->stream>>>(h->d_map, h->size, h->pitch_tiles, h->d_checksum);
-  });
-  h->launches++;
-  unsigned long long v = 0;
-  CS_CUDA(h, cudaMemcpyAsync(&v, h->d_checksum, sizeof(v), cudaMemcpyDeviceToHost, h->stream));
+  cs_status st = queue_map_checksum(h, h->d_map, 148 * 8, checksum);
+  if (st != CS_OK) return st;
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
-  *checksum = v;
   return CS_OK;
 }
 
@@ -1866,7 +1917,7 @@ cs_status cs_get_visits(cs_processor* h, int64_t* visits) {
   CS_CHECK_HANDLE(h);
   if (!visits) return fail(h, CS_ERR_INVALID_ARGUMENT, "null visits");
   long long v = 0;
-  CS_CUDA(h, cudaMemcpyAsync(&v, reinterpret_cast<uint8_t*>(h->d_sess) + offsetof(CsSession, visits_slot) + (h->step_counter & 1u) * sizeof(long long), sizeof(v),
+  CS_CUDA(h, cudaMemcpyAsync(&v, reinterpret_cast<uint8_t*>(h->d_sess) + offsetof(CsSession, visits_slot) + (h->step.step_counter & 1u) * sizeof(long long), sizeof(v),
                              cudaMemcpyDeviceToHost, h->stream));
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
   *visits = v;
@@ -2152,31 +2203,19 @@ cs_status cs_replay(cs_processor* h, const cs_scanlog* log, int32_t first, int32
   }
   for (int i = 0; i < count; i++) {
     const int sidx = first + i;
-    const bool do_search = h->scan_count >= h->search_begin;
-    CsStepArgs a{};
+    CsStepArgs a = update_args(*h, log->n_offsets > 0, log->h_hdr[sidx].n_points);
     a.hdr = log->d_hdr + sidx;
     a.points = log->d_points + (size_t)sidx * log->max_points;
     a.cand = log->n_offsets > 0 ? log->d_offsets + (size_t)sidx * log->n_offsets * 3 : nullptr;
     a.result = log->d_results + sidx;
     a.visits_out = reinterpret_cast<long long*>(reinterpret_cast<uint8_t*>(log->d_results + sidx) + offsetof(CsDevResult, visits));
-    a.scan_index = h->update_count;
-    a.cand_mode = log->n_offsets > 0 ? CS_CAND_OFFSETS : CS_CAND_PHILOX;
-    a.step_mode = CS_STEP_UPDATE;
-    a.parity = h->parity;
-    a.do_search = do_search ? 1 : 0;
-    a.n_cand = h->n_cand;
-    a.cand_first = 0;
-    a.cand_count = h->n_cand + 1;
-    a.s2_host_points = log->h_hdr[sidx].n_points;
     apply_group(h, a);
     // (the next scan's table, if the log has one: its sort is queued behind this scan's draw kernel, see Presort)
     const float* next_cand = (log->n_offsets > 0 && sidx + 1 < log->n_scans) ? log->d_offsets + (size_t)(sidx + 1) * log->n_offsets * 3 : nullptr;
     cs_status st = launch_step(h, a, log->h_hdr[sidx].n_points, rings_hint(h, log->h_max_range[sidx]), per_kernel, 2, CS_PHASE_ALL,
                                next_cand, log->generation);
     if (st != CS_OK) return st;
-    h->parity ^= 1;
-    h->update_count++;
-    if (!do_search) h->scan_count++;
+    h->step.advance(a.do_search);
   }
   if (timing && !per_kernel) cudaEventRecord(h->tm.ev[4], h->stream);
   if (results && count > 0) {
@@ -2204,32 +2243,23 @@ cs_status cs_replay(cs_processor* h, const cs_scanlog* log, int32_t first, int32
 // =====================================================================================================
 }  // extern "C"
 
-struct cs_batch {
-  int device = 0, n = 0;
-  cudaStream_t stream = nullptr;
-  bool own_stream = false, tiled = true;
-  int size = 0, pitch_tiles = 0, max_points = 0, n_cand = 0;
+struct cs_batch : CsHost {
+  int n = 0;
+  int max_points = 0;
   int user_max_points = 0;  // the caller's cfg.max_points: stride of the caller's `points` array (max_points above is the
                             // internal stride of the staging / device blocks, rounded up to even for 16-byte alignment)
-  float scale = 0.f;
-  size_t map_cells = 0;
   std::vector<CsSession> hs;
-  CsSession* d_sess = nullptr;
   uint16_t* d_maps = nullptr;
-  uint16_t* d_linear = nullptr;
   int4* d_rays = nullptr;
   int* d_batch_max = nullptr;
   unsigned long long* d_prep_words = nullptr;
-  unsigned long long* d_checksum = nullptr;
   // wedge integration scratch of all sessions (CsSession::w_*)
   int2* d_w_rk = nullptr;
   float2* d_w_bkey = nullptr;
   int* d_w_top = nullptr;
-  int w_slot = 0;
   // slab-search scratch of all sessions (CsSession::s2_*): per session 2*cap sorted + cap tmp entries, cap meta + cap acc words
   float4* d_s2_entries = nullptr;
   unsigned long long* d_s2_words = nullptr;
-  int s2_cap = 0, s2_toggle = 0;
   uint32_t flags = 0;
   // staging: [n headers][n * max_points points][n * n_cand offsets]
   size_t off_points = 0, off_cand = 0, stage_bytes = 0;
@@ -2237,12 +2267,6 @@ struct cs_batch {
   uint8_t* d_stage = nullptr;
   CsDevResult* d_results = nullptr;
   CsDevResult* h_results = nullptr;  // pinned
-  uint8_t* h_stuck = nullptr;        // CS_FLAG_DEBUG_BOUNDED_SPIN: pinned+mapped stuck-poll word (CsSpin), and its device address
-  uint8_t* d_stuck = nullptr;
-  int parity = 0, scan_count = 0, search_begin = 5;
-  unsigned update_count = 0;
-  uint64_t launches = 0;
-  unsigned step_counter = 0;
   // cs_batch_submit / cs_batch_collect: two staging + result slots, so that the host stages step k+1 while step k runs
   uint8_t* pipe_h_stage[2] = {nullptr, nullptr};
   uint8_t* pipe_d_stage[2] = {nullptr, nullptr};
@@ -2250,73 +2274,7 @@ struct cs_batch {
   CsDevResult* pipe_h_results[2] = {nullptr, nullptr};
   cudaEvent_t pipe_done[2] = {nullptr, nullptr};
   unsigned pipe_submitted = 0, pipe_collected = 0;
-  std::string error;
-  bool poisoned = false;
 };
-
-namespace {
-cs_status bfail(cs_batch* b, cs_status code, const char* fmt, ...) {
-  char buf[512];
-  va_list ap;
-  va_start(ap, fmt);
-  vsnprintf(buf, sizeof(buf), fmt, ap);
-  va_end(ap);
-  if (b) {
-    b->error = buf;
-    if (code == CS_ERR_CUDA) b->poisoned = true;
-  } else {
-    g_create_error = buf;
-  }
-  return code;
-}
-#define CS_BCUDA(b, expr)                                                                                   \
-  do {                                                                                                      \
-    cudaError_t _e = (expr);                                                                                \
-    if (_e != cudaSuccess) return bfail((b), CS_ERR_CUDA, "%s failed: %s (line %d)", #expr, cudaGetErrorString(_e), __LINE__); \
-  } while (0)
-#define CS_CHECK_BATCH(b)                                                           \
-  do {                                                                              \
-    if (!(b)) return CS_ERR_INVALID_ARGUMENT;                                       \
-    if ((b)->poisoned) return CS_ERR_CUDA;                                          \
-    CS_CHECK_STUCK(b, (b)->h_stuck, bfail);                                         \
-    if (cudaSetDevice((b)->device) != cudaSuccess) return bfail((b), CS_ERR_CUDA, "cudaSetDevice failed"); \
-  } while (0)
-
-LaunchCtx batch_ctx(cs_batch* b) {
-  LaunchCtx c{};
-  c.num_sms = device_sm_count(b->device);
-  c.stream = b->stream;
-  c.d_sess = b->d_sess;
-  c.tiled = b->tiled;
-  c.n_sessions = b->n;
-  c.launches = &b->launches;
-  c.step_counter = &b->step_counter;
-  c.w_slot = &b->w_slot;
-  c.s2_cap = b->s2_cap;
-  c.s2_min_cand = cs_s2_min_cand(b->flags, b->n);
-  c.s2_toggle = &b->s2_toggle;
-  c.hs = &b->hs[0];
-  c.stuck_dev = reinterpret_cast<volatile unsigned*>(b->d_stuck);
-  return c;
-}
-
-void batch_reset_host(cs_batch* b, const cs_config* cfgs) {
-  for (int j = 0; j < b->n; j++) {
-    CsSession& s = b->hs[j];
-    memset(s.state, 0, sizeof(s.state));
-    if (cfgs)
-      for (int k = 0; k < 3; k++) s.state[0].pose[k] = cfgs[j].start_pose[k];
-    s.key[0] = s.key[1] = ~0ull;
-    s.search_done = 0;
-    s.visits_slot[0] = s.visits_slot[1] = 0;
-    s.ring_ticket[0] = s.ring_ticket[1] = 0;
-    memset(s.ll_pose, 0, sizeof(s.ll_pose));
-  }
-  b->parity = 0;
-  b->scan_count = 0;
-  b->update_count = 0;
-}
-}  // namespace
 
 extern "C" {
 
@@ -2324,31 +2282,31 @@ const char* cs_batch_last_error(const cs_batch* b) { return b ? b->error.c_str()
 
 cs_status cs_batch_create(const cs_config* cfgs, int32_t n_sessions, cs_batch** out) {
   if (!cfgs || !out || n_sessions <= 0 || n_sessions > 65535)
-    return bfail(nullptr, CS_ERR_INVALID_ARGUMENT, "cs_batch_create: bad argument (1..65535 sessions)");
+    return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "cs_batch_create: bad argument (1..65535 sessions)");
   *out = nullptr;
   const cs_config& c0 = cfgs[0];
   if (c0.hole_map_size < 8 || c0.hole_map_size > 16384 || !(c0.physical_map_size > 0.f) || c0.iterations_per_thread < 0)
-    return bfail(nullptr, CS_ERR_INVALID_ARGUMENT, "cs_batch_create: bad map size / iterations");
+    return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "cs_batch_create: bad map size / iterations");
   for (int j = 0; j < n_sessions; j++)
     if (cfgs[j].obstacle_map_size != 0)
-      return bfail(nullptr, CS_ERR_INVALID_ARGUMENT, "cs_batch_create: session batches carry no ObstacleMap (obstacle_map_size must be 0)");
+      return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "cs_batch_create: session batches carry no ObstacleMap (obstacle_map_size must be 0)");
   for (int j = 1; j < n_sessions; j++) {
     const cs_config& c = cfgs[j];
     if (c.hole_map_size != c0.hole_map_size || c.physical_map_size != c0.physical_map_size ||
         c.iterations_per_thread != c0.iterations_per_thread || c.num_search_threads != c0.num_search_threads ||
         c.device != c0.device || c.max_points != c0.max_points || c.flags != c0.flags)
-      return bfail(nullptr, CS_ERR_INVALID_ARGUMENT,
+      return fail(nullptr, CS_ERR_INVALID_ARGUMENT,
                    "cs_batch_create: session %d differs in map size / iterations / threads / device / max_points / flags "
                    "(only start_pose, sigma_xy, sigma_theta and seed may vary)", j);
   }
   const int threads = c0.num_search_threads > 0 ? c0.num_search_threads : 1;
   const long long n_cand = (long long)threads * c0.iterations_per_thread;
-  if (n_cand > (1ll << 26)) return bfail(nullptr, CS_ERR_INVALID_ARGUMENT, "too many candidates per scan");
+  if (n_cand > (1ll << 26)) return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "too many candidates per scan");
   const int max_points = c0.max_points > 0 ? c0.max_points : 16384;
-  if (max_points > 65536) return bfail(nullptr, CS_ERR_INVALID_ARGUMENT, "max_points must be <= 65536");
+  if (max_points > 65536) return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "max_points must be <= 65536");
   int ndev = cs_device_count();
-  if (ndev <= 0) return bfail(nullptr, CS_ERR_NO_DEVICE, "no CUDA device: this library has no CPU path");
-  if (c0.device < 0 || c0.device >= ndev) return bfail(nullptr, CS_ERR_INVALID_ARGUMENT, "device %d out of range", c0.device);
+  if (ndev <= 0) return fail(nullptr, CS_ERR_NO_DEVICE, "no CUDA device: this library has no CPU path");
+  if (c0.device < 0 || c0.device >= ndev) return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "device %d out of range", c0.device);
 
   cs_batch* b = new cs_batch();
   b->device = c0.device;
@@ -2360,69 +2318,57 @@ cs_status cs_batch_create(const cs_config* cfgs, int32_t n_sessions, cs_batch** 
   b->max_points = (max_points + 1) & ~1;
   b->n_cand = (int)n_cand;
   b->scale = (float)c0.hole_map_size / c0.physical_map_size;
+  b->flags = c0.flags;
   b->map_cells = b->tiled ? (size_t)b->pitch_tiles * b->pitch_tiles * 64 : (size_t)b->size * b->size;
   b->hs.assign((size_t)n_sessions, CsSession{});
   b->off_points = align_up(sizeof(CsStepHeader) * (size_t)n_sessions, 16);
   b->off_cand = align_up(b->off_points + (size_t)n_sessions * b->max_points * 8, 16);
   b->stage_bytes = align_up(b->off_cand + (size_t)n_sessions * (size_t)n_cand * 12, 16);
 
-  bool ok = cudaSetDevice(b->device) == cudaSuccess;
-  if (ok && c0.stream) b->stream = (cudaStream_t)c0.stream;
-  else if (ok) { ok = cudaStreamCreateWithFlags(&b->stream, cudaStreamNonBlocking) == cudaSuccess; b->own_stream = ok; }
-  ok = ok && cudaMalloc(&b->d_maps, b->map_cells * sizeof(uint16_t) * (size_t)n_sessions) == cudaSuccess;
-  ok = ok && cudaMalloc(&b->d_sess, sizeof(CsSession) * (size_t)n_sessions) == cudaSuccess;
-  ok = ok && cudaMalloc(&b->d_rays, (size_t)b->max_points * sizeof(int4) * (size_t)n_sessions) == cudaSuccess;
-  ok = ok && cudaMalloc(&b->d_batch_max, ((size_t)b->max_points / 32 + 1) * sizeof(int) * (size_t)n_sessions) == cudaSuccess;
-  ok = ok && cudaMalloc(&b->d_prep_words, (size_t)n_sessions * 2 * 16 * sizeof(unsigned long long)) == cudaSuccess;
-  ok = ok && cudaMemset(b->d_prep_words, 0, (size_t)n_sessions * 2 * 16 * sizeof(unsigned long long)) == cudaSuccess;
-  ok = ok && cudaMalloc(&b->d_checksum, sizeof(unsigned long long)) == cudaSuccess;
-  ok = ok && cudaMalloc(&b->d_w_rk, (size_t)b->max_points * sizeof(int2) * (size_t)n_sessions) == cudaSuccess;
-  ok = ok && cudaMalloc(&b->d_w_bkey, ((size_t)b->max_points / 32 + 1) * sizeof(float2) * (size_t)n_sessions) == cudaSuccess;
-  ok = ok && cudaMalloc(&b->d_w_top, (size_t)n_sessions * 3 * wedge_top_words(b->size) * sizeof(int)) == cudaSuccess;
-  ok = ok && cudaMemset(b->d_w_top, 0, (size_t)n_sessions * 3 * wedge_top_words(b->size) * sizeof(int)) == cudaSuccess;
-  ok = ok && wedge_allow_shared_memory() == cudaSuccess;
-  b->flags = c0.flags;
-  {
-    const int min_cand = cs_s2_min_cand(c0.flags, n_sessions);
-    if (n_sessions > 1 && min_cand > 0 && n_cand + 1 >= min_cand && n_cand + 1 <= CS_SORT_THREADS * CS_SORT_REG) {
-      b->s2_cap = n_cand + 1;
-      const size_t cap = (size_t)b->s2_cap;
-      ok = ok && cudaMalloc(&b->d_s2_entries, (size_t)n_sessions * 3 * cap * sizeof(float4)) == cudaSuccess;
-      ok = ok && cudaMalloc(&b->d_s2_words, (size_t)n_sessions * 2 * cap * sizeof(unsigned long long)) == cudaSuccess;
-      ok = ok && cudaMemsetAsync(b->d_s2_words, 0, (size_t)n_sessions * 2 * cap * sizeof(unsigned long long), b->stream) == cudaSuccess;
-    }
-  }
-  ok = ok && cudaHostAlloc(&b->h_stage, b->stage_bytes, cudaHostAllocDefault) == cudaSuccess;
-  ok = ok && cudaMalloc(&b->d_stage, b->stage_bytes) == cudaSuccess;
-  ok = ok && cudaMalloc(&b->d_results, sizeof(CsDevResult) * (size_t)n_sessions) == cudaSuccess;
-  ok = ok && cudaHostAlloc(&b->h_results, sizeof(CsDevResult) * (size_t)n_sessions, cudaHostAllocDefault) == cudaSuccess;
-  if (b->flags & CS_FLAG_DEBUG_BOUNDED_SPIN) {
-    ok = ok && cudaHostAlloc(&b->h_stuck, 64, cudaHostAllocMapped) == cudaSuccess;
-    ok = ok && cudaHostGetDevicePointer((void**)&b->d_stuck, b->h_stuck, 0) == cudaSuccess;
-    if (ok) memset(b->h_stuck, 0, 64);
-  }
-  if (!ok) {
-    cudaError_t e = cudaGetLastError();
-    bfail(nullptr, e == cudaErrorMemoryAllocation ? CS_ERR_OUT_OF_MEMORY : CS_ERR_CUDA, "cs_batch_create: %s", cudaGetErrorString(e));
+  auto bail = [&](cs_status st) {
+    g_create_error = b->error;
     cs_batch_destroy(b);
-    return e == cudaErrorMemoryAllocation ? CS_ERR_OUT_OF_MEMORY : CS_ERR_CUDA;
+    return st;
+  };
+  CS_CREATE_CUDA(b, cudaSetDevice(b->device));
+  if (c0.stream) {
+    b->stream = (cudaStream_t)c0.stream;
+  } else {
+    CS_CREATE_CUDA(b, cudaStreamCreateWithFlags(&b->stream, cudaStreamNonBlocking));
+    b->own_stream = true;
+  }
+  CS_CREATE_CUDA(b, cudaMalloc(&b->d_maps, b->map_cells * sizeof(uint16_t) * (size_t)n_sessions));
+  CS_CREATE_CUDA(b, cudaMalloc(&b->d_sess, sizeof(CsSession) * (size_t)n_sessions));
+  CS_CREATE_CUDA(b, cudaMalloc(&b->d_rays, (size_t)b->max_points * sizeof(int4) * (size_t)n_sessions));
+  CS_CREATE_CUDA(b, cudaMalloc(&b->d_batch_max, ((size_t)b->max_points / 32 + 1) * sizeof(int) * (size_t)n_sessions));
+  CS_CREATE_CUDA(b, cudaMalloc(&b->d_prep_words, (size_t)n_sessions * 2 * 16 * sizeof(unsigned long long)));
+  CS_CREATE_CUDA(b, cudaMemset(b->d_prep_words, 0, (size_t)n_sessions * 2 * 16 * sizeof(unsigned long long)));
+  CS_CREATE_CUDA(b, cudaMalloc(&b->d_checksum, sizeof(unsigned long long)));
+  CS_CREATE_CUDA(b, cudaMalloc(&b->d_w_rk, (size_t)b->max_points * sizeof(int2) * (size_t)n_sessions));
+  CS_CREATE_CUDA(b, cudaMalloc(&b->d_w_bkey, ((size_t)b->max_points / 32 + 1) * sizeof(float2) * (size_t)n_sessions));
+  CS_CREATE_CUDA(b, cudaMalloc(&b->d_w_top, (size_t)n_sessions * 3 * wedge_top_words(b->size) * sizeof(int)));
+  CS_CREATE_CUDA(b, cudaMemset(b->d_w_top, 0, (size_t)n_sessions * 3 * wedge_top_words(b->size) * sizeof(int)));
+  CS_CREATE_CUDA(b, wedge_allow_shared_memory());
+  const int min_cand = cs_s2_min_cand(b->flags, n_sessions);
+  if (n_sessions > 1 && min_cand > 0 && n_cand + 1 >= min_cand && n_cand + 1 <= CS_SORT_THREADS * CS_SORT_REG) {
+    b->s2_cap = n_cand + 1;
+    const size_t cap = (size_t)b->s2_cap;
+    CS_CREATE_CUDA(b, cudaMalloc(&b->d_s2_entries, (size_t)n_sessions * 3 * cap * sizeof(float4)));
+    CS_CREATE_CUDA(b, cudaMalloc(&b->d_s2_words, (size_t)n_sessions * 2 * cap * sizeof(unsigned long long)));
+    CS_CREATE_CUDA(b, cudaMemsetAsync(b->d_s2_words, 0, (size_t)n_sessions * 2 * cap * sizeof(unsigned long long), b->stream));
+  }
+  CS_CREATE_CUDA(b, cudaHostAlloc(&b->h_stage, b->stage_bytes, cudaHostAllocDefault));
+  CS_CREATE_CUDA(b, cudaMalloc(&b->d_stage, b->stage_bytes));
+  CS_CREATE_CUDA(b, cudaMalloc(&b->d_results, sizeof(CsDevResult) * (size_t)n_sessions));
+  CS_CREATE_CUDA(b, cudaHostAlloc(&b->h_results, sizeof(CsDevResult) * (size_t)n_sessions, cudaHostAllocDefault));
+  if (b->flags & CS_FLAG_DEBUG_BOUNDED_SPIN) {
+    CS_CREATE_CUDA(b, cudaHostAlloc(&b->h_stuck, 64, cudaHostAllocMapped));
+    CS_CREATE_CUDA(b, cudaHostGetDevicePointer((void**)&b->d_stuck, b->h_stuck, 0));
+    memset(b->h_stuck, 0, 64);
   }
   for (int j = 0; j < n_sessions; j++) {
     CsSession& s = b->hs[j];
-    memset(&s, 0, sizeof(s));
-    s.map = b->d_maps + (size_t)j * b->map_cells;
-    s.size = b->size;
-    s.pitch_tiles = b->pitch_tiles;
-    s.scale = b->scale;
-    s.sigma_xy = cfgs[j].sigma_xy;
-    s.sigma_theta = cfgs[j].sigma_theta;
-    s.iters = c0.iterations_per_thread;
-    s.threads = c0.num_search_threads;
-    s.n_cand = b->n_cand;
-    s.quality = 50;
-    s.hole_width = 0.6f;
-    s.search_begin = 5;
-    s.seed = cfgs[j].seed;
+    init_session(s, *b, cfgs[j], b->d_maps + (size_t)j * b->map_cells);
     s.rays = b->d_rays + (size_t)j * b->max_points;
     s.batch_max = b->d_batch_max + (size_t)j * ((size_t)b->max_points / 32 + 1);
     s.ray_copies = 1;  // a session of a batch has few blocks: nothing to spread
@@ -2432,7 +2378,6 @@ cs_status cs_batch_create(const cs_config* cfgs, int32_t n_sessions, cs_batch** 
     s.w_rk = b->d_w_rk + (size_t)j * b->max_points;
     s.w_bkey = b->d_w_bkey + (size_t)j * ((size_t)b->max_points / 32 + 1);
     s.w_top = b->d_w_top + (size_t)j * 3 * wedge_top_words(b->size);
-    s.w_levels = wedge_levels(b->size);
     if (b->s2_cap > 0) {
       const size_t cap = (size_t)b->s2_cap;
       s.s2_sorted = b->d_s2_entries + (size_t)j * 3 * cap;
@@ -2441,17 +2386,13 @@ cs_status cs_batch_create(const cs_config* cfgs, int32_t n_sessions, cs_batch** 
       s.s2_acc = s.s2_meta + cap;
       s.s2_cap = b->s2_cap;
     }
+    reset_session(s, cfgs[j].start_pose);
   }
-  batch_reset_host(b, cfgs);
   cs_fill_kernel<<<148 * 8, 256, 0, b->stream>>>(b->d_maps, b->map_cells * (size_t)n_sessions,
                                                  (uint16_t)((CS_TS_OBSTACLE + CS_TS_NO_OBSTACLE) / 2));
   b->launches++;
-  cudaMemcpyAsync(b->d_sess, b->hs.data(), sizeof(CsSession) * (size_t)n_sessions, cudaMemcpyHostToDevice, b->stream);
-  if (cudaStreamSynchronize(b->stream) != cudaSuccess) {
-    bfail(nullptr, CS_ERR_CUDA, "cs_batch_create: %s", cudaGetErrorString(cudaGetLastError()));
-    cs_batch_destroy(b);
-    return CS_ERR_CUDA;
-  }
+  CS_CREATE_CUDA(b, cudaMemcpyAsync(b->d_sess, b->hs.data(), sizeof(CsSession) * (size_t)n_sessions, cudaMemcpyHostToDevice, b->stream));
+  CS_CREATE_CUDA(b, cudaStreamSynchronize(b->stream));
   *out = b;
   return CS_OK;
 }
@@ -2494,20 +2435,20 @@ int32_t cs_batch_size(const cs_batch* b) { return b ? b->n : 0; }
 
 // session < 0: all sessions.  Quality 1..255 (:76-82), HoleWidth metres (:87).
 cs_status cs_batch_set_params(cs_batch* b, int32_t session, int32_t quality, float hole_width) {
-  CS_CHECK_BATCH(b);
-  if (session >= b->n) return bfail(b, CS_ERR_INVALID_ARGUMENT, "session %d out of range", session);
-  if (quality < 1 || quality > 255) return bfail(b, CS_ERR_INVALID_ARGUMENT, "Quality must be 1..255");
-  if (!(hole_width >= 0.f) || !(hole_width * b->scale < 60000.f)) return bfail(b, CS_ERR_INVALID_ARGUMENT, "HoleWidth out of range");
-  CS_BCUDA(b, cudaStreamSynchronize(b->stream));
+  CS_CHECK_HANDLE(b);
+  if (session >= b->n) return fail(b, CS_ERR_INVALID_ARGUMENT, "session %d out of range", session);
+  if (quality < 1 || quality > 255) return fail(b, CS_ERR_INVALID_ARGUMENT, "Quality must be 1..255");
+  if (!(hole_width >= 0.f) || !(hole_width * b->scale < 60000.f)) return fail(b, CS_ERR_INVALID_ARGUMENT, "HoleWidth out of range");
+  CS_CUDA(b, cudaStreamSynchronize(b->stream));
   for (int j = (session < 0 ? 0 : session); j < (session < 0 ? b->n : session + 1); j++) {
     b->hs[j].quality = quality;
     b->hs[j].hole_width = hole_width;
-    CS_BCUDA(b, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(b->d_sess + j) + offsetof(CsSession, quality), &b->hs[j].quality,
+    CS_CUDA(b, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(b->d_sess + j) + offsetof(CsSession, quality), &b->hs[j].quality,
                                 sizeof(int), cudaMemcpyHostToDevice, b->stream));
-    CS_BCUDA(b, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(b->d_sess + j) + offsetof(CsSession, hole_width), &b->hs[j].hole_width,
+    CS_CUDA(b, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(b->d_sess + j) + offsetof(CsSession, hole_width), &b->hs[j].hole_width,
                                 sizeof(float), cudaMemcpyHostToDevice, b->stream));
   }
-  CS_BCUDA(b, cudaStreamSynchronize(b->stream));
+  CS_CUDA(b, cudaStreamSynchronize(b->stream));
   return CS_OK;
 }
 
@@ -2526,17 +2467,16 @@ namespace {
 // Stages one Update of every session into (h_stage -> d_stage) and launches its kernels; the result records go to d_results.
 cs_status batch_stage_and_launch(cs_batch* b, uint8_t* h_stage, uint8_t* d_stage, CsDevResult* d_results, const float* points,
                                  const int32_t* n_points, const float* odometry, const float* cand_offsets) {
-  const bool do_search = b->scan_count >= b->search_begin;
-  const bool with_offsets = cand_offsets != nullptr && do_search;
+  const bool with_offsets = cand_offsets != nullptr && b->step.searches();
   int max_n = 0;
   double max_range = 0.0;
   bool range_nan = false;  // a NaN point anywhere in the batch: every ring is launched (NaN does not order, so it is tracked apart)
   for (int j = 0; j < b->n; j++) {
     const int np = n_points[j];
     if (np <= 0 || np > b->user_max_points)
-      return bfail(b, CS_ERR_CAPACITY, "session %d: n_points %d outside 1..%d", j, np, b->user_max_points);
+      return fail(b, CS_ERR_CAPACITY, "session %d: n_points %d outside 1..%d", j, np, b->user_max_points);
     const float* odo = odometry + 3 * (size_t)j;
-    if (!finite3(odo)) return bfail(b, CS_ERR_INVALID_ARGUMENT, "session %d: odometry pose is NaN", j);
+    if (!finite3(odo)) return fail(b, CS_ERR_INVALID_ARGUMENT, "session %d: odometry pose is NaN", j);
     CsStepHeader* hdr = reinterpret_cast<CsStepHeader*>(h_stage) + j;
     memset(hdr, 0, sizeof(CsStepHeader));
     hdr->odo[0] = odo[0]; hdr->odo[1] = odo[1]; hdr->odo[2] = odo[2];
@@ -2551,9 +2491,9 @@ cs_status batch_stage_and_launch(cs_batch* b, uint8_t* h_stage, uint8_t* d_stage
   if (range_nan) max_range = std::numeric_limits<double>::quiet_NaN();
   if (with_offsets) memcpy(h_stage + b->off_cand, cand_offsets, (size_t)b->n * b->n_cand * 12);
   const size_t bytes = with_offsets ? b->stage_bytes : b->off_cand;
-  CS_BCUDA(b, cudaMemcpyAsync(d_stage, h_stage, bytes, cudaMemcpyHostToDevice, b->stream));
+  CS_CUDA(b, cudaMemcpyAsync(d_stage, h_stage, bytes, cudaMemcpyHostToDevice, b->stream));
 
-  CsStepArgs a{};
+  CsStepArgs a = update_args(*b, with_offsets, max_n);
   a.hdr = reinterpret_cast<const CsStepHeader*>(d_stage);
   a.hdr_stride = 1;
   a.points = reinterpret_cast<const float2*>(d_stage + b->off_points);
@@ -2562,19 +2502,9 @@ cs_status batch_stage_and_launch(cs_batch* b, uint8_t* h_stage, uint8_t* d_stage
   a.cand_stride = (size_t)b->n_cand * 3;
   a.result = d_results;
   a.result_stride = 1;
-  a.scan_index = b->update_count;
-  a.cand_mode = with_offsets ? CS_CAND_OFFSETS : CS_CAND_PHILOX;
-  a.step_mode = CS_STEP_UPDATE;
-  a.parity = b->parity;
-  a.do_search = do_search ? 1 : 0;
-  a.n_cand = b->n_cand;
-  a.cand_first = 0;
-  a.cand_count = b->n_cand + 1;
-  a.s2_host_points = max_n;
-  CS_BCUDA(b, launch_step_ctx(batch_ctx(b), a, max_n, rings_hint_of(b->size, b->scale, batch_max_hole_width(b), max_range), CS_PHASE_ALL));
-  b->parity ^= 1;
-  b->update_count++;
-  if (!do_search) b->scan_count++;
+  CS_CUDA(b, launch_step_ctx(LaunchCtx(b, b->flags, b->n, b->hs.data()), a, max_n,
+                             rings_hint_of(b->size, b->scale, batch_max_hole_width(b), max_range), CS_PHASE_ALL));
+  b->step.advance(a.do_search);
   return CS_OK;
 }
 }  // namespace
@@ -2582,19 +2512,16 @@ cs_status batch_stage_and_launch(cs_batch* b, uint8_t* h_stage, uint8_t* d_stage
 cs_status cs_batch_update(cs_batch* b, const float* points, const int32_t* n_points, const float* odometry,
                           const float* cand_offsets, cs_result* results) {
   NvtxRange nvtx_range("cs_batch_update");
-  CS_CHECK_BATCH(b);
-  if (!points || !n_points || !odometry) return bfail(b, CS_ERR_INVALID_ARGUMENT, "cs_batch_update: null argument");
+  CS_CHECK_HANDLE(b);
+  if (!points || !n_points || !odometry) return fail(b, CS_ERR_INVALID_ARGUMENT, "cs_batch_update: null argument");
   // the pinned block may still be the source of the previous call's copy
-  CS_BCUDA(b, cudaStreamSynchronize(b->stream));
+  CS_CUDA(b, cudaStreamSynchronize(b->stream));
   cs_status st = batch_stage_and_launch(b, b->h_stage, b->d_stage, b->d_results, points, n_points, odometry, cand_offsets);
   if (st != CS_OK) return st;
   if (results) {
-    CS_BCUDA(b, cudaMemcpyAsync(b->h_results, b->d_results, sizeof(CsDevResult) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
-    CS_BCUDA(b, cudaStreamSynchronize(b->stream));
-    for (int j = 0; j < b->n; j++) {
-      copy_result(results + j, b->h_results + j);
-      results[j].visits = -1;
-    }
+    CS_CUDA(b, cudaMemcpyAsync(b->h_results, b->d_results, sizeof(CsDevResult) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
+    CS_CUDA(b, cudaStreamSynchronize(b->stream));
+    copy_update_results(results, b->h_results, b->n);
   }
   return CS_OK;
 }
@@ -2606,10 +2533,10 @@ cs_status cs_batch_update(cs_batch* b, const float* points, const int32_t* n_poi
 cs_status cs_batch_submit(cs_batch* b, const float* points, const int32_t* n_points, const float* odometry,
                           const float* cand_offsets) {
   NvtxRange nvtx_range("cs_batch_submit");
-  CS_CHECK_BATCH(b);
-  if (!points || !n_points || !odometry) return bfail(b, CS_ERR_INVALID_ARGUMENT, "cs_batch_submit: null argument");
+  CS_CHECK_HANDLE(b);
+  if (!points || !n_points || !odometry) return fail(b, CS_ERR_INVALID_ARGUMENT, "cs_batch_submit: null argument");
   if (b->pipe_submitted - b->pipe_collected >= 2u)
-    return bfail(b, CS_ERR_STATE, "cs_batch_submit: two submitted steps are waiting for cs_batch_collect");
+    return fail(b, CS_ERR_STATE, "cs_batch_submit: two submitted steps are waiting for cs_batch_collect");
   const int slot = (int)(b->pipe_submitted & 1u);
   if (!b->pipe_done[slot]) {  // first use of the slot: all five resources or none (the event, created last, is the guard)
     uint8_t *hs = nullptr, *ds = nullptr;
@@ -2626,7 +2553,7 @@ cs_status cs_batch_submit(cs_batch* b, const float* points, const int32_t* n_poi
       cudaFree(ds);
       cudaFree(dr);
       cudaGetLastError();
-      return bfail(b, e == cudaErrorMemoryAllocation ? CS_ERR_OUT_OF_MEMORY : CS_ERR_CUDA, "cs_batch_submit: staging slot: %s",
+      return fail(b, e == cudaErrorMemoryAllocation ? CS_ERR_OUT_OF_MEMORY : CS_ERR_CUDA, "cs_batch_submit: staging slot: %s",
                    cudaGetErrorString(e));
     }
     b->pipe_h_stage[slot] = hs; b->pipe_d_stage[slot] = ds; b->pipe_d_results[slot] = dr; b->pipe_h_results[slot] = hr;
@@ -2637,25 +2564,20 @@ cs_status cs_batch_submit(cs_batch* b, const float* points, const int32_t* n_poi
   cs_status st = batch_stage_and_launch(b, b->pipe_h_stage[slot], b->pipe_d_stage[slot], b->pipe_d_results[slot], points, n_points,
                                         odometry, cand_offsets);
   if (st != CS_OK) return st;
-  CS_BCUDA(b, cudaMemcpyAsync(b->pipe_h_results[slot], b->pipe_d_results[slot], sizeof(CsDevResult) * (size_t)b->n,
+  CS_CUDA(b, cudaMemcpyAsync(b->pipe_h_results[slot], b->pipe_d_results[slot], sizeof(CsDevResult) * (size_t)b->n,
                               cudaMemcpyDeviceToHost, b->stream));
-  CS_BCUDA(b, cudaEventRecord(b->pipe_done[slot], b->stream));
+  CS_CUDA(b, cudaEventRecord(b->pipe_done[slot], b->stream));
   b->pipe_submitted++;
   return CS_OK;
 }
 
 cs_status cs_batch_collect(cs_batch* b, cs_result* results /* n_sessions records, or NULL to only wait */) {
   NvtxRange nvtx_range("cs_batch_collect");
-  CS_CHECK_BATCH(b);
-  if (b->pipe_collected == b->pipe_submitted) return bfail(b, CS_ERR_STATE, "cs_batch_collect: nothing was submitted");
+  CS_CHECK_HANDLE(b);
+  if (b->pipe_collected == b->pipe_submitted) return fail(b, CS_ERR_STATE, "cs_batch_collect: nothing was submitted");
   const int slot = (int)(b->pipe_collected & 1u);
-  CS_BCUDA(b, cudaEventSynchronize(b->pipe_done[slot]));
-  if (results) {
-    for (int j = 0; j < b->n; j++) {
-      copy_result(results + j, b->pipe_h_results[slot] + j);
-      results[j].visits = -1;
-    }
-  }
+  CS_CUDA(b, cudaEventSynchronize(b->pipe_done[slot]));
+  if (results) copy_update_results(results, b->pipe_h_results[slot], b->n);
   b->pipe_collected++;
   return CS_OK;
 }
@@ -2665,17 +2587,16 @@ cs_status cs_batch_collect(cs_batch* b, cs_result* results /* n_sessions records
 // n_sessions records of the LAST scan replayed.
 cs_status cs_batch_replay(cs_batch* b, const cs_scanlog* log, int32_t first, int32_t count, cs_result* results) {
   NvtxRange nvtx_range("cs_batch_replay");
-  CS_CHECK_BATCH(b);
-  if (!log || !log->uploaded) return bfail(b, CS_ERR_STATE, "scan log not uploaded");
-  if (log->device != b->device) return bfail(b, CS_ERR_INVALID_ARGUMENT, "scan log lives on another device");
-  if (first < 0 || count < 0 || first + count > log->n_scans) return bfail(b, CS_ERR_INVALID_ARGUMENT, "scan range");
-  if (log->n_offsets > 0 && log->n_offsets != b->n_cand) return bfail(b, CS_ERR_INVALID_ARGUMENT, "scan log offsets != T*I");
-  if (log->max_points > b->max_points) return bfail(b, CS_ERR_CAPACITY, "scan log max_points exceeds the batch's");
+  CS_CHECK_HANDLE(b);
+  if (!log || !log->uploaded) return fail(b, CS_ERR_STATE, "scan log not uploaded");
+  if (log->device != b->device) return fail(b, CS_ERR_INVALID_ARGUMENT, "scan log lives on another device");
+  if (first < 0 || count < 0 || first + count > log->n_scans) return fail(b, CS_ERR_INVALID_ARGUMENT, "scan range");
+  if (log->n_offsets > 0 && log->n_offsets != b->n_cand) return fail(b, CS_ERR_INVALID_ARGUMENT, "scan log offsets != T*I");
+  if (log->max_points > b->max_points) return fail(b, CS_ERR_CAPACITY, "scan log max_points exceeds the batch's");
   const float hw = batch_max_hole_width(b);
   for (int i = 0; i < count; i++) {
     const int sidx = first + i;
-    const bool do_search = b->scan_count >= b->search_begin;
-    CsStepArgs a{};
+    CsStepArgs a = update_args(*b, log->n_offsets > 0, log->h_hdr[sidx].n_points);
     a.hdr = log->d_hdr + sidx;
     a.hdr_stride = 0;
     a.points = log->d_points + (size_t)sidx * log->max_points;
@@ -2684,74 +2605,49 @@ cs_status cs_batch_replay(cs_batch* b, const cs_scanlog* log, int32_t first, int
     a.cand_stride = 0;
     a.result = b->d_results;
     a.result_stride = 1;
-    a.scan_index = b->update_count;
-    a.cand_mode = log->n_offsets > 0 ? CS_CAND_OFFSETS : CS_CAND_PHILOX;
-    a.step_mode = CS_STEP_UPDATE;
-    a.parity = b->parity;
-    a.do_search = do_search ? 1 : 0;
-    a.n_cand = b->n_cand;
-    a.cand_first = 0;
-    a.cand_count = b->n_cand + 1;
-    a.s2_host_points = log->h_hdr[sidx].n_points;
-    CS_BCUDA(b, launch_step_ctx(batch_ctx(b), a, log->h_hdr[sidx].n_points,
-                                rings_hint_of(b->size, b->scale, hw, log->h_max_range[sidx]), CS_PHASE_ALL));
-    b->parity ^= 1;
-    b->update_count++;
-    if (!do_search) b->scan_count++;
+    CS_CUDA(b, launch_step_ctx(LaunchCtx(b, b->flags, b->n, b->hs.data()), a, log->h_hdr[sidx].n_points,
+                               rings_hint_of(b->size, b->scale, hw, log->h_max_range[sidx]), CS_PHASE_ALL));
+    b->step.advance(a.do_search);
   }
   if (results && count > 0) {
-    CS_BCUDA(b, cudaMemcpyAsync(b->h_results, b->d_results, sizeof(CsDevResult) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
-    CS_BCUDA(b, cudaStreamSynchronize(b->stream));
-    for (int j = 0; j < b->n; j++) {
-      copy_result(results + j, b->h_results + j);
-      results[j].visits = -1;
-    }
+    CS_CUDA(b, cudaMemcpyAsync(b->h_results, b->d_results, sizeof(CsDevResult) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
+    CS_CUDA(b, cudaStreamSynchronize(b->stream));
+    copy_update_results(results, b->h_results, b->n);
   }  // results == NULL: fire and forget (cs_batch_sync waits)
   return CS_OK;
 }
 
 cs_status cs_batch_sync(cs_batch* b) {
-  CS_CHECK_BATCH(b);
-  CS_BCUDA(b, cudaStreamSynchronize(b->stream));
+  CS_CHECK_HANDLE(b);
+  CS_CUDA(b, cudaStreamSynchronize(b->stream));
   return CS_OK;
 }
 
 cs_status cs_batch_get_poses(cs_batch* b, float* poses /* n_sessions * 3 */) {
-  CS_CHECK_BATCH(b);
-  if (!poses) return bfail(b, CS_ERR_INVALID_ARGUMENT, "null poses");
+  CS_CHECK_HANDLE(b);
+  if (!poses) return fail(b, CS_ERR_INVALID_ARGUMENT, "null poses");
   std::vector<CsSession> tmp((size_t)b->n);
-  CS_BCUDA(b, cudaMemcpyAsync(tmp.data(), b->d_sess, sizeof(CsSession) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
-  CS_BCUDA(b, cudaStreamSynchronize(b->stream));
+  CS_CUDA(b, cudaMemcpyAsync(tmp.data(), b->d_sess, sizeof(CsSession) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
+  CS_CUDA(b, cudaStreamSynchronize(b->stream));
   for (int j = 0; j < b->n; j++)
-    for (int k = 0; k < 3; k++) poses[3 * j + k] = tmp[j].state[b->parity].pose[k];
+    for (int k = 0; k < 3; k++) poses[3 * j + k] = tmp[j].state[b->step.parity].pose[k];
   return CS_OK;
 }
 
 cs_status cs_batch_map_download(cs_batch* b, int32_t session, uint16_t* pixels) {
-  CS_CHECK_BATCH(b);
-  if (!pixels || session < 0 || session >= b->n) return bfail(b, CS_ERR_INVALID_ARGUMENT, "cs_batch_map_download: bad argument");
-  if (!b->d_linear) CS_BCUDA(b, cudaMalloc(&b->d_linear, (size_t)b->size * b->size * sizeof(uint16_t)));
-  dispatch_layout(b->tiled, [&](auto T) {
-    cs_relayout_kernel<decltype(T)::value><<<148 * 8, 256, 0, b->stream>>>(b->hs[session].map, b->d_linear, b->size, b->pitch_tiles, 0);
-  });
-  b->launches++;
-  CS_BCUDA(b, cudaMemcpyAsync(pixels, b->d_linear, (size_t)b->size * b->size * 2, cudaMemcpyDeviceToHost, b->stream));
-  CS_BCUDA(b, cudaStreamSynchronize(b->stream));
-  return CS_OK;
+  CS_CHECK_HANDLE(b);
+  if (!pixels || session < 0 || session >= b->n) return fail(b, CS_ERR_INVALID_ARGUMENT, "cs_batch_map_download: bad argument");
+  return download_map(b, b->hs[session].map, pixels);
 }
 
 cs_status cs_batch_map_checksums(cs_batch* b, uint64_t* checksums /* n_sessions */) {
-  CS_CHECK_BATCH(b);
-  if (!checksums) return bfail(b, CS_ERR_INVALID_ARGUMENT, "null checksums");
+  CS_CHECK_HANDLE(b);
+  if (!checksums) return fail(b, CS_ERR_INVALID_ARGUMENT, "null checksums");
   for (int j = 0; j < b->n; j++) {
-    CS_BCUDA(b, cudaMemsetAsync(b->d_checksum, 0, sizeof(unsigned long long), b->stream));
-    dispatch_layout(b->tiled, [&](auto T) {
-      cs_checksum_kernel<decltype(T)::value><<<148 * 4, 256, 0, b->stream>>>(b->hs[j].map, b->size, b->pitch_tiles, b->d_checksum);
-    });
-    b->launches++;
-    CS_BCUDA(b, cudaMemcpyAsync(checksums + j, b->d_checksum, sizeof(unsigned long long), cudaMemcpyDeviceToHost, b->stream));
+    cs_status st = queue_map_checksum(b, b->hs[j].map, 148 * 4, checksums + j);
+    if (st != CS_OK) return st;
   }
-  CS_BCUDA(b, cudaStreamSynchronize(b->stream));
+  CS_CUDA(b, cudaStreamSynchronize(b->stream));
   return CS_OK;
 }
 
