@@ -99,6 +99,15 @@ namespace CoreSLAM.B200
         [DllImport(Lib)] public static extern CsStatus cs_batch_sync(IntPtr batch);
         [DllImport(Lib)] public static extern CsStatus cs_batch_get_poses(IntPtr batch, float* poses3);
         [DllImport(Lib)] public static extern CsStatus cs_batch_map_download(IntPtr batch, int session, ushort* pixels);
+        // Reset() of every session at once; refused while submitted steps wait for cs_batch_collect
+        [DllImport(Lib)] public static extern CsStatus cs_batch_reset(IntPtr batch);
+        // per-session ObstacleMaps (CsConfig.ObstacleMapSize > 0, equal in all cfgs); session < 0: all sessions.
+        // unmappedHits applies at the next cs_batch_reset, maxHits from the next step
+        [DllImport(Lib)] public static extern CsStatus cs_batch_set_obstacle_params(IntPtr batch, int session, int unmappedHits, int maxHits);
+        [DllImport(Lib)] public static extern CsStatus cs_batch_obstacle_map_download(IntPtr batch, int session, sbyte* pixels);
+        [DllImport(Lib)] public static extern CsStatus cs_batch_obstacle_checksums(IntPtr batch, ulong* checksums);
+        [DllImport(Lib)] public static extern CsStatus cs_batch_get_obstacle_visits(IntPtr batch, long* touched);
+        [DllImport(Lib)] public static extern ulong cs_host_obstacle_checksum(sbyte* pixels, int size);
 
         // Candidate split over the GPUs of a node (BASELINE cfg4): one process per GPU exports the 64-byte handle of its exchange
         // table, the handles travel between the processes by any means (a pipe, a file, MPI), every process attaches all of them;

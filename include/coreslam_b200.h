@@ -268,9 +268,12 @@ cs_status cs_scanlog_file_read(const char* path, int32_t scan, float* points /* 
 cs_status cs_replay(cs_processor* h, const cs_scanlog* log, int32_t first, int32_t count, cs_result* results);
 
 /* ---- batches of independent sessions on one GPU (parameter sweeps / scan-log replays, BASELINE cfg5) ----
- * One launch per kernel for all sessions (grid.y = session); every session has its own HoleMap, pose,
- * sigma_xy / sigma_theta / seed / start_pose (cfgs[j]), Quality and HoleWidth.  Map size, iterations,
- * threads, device, max_points and flags must be equal across cfgs.  No communication between sessions. */
+ * One launch per kernel for all sessions (grid.y = session); every session has its own HoleMap, ObstacleMap (when
+ * obstacle_map_size > 0), pose, sigma_xy / sigma_theta / seed / start_pose (cfgs[j]), Quality, HoleWidth,
+ * MaxObstacleHits and UnmappedObstacleHits.  Map size, obstacle_map_size, iterations, threads, device, max_points
+ * and flags must be equal across cfgs.  No communication between sessions.  With obstacle_map_size > 0 every
+ * batched Update (cs_batch_update, cs_batch_submit, cs_batch_replay) also runs UpdateObstacleMap (:751) for every
+ * session, as cs_update does for one processor. */
 cs_status cs_batch_create(const cs_config* cfgs, int32_t n_sessions, cs_batch** out);
 cs_status cs_batch_destroy(cs_batch* b);
 const char* cs_batch_last_error(const cs_batch* b);
@@ -297,6 +300,20 @@ cs_status cs_batch_get_poses(cs_batch* b, float* poses /* n_sessions*3 */);
 cs_status cs_batch_map_download(cs_batch* b, int32_t session, uint16_t* pixels);
 cs_status cs_batch_map_checksums(cs_batch* b, uint64_t* checksums /* n_sessions */);
 cs_status cs_batch_get_launch_count(cs_batch* b, uint64_t* launches);
+/* CoreSLAMProcessor.Reset (:167-175) of every session at once (the sessions share one step state): HoleMap := 32750,
+ * ObstacleMap := the session's UnmappedObstacleHits, Pose := its cfgs[j].start_pose, lastOdometryPose := 0,
+ * scanCount := 0, and the Philox stream restarts at scan 0.  Quality, HoleWidth and MaxObstacleHits are kept.
+ * CS_ERR_STATE while submitted steps wait for cs_batch_collect. */
+cs_status cs_batch_reset(cs_batch* b);
+/* The sessions' ObstacleMaps (need obstacle_map_size > 0, CS_ERR_STATE otherwise); session < 0: all sessions.
+ * unmapped_hits: UnmappedObstacleHits (:98), sbyte, default -5, used by the next cs_batch_reset;
+ * max_hits: MaxObstacleHits (:103), sbyte, default 10, used from the next step. */
+cs_status cs_batch_set_obstacle_params(cs_batch* b, int32_t session, int32_t unmapped_hits, int32_t max_hits);
+cs_status cs_batch_obstacle_map_download(cs_batch* b, int32_t session, int8_t* pixels); /* Size*Size sbyte, [y, x] row-major */
+cs_status cs_batch_obstacle_checksums(cs_batch* b, uint64_t* checksums /* n_sessions */); /* cs_host_obstacle_checksum of each map */
+cs_status cs_batch_get_obstacle_visits(cs_batch* b, int64_t* touched /* n_sessions */);  /* as cs_get_obstacle_visits, per session */
+/* Host-only: sum over the row-major cells i of ((uint8_t)pixel + 1) * mix64(i), mod 2^64 (the hash of cs_host_map_checksum). */
+uint64_t cs_host_obstacle_checksum(const int8_t* pixels, int32_t size);
 
 /* ---- host twins of the device generators (for building verification tables; not a compute path) ----- */
 /* offsets[n*3] = the Philox deviates the device uses for candidates 0..n-1 of scan `scan_index`. */

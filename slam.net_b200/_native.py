@@ -193,6 +193,12 @@ SIGNATURES = {
     "cs_batch_map_download": (C.c_int, [_vp, C.c_int32, _vp]),
     "cs_batch_map_checksums": (C.c_int, [_vp, C.POINTER(C.c_uint64)]),
     "cs_batch_get_launch_count": (C.c_int, [_vp, C.POINTER(C.c_uint64)]),
+    "cs_batch_reset": (C.c_int, [_vp]),
+    "cs_batch_set_obstacle_params": (C.c_int, [_vp, C.c_int32, C.c_int32, C.c_int32]),
+    "cs_batch_obstacle_map_download": (C.c_int, [_vp, C.c_int32, _vp]),
+    "cs_batch_obstacle_checksums": (C.c_int, [_vp, C.POINTER(C.c_uint64)]),
+    "cs_batch_get_obstacle_visits": (C.c_int, [_vp, C.POINTER(C.c_int64)]),
+    "cs_host_obstacle_checksum": (C.c_uint64, [_vp, C.c_int32]),
     "cs_philox_offsets": (None, [C.c_uint64, C.c_uint32, C.c_int32, C.c_float, C.c_float, _fp]),
     "cs_host_sincos": (None, [_fp, C.c_int32, _fp, _fp]),
     "cs_device_sincos": (C.c_int, [C.c_int32, _fp, C.c_int32, _fp, _fp]),

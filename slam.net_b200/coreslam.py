@@ -442,11 +442,12 @@ class Processor:
 
 class Batch:
     """N independent sessions on one GPU (cs_batch_*): a parameter sweep / many replays advanced in
-    lockstep, one kernel launch per stage for all of them."""
+    lockstep, one kernel launch per stage for all of them.  obstacle_map_size > 0 gives every session its own
+    ObstacleMap, updated by every step as in a Processor."""
 
     def __init__(self, n_sessions: int, physical_map_size: float, hole_map_size: int, start_poses, sigma_xy, sigma_theta,
                  iterations_per_thread: int, num_search_threads: int, *, device: int = 0, max_points: int = 0,
-                 seeds=None, stream: int = 0, flags: int = 0):
+                 seeds=None, stream: int = 0, flags: int = 0, obstacle_map_size: int = 0):
         cfgs = (N.Config * n_sessions)()
         start_poses = np.broadcast_to(_f32(start_poses), (n_sessions, 3))
         sxy = np.broadcast_to(np.asarray(sigma_xy, dtype=np.float32), (n_sessions,))
@@ -466,10 +467,12 @@ class Batch:
             c.seed = int(seeds[j])
             c.stream = stream or None
             c.flags = flags
+            c.obstacle_map_size = obstacle_map_size
         self._h = C.c_void_p()
         N.check(N.lib().cs_batch_create(cfgs, n_sessions, C.byref(self._h)))
         self.n = n_sessions
         self.size = hole_map_size
+        self.obstacle_size = obstacle_map_size
         self.n_cand = max(num_search_threads, 1) * iterations_per_thread
         self.max_points = max_points if max_points > 0 else 16384  # stride of the points array = cfg.max_points, odd or even
         self.seeds, self.sigma_xy, self.sigma_theta = seeds, sxy, sth
@@ -553,6 +556,31 @@ class Batch:
         self._ck(N.lib().cs_batch_get_launch_count(self._h, C.byref(v)))
         return int(v.value)
 
+    def reset(self):
+        """CoreSLAMProcessor.Reset of every session: maps refilled, poses back to the start poses, scan count 0."""
+        self._ck(N.lib().cs_batch_reset(self._h))
+
+    # -- ObstacleMaps (needs obstacle_map_size > 0) -------------------------------------------------
+    def set_obstacle_params(self, session: int, unmapped_hits: int, max_hits: int):
+        """session < 0: all.  max_hits applies from the next step, unmapped_hits from the next reset()."""
+        self._ck(N.lib().cs_batch_set_obstacle_params(self._h, int(session), int(unmapped_hits), int(max_hits)))
+
+    def obstacle_map_download(self, session: int) -> np.ndarray:
+        px = np.empty((self.obstacle_size, self.obstacle_size), dtype=np.int8)
+        self._ck(N.lib().cs_batch_obstacle_map_download(self._h, int(session), px.ctypes.data))
+        return px
+
+    def obstacle_checksums(self) -> np.ndarray:
+        out = np.zeros(self.n, dtype=np.uint64)
+        self._ck(N.lib().cs_batch_obstacle_checksums(self._h, out.ctypes.data_as(C.POINTER(C.c_uint64))))
+        return out
+
+    def obstacle_visits(self) -> np.ndarray:
+        """Per session: ObstacleMap cells the rays touched since the last reset (measurement)."""
+        out = np.zeros(self.n, dtype=np.int64)
+        self._ck(N.lib().cs_batch_get_obstacle_visits(self._h, out.ctypes.data_as(C.POINTER(C.c_int64))))
+        return out
+
 
 def gather_peak(cells: int, per_thread: int = 256, repeats: int = 5, device: int = 0) -> float:
     """Measured random 2-byte gather rate (lookups/s) over a table of `cells` uint16."""
@@ -564,6 +592,14 @@ def gather_peak(cells: int, per_thread: int = 256, repeats: int = 5, device: int
 def host_map_checksum(pixels, size: int) -> int:
     px = np.ascontiguousarray(pixels, dtype=np.uint16).reshape(-1)
     return int(N.lib().cs_host_map_checksum(px.ctypes.data, size))
+
+
+def host_obstacle_checksum(pixels, size: int) -> int:
+    """The hash of Batch.obstacle_checksums() for a host ObstacleMap (size * size sbyte, row-major)."""
+    px = np.ascontiguousarray(pixels, dtype=np.int8).reshape(-1)
+    if px.size != size * size:
+        raise ValueError("expected %d pixels, got %d" % (size * size, px.size))
+    return int(N.lib().cs_host_obstacle_checksum(px.ctypes.data, size))
 
 
 def philox_offsets(seed: int, scan_index: int, n: int, sigma_xy: float, sigma_theta: float) -> np.ndarray:

@@ -791,6 +791,40 @@ cudaError_t launch_obstacle_update(cudaStream_t stream, const CsSession* d_sess,
   return cudaGetLastError();
 }
 
+// An ObstacleMap of `size` pixels per edge (ObstacleMap.cs:17-22, :103) without its buffers: rows padded to whole 8-cell
+// words and the row count to whole 4-row tiles of the no-hit bitmap.
+CsObstacle obstacle_geometry(int size, float physical_map_size) {
+  CsObstacle o{};
+  o.size = size;
+  o.pitch = (size + 7) / 8 * 8;
+  o.rows = (size + 3) / 4 * 4;
+  o.words_per_row = o.pitch / 8;
+  o.scale = (float)size / physical_map_size;  // ObstacleMap.cs:20
+  o.max_hits = 10;                            // :103
+  return o;
+}
+size_t obstacle_pixel_bytes(const CsObstacle& o) { return (size_t)o.pitch * o.rows; }
+size_t obstacle_bitmap_words(const CsObstacle& o) { return (size_t)o.words_per_row * (o.rows / 4); }
+
+// ArrayEx.Fill(ObstacleMap.Pixels, v) (:170) of n_sessions maps of the geometry `ho`: with `values`, session j's map gets
+// values[j] (device array), otherwise every map gets `value`.
+cudaError_t launch_obstacle_fill(cudaStream_t stream, const CsObstacle* d_obst, const int* values, int value, const CsObstacle& ho,
+                                 int n_sessions, uint64_t* launches) {
+  size_t blocks = (obstacle_pixel_bytes(ho) / 8 + 255) / 256;
+  if (blocks > 148 * 2) blocks = 148 * 2;
+  cs_obstacle_fill_kernel<<<dim3((unsigned)blocks, (unsigned)n_sessions), 256, 0, stream>>>(d_obst, values, value);
+  (*launches)++;
+  return cudaGetLastError();
+}
+
+// Pixels of one ObstacleMap out to `pixels` (Size * Size sbyte, [y, x]); returns once the copy is complete.
+cs_status download_obstacle_map(CsHost* h, const CsObstacle& o, int8_t* pixels) {
+  CS_CUDA(h, cudaMemcpy2DAsync(pixels, (size_t)o.size, o.pixels, (size_t)o.pitch, (size_t)o.size, (size_t)o.size,
+                               cudaMemcpyDeviceToHost, h->stream));
+  CS_CUDA(h, cudaStreamSynchronize(h->stream));
+  return CS_OK;
+}
+
 cs_status launch_step(cs_processor* h, CsStepArgs a, int n_points, int rings, bool timing, int ev_base, int phases = CS_PHASE_ALL,
                       const float* next_cand = nullptr, uint64_t log_tag = 0) {
   LaunchCtx c(h, h->cfg.flags, 1, &h->hs);
@@ -1041,17 +1075,13 @@ cs_status cs_create(const cs_config* cfg, cs_processor** out) {
   for (auto& e : h->tm.ev) CS_CREATE_CUDA(h, cudaEventCreate(&e));
   if (cfg->obstacle_map_size > 0) {  // :132-133
     CsObstacle& o = h->ho;
-    o.size = cfg->obstacle_map_size;
-    o.pitch = (o.size + 7) / 8 * 8;
-    o.rows = (o.size + 3) / 4 * 4;
-    o.words_per_row = o.pitch / 8;
-    o.scale = (float)cfg->obstacle_map_size / cfg->physical_map_size;  // ObstacleMap.cs:20
-    o.max_hits = 10;                                                   // :103
-    CS_CREATE_CUDA(h, cudaMalloc(&o.pixels, (size_t)o.pitch * o.rows));
-    CS_CREATE_CUDA(h, cudaMalloc(&o.no_hit, (size_t)o.words_per_row * (o.rows / 4) * sizeof(uint32_t)));
+    o = obstacle_geometry(cfg->obstacle_map_size, cfg->physical_map_size);
+    CS_CREATE_CUDA(h, cudaMalloc(&o.pixels, obstacle_pixel_bytes(o)));
+    CS_CREATE_CUDA(h, cudaMalloc(&o.no_hit, obstacle_bitmap_words(o) * sizeof(uint32_t)));
     CS_CREATE_CUDA(h, cudaMalloc(&o.touched, sizeof(long long)));
     CS_CREATE_CUDA(h, cudaMalloc(&h->d_obst, sizeof(CsObstacle)));
-    CS_CREATE_CUDA(h, cudaMemcpy(h->d_obst, &o, sizeof(CsObstacle), cudaMemcpyHostToDevice));
+    // (in stream order: the fill kernel of cs_reset below reads the descriptor on the handle's stream)
+    CS_CREATE_CUDA(h, cudaMemcpyAsync(h->d_obst, &o, sizeof(CsObstacle), cudaMemcpyHostToDevice, h->stream));
   }
 
   // Optional L2 persistence window over the map (the gathers are served from L2 either way when the
@@ -1165,11 +1195,8 @@ cs_status cs_reset(cs_processor* h) {  // CoreSLAMProcessor.cs:167-175
   if (st != CS_OK) return st;
   st = launch_fill(h, (uint16_t)((CS_TS_OBSTACLE + CS_TS_NO_OBSTACLE) / 2));  // :169
   if (st != CS_OK) return st;
-  if (h->d_obst) {  // :170 ArrayEx.Fill(ObstacleMap.Pixels, UnmappedObstacleHits)
-    cs_obstacle_fill_kernel<<<148 * 2, 256, 0, h->stream>>>(h->ho, h->unmapped_obstacle_hits);
-    h->launches++;
-    CS_CUDA(h, cudaGetLastError());
-  }
+  if (h->d_obst)  // :170 ArrayEx.Fill(ObstacleMap.Pixels, UnmappedObstacleHits)
+    CS_CUDA(h, launch_obstacle_fill(h->stream, h->d_obst, nullptr, h->unmapped_obstacle_hits, h->ho, 1, &h->launches));
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
   return CS_OK;
 }
@@ -1209,11 +1236,7 @@ cs_status cs_obstacle_map_download(cs_processor* h, int8_t* pixels) {
   CS_CHECK_HANDLE(h);
   CS_NEED_OBSTACLE(h);
   if (!pixels) return fail(h, CS_ERR_INVALID_ARGUMENT, "null pixels");
-  const CsObstacle& o = h->ho;
-  CS_CUDA(h, cudaMemcpy2DAsync(pixels, (size_t)o.size, o.pixels, (size_t)o.pitch, (size_t)o.size, (size_t)o.size,
-                               cudaMemcpyDeviceToHost, h->stream));
-  CS_CUDA(h, cudaStreamSynchronize(h->stream));
-  return CS_OK;
+  return download_obstacle_map(h, h->ho, pixels);
 }
 
 cs_status cs_obstacle_map_upload(cs_processor* h, const int8_t* pixels) {
@@ -1231,9 +1254,7 @@ cs_status cs_obstacle_map_fill(cs_processor* h, int32_t value) {
   CS_CHECK_HANDLE(h);
   CS_NEED_OBSTACLE(h);
   if (value < -128 || value > 127) return fail(h, CS_ERR_INVALID_ARGUMENT, "ObstacleMap pixels are sbyte");
-  cs_obstacle_fill_kernel<<<148 * 2, 256, 0, h->stream>>>(h->ho, value);
-  h->launches++;
-  CS_CUDA(h, cudaGetLastError());
+  CS_CUDA(h, launch_obstacle_fill(h->stream, h->d_obst, nullptr, value, h->ho, 1, &h->launches));
   return CS_OK;
 }
 
@@ -1888,6 +1909,13 @@ uint64_t cs_host_map_checksum(const uint16_t* pixels, int32_t size) {
   return acc;
 }
 
+uint64_t cs_host_obstacle_checksum(const int8_t* pixels, int32_t size) {
+  unsigned long long acc = 0;
+  const size_t n = size > 0 ? (size_t)size * (size_t)size : 0;
+  for (size_t i = 0; i < n; i++) acc += ((unsigned long long)(uint8_t)pixels[i] + 1ull) * cs_mix64((unsigned long long)i);
+  return acc;
+}
+
 // -----------------------------------------------------------------------------------------------------
 cs_status cs_get_timing(cs_processor* h, cs_timing* t) {
   if (!h || !t) return CS_ERR_INVALID_ARGUMENT;
@@ -2274,7 +2302,42 @@ struct cs_batch : CsHost {
   CsDevResult* pipe_h_results[2] = {nullptr, nullptr};
   cudaEvent_t pipe_done[2] = {nullptr, nullptr};
   unsigned pipe_submitted = 0, pipe_collected = 0;
+  std::vector<float> start_poses;  // n * 3: cfgs[j].start_pose, the Pose of session j after cs_batch_reset (:172)
+
+  // ObstacleMaps (cfg.obstacle_map_size > 0), one per session, all of the geometry `ho` (its pointers unused): session j's
+  // pixels, bitmap and touched counter are the j-th pieces of the three blocks below, described by obst[j] / d_obst[j]
+  CsObstacle ho{};
+  std::vector<CsObstacle> obst;
+  CsObstacle* d_obst = nullptr;
+  int8_t* d_obst_pixels = nullptr;
+  uint32_t* d_obst_no_hit = nullptr;
+  long long* d_obst_touched = nullptr;
+  std::vector<int> unmapped_obstacle_hits;  // per session, :98; the fill values of the next cs_batch_reset
+  int* d_obst_fill = nullptr;               // ... as the fill kernel reads them
+  unsigned long long* d_obst_sums = nullptr;  // cs_batch_obstacle_checksums
 };
+
+namespace {
+// The maps of Reset (:169-170) for every session: HoleMap := 32750, ObstacleMap := the session's UnmappedObstacleHits (with
+// its no-hit bitmap and touched counter cleared).  Queued on the stream; the caller synchronises.
+cs_status batch_fill_maps(cs_batch* b) {
+  cs_fill_kernel<<<148 * 8, 256, 0, b->stream>>>(b->d_maps, b->map_cells * (size_t)b->n, (uint16_t)((CS_TS_OBSTACLE + CS_TS_NO_OBSTACLE) / 2));
+  b->launches++;
+  CS_CUDA(b, cudaGetLastError());
+  if (b->d_obst) {
+    CS_CUDA(b, cudaMemcpyAsync(b->d_obst_fill, b->unmapped_obstacle_hits.data(), sizeof(int) * (size_t)b->n, cudaMemcpyHostToDevice,
+                               b->stream));
+    CS_CUDA(b, launch_obstacle_fill(b->stream, b->d_obst, b->d_obst_fill, 0, b->ho, b->n, &b->launches));
+  }
+  return CS_OK;
+}
+
+// The host-owned descriptors of all sessions' ObstacleMaps to the device (in stream order).
+cs_status batch_push_obstacles(cs_batch* b) {
+  CS_CUDA(b, cudaMemcpyAsync(b->d_obst, b->obst.data(), sizeof(CsObstacle) * (size_t)b->n, cudaMemcpyHostToDevice, b->stream));
+  return CS_OK;
+}
+}  // namespace
 
 extern "C" {
 
@@ -2287,17 +2350,17 @@ cs_status cs_batch_create(const cs_config* cfgs, int32_t n_sessions, cs_batch** 
   const cs_config& c0 = cfgs[0];
   if (c0.hole_map_size < 8 || c0.hole_map_size > 16384 || !(c0.physical_map_size > 0.f) || c0.iterations_per_thread < 0)
     return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "cs_batch_create: bad map size / iterations");
-  for (int j = 0; j < n_sessions; j++)
-    if (cfgs[j].obstacle_map_size != 0)
-      return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "cs_batch_create: session batches carry no ObstacleMap (obstacle_map_size must be 0)");
+  if (c0.obstacle_map_size < 0 || c0.obstacle_map_size > 16384)
+    return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "obstacle_map_size must be 0 (no ObstacleMap) or in [1, 16384], got %d",
+                c0.obstacle_map_size);
   for (int j = 1; j < n_sessions; j++) {
     const cs_config& c = cfgs[j];
     if (c.hole_map_size != c0.hole_map_size || c.physical_map_size != c0.physical_map_size ||
         c.iterations_per_thread != c0.iterations_per_thread || c.num_search_threads != c0.num_search_threads ||
-        c.device != c0.device || c.max_points != c0.max_points || c.flags != c0.flags)
+        c.device != c0.device || c.max_points != c0.max_points || c.flags != c0.flags || c.obstacle_map_size != c0.obstacle_map_size)
       return fail(nullptr, CS_ERR_INVALID_ARGUMENT,
-                   "cs_batch_create: session %d differs in map size / iterations / threads / device / max_points / flags "
-                   "(only start_pose, sigma_xy, sigma_theta and seed may vary)", j);
+                   "cs_batch_create: session %d differs in map size / iterations / threads / device / max_points / flags / "
+                   "obstacle_map_size (only start_pose, sigma_xy, sigma_theta and seed may vary)", j);
   }
   const int threads = c0.num_search_threads > 0 ? c0.num_search_threads : 1;
   const long long n_cand = (long long)threads * c0.iterations_per_thread;
@@ -2388,9 +2451,31 @@ cs_status cs_batch_create(const cs_config* cfgs, int32_t n_sessions, cs_batch** 
     }
     reset_session(s, cfgs[j].start_pose);
   }
-  cs_fill_kernel<<<148 * 8, 256, 0, b->stream>>>(b->d_maps, b->map_cells * (size_t)n_sessions,
-                                                 (uint16_t)((CS_TS_OBSTACLE + CS_TS_NO_OBSTACLE) / 2));
-  b->launches++;
+  b->start_poses.resize((size_t)n_sessions * 3);
+  for (int j = 0; j < n_sessions; j++)
+    for (int k = 0; k < 3; k++) b->start_poses[3 * (size_t)j + k] = cfgs[j].start_pose[k];
+  if (c0.obstacle_map_size > 0) {  // :132-133, per session
+    b->ho = obstacle_geometry(c0.obstacle_map_size, c0.physical_map_size);
+    const size_t px = obstacle_pixel_bytes(b->ho), words = obstacle_bitmap_words(b->ho);
+    CS_CREATE_CUDA(b, cudaMalloc(&b->d_obst_pixels, px * (size_t)n_sessions));
+    CS_CREATE_CUDA(b, cudaMalloc(&b->d_obst_no_hit, words * sizeof(uint32_t) * (size_t)n_sessions));
+    CS_CREATE_CUDA(b, cudaMalloc(&b->d_obst_touched, sizeof(long long) * (size_t)n_sessions));
+    CS_CREATE_CUDA(b, cudaMalloc(&b->d_obst, sizeof(CsObstacle) * (size_t)n_sessions));
+    CS_CREATE_CUDA(b, cudaMalloc(&b->d_obst_fill, sizeof(int) * (size_t)n_sessions));
+    CS_CREATE_CUDA(b, cudaMalloc(&b->d_obst_sums, sizeof(unsigned long long) * (size_t)n_sessions));
+    b->obst.assign((size_t)n_sessions, b->ho);
+    for (int j = 0; j < n_sessions; j++) {
+      CsObstacle& o = b->obst[j];
+      o.pixels = b->d_obst_pixels + (size_t)j * px;
+      o.no_hit = b->d_obst_no_hit + (size_t)j * words;
+      o.touched = b->d_obst_touched + j;
+    }
+    b->unmapped_obstacle_hits.assign((size_t)n_sessions, -5);  // :98
+    const cs_status st = batch_push_obstacles(b);
+    if (st != CS_OK) return bail(st);
+  }
+  const cs_status st = batch_fill_maps(b);
+  if (st != CS_OK) return bail(st);
   CS_CREATE_CUDA(b, cudaMemcpyAsync(b->d_sess, b->hs.data(), sizeof(CsSession) * (size_t)n_sessions, cudaMemcpyHostToDevice, b->stream));
   CS_CREATE_CUDA(b, cudaStreamSynchronize(b->stream));
   *out = b;
@@ -2413,6 +2498,12 @@ cs_status cs_batch_destroy(cs_batch* b) {
   cudaFree(b->d_w_top);
   cudaFree(b->d_s2_entries);
   cudaFree(b->d_s2_words);
+  cudaFree(b->d_obst);
+  cudaFree(b->d_obst_pixels);
+  cudaFree(b->d_obst_no_hit);
+  cudaFree(b->d_obst_touched);
+  cudaFree(b->d_obst_fill);
+  cudaFree(b->d_obst_sums);
   cudaFree(b->d_stage);
   cudaFree(b->d_results);
   if (b->h_stage) cudaFreeHost(b->h_stage);
@@ -2464,6 +2555,14 @@ static float batch_max_hole_width(const cs_batch* b) {
 //   cand_offsets  n_sessions * T*I * (dx, dy, dtheta) verification tables, or NULL: per-session Philox streams
 //   results       optional, n_sessions records (blocks until the poses are back)
 namespace {
+// UpdateObstacleMap (:751) of every session behind the draw kernel of the step `a` (same pose, same cloud, as launch_step
+// does for one processor): one launch of each obstacle kernel for all sessions.  Nothing without ObstacleMaps or points.
+cs_status batch_obstacle_update(cs_batch* b, const CsStepArgs& a, int n_points) {
+  if (!b->d_obst || n_points <= 0) return CS_OK;
+  CS_CUDA(b, launch_obstacle_update(b->stream, b->d_sess, b->d_obst, b->ho, a, n_points, b->n, device_sm_count(b->device), &b->launches));
+  return CS_OK;
+}
+
 // Stages one Update of every session into (h_stage -> d_stage) and launches its kernels; the result records go to d_results.
 cs_status batch_stage_and_launch(cs_batch* b, uint8_t* h_stage, uint8_t* d_stage, CsDevResult* d_results, const float* points,
                                  const int32_t* n_points, const float* odometry, const float* cand_offsets) {
@@ -2504,6 +2603,8 @@ cs_status batch_stage_and_launch(cs_batch* b, uint8_t* h_stage, uint8_t* d_stage
   a.result_stride = 1;
   CS_CUDA(b, launch_step_ctx(LaunchCtx(b, b->flags, b->n, b->hs.data()), a, max_n,
                              rings_hint_of(b->size, b->scale, batch_max_hole_width(b), max_range), CS_PHASE_ALL));
+  cs_status st = batch_obstacle_update(b, a, max_n);
+  if (st != CS_OK) return st;
   b->step.advance(a.do_search);
   return CS_OK;
 }
@@ -2607,6 +2708,8 @@ cs_status cs_batch_replay(cs_batch* b, const cs_scanlog* log, int32_t first, int
     a.result_stride = 1;
     CS_CUDA(b, launch_step_ctx(LaunchCtx(b, b->flags, b->n, b->hs.data()), a, log->h_hdr[sidx].n_points,
                                rings_hint_of(b->size, b->scale, hw, log->h_max_range[sidx]), CS_PHASE_ALL));
+    cs_status st = batch_obstacle_update(b, a, log->h_hdr[sidx].n_points);
+    if (st != CS_OK) return st;
     b->step.advance(a.do_search);
   }
   if (results && count > 0) {
@@ -2654,6 +2757,76 @@ cs_status cs_batch_map_checksums(cs_batch* b, uint64_t* checksums /* n_sessions 
 cs_status cs_batch_get_launch_count(cs_batch* b, uint64_t* launches) {
   if (!b || !launches) return CS_ERR_INVALID_ARGUMENT;
   *launches = b->launches;
+  return CS_OK;
+}
+
+// CoreSLAMProcessor.Reset (:167-175) of every session: the batch steps all sessions with one step state, so they reset together.
+cs_status cs_batch_reset(cs_batch* b) {
+  CS_CHECK_HANDLE(b);
+  if (b->pipe_submitted != b->pipe_collected)
+    return fail(b, CS_ERR_STATE, "cs_batch_reset: submitted steps are waiting for cs_batch_collect");
+  CS_CUDA(b, cudaStreamSynchronize(b->stream));  // the host mirrors are the source of the uploads below
+  for (int j = 0; j < b->n; j++) reset_session(b->hs[j], &b->start_poses[3 * (size_t)j]);  // :172-174
+  b->step.parity = 0;
+  b->step.scan_count = 0;
+  b->step.update_count = 0;
+  CS_CUDA(b, cudaMemcpyAsync(b->d_sess, b->hs.data(), sizeof(CsSession) * (size_t)b->n, cudaMemcpyHostToDevice, b->stream));
+  cs_status st = batch_fill_maps(b);  // :169-170
+  if (st != CS_OK) return st;
+  CS_CUDA(b, cudaStreamSynchronize(b->stream));
+  return CS_OK;
+}
+
+// ---- the sessions' ObstacleMaps (cfg.obstacle_map_size > 0; CoreSLAM/ObstacleMap.cs, CoreSLAMProcessor.cs:98, :103) ----
+// session < 0: all sessions.  MaxObstacleHits applies from the next step, UnmappedObstacleHits from the next cs_batch_reset.
+cs_status cs_batch_set_obstacle_params(cs_batch* b, int32_t session, int32_t unmapped_hits, int32_t max_hits) {
+  CS_CHECK_HANDLE(b);
+  CS_NEED_OBSTACLE(b);
+  if (session >= b->n) return fail(b, CS_ERR_INVALID_ARGUMENT, "session %d out of range", session);
+  if (unmapped_hits < -128 || unmapped_hits > 127) return fail(b, CS_ERR_INVALID_ARGUMENT, "UnmappedObstacleHits is an sbyte");
+  if (max_hits < -128 || max_hits > 127) return fail(b, CS_ERR_INVALID_ARGUMENT, "MaxObstacleHits is an sbyte");
+  for (int j = (session < 0 ? 0 : session); j < (session < 0 ? b->n : session + 1); j++) {
+    b->unmapped_obstacle_hits[j] = unmapped_hits;
+    b->obst[j].max_hits = max_hits;
+  }
+  cs_status st = batch_push_obstacles(b);  // in stream order: steps already queued keep the values they were queued with
+  if (st != CS_OK) return st;
+  CS_CUDA(b, cudaStreamSynchronize(b->stream));
+  return CS_OK;
+}
+
+cs_status cs_batch_obstacle_map_download(cs_batch* b, int32_t session, int8_t* pixels) {
+  CS_CHECK_HANDLE(b);
+  CS_NEED_OBSTACLE(b);
+  if (!pixels || session < 0 || session >= b->n)
+    return fail(b, CS_ERR_INVALID_ARGUMENT, "cs_batch_obstacle_map_download: bad argument");
+  return download_obstacle_map(b, b->obst[session], pixels);
+}
+
+cs_status cs_batch_obstacle_checksums(cs_batch* b, uint64_t* checksums /* n_sessions */) {
+  CS_CHECK_HANDLE(b);
+  CS_NEED_OBSTACLE(b);
+  if (!checksums) return fail(b, CS_ERR_INVALID_ARGUMENT, "null checksums");
+  const unsigned cells = (unsigned)b->ho.size * (unsigned)b->ho.size;
+  const int sms = device_sm_count(b->device);
+  unsigned blocks = (unsigned)((sms * 8 + b->n - 1) / b->n);  // about eight blocks per SM over all sessions
+  if (blocks > (cells + 255) / 256) blocks = (cells + 255) / 256;
+  CS_CUDA(b, cudaMemsetAsync(b->d_obst_sums, 0, sizeof(unsigned long long) * (size_t)b->n, b->stream));
+  cs_obstacle_checksum_kernel<<<dim3(blocks, (unsigned)b->n), 256, 0, b->stream>>>(b->d_obst, b->d_obst_sums);
+  b->launches++;
+  CS_CUDA(b, cudaGetLastError());
+  CS_CUDA(b, cudaMemcpyAsync(checksums, b->d_obst_sums, sizeof(unsigned long long) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
+  CS_CUDA(b, cudaStreamSynchronize(b->stream));
+  return CS_OK;
+}
+
+cs_status cs_batch_get_obstacle_visits(cs_batch* b, int64_t* touched /* n_sessions */) {
+  CS_CHECK_HANDLE(b);
+  CS_NEED_OBSTACLE(b);
+  if (!touched) return fail(b, CS_ERR_INVALID_ARGUMENT, "null out");
+  static_assert(sizeof(long long) == sizeof(int64_t), "touched counters");
+  CS_CUDA(b, cudaMemcpyAsync(touched, b->d_obst_touched, sizeof(long long) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
+  CS_CUDA(b, cudaStreamSynchronize(b->stream));
   return CS_OK;
 }
 

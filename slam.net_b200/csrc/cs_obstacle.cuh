@@ -3,6 +3,10 @@
 //   cs_obstacle_rays_kernel    UpdateObstacleMap's ray loop (CoreSLAM/CoreSLAMProcessor.cs:540-571) with
 //                              DrawLaserRayOnObstacleMap (:456-490): one warp per ray, lanes over the steps
 //   cs_obstacle_sweep_kernel   the no-hit sweep (:576-592), only over the cells the rays marked
+//   cs_obstacle_fill_kernel    Reset's fill (:170) and cs_obstacle_map_fill
+//   cs_obstacle_checksum_kernel  a hash of each map (session batches: all sessions in one launch)
+// Every kernel takes an array of CsObstacle descriptors and works on descriptor blockIdx.y: a processor launches them with
+// one, a session batch with one per session.
 //
 // The reference walks each ray with a loop-carried error term and finishes with an O(Size^2) pass over a
 // bool[,] noHitMap.  Here
@@ -155,7 +159,11 @@ cs_obstacle_sweep_kernel(const CsObstacle* __restrict__ obstacles) {
   }
 }
 
-__global__ void cs_obstacle_fill_kernel(CsObstacle O, int value) {
+// ArrayEx.Fill(ObstacleMap.Pixels, v) (:170), with the no-hit bitmap and the touched counter cleared: one ObstacleMap per
+// blockIdx.y, filled with values[blockIdx.y] (a batch's per-session UnmappedObstacleHits) or, without values, with `value`.
+__global__ void cs_obstacle_fill_kernel(const CsObstacle* __restrict__ obstacles, const int* __restrict__ values, int value) {
+  const CsObstacle O = obstacles[blockIdx.y];
+  if (values) value = values[blockIdx.y];
   const size_t n8 = (size_t)O.pitch * O.rows / 8;
   const unsigned long long b = (unsigned long long)((unsigned)value & 0xffu) * 0x0101010101010101ull;
   unsigned long long* q = reinterpret_cast<unsigned long long*>(O.pixels);
@@ -163,4 +171,21 @@ __global__ void cs_obstacle_fill_kernel(CsObstacle O, int value) {
   const size_t nw = (size_t)O.words_per_row * (O.rows >> 2);
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < nw; i += (size_t)gridDim.x * blockDim.x) O.no_hit[i] = 0u;
   if (blockIdx.x == 0 && threadIdx.x == 0 && O.touched) *O.touched = 0;
+}
+
+// Position-dependent hash of every ObstacleMap, one per blockIdx.y: out[blockIdx.y] += sum over the row-major cells i of
+// ((uint8_t)pixel + 1) * cs_mix64(i), mod 2^64 (cs_host_obstacle_checksum; the caller zeroes `out`).
+__global__ void __launch_bounds__(256)
+cs_obstacle_checksum_kernel(const CsObstacle* __restrict__ obstacles, unsigned long long* __restrict__ out) {
+  const CsObstacle O = obstacles[blockIdx.y];
+  const unsigned size = (unsigned)O.size, n = size * size;  // size <= 16384: n < 2^32
+  unsigned long long acc = 0;
+  for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const unsigned y = i / size, x = i - y * size;
+    const unsigned long long v = (unsigned char)O.pixels[(size_t)y * O.pitch + x];
+    acc += (v + 1ull) * cs_mix64((unsigned long long)i);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  if ((threadIdx.x & 31) == 0 && acc) atomicAdd(out + blockIdx.y, acc);
 }
