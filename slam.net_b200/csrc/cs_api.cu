@@ -16,6 +16,7 @@
 #include <cstring>
 #include <atomic>
 #include <exception>
+#include <memory>
 #include <string>
 #include <type_traits>
 #include <vector>
@@ -44,9 +45,46 @@ constexpr int kRayCopies = 8;  // copies of the per-ray draw parameters of a sta
 
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// Owners of the CUDA resources a handle allocates: released when the owner goes, so a failed create, a destroy and an
+// early return all give back what was allocated.  The descriptors copied to the device (CsSession, CsObstacle,
+// CsStepArgs) hold plain pointers into these blocks.
+struct DevFree { void operator()(void* p) const { cudaFree(p); } };
+struct HostFree { void operator()(void* p) const { cudaFreeHost(p); } };  // pinned, plain or mapped
+struct StreamDestroy { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
+struct EventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+template <typename T> using DevBuf = std::unique_ptr<T[], DevFree>;
+template <typename T> using HostBuf = std::unique_ptr<T[], HostFree>;
+using Stream = std::unique_ptr<CUstream_st, StreamDestroy>;
+using Event = std::unique_ptr<CUevent_st, EventDestroy>;
+
+// `count` elements of T into an empty owner.
+template <typename T> cudaError_t alloc(DevBuf<T>& buf, size_t count) {
+  T* p = nullptr;
+  const cudaError_t e = cudaMalloc(&p, count * sizeof(T));
+  buf.reset(p);
+  return e;
+}
+template <typename T> cudaError_t alloc(HostBuf<T>& buf, size_t count, unsigned flags = cudaHostAllocDefault) {
+  T* p = nullptr;
+  const cudaError_t e = cudaHostAlloc(&p, count * sizeof(T), flags);
+  buf.reset(p);
+  return e;
+}
+cudaError_t create(Stream& s) {
+  cudaStream_t p = nullptr;
+  const cudaError_t e = cudaStreamCreateWithFlags(&p, cudaStreamNonBlocking);
+  s.reset(p);
+  return e;
+}
+cudaError_t create(Event& ev, unsigned flags = cudaEventDisableTiming) {
+  cudaEvent_t p = nullptr;
+  const cudaError_t e = cudaEventCreateWithFlags(&p, flags);
+  ev.reset(p);
+  return e;
+}
+
 struct Timing {
-  cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-  bool valid = false;
+  Event ev[5];
 };
 
 }  // namespace
@@ -90,14 +128,29 @@ struct StepState {
 struct CsHost {
   int device = 0;
   cudaStream_t stream = nullptr;
-  bool own_stream = false;
+  Stream own_stream;  // the stream above when the library created it (never one the caller passed in cfg.stream)
   bool tiled = true;
   int size = 0, pitch_tiles = 0, n_cand = 0;
   float scale = 0.f;
   size_t map_cells = 0;  // allocated cells of one map (tiled: pitch_tiles^2 * 64)
-  CsSession* d_sess = nullptr;
-  uint16_t* d_linear = nullptr;  // lazily allocated row-major scratch for upload/download
-  unsigned long long* d_checksum = nullptr;
+  DevBuf<CsSession> d_sess;
+  DevBuf<uint16_t> d_linear;  // lazily allocated row-major scratch for upload/download
+  DevBuf<unsigned long long> d_checksum;
+  // ray and wedge scratch of all sessions (CsSession::rays .. w_top, alloc_ray_scratch)
+  DevBuf<int4> d_rays;
+  DevBuf<int> d_batch_max;
+  DevBuf<unsigned long long> d_prep_words;
+  DevBuf<int2> d_w_rk;
+  DevBuf<float2> d_w_bkey;
+  DevBuf<int> d_w_top;
+  // ObstacleMaps (cfg.obstacle_map_size > 0), one per session, all of the geometry `ho` (alloc_obstacle_maps): session j's
+  // pixels, bitmap and touched counter are the j-th pieces of the three blocks, described by d_obst[j] (host mirrors: a
+  // processor's `ho` itself, a batch's cs_batch::obst)
+  CsObstacle ho{};
+  DevBuf<CsObstacle> d_obst;
+  DevBuf<int8_t> d_obst_pixels;
+  DevBuf<uint32_t> d_obst_no_hit;
+  DevBuf<long long> d_obst_touched;
   int s2_cap = 0;                // slab-search capacity of one session (0: no slab-search scratch)
   StepState step;
   // stuck-poll word (CsSpin) in pinned+mapped memory, and its device address: a processor's lies in its result slot, a
@@ -114,56 +167,47 @@ struct cs_processor : CsHost {
   int max_points = 0;
 
   CsSession hs{};            // host mirror of the session descriptor
-  uint16_t* d_map = nullptr;
-  uint8_t* d_packed = nullptr;
-  int4* d_rays = nullptr;       // kRayCopies copies of ray_stride entries
-  int* d_batch_max = nullptr;   // kRayCopies copies of batch_stride entries
-  unsigned long long* d_prep_words = nullptr;
-  int ray_stride = 0, batch_stride = 0;
-  int* d_ray_dbg = nullptr;
-  int* d_distances = nullptr;
-  // wedge integration scratch (CsSession::w_*)
-  int2* d_w_rk = nullptr;
-  float2* d_w_bkey = nullptr;
-  int* d_w_top = nullptr;
-  unsigned long long* d_spec = nullptr;  // glue table (CsStepArgs::spec): 8 words per flat candidate
-  long long* d_ring_cycles = nullptr;
+  DevBuf<uint16_t> d_map;
+  DevBuf<uint8_t> d_packed;
+  DevBuf<int> d_ray_dbg;
+  DevBuf<int> d_distances;
+  DevBuf<unsigned long long> d_spec;  // glue table (CsStepArgs::spec): 8 words per flat candidate
+  DevBuf<long long> d_ring_cycles;
 
   // slab search scratch (CsSession::s2_*), allocated when the handle has enough candidates for it to pay
-  float4* d_s2_sorted = nullptr;
-  float4* d_s2_tmp = nullptr;
-  unsigned long long* d_s2_meta = nullptr;
-  unsigned long long* d_s2_acc = nullptr;
-  unsigned* d_s2_ghist = nullptr;
+  DevBuf<float4> d_s2_sorted;
+  DevBuf<float4> d_s2_tmp;
+  DevBuf<unsigned long long> d_s2_meta;
+  DevBuf<unsigned long long> d_s2_acc;
+  DevBuf<unsigned> d_s2_ghist;
   Presort presort;
 
-  // ObstacleMap (cfg.obstacle_map_size > 0): CoreSLAM/ObstacleMap.cs, CoreSLAMProcessor.cs:53, :132-133
-  CsObstacle ho{};               // host mirror of the descriptor
-  CsObstacle* d_obst = nullptr;
+  // ObstacleMap (cfg.obstacle_map_size > 0; CoreSLAM/ObstacleMap.cs, CoreSLAMProcessor.cs:53, :132-133): CsHost::ho is the
+  // host mirror of its descriptor
   int unmapped_obstacle_hits = -5;  // :98
 
   // asynchronous map export (cs_map_export_begin / _wait): snapshot on the main stream, D2H on a side stream
-  cudaStream_t export_stream = nullptr;
-  cudaEvent_t ev_export_snap = nullptr, ev_export_done = nullptr;
+  Stream export_stream;
+  Event ev_export_snap, ev_export_done;
   bool export_busy = false;
-  int8_t* d_obst_snap = nullptr;
+  DevBuf<int8_t> d_obst_snap;
 
-  float2* d_cloud = nullptr;  // scan points computed on the device from raw segments (cs_update_segments)
+  DevBuf<float2> d_cloud;  // scan points computed on the device from raw segments (cs_update_segments)
 
   // staging: [hdr 64][points][cand][cand_cs]; segments path: [hdr 64][rays][seg_first][seg_poses][cand]
   size_t stage_bytes = 0;
-  uint8_t* h_stage = nullptr;  // pinned
-  uint8_t* d_stage = nullptr;
+  HostBuf<uint8_t> h_stage;  // pinned
+  DevBuf<uint8_t> d_stage;
   // cs_update's staging runs ahead of the stream: the H2D copy of scan k goes through a copy stream into the buffer scan
   // k-1 is NOT using (d_stage / d_stage_b alternate), so it overlaps the integration of scan k-1 instead of queueing
   // behind it; the main stream only waits for the copy's event.  ev_stage_free[i]: last step that reads buffer i is enqueued.
-  uint8_t* d_stage_b = nullptr;
-  cudaStream_t copy_stream = nullptr;
-  cudaEvent_t ev_copy = nullptr, ev_stage_free[2] = {nullptr, nullptr};
+  DevBuf<uint8_t> d_stage_b;
+  Stream copy_stream;
+  Event ev_copy, ev_stage_free[2];
   int stage_flip = 0, stage_cur = 0;
 
   // mapped result slot
-  uint8_t* h_slot = nullptr;  // pinned+mapped: CsDevResult at 0, seq flag at 64, stuck-poll word (CsSpin) at 96
+  HostBuf<uint8_t> h_slot;  // pinned+mapped: CsDevResult at 0, seq flag at 64, stuck-poll word (CsSpin) at 96
   uint8_t* d_slot = nullptr;
   unsigned seq = 0;
 
@@ -176,12 +220,22 @@ struct cs_processor : CsHost {
   int group_rank = 0, group_world = 0;
   bool group_shares_device = false;  // another rank of the group runs on this handle's device (same process)
   unsigned xchg_seq = 0;
-  unsigned long long* d_xchg = nullptr;
+  DevBuf<unsigned long long> d_xchg;
   unsigned long long* xchg_peer[CS_GROUP_MAX] = {};
   bool xchg_ipc[CS_GROUP_MAX] = {};  // opened with cudaIpcOpenMemHandle (to be closed on detach)
 
   Timing tm;
   cs_timing last_timing{};
+
+  // The owners release after this: on the handle's device, once every stream the handle queues work on has drained (the
+  // export stream's copy writes caller memory) and the peers' exchange tables are unmapped.
+  ~cs_processor() {
+    cudaSetDevice(device);
+    for (cudaStream_t s : {stream, copy_stream.get(), export_stream.get()})
+      if (s) cudaStreamSynchronize(s);
+    for (int p = 0; p < CS_GROUP_MAX; p++)
+      if (xchg_ipc[p] && xchg_peer[p]) cudaIpcCloseMemHandle(xchg_peer[p]);
+  }
 };
 
 struct cs_scanlog {
@@ -190,12 +244,14 @@ struct cs_scanlog {
   std::vector<float> h_points;   // n_scans * max_points * 2
   std::vector<float> h_offsets;  // n_scans * n_offsets * 3
   std::vector<double> h_max_range;  // per scan, sizes the update kernel's grid
-  CsStepHeader* d_hdr = nullptr;
-  float2* d_points = nullptr;
-  float* d_offsets = nullptr;
-  CsDevResult* d_results = nullptr;
+  DevBuf<CsStepHeader> d_hdr;
+  DevBuf<float2> d_points;
+  DevBuf<float> d_offsets;
+  DevBuf<CsDevResult> d_results;
   bool uploaded = false;
   uint64_t generation = 0;  // counts the uploads: what a handle sorted ahead from this log is only good for the same upload
+
+  ~cs_scanlog() { cudaSetDevice(device); }  // (the owners release on the log's device)
 };
 
 namespace {
@@ -261,13 +317,13 @@ const char* stuck_site_name(unsigned w) {
   } while (0)
 
 cs_status push_session(cs_processor* h) {
-  CS_CUDA(h, cudaMemcpyAsync(h->d_sess, &h->hs, sizeof(CsSession), cudaMemcpyHostToDevice, h->stream));
+  CS_CUDA(h, cudaMemcpyAsync(h->d_sess.get(), &h->hs, sizeof(CsSession), cudaMemcpyHostToDevice, h->stream));
   return CS_OK;
 }
 
 // session fields the host owns; state/key/x1.. are device-owned, so properties are patched individually
 cs_status patch_session(cs_processor* h, size_t offset, const void* src, size_t bytes) {
-  CS_CUDA(h, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(h->d_sess) + offset, src, bytes, cudaMemcpyHostToDevice,
+  CS_CUDA(h, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(h->d_sess.get()) + offset, src, bytes, cudaMemcpyHostToDevice,
                              h->stream));
   CS_CUDA(h, cudaStreamSynchronize(h->stream));  // src may be a stack temporary
   return CS_OK;
@@ -280,7 +336,7 @@ void dispatch_layout(bool tiled, F&& f) {
 }
 
 cs_status launch_fill(cs_processor* h, uint16_t value) {
-  cs_fill_kernel<<<148 * 4, 256, 0, h->stream>>>(h->d_map, h->map_cells, value);
+  cs_fill_kernel<<<148 * 4, 256, 0, h->stream>>>(h->d_map.get(), h->map_cells, value);
   h->launches++;
   CS_CUDA(h, cudaGetLastError());
   return CS_OK;
@@ -553,7 +609,7 @@ struct LaunchCtx {
   // what a step of either handle is launched on; launch_step adds what only a processor has
   LaunchCtx(CsHost* h, uint32_t flags, int sessions, const CsSession* host_sessions)
       : s2_cap(h->s2_cap), s2_min_cand(cs_s2_min_cand(flags, sessions)), hs(host_sessions), num_sms(device_sm_count(h->device)),
-        stream(h->stream), d_sess(h->d_sess), tiled(h->tiled), n_sessions(sessions), launches(&h->launches), step(&h->step) {
+        stream(h->stream), d_sess(h->d_sess.get()), tiled(h->tiled), n_sessions(sessions), launches(&h->launches), step(&h->step) {
     if (flags & CS_FLAG_DEBUG_BOUNDED_SPIN) stuck_dev = reinterpret_cast<volatile unsigned*>(h->d_stuck);
   }
 };
@@ -831,20 +887,20 @@ cs_status launch_step(cs_processor* h, CsStepArgs a, int n_points, int rings, bo
   c.presort = &h->presort;
   c.next_cand = next_cand;
   c.log_tag = log_tag;
-  c.spec = h->d_spec;
-  c.diag = h->d_ring_cycles;
+  c.spec = h->d_spec.get();
+  c.diag = h->d_ring_cycles.get();
   c.diag_rings = h->size;
   a.hdr_stride = 1;
   const bool want_pose_event = timing || (a.seq_flag && (h->cfg.flags & CS_FLAG_NO_HOST_SPIN));
-  c.ev_pose = (want_pose_event && (phases & CS_PHASE_FINISH)) ? h->tm.ev[ev_base + 0] : nullptr;
-  c.ev_done = (timing && (phases & CS_PHASE_FINISH)) ? h->tm.ev[ev_base + 1] : nullptr;
+  c.ev_pose = (want_pose_event && (phases & CS_PHASE_FINISH)) ? h->tm.ev[ev_base + 0].get() : nullptr;
+  c.ev_done = (timing && (phases & CS_PHASE_FINISH)) ? h->tm.ev[ev_base + 1].get() : nullptr;
   CS_CUDA(h, launch_step_ctx(c, a, n_points, rings, phases));
   if (h->d_obst && (phases & CS_PHASE_FINISH) && a.step_mode != CS_STEP_SEARCH_ONLY && n_points > 0) {
     // UpdateObstacleMap (:751) follows UpdateHoleMap (:750): same pose (CsSession::cur_pose), same cloud
-    CS_CUDA(h, launch_obstacle_update(c.stream, h->d_sess, h->d_obst, h->ho, a, n_points, 1, c.num_sms, &h->launches));
+    CS_CUDA(h, launch_obstacle_update(c.stream, h->d_sess.get(), h->d_obst.get(), h->ho, a, n_points, 1, c.num_sms, &h->launches));
   }
-  if (c.ev_done) cudaEventRecord(h->tm.ev[ev_base + 2], h->stream);
-  if (h->copy_stream) CS_CUDA(h, cudaEventRecord(h->ev_stage_free[h->stage_cur], h->stream));  // this step's readers of its staging buffer are enqueued
+  if (c.ev_done) cudaEventRecord(h->tm.ev[ev_base + 2].get(), h->stream);
+  if (h->copy_stream) CS_CUDA(h, cudaEventRecord(h->ev_stage_free[h->stage_cur].get(), h->stream));  // this step's readers of its staging buffer are enqueued
   return CS_OK;
 }
 
@@ -869,7 +925,7 @@ cs_status wait_for_pose(cs_processor* h, unsigned seq, cudaEvent_t fallback_even
   if (h->cfg.flags & CS_FLAG_NO_HOST_SPIN) {
     CS_CUDA(h, cudaEventSynchronize(fallback_event));
   } else {
-    volatile unsigned* flag = reinterpret_cast<volatile unsigned*>(h->h_slot + 64);
+    volatile unsigned* flag = reinterpret_cast<volatile unsigned*>(h->h_slot.get() + 64);
     unsigned spins = 0;
     while (*flag != seq) {
       if ((++spins & 0x3fff) == 0) {
@@ -924,7 +980,7 @@ CsStepArgs update_args(const CsHost& h, bool with_offsets, int n_points) {
 }
 
 cs_status ensure_linear(CsHost* h) {
-  if (!h->d_linear) CS_CUDA(h, cudaMalloc(&h->d_linear, (size_t)h->size * h->size * sizeof(uint16_t)));
+  if (!h->d_linear) CS_CUDA(h, alloc(h->d_linear, (size_t)h->size * h->size));
   return CS_OK;
 }
 
@@ -933,7 +989,7 @@ cs_status relayout_to_linear(CsHost* h, uint16_t* map) {
   cs_status st = ensure_linear(h);
   if (st != CS_OK) return st;
   dispatch_layout(h->tiled, [&](auto T) {
-    cs_relayout_kernel<decltype(T)::value><<<148 * 8, 256, 0, h->stream>>>(map, h->d_linear, h->size, h->pitch_tiles, 0);
+    cs_relayout_kernel<decltype(T)::value><<<148 * 8, 256, 0, h->stream>>>(map, h->d_linear.get(), h->size, h->pitch_tiles, 0);
   });
   h->launches++;
   return CS_OK;
@@ -943,26 +999,101 @@ cs_status relayout_to_linear(CsHost* h, uint16_t* map) {
 cs_status download_map(CsHost* h, uint16_t* map, uint16_t* pixels) {
   cs_status st = relayout_to_linear(h, map);
   if (st != CS_OK) return st;
-  CS_CUDA(h, cudaMemcpyAsync(pixels, h->d_linear, (size_t)h->size * h->size * 2, cudaMemcpyDeviceToHost, h->stream));
+  CS_CUDA(h, cudaMemcpyAsync(pixels, h->d_linear.get(), (size_t)h->size * h->size * 2, cudaMemcpyDeviceToHost, h->stream));
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
   return CS_OK;
 }
 
 cs_status collect_timing(cs_processor* h, bool had_h2d) {
-  CS_CUDA(h, cudaEventSynchronize(h->tm.ev[4]));
+  CS_CUDA(h, cudaEventSynchronize(h->tm.ev[4].get()));
   float ms = 0;
   cs_timing& t = h->last_timing;
-  if (had_h2d) { cudaEventElapsedTime(&ms, h->tm.ev[0], h->tm.ev[1]); t.h2d_ms = ms; } else t.h2d_ms = 0;
-  cudaEventElapsedTime(&ms, h->tm.ev[1], h->tm.ev[2]); t.search_ms = ms;
-  cudaEventElapsedTime(&ms, h->tm.ev[2], h->tm.ev[3]); t.integrate_ms = ms;  // the draw kernel
+  if (had_h2d) { cudaEventElapsedTime(&ms, h->tm.ev[0].get(), h->tm.ev[1].get()); t.h2d_ms = ms; } else t.h2d_ms = 0;
+  cudaEventElapsedTime(&ms, h->tm.ev[1].get(), h->tm.ev[2].get()); t.search_ms = ms;
+  cudaEventElapsedTime(&ms, h->tm.ev[2].get(), h->tm.ev[3].get()); t.integrate_ms = ms;  // the draw kernel
   t.finalize_ms = 0.f;
-  cudaEventElapsedTime(&ms, h->tm.ev[0], h->tm.ev[4]); t.total_device_ms = ms;
+  cudaEventElapsedTime(&ms, h->tm.ev[0].get(), h->tm.ev[4].get()); t.total_device_ms = ms;
   t.obstacle_ms = 0.f;
-  if (h->d_obst) { cudaEventElapsedTime(&ms, h->tm.ev[3], h->tm.ev[4]); t.obstacle_ms = ms; }
+  if (h->d_obst) { cudaEventElapsedTime(&ms, h->tm.ev[3].get(), h->tm.ev[4].get()); t.obstacle_ms = ms; }
   return CS_OK;
 }
 
 bool finite3(const float* p) { return p[0] == p[0] && p[1] == p[1] && p[2] == p[2]; }
+
+// What cs_create and cs_batch_create both require of a configuration (of a batch: of its first session's).  On success,
+// the candidates per scan (T*I) and the point capacity.
+cs_status check_config(const cs_config& cfg, long long* n_cand, int* max_points) {
+  if (cfg.hole_map_size < 8 || cfg.hole_map_size > 16384)
+    return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "hole_map_size must be in [8, 16384], got %d", cfg.hole_map_size);
+  if (!(cfg.physical_map_size > 0.f))
+    return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "physical_map_size must be positive");
+  if (cfg.iterations_per_thread < 0) return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "iterations_per_thread out of range");
+  const int threads = cfg.num_search_threads > 0 ? cfg.num_search_threads : 1;
+  *n_cand = (long long)threads * cfg.iterations_per_thread;
+  if (*n_cand > (1ll << 26)) return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "too many candidates per scan");
+  *max_points = cfg.max_points > 0 ? cfg.max_points : 16384;
+  if (*max_points > 65536) return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "max_points must be <= 65536");
+  if (cfg.obstacle_map_size < 0 || cfg.obstacle_map_size > 16384)
+    return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "obstacle_map_size must be 0 (no ObstacleMap) or in [1, 16384], got %d",
+                cfg.obstacle_map_size);
+  const int ndev = cs_device_count();
+  if (ndev <= 0)
+    return fail(nullptr, CS_ERR_NO_DEVICE, "no CUDA device: this library has no CPU path (cudaGetDeviceCount = 0)");
+  if (cfg.device < 0 || cfg.device >= ndev)
+    return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "device %d out of range (have %d)", cfg.device, ndev);
+  return CS_OK;
+}
+
+// The ray and wedge scratch of the n sessions sess[0..n) (CsSession::rays .. w_top), each session pointed at its slice:
+// `copies` copies of ray_stride rays and of batch_stride batch maxima, and the wedge tables of ray_stride rays on a map of
+// h.size.  The words a step expects zeroed are zeroed.
+cudaError_t alloc_ray_scratch(CsHost& h, CsSession* sess, int n, int copies, int ray_stride, int batch_stride) {
+  const size_t rays = (size_t)copies * ray_stride, maxima = (size_t)copies * batch_stride, prep = (size_t)2 * copies * 16;
+  const size_t bkeys = (size_t)(ray_stride / 32 + 1), top = 3 * wedge_top_words(h.size);
+  cudaError_t e = alloc(h.d_rays, rays * n);
+  if (e == cudaSuccess) e = alloc(h.d_batch_max, maxima * n);
+  if (e == cudaSuccess) e = alloc(h.d_prep_words, prep * n);
+  if (e == cudaSuccess) e = cudaMemset(h.d_prep_words.get(), 0, prep * n * sizeof(unsigned long long));
+  if (e == cudaSuccess) e = alloc(h.d_w_rk, (size_t)ray_stride * n);
+  if (e == cudaSuccess) e = alloc(h.d_w_bkey, bkeys * n);
+  if (e == cudaSuccess) e = alloc(h.d_w_top, top * n);
+  if (e == cudaSuccess) e = cudaMemset(h.d_w_top.get(), 0, top * n * sizeof(int));
+  if (e != cudaSuccess) return e;
+  for (int j = 0; j < n; j++) {
+    CsSession& s = sess[j];
+    s.rays = h.d_rays.get() + j * rays;
+    s.batch_max = h.d_batch_max.get() + j * maxima;
+    s.ray_copies = copies;
+    s.ray_stride = ray_stride;
+    s.batch_stride = batch_stride;
+    s.prep_words = h.d_prep_words.get() + j * prep;
+    s.w_rk = h.d_w_rk.get() + (size_t)j * ray_stride;
+    s.w_bkey = h.d_w_bkey.get() + j * bkeys;
+    s.w_top = h.d_w_top.get() + j * top;
+  }
+  return cudaSuccess;
+}
+
+// n ObstacleMaps of `size` pixels per edge (:132-133): h.ho becomes their geometry, and desc[0..n) the host descriptors of
+// the maps, each with its pieces of the pixel, no-hit bitmap and touched-counter blocks.  The device descriptor array
+// d_obst is allocated; the caller uploads desc into it.
+cudaError_t alloc_obstacle_maps(CsHost& h, CsObstacle* desc, int n, int size, float physical_map_size) {
+  h.ho = obstacle_geometry(size, physical_map_size);
+  const size_t px = obstacle_pixel_bytes(h.ho), words = obstacle_bitmap_words(h.ho);
+  cudaError_t e = alloc(h.d_obst_pixels, px * n);
+  if (e == cudaSuccess) e = alloc(h.d_obst_no_hit, words * n);
+  if (e == cudaSuccess) e = alloc(h.d_obst_touched, (size_t)n);
+  if (e == cudaSuccess) e = alloc(h.d_obst, (size_t)n);
+  if (e != cudaSuccess) return e;
+  for (int j = 0; j < n; j++) {
+    CsObstacle& o = desc[j];
+    o = h.ho;
+    o.pixels = h.d_obst_pixels.get() + j * px;
+    o.no_hit = h.d_obst_no_hit.get() + j * words;
+    o.touched = h.d_obst_touched.get() + j;
+  }
+  return cudaSuccess;
+}
 
 }  // namespace
 
@@ -985,26 +1116,11 @@ int32_t cs_device_count(void) {
 cs_status cs_create(const cs_config* cfg, cs_processor** out) {
   if (!cfg || !out) return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "cs_create: null argument");
   *out = nullptr;
-  if (cfg->hole_map_size < 8 || cfg->hole_map_size > 16384)
-    return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "hole_map_size must be in [8, 16384], got %d", cfg->hole_map_size);
-  if (!(cfg->physical_map_size > 0.f))
-    return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "physical_map_size must be positive");
-  if (cfg->iterations_per_thread < 0 || cfg->iterations_per_thread > (1 << 24))
-    return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "iterations_per_thread out of range");
-  const int threads = cfg->num_search_threads > 0 ? cfg->num_search_threads : 1;
-  const long long n_cand = (long long)threads * cfg->iterations_per_thread;
-  if (n_cand > (1ll << 26)) return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "too many candidates per scan");
-  const int max_points = cfg->max_points > 0 ? cfg->max_points : 16384;
-  if (max_points > 65536) return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "max_points must be <= 65536");
-  if (cfg->obstacle_map_size < 0 || cfg->obstacle_map_size > 16384)
-    return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "obstacle_map_size must be 0 (no ObstacleMap) or in [1, 16384], got %d",
-                cfg->obstacle_map_size);
-
-  int ndev = cs_device_count();
-  if (ndev <= 0)
-    return fail(nullptr, CS_ERR_NO_DEVICE, "no CUDA device: this library has no CPU path (cudaGetDeviceCount = 0)");
-  if (cfg->device < 0 || cfg->device >= ndev)
-    return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "device %d out of range (have %d)", cfg->device, ndev);
+  if (cfg->iterations_per_thread > (1 << 24)) return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "iterations_per_thread out of range");
+  long long n_cand = 0;
+  int max_points = 0;
+  const cs_status cst = check_config(*cfg, &n_cand, &max_points);
+  if (cst != CS_OK) return cst;
 
   cs_processor* h = new cs_processor();
   h->cfg = *cfg;
@@ -1026,62 +1142,53 @@ cs_status cs_create(const cs_config* cfg, cs_processor** out) {
   if (cfg->stream) {
     h->stream = (cudaStream_t)cfg->stream;
   } else {
-    CS_CREATE_CUDA(h, cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
-    h->own_stream = true;
+    CS_CREATE_CUDA(h, create(h->own_stream));
+    h->stream = h->own_stream.get();
   }
-  CS_CREATE_CUDA(h, cudaMalloc(&h->d_map, h->map_cells * sizeof(uint16_t)));
-  CS_CREATE_CUDA(h, cudaMalloc(&h->d_sess, sizeof(CsSession)));
-  if (cfg->flags & CS_FLAG_DEBUG_RAYS) CS_CREATE_CUDA(h, cudaMalloc(&h->d_ray_dbg, (size_t)max_points * 6 * sizeof(int)));
-  h->ray_stride = (max_points + 31) / 32 * 32;
-  h->batch_stride = (h->ray_stride / 32 + 31) / 32 * 32;  // whole 128-byte lines per copy
-  CS_CREATE_CUDA(h, cudaMalloc(&h->d_rays, (size_t)kRayCopies * h->ray_stride * sizeof(int4)));
-  CS_CREATE_CUDA(h, cudaMalloc(&h->d_batch_max, (size_t)kRayCopies * h->batch_stride * sizeof(int)));
-  CS_CREATE_CUDA(h, cudaMalloc(&h->d_prep_words, (size_t)2 * kRayCopies * 16 * sizeof(unsigned long long)));
-  CS_CREATE_CUDA(h, cudaMemset(h->d_prep_words, 0, (size_t)2 * kRayCopies * 16 * sizeof(unsigned long long)));
-  CS_CREATE_CUDA(h, cudaMalloc(&h->d_w_rk, (size_t)h->ray_stride * sizeof(int2)));
-  CS_CREATE_CUDA(h, cudaMalloc(&h->d_w_bkey, (size_t)(h->ray_stride / 32 + 1) * sizeof(float2)));
-  CS_CREATE_CUDA(h, cudaMalloc(&h->d_w_top, (size_t)3 * wedge_top_words(h->size) * sizeof(int)));
-  CS_CREATE_CUDA(h, cudaMemset(h->d_w_top, 0, (size_t)3 * wedge_top_words(h->size) * sizeof(int)));
+  CS_CREATE_CUDA(h, alloc(h->d_map, h->map_cells));
+  CS_CREATE_CUDA(h, alloc(h->d_sess, 1));
+  CsSession& s = h->hs;
+  init_session(s, *h, *cfg, h->d_map.get());
+  if (cfg->flags & CS_FLAG_DEBUG_RAYS) CS_CREATE_CUDA(h, alloc(h->d_ray_dbg, (size_t)max_points * 6));
+  const int ray_stride = (max_points + 31) / 32 * 32;
+  const int batch_stride = (ray_stride / 32 + 31) / 32 * 32;  // whole 128-byte lines per copy
+  CS_CREATE_CUDA(h, alloc_ray_scratch(*h, &s, 1, kRayCopies, ray_stride, batch_stride));
   CS_CREATE_CUDA(h, wedge_allow_shared_memory());
-  CS_CREATE_CUDA(h, cudaMalloc(&h->d_spec, ((size_t)n_cand + 1) * 8 * sizeof(unsigned long long)));
-  CS_CREATE_CUDA(h, cudaMemset(h->d_spec, 0, ((size_t)n_cand + 1) * 8 * sizeof(unsigned long long)));  // (tag 0 is never a step's)
-  CS_CREATE_CUDA(h, cudaMalloc(&h->d_distances, ((size_t)n_cand + 1) * sizeof(int)));
-  CS_CREATE_CUDA(h, cudaMalloc(&h->d_checksum, sizeof(unsigned long long)));
+  CS_CREATE_CUDA(h, alloc(h->d_spec, ((size_t)n_cand + 1) * 8));
+  CS_CREATE_CUDA(h, cudaMemset(h->d_spec.get(), 0, ((size_t)n_cand + 1) * 8 * sizeof(unsigned long long)));  // (tag 0 is never a step's)
+  CS_CREATE_CUDA(h, alloc(h->d_distances, (size_t)n_cand + 1));
+  CS_CREATE_CUDA(h, alloc(h->d_checksum, 1));
   if (cs_s2_min_cand(cfg->flags) > 0 && n_cand + 1 >= cs_s2_min_cand(cfg->flags)) {
     h->s2_cap = (int)n_cand + 1;
-    CS_CREATE_CUDA(h, cudaMalloc(&h->d_s2_sorted, (size_t)2 * h->s2_cap * sizeof(float4)));
-    CS_CREATE_CUDA(h, cudaMalloc(&h->d_s2_tmp, (size_t)h->s2_cap * sizeof(float4)));
-    CS_CREATE_CUDA(h, cudaMalloc(&h->d_s2_meta, (size_t)h->s2_cap * sizeof(unsigned long long)));
-    CS_CREATE_CUDA(h, cudaMalloc(&h->d_s2_acc, (size_t)h->s2_cap * sizeof(unsigned long long)));
-    CS_CREATE_CUDA(h, cudaMemsetAsync(h->d_s2_acc, 0, (size_t)h->s2_cap * sizeof(unsigned long long), h->stream));
-    CS_CREATE_CUDA(h, cudaMalloc(&h->d_s2_ghist, (size_t)(CS_SORT_BINS + 1) * sizeof(unsigned)));
-    CS_CREATE_CUDA(h, cudaMemsetAsync(h->d_s2_ghist, 0, (size_t)(CS_SORT_BINS + 1) * sizeof(unsigned), h->stream));
+    const size_t cap = (size_t)h->s2_cap;
+    CS_CREATE_CUDA(h, alloc(h->d_s2_sorted, 2 * cap));
+    CS_CREATE_CUDA(h, alloc(h->d_s2_tmp, cap));
+    CS_CREATE_CUDA(h, alloc(h->d_s2_meta, cap));
+    CS_CREATE_CUDA(h, alloc(h->d_s2_acc, cap));
+    CS_CREATE_CUDA(h, cudaMemsetAsync(h->d_s2_acc.get(), 0, cap * sizeof(unsigned long long), h->stream));
+    CS_CREATE_CUDA(h, alloc(h->d_s2_ghist, (size_t)CS_SORT_BINS + 1));
+    CS_CREATE_CUDA(h, cudaMemsetAsync(h->d_s2_ghist.get(), 0, (size_t)(CS_SORT_BINS + 1) * sizeof(unsigned), h->stream));
   }
   h->stage_bytes = plan_stage(max_points, (int)n_cand, true).total + 16 * ((size_t)max_points + 1) + 64;  // + segment tables
-  CS_CREATE_CUDA(h, cudaMalloc(&h->d_cloud, (size_t)max_points * sizeof(float2)));
-  CS_CREATE_CUDA(h, cudaHostAlloc(&h->h_stage, h->stage_bytes, cudaHostAllocDefault));
-  CS_CREATE_CUDA(h, cudaMalloc(&h->d_stage, h->stage_bytes));
+  CS_CREATE_CUDA(h, alloc(h->d_cloud, (size_t)max_points));
+  CS_CREATE_CUDA(h, alloc(h->h_stage, h->stage_bytes));
+  CS_CREATE_CUDA(h, alloc(h->d_stage, h->stage_bytes));
   if (tune().copy_stream >= 0) {
-    CS_CREATE_CUDA(h, cudaMalloc(&h->d_stage_b, h->stage_bytes));
-    CS_CREATE_CUDA(h, cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
-    CS_CREATE_CUDA(h, cudaEventCreateWithFlags(&h->ev_copy, cudaEventDisableTiming));
-    for (auto& e : h->ev_stage_free) CS_CREATE_CUDA(h, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    CS_CREATE_CUDA(h, alloc(h->d_stage_b, h->stage_bytes));
+    CS_CREATE_CUDA(h, create(h->copy_stream));
+    CS_CREATE_CUDA(h, create(h->ev_copy));
+    for (Event& e : h->ev_stage_free) CS_CREATE_CUDA(h, create(e));
   }
-  CS_CREATE_CUDA(h, cudaHostAlloc(&h->h_slot, 128, cudaHostAllocMapped));
-  CS_CREATE_CUDA(h, cudaHostGetDevicePointer((void**)&h->d_slot, h->h_slot, 0));
-  memset(h->h_slot, 0, 128);
-  h->h_stuck = h->h_slot + 96;
+  CS_CREATE_CUDA(h, alloc(h->h_slot, 128, cudaHostAllocMapped));
+  CS_CREATE_CUDA(h, cudaHostGetDevicePointer((void**)&h->d_slot, h->h_slot.get(), 0));
+  memset(h->h_slot.get(), 0, 128);
+  h->h_stuck = h->h_slot.get() + 96;
   h->d_stuck = h->d_slot + 96;
-  for (auto& e : h->tm.ev) CS_CREATE_CUDA(h, cudaEventCreate(&e));
+  for (Event& e : h->tm.ev) CS_CREATE_CUDA(h, create(e, cudaEventDefault));
   if (cfg->obstacle_map_size > 0) {  // :132-133
-    CsObstacle& o = h->ho;
-    o = obstacle_geometry(cfg->obstacle_map_size, cfg->physical_map_size);
-    CS_CREATE_CUDA(h, cudaMalloc(&o.pixels, obstacle_pixel_bytes(o)));
-    CS_CREATE_CUDA(h, cudaMalloc(&o.no_hit, obstacle_bitmap_words(o) * sizeof(uint32_t)));
-    CS_CREATE_CUDA(h, cudaMalloc(&o.touched, sizeof(long long)));
-    CS_CREATE_CUDA(h, cudaMalloc(&h->d_obst, sizeof(CsObstacle)));
+    CS_CREATE_CUDA(h, alloc_obstacle_maps(*h, &h->ho, 1, cfg->obstacle_map_size, cfg->physical_map_size));
     // (in stream order: the fill kernel of cs_reset below reads the descriptor on the handle's stream)
-    CS_CREATE_CUDA(h, cudaMemcpyAsync(h->d_obst, &o, sizeof(CsObstacle), cudaMemcpyHostToDevice, h->stream));
+    CS_CREATE_CUDA(h, cudaMemcpyAsync(h->d_obst.get(), &h->ho, sizeof(CsObstacle), cudaMemcpyHostToDevice, h->stream));
   }
 
   // Optional L2 persistence window over the map (the gathers are served from L2 either way when the
@@ -1095,7 +1202,7 @@ cs_status cs_create(const cs_config* cfg, cs_processor** out) {
       size_t carve = win < (size_t)prop.persistingL2CacheMaxSize ? win : (size_t)prop.persistingL2CacheMaxSize;
       if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, carve) == cudaSuccess) {
         cudaStreamAttrValue attr{};
-        attr.accessPolicyWindow.base_ptr = h->d_map;
+        attr.accessPolicyWindow.base_ptr = h->d_map.get();
         attr.accessPolicyWindow.num_bytes = win;
         attr.accessPolicyWindow.hitRatio = win <= carve ? 1.0f : (float)carve / (float)win;
         attr.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
@@ -1106,25 +1213,14 @@ cs_status cs_create(const cs_config* cfg, cs_processor** out) {
     }
   }
 
-  CsSession& s = h->hs;
-  init_session(s, *h, *cfg, h->d_map);
-  s.rays = h->d_rays;
-  s.batch_max = h->d_batch_max;
-  s.ray_copies = kRayCopies;
-  s.ray_stride = h->ray_stride;
-  s.batch_stride = h->batch_stride;
-  s.prep_words = h->d_prep_words;
-  s.w_rk = h->d_w_rk;
-  s.w_bkey = h->d_w_bkey;
-  s.w_top = h->d_w_top;
-  s.s2_sorted = h->d_s2_sorted;
-  s.s2_tmp = h->d_s2_tmp;
-  s.s2_meta = h->d_s2_meta;
-  s.s2_acc = h->d_s2_acc;
-  s.s2_ghist = h->d_s2_ghist;
+  s.s2_sorted = h->d_s2_sorted.get();
+  s.s2_tmp = h->d_s2_tmp.get();
+  s.s2_meta = h->d_s2_meta.get();
+  s.s2_acc = h->d_s2_acc.get();
+  s.s2_ghist = h->d_s2_ghist.get();
   s.s2_cap = h->s2_cap;
-  s.ray_dbg = h->d_ray_dbg;
-  s.distances = (cfg->flags & CS_FLAG_KEEP_DISTANCES) ? h->d_distances : nullptr;
+  s.ray_dbg = h->d_ray_dbg.get();
+  s.distances = (cfg->flags & CS_FLAG_KEEP_DISTANCES) ? h->d_distances.get() : nullptr;
   cs_status st = cs_reset(h);
   if (st != CS_OK) return bail(st);
   *out = h;
@@ -1133,54 +1229,8 @@ cs_status cs_create(const cs_config* cfg, cs_processor** out) {
 
 cs_status cs_destroy(cs_processor* h) {
   if (!h) return CS_OK;
-  cudaSetDevice(h->device);
-  if (h->stream) cudaStreamSynchronize(h->stream);
-  for (auto& e : h->tm.ev)
-    if (e) cudaEventDestroy(e);
-  cudaFree(h->d_map);
-  cudaFree(h->d_linear);
-  cudaFree(h->d_packed);
-  cudaFree(h->d_sess);
-  cudaFree(h->d_rays);
-  cudaFree(h->d_batch_max);
-  cudaFree(h->d_prep_words);
-  for (int p = 0; p < CS_GROUP_MAX; p++)
-    if (h->xchg_ipc[p] && h->xchg_peer[p]) cudaIpcCloseMemHandle(h->xchg_peer[p]);
-  cudaFree(h->d_xchg);
-  cudaFree(h->d_ray_dbg);
-  cudaFree(h->d_w_rk);
-  cudaFree(h->d_w_bkey);
-  cudaFree(h->d_w_top);
-  cudaFree(h->d_spec);
-  cudaFree(h->d_distances);
-  cudaFree(h->d_ring_cycles);
-  cudaFree(h->d_checksum);
-  cudaFree(h->d_cloud);
-  if (h->export_stream) cudaStreamSynchronize(h->export_stream);
-  if (h->ev_export_snap) cudaEventDestroy(h->ev_export_snap);
-  if (h->ev_export_done) cudaEventDestroy(h->ev_export_done);
-  if (h->export_stream) cudaStreamDestroy(h->export_stream);
-  cudaFree(h->d_obst_snap);
-  cudaFree(h->d_s2_sorted);
-  cudaFree(h->d_s2_tmp);
-  cudaFree(h->d_s2_meta);
-  cudaFree(h->d_s2_acc);
-  cudaFree(h->d_s2_ghist);
-  cudaFree(h->d_stage);
-  cudaFree(h->d_stage_b);
-  if (h->copy_stream) { cudaStreamSynchronize(h->copy_stream); cudaStreamDestroy(h->copy_stream); }
-  if (h->ev_copy) cudaEventDestroy(h->ev_copy);
-  for (auto& e : h->ev_stage_free)
-    if (e) cudaEventDestroy(e);
-  cudaFree(h->ho.pixels);
-  cudaFree(h->ho.no_hit);
-  cudaFree(h->ho.touched);
-  cudaFree(h->d_obst);
-  if (h->h_stage) cudaFreeHost(h->h_stage);
-  if (h->h_slot) cudaFreeHost(h->h_slot);
-  if (h->own_stream && h->stream) cudaStreamDestroy(h->stream);
+  delete h;  // ~cs_processor drains the handle's streams; then every owner releases
   cudaGetLastError();
-  delete h;
   return CS_OK;
 }
 
@@ -1196,7 +1246,7 @@ cs_status cs_reset(cs_processor* h) {  // CoreSLAMProcessor.cs:167-175
   st = launch_fill(h, (uint16_t)((CS_TS_OBSTACLE + CS_TS_NO_OBSTACLE) / 2));  // :169
   if (st != CS_OK) return st;
   if (h->d_obst)  // :170 ArrayEx.Fill(ObstacleMap.Pixels, UnmappedObstacleHits)
-    CS_CUDA(h, launch_obstacle_fill(h->stream, h->d_obst, nullptr, h->unmapped_obstacle_hits, h->ho, 1, &h->launches));
+    CS_CUDA(h, launch_obstacle_fill(h->stream, h->d_obst.get(), nullptr, h->unmapped_obstacle_hits, h->ho, 1, &h->launches));
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
   return CS_OK;
 }
@@ -1219,7 +1269,7 @@ cs_status cs_set_max_obstacle_hits(cs_processor* h, int32_t hits) {
   if (hits < -128 || hits > 127) return fail(h, CS_ERR_INVALID_ARGUMENT, "MaxObstacleHits is an sbyte");
   h->ho.max_hits = hits;
   if (!h->d_obst) return CS_OK;
-  CS_CUDA(h, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(h->d_obst) + offsetof(CsObstacle, max_hits), &h->ho.max_hits, sizeof(int),
+  CS_CUDA(h, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(h->d_obst.get()) + offsetof(CsObstacle, max_hits), &h->ho.max_hits, sizeof(int),
                              cudaMemcpyHostToDevice, h->stream));
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
   return CS_OK;
@@ -1254,7 +1304,7 @@ cs_status cs_obstacle_map_fill(cs_processor* h, int32_t value) {
   CS_CHECK_HANDLE(h);
   CS_NEED_OBSTACLE(h);
   if (value < -128 || value > 127) return fail(h, CS_ERR_INVALID_ARGUMENT, "ObstacleMap pixels are sbyte");
-  CS_CUDA(h, launch_obstacle_fill(h->stream, h->d_obst, nullptr, value, h->ho, 1, &h->launches));
+  CS_CUDA(h, launch_obstacle_fill(h->stream, h->d_obst.get(), nullptr, value, h->ho, 1, &h->launches));
   return CS_OK;
 }
 
@@ -1295,7 +1345,7 @@ cs_status cs_get_pose(cs_processor* h, float pose[3]) {
   CS_CHECK_HANDLE(h);
   if (!pose) return fail(h, CS_ERR_INVALID_ARGUMENT, "null pose");
   CsState st;
-  CS_CUDA(h, cudaMemcpyAsync(&st, reinterpret_cast<uint8_t*>(h->d_sess) + offsetof(CsSession, state) + h->step.parity * sizeof(CsState),
+  CS_CUDA(h, cudaMemcpyAsync(&st, reinterpret_cast<uint8_t*>(h->d_sess.get()) + offsetof(CsSession, state) + h->step.parity * sizeof(CsState),
                              sizeof(CsState), cudaMemcpyDeviceToHost, h->stream));
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
   pose[0] = st.pose[0]; pose[1] = st.pose[1]; pose[2] = st.pose[2];
@@ -1332,27 +1382,27 @@ cs_status cs_search(cs_processor* h, const float* points, int32_t n_points, cons
 
   StagePlan sp = plan_stage(n_points, n_cand, cand_cs != nullptr);
   h->stage_cur = 0;
-  CsStepHeader* hdr = reinterpret_cast<CsStepHeader*>(h->h_stage);
+  CsStepHeader* hdr = reinterpret_cast<CsStepHeader*>(h->h_stage.get());
   memset(hdr, 0, kHdrBytes);
   hdr->odo[0] = search_pose[0]; hdr->odo[1] = search_pose[1]; hdr->odo[2] = search_pose[2];
   hdr->n_points = n_points;
-  memcpy(h->h_stage + sp.off_points, points, (size_t)n_points * 8);
-  if (cand_poses) memcpy(h->h_stage + sp.off_cand, cand_poses, (size_t)n_cand * 12);
-  if (cand_cs) memcpy(h->h_stage + sp.off_cs, cand_cs, (size_t)(n_cand + 1) * 8);
-  CS_CUDA(h, cudaMemcpyAsync(h->d_stage, h->h_stage, sp.total, cudaMemcpyHostToDevice, h->stream));
+  memcpy(h->h_stage.get() + sp.off_points, points, (size_t)n_points * 8);
+  if (cand_poses) memcpy(h->h_stage.get() + sp.off_cand, cand_poses, (size_t)n_cand * 12);
+  if (cand_cs) memcpy(h->h_stage.get() + sp.off_cs, cand_cs, (size_t)(n_cand + 1) * 8);
+  CS_CUDA(h, cudaMemcpyAsync(h->d_stage.get(), h->h_stage.get(), sp.total, cudaMemcpyHostToDevice, h->stream));
 
   // distances requested: point the session at the buffer for this call
-  int* dist_ptr = distances ? h->d_distances : h->hs.distances;
+  int* dist_ptr = distances ? h->d_distances.get() : h->hs.distances;
   if (dist_ptr != h->hs.distances) {
-    CS_CUDA(h, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(h->d_sess) + offsetof(CsSession, distances), &dist_ptr,
+    CS_CUDA(h, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(h->d_sess.get()) + offsetof(CsSession, distances), &dist_ptr,
                                sizeof(int*), cudaMemcpyHostToDevice, h->stream));
   }
 
   CsStepArgs a{};
-  a.hdr = reinterpret_cast<const CsStepHeader*>(h->d_stage);
-  a.points = reinterpret_cast<const float2*>(h->d_stage + sp.off_points);
-  a.cand = cand_poses ? reinterpret_cast<const float*>(h->d_stage + sp.off_cand) : nullptr;
-  a.cand_cs = cand_cs ? reinterpret_cast<const float*>(h->d_stage + sp.off_cs) : nullptr;
+  a.hdr = reinterpret_cast<const CsStepHeader*>(h->d_stage.get());
+  a.points = reinterpret_cast<const float2*>(h->d_stage.get() + sp.off_points);
+  a.cand = cand_poses ? reinterpret_cast<const float*>(h->d_stage.get() + sp.off_cand) : nullptr;
+  a.cand_cs = cand_cs ? reinterpret_cast<const float*>(h->d_stage.get() + sp.off_cs) : nullptr;
   a.result = reinterpret_cast<CsDevResult*>(h->d_slot);
   a.seq_flag = reinterpret_cast<volatile unsigned*>(h->d_slot + 64);
   a.seq_value = ++h->seq;
@@ -1368,14 +1418,14 @@ cs_status cs_search(cs_processor* h, const float* points, int32_t n_points, cons
   cs_status st = launch_step(h, a, 0, 0, false, 0);
   if (st != CS_OK) return st;
   if (distances) {
-    CS_CUDA(h, cudaMemcpyAsync(distances, h->d_distances, (size_t)(n_cand + 1) * sizeof(int), cudaMemcpyDeviceToHost,
+    CS_CUDA(h, cudaMemcpyAsync(distances, h->d_distances.get(), (size_t)(n_cand + 1) * sizeof(int), cudaMemcpyDeviceToHost,
                                h->stream));
     int* restore = h->hs.distances;
-    CS_CUDA(h, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(h->d_sess) + offsetof(CsSession, distances), &restore,
+    CS_CUDA(h, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(h->d_sess.get()) + offsetof(CsSession, distances), &restore,
                                sizeof(int*), cudaMemcpyHostToDevice, h->stream));
   }
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
-  copy_result(best, reinterpret_cast<const CsDevResult*>(h->h_slot));
+  copy_result(best, reinterpret_cast<const CsDevResult*>(h->h_slot.get()));
   best->visits = 0;
   return CS_OK;
 }
@@ -1391,16 +1441,16 @@ cs_status cs_integrate(cs_processor* h, const float* points, int32_t n_points, c
   // protected by stream order.
   StagePlan sp = plan_stage(n_points, 0, false);
   h->stage_cur = 0;
-  CsStepHeader* hdr = reinterpret_cast<CsStepHeader*>(h->h_stage);
+  CsStepHeader* hdr = reinterpret_cast<CsStepHeader*>(h->h_stage.get());
   memset(hdr, 0, kHdrBytes);
   hdr->odo[0] = pose[0]; hdr->odo[1] = pose[1]; hdr->odo[2] = pose[2];
   hdr->n_points = n_points;
   if (pose_cs) { hdr->cs[0] = pose_cs[0]; hdr->cs[1] = pose_cs[1]; hdr->has_cs = 1; }
-  memcpy(h->h_stage + sp.off_points, points, (size_t)n_points * 8);
-  CS_CUDA(h, cudaMemcpyAsync(h->d_stage, h->h_stage, sp.total, cudaMemcpyHostToDevice, h->stream));
+  memcpy(h->h_stage.get() + sp.off_points, points, (size_t)n_points * 8);
+  CS_CUDA(h, cudaMemcpyAsync(h->d_stage.get(), h->h_stage.get(), sp.total, cudaMemcpyHostToDevice, h->stream));
   CsStepArgs a{};
-  a.hdr = reinterpret_cast<const CsStepHeader*>(h->d_stage);
-  a.points = reinterpret_cast<const float2*>(h->d_stage + sp.off_points);
+  a.hdr = reinterpret_cast<const CsStepHeader*>(h->d_stage.get());
+  a.points = reinterpret_cast<const float2*>(h->d_stage.get() + sp.off_points);
   a.result = reinterpret_cast<CsDevResult*>(h->d_slot);
   a.step_mode = CS_STEP_INTEGRATE_ONLY;
   a.parity = h->step.parity;
@@ -1408,7 +1458,7 @@ cs_status cs_integrate(cs_processor* h, const float* points, int32_t n_points, c
   if (st != CS_OK) return st;
   if (visits) {
     long long v = 0;
-    CS_CUDA(h, cudaMemcpyAsync(&v, reinterpret_cast<uint8_t*>(h->d_sess) + offsetof(CsSession, visits_slot) + (h->step.step_counter & 1u) * sizeof(long long), sizeof(v),
+    CS_CUDA(h, cudaMemcpyAsync(&v, reinterpret_cast<uint8_t*>(h->d_sess.get()) + offsetof(CsSession, visits_slot) + (h->step.step_counter & 1u) * sizeof(long long), sizeof(v),
                                cudaMemcpyDeviceToHost, h->stream));
     CS_CUDA(h, cudaStreamSynchronize(h->stream));
     *visits = v;
@@ -1429,7 +1479,7 @@ static cs_status launch_cloud(cs_processor* h, const uint8_t* d_rays, const uint
                               int n_segments, const float odo[3]) {
   cs_cloud_kernel<<<(n_rays + CS_CLOUD_THREADS - 1) / CS_CLOUD_THREADS, CS_CLOUD_THREADS, 0, h->stream>>>(
       reinterpret_cast<const float2*>(d_rays), reinterpret_cast<const int*>(d_first), reinterpret_cast<const float*>(d_poses),
-      n_segments, n_rays, odo[0], odo[1], odo[2], h->d_cloud);
+      n_segments, n_rays, odo[0], odo[1], odo[2], h->d_cloud.get());
   h->launches++;
   CS_CUDA(h, cudaGetLastError());
   return CS_OK;
@@ -1478,37 +1528,37 @@ static cs_status stage_update(cs_processor* h, const float* points, int32_t n_po
   const bool do_search = h->step.searches();
   const bool with_offsets = cand_offsets != nullptr && do_search;
   StagePlan sp = plan_stage(n_points, with_offsets ? h->n_cand : 0, false);
-  CsStepHeader* hdr = reinterpret_cast<CsStepHeader*>(h->h_stage);
+  CsStepHeader* hdr = reinterpret_cast<CsStepHeader*>(h->h_stage.get());
   memset(hdr, 0, kHdrBytes);
   hdr->odo[0] = odometry_pose[0]; hdr->odo[1] = odometry_pose[1]; hdr->odo[2] = odometry_pose[2];
   hdr->n_points = n_points;
   size_t off_first = 0, off_poses = 0;
   if (seg) {  // the points slot carries the raw rays; the segment tables go behind the candidate table
-    if (n_points > 0) memcpy(h->h_stage + sp.off_points, seg->rays, (size_t)n_points * 8);
+    if (n_points > 0) memcpy(h->h_stage.get() + sp.off_points, seg->rays, (size_t)n_points * 8);
     off_first = sp.total;
     off_poses = align_up(off_first + (size_t)(seg->n_segments + 1) * 4, 16);
     sp.total = align_up(off_poses + (size_t)seg->n_segments * 12, 16);
-    memcpy(h->h_stage + off_first, seg->seg_first, (size_t)(seg->n_segments + 1) * 4);
-    memcpy(h->h_stage + off_poses, seg->seg_poses, (size_t)seg->n_segments * 12);
+    memcpy(h->h_stage.get() + off_first, seg->seg_first, (size_t)(seg->n_segments + 1) * 4);
+    memcpy(h->h_stage.get() + off_poses, seg->seg_poses, (size_t)seg->n_segments * 12);
   } else if (n_points > 0) {
-    memcpy(h->h_stage + sp.off_points, points, (size_t)n_points * 8);
+    memcpy(h->h_stage.get() + sp.off_points, points, (size_t)n_points * 8);
   }
-  if (with_offsets) memcpy(h->h_stage + sp.off_cand, cand_offsets, (size_t)h->n_cand * 12);
+  if (with_offsets) memcpy(h->h_stage.get() + sp.off_cand, cand_offsets, (size_t)h->n_cand * 12);
 
-  if (timing) cudaEventRecord(h->tm.ev[0], h->stream);
-  uint8_t* d_base = h->d_stage;
+  if (timing) cudaEventRecord(h->tm.ev[0].get(), h->stream);
+  uint8_t* d_base = h->d_stage.get();
   if (h->copy_stream) {
     // run ahead of the stream: copy into the buffer the scan in flight is not reading, behind nothing but that buffer's
     // last readers (two scans ago); the main stream picks the copy up through its event
     h->stage_cur = (h->stage_flip ^= 1);
-    d_base = h->stage_cur ? h->d_stage_b : h->d_stage;
-    CS_CUDA(h, cudaStreamWaitEvent(h->copy_stream, h->ev_stage_free[h->stage_cur], 0));
-    CS_CUDA(h, cudaMemcpyAsync(d_base, h->h_stage, sp.total, cudaMemcpyHostToDevice, h->copy_stream));
-    CS_CUDA(h, cudaEventRecord(h->ev_copy, h->copy_stream));
-    CS_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_copy, 0));
+    d_base = h->stage_cur ? h->d_stage_b.get() : h->d_stage.get();
+    CS_CUDA(h, cudaStreamWaitEvent(h->copy_stream.get(), h->ev_stage_free[h->stage_cur].get(), 0));
+    CS_CUDA(h, cudaMemcpyAsync(d_base, h->h_stage.get(), sp.total, cudaMemcpyHostToDevice, h->copy_stream.get()));
+    CS_CUDA(h, cudaEventRecord(h->ev_copy.get(), h->copy_stream.get()));
+    CS_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_copy.get(), 0));
   } else {
     h->stage_cur = 0;
-    CS_CUDA(h, cudaMemcpyAsync(d_base, h->h_stage, sp.total, cudaMemcpyHostToDevice, h->stream));
+    CS_CUDA(h, cudaMemcpyAsync(d_base, h->h_stage.get(), sp.total, cudaMemcpyHostToDevice, h->stream));
   }
   if (seg && n_points > 0) {  // ScanSegmentsToCloud (:723) on the device; the step's first kernel must not start before it is complete
     cs_status cst = launch_cloud(h, d_base + sp.off_points, d_base + off_first, d_base + off_poses, n_points,
@@ -1516,11 +1566,11 @@ static cs_status stage_update(cs_processor* h, const float* points, int32_t n_po
     if (cst != CS_OK) return cst;
     g_next_launch_plain = true;
   }
-  if (timing) cudaEventRecord(h->tm.ev[1], h->stream);
+  if (timing) cudaEventRecord(h->tm.ev[1].get(), h->stream);
 
   CsStepArgs a = update_args(*h, with_offsets, n_points);
   a.hdr = reinterpret_cast<const CsStepHeader*>(d_base);
-  a.points = seg ? h->d_cloud : reinterpret_cast<const float2*>(d_base + sp.off_points);
+  a.points = seg ? h->d_cloud.get() : reinterpret_cast<const float2*>(d_base + sp.off_points);
   a.cand = with_offsets ? reinterpret_cast<const float*>(d_base + sp.off_cand) : nullptr;
   a.result = reinterpret_cast<CsDevResult*>(h->d_slot);
   a.seq_flag = reinterpret_cast<volatile unsigned*>(h->d_slot + 64);
@@ -1534,21 +1584,21 @@ static cs_status stage_update(cs_processor* h, const float* points, int32_t n_po
 // Host-side bookkeeping after an Update has been enqueued, the wait for the pose, and the result copy.
 static cs_status complete_update(cs_processor* h, const CsStepArgs& a, bool timing, cs_result* out) {
   h->step.advance(a.do_search);
-  cs_status st = wait_for_pose(h, a.seq_value, h->tm.ev[2]);
+  cs_status st = wait_for_pose(h, a.seq_value, h->tm.ev[2].get());
   if (st != CS_OK) return st;
   if (timing) {
     st = collect_timing(h, true);
     if (st != CS_OK) return st;
   }
   CS_CHECK_STUCK(h);
-  if (reinterpret_cast<const CsDevResult*>(h->h_slot)->searched < 0)
+  if (reinterpret_cast<const CsDevResult*>(h->h_slot.get())->searched < 0)
     return fail(h, CS_ERR_NCCL, "candidate-split group: a rank never delivered its arg-min (exchange timed out after %.1f s)",
                 (double)CS_XCHG_TIMEOUT_NS * 1e-9);
   if (out) {
-    copy_update_results(out, reinterpret_cast<const CsDevResult*>(h->h_slot), 1);
+    copy_update_results(out, reinterpret_cast<const CsDevResult*>(h->h_slot.get()), 1);
     if (timing) {
       long long v = 0;
-      CS_CUDA(h, cudaMemcpyAsync(&v, reinterpret_cast<uint8_t*>(h->d_sess) + offsetof(CsSession, visits_slot) + (h->step.step_counter & 1u) * sizeof(long long), sizeof(v),
+      CS_CUDA(h, cudaMemcpyAsync(&v, reinterpret_cast<uint8_t*>(h->d_sess.get()) + offsetof(CsSession, visits_slot) + (h->step.step_counter & 1u) * sizeof(long long), sizeof(v),
                                  cudaMemcpyDeviceToHost, h->stream));
       CS_CUDA(h, cudaStreamSynchronize(h->stream));
       out->visits = v;
@@ -1600,13 +1650,13 @@ cs_status cs_segments_to_cloud(cs_processor* h, const float* rays, const int32_t
   const size_t off_first = align_up(off_rays + (size_t)n_rays * 8, 16);
   const size_t off_poses = align_up(off_first + (size_t)(n_segments + 1) * 4, 16);
   const size_t total = align_up(off_poses + (size_t)n_segments * 12, 16);
-  memcpy(h->h_stage + off_rays, rays, (size_t)n_rays * 8);
-  memcpy(h->h_stage + off_first, seg_first, (size_t)(n_segments + 1) * 4);
-  memcpy(h->h_stage + off_poses, seg_poses, (size_t)n_segments * 12);
-  CS_CUDA(h, cudaMemcpyAsync(h->d_stage, h->h_stage, total, cudaMemcpyHostToDevice, h->stream));
-  st = launch_cloud(h, h->d_stage + off_rays, h->d_stage + off_first, h->d_stage + off_poses, n_rays, n_segments, odometry_pose);
+  memcpy(h->h_stage.get() + off_rays, rays, (size_t)n_rays * 8);
+  memcpy(h->h_stage.get() + off_first, seg_first, (size_t)(n_segments + 1) * 4);
+  memcpy(h->h_stage.get() + off_poses, seg_poses, (size_t)n_segments * 12);
+  CS_CUDA(h, cudaMemcpyAsync(h->d_stage.get(), h->h_stage.get(), total, cudaMemcpyHostToDevice, h->stream));
+  st = launch_cloud(h, h->d_stage.get() + off_rays, h->d_stage.get() + off_first, h->d_stage.get() + off_poses, n_rays, n_segments, odometry_pose);
   if (st != CS_OK) return st;
-  CS_CUDA(h, cudaMemcpyAsync(points_out, h->d_cloud, (size_t)n_rays * 8, cudaMemcpyDeviceToHost, h->stream));
+  CS_CUDA(h, cudaMemcpyAsync(points_out, h->d_cloud.get(), (size_t)n_rays * 8, cudaMemcpyDeviceToHost, h->stream));
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
   return CS_OK;
 }
@@ -1635,7 +1685,7 @@ cs_status cs_update_begin(cs_processor* h, const float* points, int32_t n_points
   h->pending_rings = rings;
   if (key_device)  // NULL when this scan runs no search (:726): nothing to exchange
     *key_device = (a.do_search && cand_count > 0)
-                      ? reinterpret_cast<uint64_t*>(reinterpret_cast<uint8_t*>(h->d_sess) + offsetof(CsSession, key) +
+                      ? reinterpret_cast<uint64_t*>(reinterpret_cast<uint8_t*>(h->d_sess.get()) + offsetof(CsSession, key) +
                                                     sizeof(unsigned long long) * (size_t)a.parity)
                       : nullptr;
   return CS_OK;
@@ -1655,9 +1705,9 @@ cs_status cs_update_finish(cs_processor* h, cs_result* out) {
 // ---- candidate-split group with the exchange inside the search kernel (SURVEY 8b "cs_group_create", 8e) ------------------
 static cs_status group_table(cs_processor* h) {
   if (!h->d_xchg) {
-    const size_t bytes = (size_t)2 * CS_GROUP_MAX * 2 * sizeof(unsigned long long);
-    CS_CUDA(h, cudaMalloc(&h->d_xchg, bytes));
-    CS_CUDA(h, cudaMemset(h->d_xchg, 0, bytes));
+    const size_t words = (size_t)2 * CS_GROUP_MAX * 2;
+    CS_CUDA(h, alloc(h->d_xchg, words));
+    CS_CUDA(h, cudaMemset(h->d_xchg.get(), 0, words * sizeof(unsigned long long)));
   }
   return CS_OK;
 }
@@ -1669,7 +1719,7 @@ cs_status cs_group_export(cs_processor* h, cs_ipc_handle* out) {
   if (st != CS_OK) return st;
   static_assert(sizeof(cudaIpcMemHandle_t) <= sizeof(cs_ipc_handle), "cs_ipc_handle too small");
   cudaIpcMemHandle_t mh;
-  CS_CUDA(h, cudaIpcGetMemHandle(&mh, h->d_xchg));
+  CS_CUDA(h, cudaIpcGetMemHandle(&mh, h->d_xchg.get()));
   memset(out, 0, sizeof(*out));
   memcpy(out, &mh, sizeof(mh));
   return CS_OK;
@@ -1687,7 +1737,7 @@ cs_status cs_group_detach(cs_processor* h) {
   h->group_rank = 0;
   h->group_shares_device = false;
   h->xchg_seq = 0;
-  if (h->d_xchg) CS_CUDA(h, cudaMemset(h->d_xchg, 0, (size_t)2 * CS_GROUP_MAX * 2 * sizeof(unsigned long long)));
+  if (h->d_xchg) CS_CUDA(h, cudaMemset(h->d_xchg.get(), 0, (size_t)2 * CS_GROUP_MAX * 2 * sizeof(unsigned long long)));
   cudaGetLastError();
   return CS_OK;
 }
@@ -1709,7 +1759,7 @@ cs_status cs_group_attach(cs_processor* h, int32_t rank, int32_t world, const cs
   if (st == CS_OK) st = group_table(h);
   if (st != CS_OK) return st;
   for (int p = 0; p < world; p++) {
-    if (p == rank) { h->xchg_peer[p] = h->d_xchg; continue; }
+    if (p == rank) { h->xchg_peer[p] = h->d_xchg.get(); continue; }
     cudaIpcMemHandle_t mh;
     memcpy(&mh, &handles[p], sizeof(mh));
     void* ptr = nullptr;
@@ -1756,7 +1806,7 @@ cs_status cs_group_attach_local(cs_processor* h, int32_t rank, int32_t world, cs
         cudaGetLastError();
       }
     }
-    h->xchg_peer[p] = q->d_xchg;
+    h->xchg_peer[p] = q->d_xchg.get();
   }
   h->group_rank = rank;
   h->group_world = world;
@@ -1772,7 +1822,7 @@ cs_status cs_sync(cs_processor* h) {
 // -----------------------------------------------------------------------------------------------------
 static cs_status export_wait(cs_processor* h) {
   if (h->export_busy) {
-    CS_CUDA(h, cudaEventSynchronize(h->ev_export_done));
+    CS_CUDA(h, cudaEventSynchronize(h->ev_export_done.get()));
     h->export_busy = false;
   }
   return CS_OK;
@@ -1784,7 +1834,7 @@ cs_status cs_map_download(cs_processor* h, uint16_t* pixels) {
   if (!pixels) return fail(h, CS_ERR_INVALID_ARGUMENT, "null pixels");
   cs_status st = export_wait(h);  // d_linear may still be read by an export's D2H copy
   if (st != CS_OK) return st;
-  return download_map(h, h->d_map, pixels);
+  return download_map(h, h->d_map.get(), pixels);
 }
 
 cs_status cs_map_upload(cs_processor* h, const uint16_t* pixels) {
@@ -1794,9 +1844,9 @@ cs_status cs_map_upload(cs_processor* h, const uint16_t* pixels) {
   cs_status st = export_wait(h);  // d_linear may still be read by an export's D2H copy
   if (st == CS_OK) st = ensure_linear(h);
   if (st != CS_OK) return st;
-  CS_CUDA(h, cudaMemcpyAsync(h->d_linear, pixels, (size_t)h->size * h->size * 2, cudaMemcpyHostToDevice, h->stream));
+  CS_CUDA(h, cudaMemcpyAsync(h->d_linear.get(), pixels, (size_t)h->size * h->size * 2, cudaMemcpyHostToDevice, h->stream));
   dispatch_layout(h->tiled, [&](auto T) {
-    cs_relayout_kernel<decltype(T)::value><<<148 * 8, 256, 0, h->stream>>>(h->d_map, h->d_linear, h->size, h->pitch_tiles, 1);
+    cs_relayout_kernel<decltype(T)::value><<<148 * 8, 256, 0, h->stream>>>(h->d_map.get(), h->d_linear.get(), h->size, h->pitch_tiles, 1);
   });
   h->launches++;
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
@@ -1819,12 +1869,12 @@ cs_status cs_map_packed(cs_processor* h, uint8_t* packed) {
     if (wst != CS_OK) return wst;
   }
   size_t n = ((size_t)h->size * h->size) / 2;
-  if (!h->d_packed) CS_CUDA(h, cudaMalloc(&h->d_packed, n));
+  if (!h->d_packed) CS_CUDA(h, alloc(h->d_packed, n));
   dispatch_layout(h->tiled, [&](auto T) {
-    cs_pack_kernel<decltype(T)::value><<<148 * 8, 256, 0, h->stream>>>(h->d_map, h->size, h->pitch_tiles, h->d_packed);
+    cs_pack_kernel<decltype(T)::value><<<148 * 8, 256, 0, h->stream>>>(h->d_map.get(), h->size, h->pitch_tiles, h->d_packed.get());
   });
   h->launches++;
-  CS_CUDA(h, cudaMemcpyAsync(packed, h->d_packed, n, cudaMemcpyDeviceToHost, h->stream));
+  CS_CUDA(h, cudaMemcpyAsync(packed, h->d_packed.get(), n, cudaMemcpyDeviceToHost, h->stream));
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
   return CS_OK;
 }
@@ -1840,39 +1890,39 @@ cs_status cs_map_export_begin(cs_processor* h, int32_t format, void* dst) {
   if (format < CS_EXPORT_GRAY16 || format > CS_EXPORT_OBSTACLE_I8) return fail(h, CS_ERR_INVALID_ARGUMENT, "unknown export format %d", format);
   if (format == CS_EXPORT_OBSTACLE_I8 && !h->d_obst) return fail(h, CS_ERR_STATE, "this processor has no ObstacleMap");
   if (!h->export_stream) {
-    CS_CUDA(h, cudaStreamCreateWithFlags(&h->export_stream, cudaStreamNonBlocking));
-    CS_CUDA(h, cudaEventCreateWithFlags(&h->ev_export_snap, cudaEventDisableTiming));
-    CS_CUDA(h, cudaEventCreateWithFlags(&h->ev_export_done, cudaEventDisableTiming));
+    CS_CUDA(h, create(h->export_stream));
+    CS_CUDA(h, create(h->ev_export_snap));
+    CS_CUDA(h, create(h->ev_export_done));
   }
   // the previous export's copy must be through with the snapshot buffers before they are overwritten (device-side wait)
-  if (h->export_busy) CS_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_export_done, 0));
+  if (h->export_busy) CS_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_export_done.get(), 0));
   const size_t cells = (size_t)h->size * h->size;
   const void* src = nullptr;
   size_t bytes = 0;
   if (format == CS_EXPORT_GRAY16) {
-    cs_status st = relayout_to_linear(h, h->d_map);
+    cs_status st = relayout_to_linear(h, h->d_map.get());
     if (st != CS_OK) return st;
-    src = h->d_linear; bytes = cells * 2;
+    src = h->d_linear.get(); bytes = cells * 2;
   } else if (format == CS_EXPORT_PACKED4) {
-    if (!h->d_packed) CS_CUDA(h, cudaMalloc(&h->d_packed, cells / 2));
+    if (!h->d_packed) CS_CUDA(h, alloc(h->d_packed, cells / 2));
     dispatch_layout(h->tiled, [&](auto T) {
-      cs_pack_kernel<decltype(T)::value><<<148 * 8, 256, 0, h->stream>>>(h->d_map, h->size, h->pitch_tiles, h->d_packed);
+      cs_pack_kernel<decltype(T)::value><<<148 * 8, 256, 0, h->stream>>>(h->d_map.get(), h->size, h->pitch_tiles, h->d_packed.get());
     });
     h->launches++;
-    src = h->d_packed; bytes = cells / 2;
+    src = h->d_packed.get(); bytes = cells / 2;
   } else {
     const CsObstacle& o = h->ho;
     bytes = (size_t)o.size * o.size;
-    if (!h->d_obst_snap) CS_CUDA(h, cudaMalloc(&h->d_obst_snap, bytes));
-    CS_CUDA(h, cudaMemcpy2DAsync(h->d_obst_snap, (size_t)o.size, o.pixels, (size_t)o.pitch, (size_t)o.size, (size_t)o.size,
+    if (!h->d_obst_snap) CS_CUDA(h, alloc(h->d_obst_snap, bytes));
+    CS_CUDA(h, cudaMemcpy2DAsync(h->d_obst_snap.get(), (size_t)o.size, o.pixels, (size_t)o.pitch, (size_t)o.size, (size_t)o.size,
                                  cudaMemcpyDeviceToDevice, h->stream));
-    src = h->d_obst_snap;
+    src = h->d_obst_snap.get();
   }
   CS_CUDA(h, cudaGetLastError());
-  CS_CUDA(h, cudaEventRecord(h->ev_export_snap, h->stream));
-  CS_CUDA(h, cudaStreamWaitEvent(h->export_stream, h->ev_export_snap, 0));
-  CS_CUDA(h, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, h->export_stream));
-  CS_CUDA(h, cudaEventRecord(h->ev_export_done, h->export_stream));
+  CS_CUDA(h, cudaEventRecord(h->ev_export_snap.get(), h->stream));
+  CS_CUDA(h, cudaStreamWaitEvent(h->export_stream.get(), h->ev_export_snap.get(), 0));
+  CS_CUDA(h, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, h->export_stream.get()));
+  CS_CUDA(h, cudaEventRecord(h->ev_export_done.get(), h->export_stream.get()));
   h->export_busy = true;
   return CS_OK;
 }
@@ -1884,19 +1934,19 @@ cs_status cs_map_export_wait(cs_processor* h) {
 
 // Queues the checksum of `map` (cs_host_map_checksum of its row-major pixels) into *out; the caller synchronises.
 static cs_status queue_map_checksum(CsHost* h, const uint16_t* map, int blocks, uint64_t* out) {
-  CS_CUDA(h, cudaMemsetAsync(h->d_checksum, 0, sizeof(unsigned long long), h->stream));
+  CS_CUDA(h, cudaMemsetAsync(h->d_checksum.get(), 0, sizeof(unsigned long long), h->stream));
   dispatch_layout(h->tiled, [&](auto T) {
-    cs_checksum_kernel<decltype(T)::value><<<blocks, 256, 0, h->stream>>>(map, h->size, h->pitch_tiles, h->d_checksum);
+    cs_checksum_kernel<decltype(T)::value><<<blocks, 256, 0, h->stream>>>(map, h->size, h->pitch_tiles, h->d_checksum.get());
   });
   h->launches++;
-  CS_CUDA(h, cudaMemcpyAsync(out, h->d_checksum, sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+  CS_CUDA(h, cudaMemcpyAsync(out, h->d_checksum.get(), sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
   return CS_OK;
 }
 
 cs_status cs_map_checksum(cs_processor* h, uint64_t* checksum) {
   CS_CHECK_HANDLE(h);
   if (!checksum) return fail(h, CS_ERR_INVALID_ARGUMENT, "null checksum");
-  cs_status st = queue_map_checksum(h, h->d_map, 148 * 8, checksum);
+  cs_status st = queue_map_checksum(h, h->d_map.get(), 148 * 8, checksum);
   if (st != CS_OK) return st;
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
   return CS_OK;
@@ -1927,7 +1977,7 @@ cs_status cs_get_distances(cs_processor* h, int32_t* distances, int32_t count) {
   CS_CHECK_HANDLE(h);
   if (!h->hs.distances) return fail(h, CS_ERR_STATE, "handle was created without CS_FLAG_KEEP_DISTANCES");
   if (!distances || count < 0 || count > h->n_cand + 1) return fail(h, CS_ERR_INVALID_ARGUMENT, "bad count");
-  CS_CUDA(h, cudaMemcpyAsync(distances, h->d_distances, (size_t)count * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  CS_CUDA(h, cudaMemcpyAsync(distances, h->d_distances.get(), (size_t)count * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
   return CS_OK;
 }
@@ -1936,7 +1986,7 @@ cs_status cs_get_rays(cs_processor* h, int32_t* rays, int32_t n_points) {
   CS_CHECK_HANDLE(h);
   if (!h->d_ray_dbg) return fail(h, CS_ERR_STATE, "handle was created without CS_FLAG_DEBUG_RAYS");
   if (!rays || n_points < 0 || n_points > h->max_points) return fail(h, CS_ERR_INVALID_ARGUMENT, "bad n_points");
-  CS_CUDA(h, cudaMemcpyAsync(rays, h->d_ray_dbg, (size_t)n_points * 6 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  CS_CUDA(h, cudaMemcpyAsync(rays, h->d_ray_dbg.get(), (size_t)n_points * 6 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
   return CS_OK;
 }
@@ -1945,7 +1995,7 @@ cs_status cs_get_visits(cs_processor* h, int64_t* visits) {
   CS_CHECK_HANDLE(h);
   if (!visits) return fail(h, CS_ERR_INVALID_ARGUMENT, "null visits");
   long long v = 0;
-  CS_CUDA(h, cudaMemcpyAsync(&v, reinterpret_cast<uint8_t*>(h->d_sess) + offsetof(CsSession, visits_slot) + (h->step.step_counter & 1u) * sizeof(long long), sizeof(v),
+  CS_CUDA(h, cudaMemcpyAsync(&v, reinterpret_cast<uint8_t*>(h->d_sess.get()) + offsetof(CsSession, visits_slot) + (h->step.step_counter & 1u) * sizeof(long long), sizeof(v),
                              cudaMemcpyDeviceToHost, h->stream));
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
   *visits = v;
@@ -1957,13 +2007,13 @@ cs_status cs_get_ring_cycles(cs_processor* h, int64_t* cycles, int32_t count) {
   const size_t slots = ((size_t)h->size + CS_DIAG_SEARCH_BLOCKS) * 8;
   if (count < 0 || (size_t)count > slots) return fail(h, CS_ERR_INVALID_ARGUMENT, "bad count");
   if (!h->d_ring_cycles) {  // first call switches the diagnostics on
-    CS_CUDA(h, cudaMalloc(&h->d_ring_cycles, slots * sizeof(long long)));
-    CS_CUDA(h, cudaMemsetAsync(h->d_ring_cycles, 0, slots * sizeof(long long), h->stream));
-    h->hs.ring_cycles = h->d_ring_cycles;
+    CS_CUDA(h, alloc(h->d_ring_cycles, slots));
+    CS_CUDA(h, cudaMemsetAsync(h->d_ring_cycles.get(), 0, slots * sizeof(long long), h->stream));
+    h->hs.ring_cycles = h->d_ring_cycles.get();
     return patch_session(h, offsetof(CsSession, ring_cycles), &h->hs.ring_cycles, sizeof(long long*));
   }
   if (cycles && count > 0) {
-    CS_CUDA(h, cudaMemcpyAsync(cycles, h->d_ring_cycles, (size_t)count * sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
+    CS_CUDA(h, cudaMemcpyAsync(cycles, h->d_ring_cycles.get(), (size_t)count * sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
     CS_CUDA(h, cudaStreamSynchronize(h->stream));
   }
   return CS_OK;
@@ -2003,7 +2053,7 @@ cs_status cs_pinned_alloc(void** ptr, uint64_t bytes) {
 }
 
 cs_status cs_pinned_free(void* ptr) {
-  if (ptr) cudaFreeHost(ptr);
+  if (ptr) HostFree()(ptr);
   return CS_OK;
 }
 
@@ -2013,9 +2063,9 @@ cs_status cs_scanlog_create(int32_t device, int32_t n_scans, int32_t max_points,
     return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "cs_scanlog_create: bad argument");
   *out = nullptr;
   if (cs_device_count() <= device) return fail(nullptr, CS_ERR_NO_DEVICE, "no such CUDA device");
-  cs_scanlog* log = nullptr;
+  std::unique_ptr<cs_scanlog> log;  // (a failed create releases what it allocated)
   try {  // a file header with a huge n_scans must come back as a status, not as std::bad_alloc through the C boundary
-    log = new cs_scanlog();
+    log.reset(new cs_scanlog());
     log->device = device;
     log->n_scans = n_scans;
     log->max_points = (max_points + 1) & ~1;  // keep every scan's points 16-byte aligned
@@ -2025,21 +2075,19 @@ cs_status cs_scanlog_create(int32_t device, int32_t n_scans, int32_t max_points,
     log->h_offsets.assign((size_t)n_scans * n_offsets * 3, 0.f);
     log->h_max_range.assign((size_t)n_scans, 0.0);
   } catch (const std::exception&) {  // bad_alloc, length_error
-    delete log;
     return fail(nullptr, CS_ERR_OUT_OF_MEMORY, "cs_scanlog_create: host allocation failed (%d scans x %d points, %d offsets)", n_scans,
                 max_points, n_offsets);
   }
   cudaSetDevice(device);
-  bool ok = cudaMalloc(&log->d_hdr, sizeof(CsStepHeader) * n_scans) == cudaSuccess &&
-            cudaMalloc(&log->d_points, sizeof(float2) * (size_t)n_scans * log->max_points) == cudaSuccess &&
-            cudaMalloc(&log->d_offsets, sizeof(float) * 3 * (size_t)n_scans * (n_offsets > 0 ? n_offsets : 1)) == cudaSuccess &&
-            cudaMalloc(&log->d_results, sizeof(CsDevResult) * n_scans) == cudaSuccess;
+  const bool ok = alloc(log->d_hdr, (size_t)n_scans) == cudaSuccess &&
+                  alloc(log->d_points, (size_t)n_scans * log->max_points) == cudaSuccess &&
+                  alloc(log->d_offsets, 3 * (size_t)n_scans * (n_offsets > 0 ? n_offsets : 1)) == cudaSuccess &&
+                  alloc(log->d_results, (size_t)n_scans) == cudaSuccess;
   if (!ok) {
     cudaGetLastError();
-    cs_scanlog_destroy(log);
     return fail(nullptr, CS_ERR_OUT_OF_MEMORY, "cs_scanlog_create: device allocation failed");
   }
-  *out = log;
+  *out = log.release();
   return CS_OK;
 }
 
@@ -2062,10 +2110,10 @@ cs_status cs_scanlog_set(cs_scanlog* log, int32_t scan, const float* points, int
 cs_status cs_scanlog_upload(cs_scanlog* log) {
   if (!log) return CS_ERR_INVALID_ARGUMENT;
   cudaSetDevice(log->device);
-  bool ok = cudaMemcpy(log->d_hdr, log->h_hdr.data(), sizeof(CsStepHeader) * log->n_scans, cudaMemcpyHostToDevice) == cudaSuccess &&
-            cudaMemcpy(log->d_points, log->h_points.data(), log->h_points.size() * sizeof(float), cudaMemcpyHostToDevice) == cudaSuccess;
+  bool ok = cudaMemcpy(log->d_hdr.get(), log->h_hdr.data(), sizeof(CsStepHeader) * log->n_scans, cudaMemcpyHostToDevice) == cudaSuccess &&
+            cudaMemcpy(log->d_points.get(), log->h_points.data(), log->h_points.size() * sizeof(float), cudaMemcpyHostToDevice) == cudaSuccess;
   if (ok && log->n_offsets > 0)
-    ok = cudaMemcpy(log->d_offsets, log->h_offsets.data(), log->h_offsets.size() * sizeof(float), cudaMemcpyHostToDevice) == cudaSuccess;
+    ok = cudaMemcpy(log->d_offsets.get(), log->h_offsets.data(), log->h_offsets.size() * sizeof(float), cudaMemcpyHostToDevice) == cudaSuccess;
   if (!ok) return fail(nullptr, CS_ERR_CUDA, "cs_scanlog_upload: %s", cudaGetErrorString(cudaGetLastError()));
   log->uploaded = true;
   static std::atomic<uint64_t> g_log_generation{1};
@@ -2204,13 +2252,8 @@ cs_status cs_scanlog_load(int32_t device, const char* path, cs_scanlog** out) {
 
 cs_status cs_scanlog_destroy(cs_scanlog* log) {
   if (!log) return CS_OK;
-  cudaSetDevice(log->device);
-  cudaFree(log->d_hdr);
-  cudaFree(log->d_points);
-  cudaFree(log->d_offsets);
-  cudaFree(log->d_results);
-  cudaGetLastError();
   delete log;
+  cudaGetLastError();
   return CS_OK;
 }
 
@@ -2226,29 +2269,29 @@ cs_status cs_replay(cs_processor* h, const cs_scanlog* log, int32_t first, int32
   const bool timing = (h->cfg.flags & CS_FLAG_TIMING) != 0;
   const bool per_kernel = timing && count == 1;
   if (timing) {
-    cudaEventRecord(h->tm.ev[0], h->stream);
-    if (per_kernel) cudaEventRecord(h->tm.ev[1], h->stream);
+    cudaEventRecord(h->tm.ev[0].get(), h->stream);
+    if (per_kernel) cudaEventRecord(h->tm.ev[1].get(), h->stream);
   }
   for (int i = 0; i < count; i++) {
     const int sidx = first + i;
     CsStepArgs a = update_args(*h, log->n_offsets > 0, log->h_hdr[sidx].n_points);
-    a.hdr = log->d_hdr + sidx;
-    a.points = log->d_points + (size_t)sidx * log->max_points;
-    a.cand = log->n_offsets > 0 ? log->d_offsets + (size_t)sidx * log->n_offsets * 3 : nullptr;
-    a.result = log->d_results + sidx;
-    a.visits_out = reinterpret_cast<long long*>(reinterpret_cast<uint8_t*>(log->d_results + sidx) + offsetof(CsDevResult, visits));
+    a.hdr = log->d_hdr.get() + sidx;
+    a.points = log->d_points.get() + (size_t)sidx * log->max_points;
+    a.cand = log->n_offsets > 0 ? log->d_offsets.get() + (size_t)sidx * log->n_offsets * 3 : nullptr;
+    a.result = log->d_results.get() + sidx;
+    a.visits_out = reinterpret_cast<long long*>(reinterpret_cast<uint8_t*>(log->d_results.get() + sidx) + offsetof(CsDevResult, visits));
     apply_group(h, a);
     // (the next scan's table, if the log has one: its sort is queued behind this scan's draw kernel, see Presort)
-    const float* next_cand = (log->n_offsets > 0 && sidx + 1 < log->n_scans) ? log->d_offsets + (size_t)(sidx + 1) * log->n_offsets * 3 : nullptr;
+    const float* next_cand = (log->n_offsets > 0 && sidx + 1 < log->n_scans) ? log->d_offsets.get() + (size_t)(sidx + 1) * log->n_offsets * 3 : nullptr;
     cs_status st = launch_step(h, a, log->h_hdr[sidx].n_points, rings_hint(h, log->h_max_range[sidx]), per_kernel, 2, CS_PHASE_ALL,
                                next_cand, log->generation);
     if (st != CS_OK) return st;
     h->step.advance(a.do_search);
   }
-  if (timing && !per_kernel) cudaEventRecord(h->tm.ev[4], h->stream);
+  if (timing && !per_kernel) cudaEventRecord(h->tm.ev[4].get(), h->stream);
   if (results && count > 0) {
     static_assert(sizeof(cs_result) == sizeof(CsDevResult), "");
-    CS_CUDA(h, cudaMemcpyAsync(results, log->d_results + first, sizeof(CsDevResult) * count, cudaMemcpyDeviceToHost, h->stream));
+    CS_CUDA(h, cudaMemcpyAsync(results, log->d_results.get() + first, sizeof(CsDevResult) * count, cudaMemcpyDeviceToHost, h->stream));
   }
   // results == NULL: fire and forget — the scans stay queued on the stream (cs_sync / cs_get_pose wait for them)
   if (results || timing) CS_CUDA(h, cudaStreamSynchronize(h->stream));
@@ -2257,7 +2300,7 @@ cs_status cs_replay(cs_processor* h, const cs_scanlog* log, int32_t first, int32
     if (st != CS_OK) return st;
   } else if (timing) {
     float ms = 0;
-    cudaEventElapsedTime(&ms, h->tm.ev[0], h->tm.ev[4]);
+    cudaEventElapsedTime(&ms, h->tm.ev[0].get(), h->tm.ev[4].get());
     h->last_timing = cs_timing{};
     h->last_timing.total_device_ms = ms;
   }
@@ -2277,64 +2320,58 @@ struct cs_batch : CsHost {
   int user_max_points = 0;  // the caller's cfg.max_points: stride of the caller's `points` array (max_points above is the
                             // internal stride of the staging / device blocks, rounded up to even for 16-byte alignment)
   std::vector<CsSession> hs;
-  uint16_t* d_maps = nullptr;
-  int4* d_rays = nullptr;
-  int* d_batch_max = nullptr;
-  unsigned long long* d_prep_words = nullptr;
-  // wedge integration scratch of all sessions (CsSession::w_*)
-  int2* d_w_rk = nullptr;
-  float2* d_w_bkey = nullptr;
-  int* d_w_top = nullptr;
+  DevBuf<uint16_t> d_maps;
   // slab-search scratch of all sessions (CsSession::s2_*): per session 2*cap sorted + cap tmp entries, cap meta + cap acc words
-  float4* d_s2_entries = nullptr;
-  unsigned long long* d_s2_words = nullptr;
+  DevBuf<float4> d_s2_entries;
+  DevBuf<unsigned long long> d_s2_words;
   uint32_t flags = 0;
   // staging: [n headers][n * max_points points][n * n_cand offsets]
   size_t off_points = 0, off_cand = 0, stage_bytes = 0;
-  uint8_t* h_stage = nullptr;
-  uint8_t* d_stage = nullptr;
-  CsDevResult* d_results = nullptr;
-  CsDevResult* h_results = nullptr;  // pinned
+  HostBuf<uint8_t> h_stage;
+  DevBuf<uint8_t> d_stage;
+  DevBuf<CsDevResult> d_results;
+  HostBuf<CsDevResult> h_results;
+  HostBuf<uint8_t> stuck_word;  // CS_FLAG_DEBUG_BOUNDED_SPIN: the block CsHost::h_stuck / d_stuck point into
   // cs_batch_submit / cs_batch_collect: two staging + result slots, so that the host stages step k+1 while step k runs
-  uint8_t* pipe_h_stage[2] = {nullptr, nullptr};
-  uint8_t* pipe_d_stage[2] = {nullptr, nullptr};
-  CsDevResult* pipe_d_results[2] = {nullptr, nullptr};
-  CsDevResult* pipe_h_results[2] = {nullptr, nullptr};
-  cudaEvent_t pipe_done[2] = {nullptr, nullptr};
+  struct PipeSlot {
+    HostBuf<uint8_t> h_stage;
+    DevBuf<uint8_t> d_stage;
+    DevBuf<CsDevResult> d_results;
+    HostBuf<CsDevResult> h_results;
+    Event done;
+  } pipe[2];
   unsigned pipe_submitted = 0, pipe_collected = 0;
   std::vector<float> start_poses;  // n * 3: cfgs[j].start_pose, the Pose of session j after cs_batch_reset (:172)
 
-  // ObstacleMaps (cfg.obstacle_map_size > 0), one per session, all of the geometry `ho` (its pointers unused): session j's
-  // pixels, bitmap and touched counter are the j-th pieces of the three blocks below, described by obst[j] / d_obst[j]
-  CsObstacle ho{};
-  std::vector<CsObstacle> obst;
-  CsObstacle* d_obst = nullptr;
-  int8_t* d_obst_pixels = nullptr;
-  uint32_t* d_obst_no_hit = nullptr;
-  long long* d_obst_touched = nullptr;
+  std::vector<CsObstacle> obst;  // host descriptors of the sessions' ObstacleMaps (CsHost::d_obst)
   std::vector<int> unmapped_obstacle_hits;  // per session, :98; the fill values of the next cs_batch_reset
-  int* d_obst_fill = nullptr;               // ... as the fill kernel reads them
-  unsigned long long* d_obst_sums = nullptr;  // cs_batch_obstacle_checksums
+  DevBuf<int> d_obst_fill;                  // ... as the fill kernel reads them
+  DevBuf<unsigned long long> d_obst_sums;   // cs_batch_obstacle_checksums
+
+  ~cs_batch() {  // the owners release after this, on the batch's device, once its stream has drained
+    cudaSetDevice(device);
+    if (stream) cudaStreamSynchronize(stream);
+  }
 };
 
 namespace {
 // The maps of Reset (:169-170) for every session: HoleMap := 32750, ObstacleMap := the session's UnmappedObstacleHits (with
 // its no-hit bitmap and touched counter cleared).  Queued on the stream; the caller synchronises.
 cs_status batch_fill_maps(cs_batch* b) {
-  cs_fill_kernel<<<148 * 8, 256, 0, b->stream>>>(b->d_maps, b->map_cells * (size_t)b->n, (uint16_t)((CS_TS_OBSTACLE + CS_TS_NO_OBSTACLE) / 2));
+  cs_fill_kernel<<<148 * 8, 256, 0, b->stream>>>(b->d_maps.get(), b->map_cells * (size_t)b->n, (uint16_t)((CS_TS_OBSTACLE + CS_TS_NO_OBSTACLE) / 2));
   b->launches++;
   CS_CUDA(b, cudaGetLastError());
   if (b->d_obst) {
-    CS_CUDA(b, cudaMemcpyAsync(b->d_obst_fill, b->unmapped_obstacle_hits.data(), sizeof(int) * (size_t)b->n, cudaMemcpyHostToDevice,
+    CS_CUDA(b, cudaMemcpyAsync(b->d_obst_fill.get(), b->unmapped_obstacle_hits.data(), sizeof(int) * (size_t)b->n, cudaMemcpyHostToDevice,
                                b->stream));
-    CS_CUDA(b, launch_obstacle_fill(b->stream, b->d_obst, b->d_obst_fill, 0, b->ho, b->n, &b->launches));
+    CS_CUDA(b, launch_obstacle_fill(b->stream, b->d_obst.get(), b->d_obst_fill.get(), 0, b->ho, b->n, &b->launches));
   }
   return CS_OK;
 }
 
 // The host-owned descriptors of all sessions' ObstacleMaps to the device (in stream order).
 cs_status batch_push_obstacles(cs_batch* b) {
-  CS_CUDA(b, cudaMemcpyAsync(b->d_obst, b->obst.data(), sizeof(CsObstacle) * (size_t)b->n, cudaMemcpyHostToDevice, b->stream));
+  CS_CUDA(b, cudaMemcpyAsync(b->d_obst.get(), b->obst.data(), sizeof(CsObstacle) * (size_t)b->n, cudaMemcpyHostToDevice, b->stream));
   return CS_OK;
 }
 }  // namespace
@@ -2348,11 +2385,6 @@ cs_status cs_batch_create(const cs_config* cfgs, int32_t n_sessions, cs_batch** 
     return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "cs_batch_create: bad argument (1..65535 sessions)");
   *out = nullptr;
   const cs_config& c0 = cfgs[0];
-  if (c0.hole_map_size < 8 || c0.hole_map_size > 16384 || !(c0.physical_map_size > 0.f) || c0.iterations_per_thread < 0)
-    return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "cs_batch_create: bad map size / iterations");
-  if (c0.obstacle_map_size < 0 || c0.obstacle_map_size > 16384)
-    return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "obstacle_map_size must be 0 (no ObstacleMap) or in [1, 16384], got %d",
-                c0.obstacle_map_size);
   for (int j = 1; j < n_sessions; j++) {
     const cs_config& c = cfgs[j];
     if (c.hole_map_size != c0.hole_map_size || c.physical_map_size != c0.physical_map_size ||
@@ -2362,14 +2394,10 @@ cs_status cs_batch_create(const cs_config* cfgs, int32_t n_sessions, cs_batch** 
                    "cs_batch_create: session %d differs in map size / iterations / threads / device / max_points / flags / "
                    "obstacle_map_size (only start_pose, sigma_xy, sigma_theta and seed may vary)", j);
   }
-  const int threads = c0.num_search_threads > 0 ? c0.num_search_threads : 1;
-  const long long n_cand = (long long)threads * c0.iterations_per_thread;
-  if (n_cand > (1ll << 26)) return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "too many candidates per scan");
-  const int max_points = c0.max_points > 0 ? c0.max_points : 16384;
-  if (max_points > 65536) return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "max_points must be <= 65536");
-  int ndev = cs_device_count();
-  if (ndev <= 0) return fail(nullptr, CS_ERR_NO_DEVICE, "no CUDA device: this library has no CPU path");
-  if (c0.device < 0 || c0.device >= ndev) return fail(nullptr, CS_ERR_INVALID_ARGUMENT, "device %d out of range", c0.device);
+  long long n_cand = 0;
+  int max_points = 0;
+  const cs_status cst = check_config(c0, &n_cand, &max_points);
+  if (cst != CS_OK) return cst;
 
   cs_batch* b = new cs_batch();
   b->device = c0.device;
@@ -2397,55 +2425,41 @@ cs_status cs_batch_create(const cs_config* cfgs, int32_t n_sessions, cs_batch** 
   if (c0.stream) {
     b->stream = (cudaStream_t)c0.stream;
   } else {
-    CS_CREATE_CUDA(b, cudaStreamCreateWithFlags(&b->stream, cudaStreamNonBlocking));
-    b->own_stream = true;
+    CS_CREATE_CUDA(b, create(b->own_stream));
+    b->stream = b->own_stream.get();
   }
-  CS_CREATE_CUDA(b, cudaMalloc(&b->d_maps, b->map_cells * sizeof(uint16_t) * (size_t)n_sessions));
-  CS_CREATE_CUDA(b, cudaMalloc(&b->d_sess, sizeof(CsSession) * (size_t)n_sessions));
-  CS_CREATE_CUDA(b, cudaMalloc(&b->d_rays, (size_t)b->max_points * sizeof(int4) * (size_t)n_sessions));
-  CS_CREATE_CUDA(b, cudaMalloc(&b->d_batch_max, ((size_t)b->max_points / 32 + 1) * sizeof(int) * (size_t)n_sessions));
-  CS_CREATE_CUDA(b, cudaMalloc(&b->d_prep_words, (size_t)n_sessions * 2 * 16 * sizeof(unsigned long long)));
-  CS_CREATE_CUDA(b, cudaMemset(b->d_prep_words, 0, (size_t)n_sessions * 2 * 16 * sizeof(unsigned long long)));
-  CS_CREATE_CUDA(b, cudaMalloc(&b->d_checksum, sizeof(unsigned long long)));
-  CS_CREATE_CUDA(b, cudaMalloc(&b->d_w_rk, (size_t)b->max_points * sizeof(int2) * (size_t)n_sessions));
-  CS_CREATE_CUDA(b, cudaMalloc(&b->d_w_bkey, ((size_t)b->max_points / 32 + 1) * sizeof(float2) * (size_t)n_sessions));
-  CS_CREATE_CUDA(b, cudaMalloc(&b->d_w_top, (size_t)n_sessions * 3 * wedge_top_words(b->size) * sizeof(int)));
-  CS_CREATE_CUDA(b, cudaMemset(b->d_w_top, 0, (size_t)n_sessions * 3 * wedge_top_words(b->size) * sizeof(int)));
+  CS_CREATE_CUDA(b, alloc(b->d_maps, b->map_cells * (size_t)n_sessions));
+  CS_CREATE_CUDA(b, alloc(b->d_sess, (size_t)n_sessions));
+  for (int j = 0; j < n_sessions; j++) init_session(b->hs[j], *b, cfgs[j], b->d_maps.get() + (size_t)j * b->map_cells);
+  // (a session of a batch has few blocks: one copy of its rays, nothing to spread)
+  CS_CREATE_CUDA(b, alloc_ray_scratch(*b, b->hs.data(), n_sessions, 1, b->max_points, b->max_points / 32 + 1));
+  CS_CREATE_CUDA(b, alloc(b->d_checksum, 1));
   CS_CREATE_CUDA(b, wedge_allow_shared_memory());
   const int min_cand = cs_s2_min_cand(b->flags, n_sessions);
   if (n_sessions > 1 && min_cand > 0 && n_cand + 1 >= min_cand && n_cand + 1 <= CS_SORT_THREADS * CS_SORT_REG) {
     b->s2_cap = n_cand + 1;
     const size_t cap = (size_t)b->s2_cap;
-    CS_CREATE_CUDA(b, cudaMalloc(&b->d_s2_entries, (size_t)n_sessions * 3 * cap * sizeof(float4)));
-    CS_CREATE_CUDA(b, cudaMalloc(&b->d_s2_words, (size_t)n_sessions * 2 * cap * sizeof(unsigned long long)));
-    CS_CREATE_CUDA(b, cudaMemsetAsync(b->d_s2_words, 0, (size_t)n_sessions * 2 * cap * sizeof(unsigned long long), b->stream));
+    CS_CREATE_CUDA(b, alloc(b->d_s2_entries, (size_t)n_sessions * 3 * cap));
+    CS_CREATE_CUDA(b, alloc(b->d_s2_words, (size_t)n_sessions * 2 * cap));
+    CS_CREATE_CUDA(b, cudaMemsetAsync(b->d_s2_words.get(), 0, (size_t)n_sessions * 2 * cap * sizeof(unsigned long long), b->stream));
   }
-  CS_CREATE_CUDA(b, cudaHostAlloc(&b->h_stage, b->stage_bytes, cudaHostAllocDefault));
-  CS_CREATE_CUDA(b, cudaMalloc(&b->d_stage, b->stage_bytes));
-  CS_CREATE_CUDA(b, cudaMalloc(&b->d_results, sizeof(CsDevResult) * (size_t)n_sessions));
-  CS_CREATE_CUDA(b, cudaHostAlloc(&b->h_results, sizeof(CsDevResult) * (size_t)n_sessions, cudaHostAllocDefault));
+  CS_CREATE_CUDA(b, alloc(b->h_stage, b->stage_bytes));
+  CS_CREATE_CUDA(b, alloc(b->d_stage, b->stage_bytes));
+  CS_CREATE_CUDA(b, alloc(b->d_results, (size_t)n_sessions));
+  CS_CREATE_CUDA(b, alloc(b->h_results, (size_t)n_sessions));
   if (b->flags & CS_FLAG_DEBUG_BOUNDED_SPIN) {
-    CS_CREATE_CUDA(b, cudaHostAlloc(&b->h_stuck, 64, cudaHostAllocMapped));
+    CS_CREATE_CUDA(b, alloc(b->stuck_word, 64, cudaHostAllocMapped));
+    b->h_stuck = b->stuck_word.get();
     CS_CREATE_CUDA(b, cudaHostGetDevicePointer((void**)&b->d_stuck, b->h_stuck, 0));
     memset(b->h_stuck, 0, 64);
   }
   for (int j = 0; j < n_sessions; j++) {
     CsSession& s = b->hs[j];
-    init_session(s, *b, cfgs[j], b->d_maps + (size_t)j * b->map_cells);
-    s.rays = b->d_rays + (size_t)j * b->max_points;
-    s.batch_max = b->d_batch_max + (size_t)j * ((size_t)b->max_points / 32 + 1);
-    s.ray_copies = 1;  // a session of a batch has few blocks: nothing to spread
-    s.ray_stride = b->max_points;
-    s.batch_stride = b->max_points / 32 + 1;
-    s.prep_words = b->d_prep_words + (size_t)j * 2 * 16;
-    s.w_rk = b->d_w_rk + (size_t)j * b->max_points;
-    s.w_bkey = b->d_w_bkey + (size_t)j * ((size_t)b->max_points / 32 + 1);
-    s.w_top = b->d_w_top + (size_t)j * 3 * wedge_top_words(b->size);
     if (b->s2_cap > 0) {
       const size_t cap = (size_t)b->s2_cap;
-      s.s2_sorted = b->d_s2_entries + (size_t)j * 3 * cap;
+      s.s2_sorted = b->d_s2_entries.get() + (size_t)j * 3 * cap;
       s.s2_tmp = s.s2_sorted + 2 * cap;
-      s.s2_meta = b->d_s2_words + (size_t)j * 2 * cap;
+      s.s2_meta = b->d_s2_words.get() + (size_t)j * 2 * cap;
       s.s2_acc = s.s2_meta + cap;
       s.s2_cap = b->s2_cap;
     }
@@ -2455,28 +2469,17 @@ cs_status cs_batch_create(const cs_config* cfgs, int32_t n_sessions, cs_batch** 
   for (int j = 0; j < n_sessions; j++)
     for (int k = 0; k < 3; k++) b->start_poses[3 * (size_t)j + k] = cfgs[j].start_pose[k];
   if (c0.obstacle_map_size > 0) {  // :132-133, per session
-    b->ho = obstacle_geometry(c0.obstacle_map_size, c0.physical_map_size);
-    const size_t px = obstacle_pixel_bytes(b->ho), words = obstacle_bitmap_words(b->ho);
-    CS_CREATE_CUDA(b, cudaMalloc(&b->d_obst_pixels, px * (size_t)n_sessions));
-    CS_CREATE_CUDA(b, cudaMalloc(&b->d_obst_no_hit, words * sizeof(uint32_t) * (size_t)n_sessions));
-    CS_CREATE_CUDA(b, cudaMalloc(&b->d_obst_touched, sizeof(long long) * (size_t)n_sessions));
-    CS_CREATE_CUDA(b, cudaMalloc(&b->d_obst, sizeof(CsObstacle) * (size_t)n_sessions));
-    CS_CREATE_CUDA(b, cudaMalloc(&b->d_obst_fill, sizeof(int) * (size_t)n_sessions));
-    CS_CREATE_CUDA(b, cudaMalloc(&b->d_obst_sums, sizeof(unsigned long long) * (size_t)n_sessions));
-    b->obst.assign((size_t)n_sessions, b->ho);
-    for (int j = 0; j < n_sessions; j++) {
-      CsObstacle& o = b->obst[j];
-      o.pixels = b->d_obst_pixels + (size_t)j * px;
-      o.no_hit = b->d_obst_no_hit + (size_t)j * words;
-      o.touched = b->d_obst_touched + j;
-    }
+    b->obst.resize((size_t)n_sessions);
+    CS_CREATE_CUDA(b, alloc_obstacle_maps(*b, b->obst.data(), n_sessions, c0.obstacle_map_size, c0.physical_map_size));
+    CS_CREATE_CUDA(b, alloc(b->d_obst_fill, (size_t)n_sessions));
+    CS_CREATE_CUDA(b, alloc(b->d_obst_sums, (size_t)n_sessions));
     b->unmapped_obstacle_hits.assign((size_t)n_sessions, -5);  // :98
     const cs_status st = batch_push_obstacles(b);
     if (st != CS_OK) return bail(st);
   }
   const cs_status st = batch_fill_maps(b);
   if (st != CS_OK) return bail(st);
-  CS_CREATE_CUDA(b, cudaMemcpyAsync(b->d_sess, b->hs.data(), sizeof(CsSession) * (size_t)n_sessions, cudaMemcpyHostToDevice, b->stream));
+  CS_CREATE_CUDA(b, cudaMemcpyAsync(b->d_sess.get(), b->hs.data(), sizeof(CsSession) * (size_t)n_sessions, cudaMemcpyHostToDevice, b->stream));
   CS_CREATE_CUDA(b, cudaStreamSynchronize(b->stream));
   *out = b;
   return CS_OK;
@@ -2484,41 +2487,8 @@ cs_status cs_batch_create(const cs_config* cfgs, int32_t n_sessions, cs_batch** 
 
 cs_status cs_batch_destroy(cs_batch* b) {
   if (!b) return CS_OK;
-  cudaSetDevice(b->device);
-  if (b->stream) cudaStreamSynchronize(b->stream);
-  cudaFree(b->d_maps);
-  cudaFree(b->d_linear);
-  cudaFree(b->d_sess);
-  cudaFree(b->d_rays);
-  cudaFree(b->d_batch_max);
-  cudaFree(b->d_prep_words);
-  cudaFree(b->d_checksum);
-  cudaFree(b->d_w_rk);
-  cudaFree(b->d_w_bkey);
-  cudaFree(b->d_w_top);
-  cudaFree(b->d_s2_entries);
-  cudaFree(b->d_s2_words);
-  cudaFree(b->d_obst);
-  cudaFree(b->d_obst_pixels);
-  cudaFree(b->d_obst_no_hit);
-  cudaFree(b->d_obst_touched);
-  cudaFree(b->d_obst_fill);
-  cudaFree(b->d_obst_sums);
-  cudaFree(b->d_stage);
-  cudaFree(b->d_results);
-  if (b->h_stage) cudaFreeHost(b->h_stage);
-  if (b->h_results) cudaFreeHost(b->h_results);
-  if (b->h_stuck) cudaFreeHost(b->h_stuck);
-  for (int i = 0; i < 2; i++) {
-    cudaFree(b->pipe_d_stage[i]);
-    cudaFree(b->pipe_d_results[i]);
-    if (b->pipe_h_stage[i]) cudaFreeHost(b->pipe_h_stage[i]);
-    if (b->pipe_h_results[i]) cudaFreeHost(b->pipe_h_results[i]);
-    if (b->pipe_done[i]) cudaEventDestroy(b->pipe_done[i]);
-  }
-  if (b->own_stream && b->stream) cudaStreamDestroy(b->stream);
+  delete b;  // ~cs_batch drains the stream; then every owner releases
   cudaGetLastError();
-  delete b;
   return CS_OK;
 }
 
@@ -2534,9 +2504,9 @@ cs_status cs_batch_set_params(cs_batch* b, int32_t session, int32_t quality, flo
   for (int j = (session < 0 ? 0 : session); j < (session < 0 ? b->n : session + 1); j++) {
     b->hs[j].quality = quality;
     b->hs[j].hole_width = hole_width;
-    CS_CUDA(b, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(b->d_sess + j) + offsetof(CsSession, quality), &b->hs[j].quality,
+    CS_CUDA(b, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(b->d_sess.get() + j) + offsetof(CsSession, quality), &b->hs[j].quality,
                                 sizeof(int), cudaMemcpyHostToDevice, b->stream));
-    CS_CUDA(b, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(b->d_sess + j) + offsetof(CsSession, hole_width), &b->hs[j].hole_width,
+    CS_CUDA(b, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(b->d_sess.get() + j) + offsetof(CsSession, hole_width), &b->hs[j].hole_width,
                                 sizeof(float), cudaMemcpyHostToDevice, b->stream));
   }
   CS_CUDA(b, cudaStreamSynchronize(b->stream));
@@ -2559,7 +2529,7 @@ namespace {
 // does for one processor): one launch of each obstacle kernel for all sessions.  Nothing without ObstacleMaps or points.
 cs_status batch_obstacle_update(cs_batch* b, const CsStepArgs& a, int n_points) {
   if (!b->d_obst || n_points <= 0) return CS_OK;
-  CS_CUDA(b, launch_obstacle_update(b->stream, b->d_sess, b->d_obst, b->ho, a, n_points, b->n, device_sm_count(b->device), &b->launches));
+  CS_CUDA(b, launch_obstacle_update(b->stream, b->d_sess.get(), b->d_obst.get(), b->ho, a, n_points, b->n, device_sm_count(b->device), &b->launches));
   return CS_OK;
 }
 
@@ -2617,12 +2587,12 @@ cs_status cs_batch_update(cs_batch* b, const float* points, const int32_t* n_poi
   if (!points || !n_points || !odometry) return fail(b, CS_ERR_INVALID_ARGUMENT, "cs_batch_update: null argument");
   // the pinned block may still be the source of the previous call's copy
   CS_CUDA(b, cudaStreamSynchronize(b->stream));
-  cs_status st = batch_stage_and_launch(b, b->h_stage, b->d_stage, b->d_results, points, n_points, odometry, cand_offsets);
+  cs_status st = batch_stage_and_launch(b, b->h_stage.get(), b->d_stage.get(), b->d_results.get(), points, n_points, odometry, cand_offsets);
   if (st != CS_OK) return st;
   if (results) {
-    CS_CUDA(b, cudaMemcpyAsync(b->h_results, b->d_results, sizeof(CsDevResult) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
+    CS_CUDA(b, cudaMemcpyAsync(b->h_results.get(), b->d_results.get(), sizeof(CsDevResult) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
     CS_CUDA(b, cudaStreamSynchronize(b->stream));
-    copy_update_results(results, b->h_results, b->n);
+    copy_update_results(results, b->h_results.get(), b->n);
   }
   return CS_OK;
 }
@@ -2638,36 +2608,28 @@ cs_status cs_batch_submit(cs_batch* b, const float* points, const int32_t* n_poi
   if (!points || !n_points || !odometry) return fail(b, CS_ERR_INVALID_ARGUMENT, "cs_batch_submit: null argument");
   if (b->pipe_submitted - b->pipe_collected >= 2u)
     return fail(b, CS_ERR_STATE, "cs_batch_submit: two submitted steps are waiting for cs_batch_collect");
-  const int slot = (int)(b->pipe_submitted & 1u);
-  if (!b->pipe_done[slot]) {  // first use of the slot: all five resources or none (the event, created last, is the guard)
-    uint8_t *hs = nullptr, *ds = nullptr;
-    CsDevResult *dr = nullptr, *hr = nullptr;
-    cudaEvent_t ev = nullptr;
-    cudaError_t e = cudaHostAlloc(&hs, b->stage_bytes, cudaHostAllocDefault);
-    if (e == cudaSuccess) e = cudaMalloc(&ds, b->stage_bytes);
-    if (e == cudaSuccess) e = cudaMalloc(&dr, sizeof(CsDevResult) * (size_t)b->n);
-    if (e == cudaSuccess) e = cudaHostAlloc(&hr, sizeof(CsDevResult) * (size_t)b->n, cudaHostAllocDefault);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+  cs_batch::PipeSlot& p = b->pipe[b->pipe_submitted & 1u];
+  if (!p.done) {  // first use of the slot: all five resources or none (the event, created last, is the guard)
+    cs_batch::PipeSlot fresh;
+    cudaError_t e = alloc(fresh.h_stage, b->stage_bytes);
+    if (e == cudaSuccess) e = alloc(fresh.d_stage, b->stage_bytes);
+    if (e == cudaSuccess) e = alloc(fresh.d_results, (size_t)b->n);
+    if (e == cudaSuccess) e = alloc(fresh.h_results, (size_t)b->n);
+    if (e == cudaSuccess) e = create(fresh.done);
     if (e != cudaSuccess) {
-      if (hs) cudaFreeHost(hs);
-      if (hr) cudaFreeHost(hr);
-      cudaFree(ds);
-      cudaFree(dr);
       cudaGetLastError();
       return fail(b, e == cudaErrorMemoryAllocation ? CS_ERR_OUT_OF_MEMORY : CS_ERR_CUDA, "cs_batch_submit: staging slot: %s",
                    cudaGetErrorString(e));
     }
-    b->pipe_h_stage[slot] = hs; b->pipe_d_stage[slot] = ds; b->pipe_d_results[slot] = dr; b->pipe_h_results[slot] = hr;
-    b->pipe_done[slot] = ev;
+    p = std::move(fresh);
   }
-  // The slot's pinned block was the source of the copy two submits ago; that step has been collected (its pipe_done event,
+  // The slot's pinned block was the source of the copy two submits ago; that step has been collected (its `done` event,
   // recorded after the copy, was waited for), so the block is free.  The device block is protected by stream order.
-  cs_status st = batch_stage_and_launch(b, b->pipe_h_stage[slot], b->pipe_d_stage[slot], b->pipe_d_results[slot], points, n_points,
-                                        odometry, cand_offsets);
+  cs_status st = batch_stage_and_launch(b, p.h_stage.get(), p.d_stage.get(), p.d_results.get(), points, n_points, odometry, cand_offsets);
   if (st != CS_OK) return st;
-  CS_CUDA(b, cudaMemcpyAsync(b->pipe_h_results[slot], b->pipe_d_results[slot], sizeof(CsDevResult) * (size_t)b->n,
-                              cudaMemcpyDeviceToHost, b->stream));
-  CS_CUDA(b, cudaEventRecord(b->pipe_done[slot], b->stream));
+  CS_CUDA(b, cudaMemcpyAsync(p.h_results.get(), p.d_results.get(), sizeof(CsDevResult) * (size_t)b->n, cudaMemcpyDeviceToHost,
+                             b->stream));
+  CS_CUDA(b, cudaEventRecord(p.done.get(), b->stream));
   b->pipe_submitted++;
   return CS_OK;
 }
@@ -2676,9 +2638,9 @@ cs_status cs_batch_collect(cs_batch* b, cs_result* results /* n_sessions records
   NvtxRange nvtx_range("cs_batch_collect");
   CS_CHECK_HANDLE(b);
   if (b->pipe_collected == b->pipe_submitted) return fail(b, CS_ERR_STATE, "cs_batch_collect: nothing was submitted");
-  const int slot = (int)(b->pipe_collected & 1u);
-  CS_CUDA(b, cudaEventSynchronize(b->pipe_done[slot]));
-  if (results) copy_update_results(results, b->pipe_h_results[slot], b->n);
+  const cs_batch::PipeSlot& p = b->pipe[b->pipe_collected & 1u];
+  CS_CUDA(b, cudaEventSynchronize(p.done.get()));
+  if (results) copy_update_results(results, p.h_results.get(), b->n);
   b->pipe_collected++;
   return CS_OK;
 }
@@ -2698,13 +2660,13 @@ cs_status cs_batch_replay(cs_batch* b, const cs_scanlog* log, int32_t first, int
   for (int i = 0; i < count; i++) {
     const int sidx = first + i;
     CsStepArgs a = update_args(*b, log->n_offsets > 0, log->h_hdr[sidx].n_points);
-    a.hdr = log->d_hdr + sidx;
+    a.hdr = log->d_hdr.get() + sidx;
     a.hdr_stride = 0;
-    a.points = log->d_points + (size_t)sidx * log->max_points;
+    a.points = log->d_points.get() + (size_t)sidx * log->max_points;
     a.points_stride = 0;
-    a.cand = log->n_offsets > 0 ? log->d_offsets + (size_t)sidx * log->n_offsets * 3 : nullptr;
+    a.cand = log->n_offsets > 0 ? log->d_offsets.get() + (size_t)sidx * log->n_offsets * 3 : nullptr;
     a.cand_stride = 0;
-    a.result = b->d_results;
+    a.result = b->d_results.get();
     a.result_stride = 1;
     CS_CUDA(b, launch_step_ctx(LaunchCtx(b, b->flags, b->n, b->hs.data()), a, log->h_hdr[sidx].n_points,
                                rings_hint_of(b->size, b->scale, hw, log->h_max_range[sidx]), CS_PHASE_ALL));
@@ -2713,9 +2675,9 @@ cs_status cs_batch_replay(cs_batch* b, const cs_scanlog* log, int32_t first, int
     b->step.advance(a.do_search);
   }
   if (results && count > 0) {
-    CS_CUDA(b, cudaMemcpyAsync(b->h_results, b->d_results, sizeof(CsDevResult) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
+    CS_CUDA(b, cudaMemcpyAsync(b->h_results.get(), b->d_results.get(), sizeof(CsDevResult) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
     CS_CUDA(b, cudaStreamSynchronize(b->stream));
-    copy_update_results(results, b->h_results, b->n);
+    copy_update_results(results, b->h_results.get(), b->n);
   }  // results == NULL: fire and forget (cs_batch_sync waits)
   return CS_OK;
 }
@@ -2730,7 +2692,7 @@ cs_status cs_batch_get_poses(cs_batch* b, float* poses /* n_sessions * 3 */) {
   CS_CHECK_HANDLE(b);
   if (!poses) return fail(b, CS_ERR_INVALID_ARGUMENT, "null poses");
   std::vector<CsSession> tmp((size_t)b->n);
-  CS_CUDA(b, cudaMemcpyAsync(tmp.data(), b->d_sess, sizeof(CsSession) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
+  CS_CUDA(b, cudaMemcpyAsync(tmp.data(), b->d_sess.get(), sizeof(CsSession) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
   CS_CUDA(b, cudaStreamSynchronize(b->stream));
   for (int j = 0; j < b->n; j++)
     for (int k = 0; k < 3; k++) poses[3 * j + k] = tmp[j].state[b->step.parity].pose[k];
@@ -2770,7 +2732,7 @@ cs_status cs_batch_reset(cs_batch* b) {
   b->step.parity = 0;
   b->step.scan_count = 0;
   b->step.update_count = 0;
-  CS_CUDA(b, cudaMemcpyAsync(b->d_sess, b->hs.data(), sizeof(CsSession) * (size_t)b->n, cudaMemcpyHostToDevice, b->stream));
+  CS_CUDA(b, cudaMemcpyAsync(b->d_sess.get(), b->hs.data(), sizeof(CsSession) * (size_t)b->n, cudaMemcpyHostToDevice, b->stream));
   cs_status st = batch_fill_maps(b);  // :169-170
   if (st != CS_OK) return st;
   CS_CUDA(b, cudaStreamSynchronize(b->stream));
@@ -2811,11 +2773,11 @@ cs_status cs_batch_obstacle_checksums(cs_batch* b, uint64_t* checksums /* n_sess
   const int sms = device_sm_count(b->device);
   unsigned blocks = (unsigned)((sms * 8 + b->n - 1) / b->n);  // about eight blocks per SM over all sessions
   if (blocks > (cells + 255) / 256) blocks = (cells + 255) / 256;
-  CS_CUDA(b, cudaMemsetAsync(b->d_obst_sums, 0, sizeof(unsigned long long) * (size_t)b->n, b->stream));
-  cs_obstacle_checksum_kernel<<<dim3(blocks, (unsigned)b->n), 256, 0, b->stream>>>(b->d_obst, b->d_obst_sums);
+  CS_CUDA(b, cudaMemsetAsync(b->d_obst_sums.get(), 0, sizeof(unsigned long long) * (size_t)b->n, b->stream));
+  cs_obstacle_checksum_kernel<<<dim3(blocks, (unsigned)b->n), 256, 0, b->stream>>>(b->d_obst.get(), b->d_obst_sums.get());
   b->launches++;
   CS_CUDA(b, cudaGetLastError());
-  CS_CUDA(b, cudaMemcpyAsync(checksums, b->d_obst_sums, sizeof(unsigned long long) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
+  CS_CUDA(b, cudaMemcpyAsync(checksums, b->d_obst_sums.get(), sizeof(unsigned long long) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
   CS_CUDA(b, cudaStreamSynchronize(b->stream));
   return CS_OK;
 }
@@ -2825,7 +2787,7 @@ cs_status cs_batch_get_obstacle_visits(cs_batch* b, int64_t* touched /* n_sessio
   CS_NEED_OBSTACLE(b);
   if (!touched) return fail(b, CS_ERR_INVALID_ARGUMENT, "null out");
   static_assert(sizeof(long long) == sizeof(int64_t), "touched counters");
-  CS_CUDA(b, cudaMemcpyAsync(touched, b->d_obst_touched, sizeof(long long) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
+  CS_CUDA(b, cudaMemcpyAsync(touched, b->d_obst_touched.get(), sizeof(long long) * (size_t)b->n, cudaMemcpyDeviceToHost, b->stream));
   CS_CUDA(b, cudaStreamSynchronize(b->stream));
   return CS_OK;
 }
@@ -2836,7 +2798,7 @@ cs_status cs_set_flags(cs_processor* h, uint32_t flags) {
   if ((flags & fixed) != (h->cfg.flags & fixed))
     return fail(h, CS_ERR_INVALID_ARGUMENT, "map layout / L2 window / debug rays / search kernel choice are fixed at creation");
   h->cfg.flags = flags;
-  int* dist = (flags & CS_FLAG_KEEP_DISTANCES) ? h->d_distances : nullptr;
+  int* dist = (flags & CS_FLAG_KEEP_DISTANCES) ? h->d_distances.get() : nullptr;
   h->hs.distances = dist;
   return patch_session(h, offsetof(CsSession, distances), &dist, sizeof(int*));
 }
@@ -2874,34 +2836,29 @@ cs_status cs_gather_peak(int32_t device, int64_t cells, int32_t per_thread, int3
   cudaSetDevice(device);
   unsigned pow2 = 1024;
   while ((int64_t)pow2 * 2 <= cells && pow2 < (1u << 30)) pow2 *= 2;
-  uint16_t* table = nullptr;
-  unsigned long long* sink = nullptr;
-  cudaEvent_t e0, e1;
-  if (cudaMalloc(&table, (size_t)pow2 * 2) != cudaSuccess || cudaMalloc(&sink, 8) != cudaSuccess) {
+  DevBuf<uint16_t> table;
+  DevBuf<unsigned long long> sink;
+  Event e0, e1;
+  if (alloc(table, pow2) != cudaSuccess || alloc(sink, 1) != cudaSuccess) {
     cudaGetLastError();
-    cudaFree(table);
     return fail(nullptr, CS_ERR_OUT_OF_MEMORY, "cs_gather_peak: allocation failed");
   }
-  cudaMemset(table, 1, (size_t)pow2 * 2);
-  cudaMemset(sink, 0, 8);
-  cudaEventCreate(&e0);
-  cudaEventCreate(&e1);
+  cudaMemset(table.get(), 1, (size_t)pow2 * 2);
+  cudaMemset(sink.get(), 0, 8);
+  create(e0, cudaEventDefault);
+  create(e1, cudaEventDefault);
   const int blocks = 148 * 8, threads = 256;
   double best = 0;
   for (int r = 0; r < repeats + 2; r++) {
-    cudaEventRecord(e0);
-    cs_gather_peak_kernel<<<blocks, threads>>>(table, pow2 - 1, per_thread, sink);
-    cudaEventRecord(e1);
-    cudaEventSynchronize(e1);
+    cudaEventRecord(e0.get());
+    cs_gather_peak_kernel<<<blocks, threads>>>(table.get(), pow2 - 1, per_thread, sink.get());
+    cudaEventRecord(e1.get());
+    cudaEventSynchronize(e1.get());
     float ms = 0;
-    cudaEventElapsedTime(&ms, e0, e1);
+    cudaEventElapsedTime(&ms, e0.get(), e1.get());
     double rate = (double)blocks * threads * (double)(per_thread / 8 * 8) / (ms * 1e-3);
     if (r >= 2 && rate > best) best = rate;
   }
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
-  cudaFree(table);
-  cudaFree(sink);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return fail(nullptr, CS_ERR_CUDA, "cs_gather_peak: %s", cudaGetErrorString(e));
   *lookups_per_s = best;
@@ -2926,16 +2883,15 @@ cs_status cs_device_sincos(int32_t device, const float* angles, int32_t n, float
   if (!angles || !cos_out || !sin_out || n <= 0) return CS_ERR_INVALID_ARGUMENT;
   if (cs_device_count() <= device) return fail(nullptr, CS_ERR_NO_DEVICE, "no such CUDA device");
   cudaSetDevice(device);
-  float *d_in = nullptr, *d_c = nullptr, *d_s = nullptr;
+  DevBuf<float> d_in, d_c, d_s;
   size_t bytes = (size_t)n * sizeof(float);
-  bool ok = cudaMalloc(&d_in, bytes) == cudaSuccess && cudaMalloc(&d_c, bytes) == cudaSuccess &&
-            cudaMalloc(&d_s, bytes) == cudaSuccess && cudaMemcpy(d_in, angles, bytes, cudaMemcpyHostToDevice) == cudaSuccess;
+  bool ok = alloc(d_in, (size_t)n) == cudaSuccess && alloc(d_c, (size_t)n) == cudaSuccess && alloc(d_s, (size_t)n) == cudaSuccess &&
+            cudaMemcpy(d_in.get(), angles, bytes, cudaMemcpyHostToDevice) == cudaSuccess;
   if (ok) {
-    cs_sincos_kernel<<<(n + 255) / 256, 256>>>(d_in, n, d_c, d_s);
-    ok = cudaMemcpy(cos_out, d_c, bytes, cudaMemcpyDeviceToHost) == cudaSuccess &&
-         cudaMemcpy(sin_out, d_s, bytes, cudaMemcpyDeviceToHost) == cudaSuccess;
+    cs_sincos_kernel<<<(n + 255) / 256, 256>>>(d_in.get(), n, d_c.get(), d_s.get());
+    ok = cudaMemcpy(cos_out, d_c.get(), bytes, cudaMemcpyDeviceToHost) == cudaSuccess &&
+         cudaMemcpy(sin_out, d_s.get(), bytes, cudaMemcpyDeviceToHost) == cudaSuccess;
   }
-  cudaFree(d_in); cudaFree(d_c); cudaFree(d_s);
   if (!ok) return fail(nullptr, CS_ERR_CUDA, "cs_device_sincos: %s", cudaGetErrorString(cudaGetLastError()));
   return CS_OK;
 }
