@@ -173,6 +173,41 @@ namespace CoreSLAM.B200
             // UpdateObstacleMap (:751) ran on the device too when the handle was created with obstacle_map_size > 0
         }
 
+        // ---- relocalisation (no counterpart in the reference: its simulator only offers Reset).  After a restart, or when the
+        // robot was carried elsewhere, find where a scan lies on the current HoleMap, then resume tracking there.
+        /// <summary>The k best poses of the lattice origin + (ix, iy, it) * step (count poses per axis) that are strict local
+        /// minima of (distance, flat index) within +-window steps; best first.  points: ScanCloud.Points of one scan.
+        /// distances (optional): Count[0]*Count[1]*Count[2] values in flat order.  Changes nothing; adopt a hit with ResumeAt.</summary>
+        public CsLatticeHit[] Relocalize(Vector2[] points, Vector3 origin, Vector3 step, int countX, int countY, int countTheta,
+                                         int window, int k, int[] distances = null)
+        {
+            var lattice = new CsLattice();
+            lattice.Origin[0] = origin.X; lattice.Origin[1] = origin.Y; lattice.Origin[2] = origin.Z;
+            lattice.Step[0] = step.X; lattice.Step[1] = step.Y; lattice.Step[2] = step.Z;
+            lattice.Count[0] = countX; lattice.Count[1] = countY; lattice.Count[2] = countTheta;
+            if (distances != null && distances.LongLength != (long)countX * countY * countTheta)
+                throw new ArgumentException("distances needs countX*countY*countTheta entries");
+            var hits = new CsLatticeHit[Native.LatticeMaxHits];
+            int n;
+            fixed (Vector2* p = points)
+            fixed (CsLatticeHit* h = hits)
+            fixed (int* d = distances)
+                Native.Check(Native.cs_relocalize(handle, (float*)p, points.Length, ref lattice, window, k, h, out n, d), handle);
+            return hits.Take(n).ToArray();
+        }
+
+        /// <summary>Continue tracking from `pose` (e.g. the best Relocalize hit, refined): odometryPose is the odometry of the
+        /// scan that pose belongs to.  The next Update searches around pose + (odometry - odometryPose).</summary>
+        public void ResumeAt(Vector3 pose, Vector3 odometryPose)
+        {
+            float* p = stackalloc float[3];
+            float* o = stackalloc float[3];
+            p[0] = pose.X; p[1] = pose.Y; p[2] = pose.Z;
+            o[0] = odometryPose.X; o[1] = odometryPose.Y; o[2] = odometryPose.Z;
+            Native.Check(Native.cs_set_pose(handle, p, o, positionSearchBeginning), handle);
+            Pose = pose;
+        }
+
         // ---- candidate split over the GPUs of a node (no counterpart in the reference: its split is over CPU threads,
         // ParallelMonteCarloSearch :674-710).  One CoreSLAMProcessor per GPU, all fed the same scans in the same order; after
         // AttachGroup every Update evaluates this rank's slice of the candidates and ends on the group's winner.

@@ -47,8 +47,27 @@ namespace CoreSLAM.B200
         public long Visits;
     }
 
+    [StructLayout(LayoutKind.Sequential)]
+    public unsafe struct CsLattice         // cs_lattice, 36 bytes
+    {
+        public fixed float Origin[3];      // pose of lattice point (0,0,0): x, y (m), theta (rad)
+        public fixed float Step[3];        // spacing along x, y (m), theta (rad)
+        public fixed int Count[3];         // points along x, y, theta; each >= 1
+    }
+
+    [StructLayout(LayoutKind.Sequential)]
+    public unsafe struct CsLatticeHit      // cs_lattice_hit, 20 bytes
+    {
+        public fixed float Pose[3];        // the lattice pose as evaluated (theta not normalised)
+        public int Distance;               // CalculateDistanceSISD at that pose
+        public int Index;                  // flat lattice index
+    }
+
     internal static unsafe class Native
     {
+        public const int LatticeMaxPoses = 1 << 28;   // CS_LATTICE_MAX_POSES
+        public const int LatticeMaxHits = 64;         // CS_LATTICE_MAX_HITS
+
         private const string Lib = "coreslam_b200";   // libcoreslam_b200.so / coreslam_b200.dll
 
         [DllImport(Lib)] public static extern int cs_abi_version();
@@ -61,6 +80,7 @@ namespace CoreSLAM.B200
         [DllImport(Lib)] public static extern CsStatus cs_set_hole_width(IntPtr h, float metres);
         [DllImport(Lib)] public static extern CsStatus cs_set_position_search_beginning(IntPtr h, int scans);
         [DllImport(Lib)] public static extern CsStatus cs_get_pose(IntPtr h, float* pose3);
+        [DllImport(Lib)] public static extern CsStatus cs_set_pose(IntPtr h, float* pose3, float* lastOdometry3, int scanCount);
         [DllImport(Lib)] public static extern CsStatus cs_update(IntPtr h, float* pointsXY, int nPoints, float* odometryPose3,
                                                                  float* candOffsets /* T*I*3 or null */, out CsResult result);
         [DllImport(Lib)] public static extern CsStatus cs_update_segments(IntPtr h, float* raysAngleRadius, int* segFirst, float* segPoses3,
@@ -70,6 +90,10 @@ namespace CoreSLAM.B200
         [DllImport(Lib)] public static extern CsStatus cs_search(IntPtr h, float* pointsXY, int nPoints, float* searchPose3,
                                                                  float* candPoses, float* candCosSin, int nCand, uint scanIndex,
                                                                  out CsResult best, int* distances);
+        // relocalisation on the current HoleMap (no reference counterpart): the k best window minima of the distance over a
+        // pose lattice; distances (optional) receives Count[0]*Count[1]*Count[2] values in flat order
+        [DllImport(Lib)] public static extern CsStatus cs_relocalize(IntPtr h, float* pointsXY, int nPoints, ref CsLattice lattice, int window,
+                                                                     int k, CsLatticeHit* hits, out int nHits, int* distances);
         [DllImport(Lib)] public static extern CsStatus cs_integrate(IntPtr h, float* pointsXY, int nPoints, float* pose3,
                                                                     float* poseCosSin, long* visits);
         [DllImport(Lib)] public static extern CsStatus cs_sync(IntPtr h);

@@ -139,6 +139,54 @@ cs_status cs_search(cs_processor* h, const float* points, int32_t n_points, cons
                     const float* cand_poses, const float* cand_cs, int32_t n_cand, uint32_t scan_index,
                     cs_result* best, int32_t* distances);
 
+/* ---- relocalisation on an existing map (no reference counterpart: its simulator only offers Reset) ----------------------
+ * Where is this scan on the handle's map, from a pose nobody knows (a restart, a robot carried elsewhere, lost tracking)?
+ * cs_relocalize evaluates CalculateDistanceSISD (:226-259) at every pose of a regular (x, y, theta) lattice on the device
+ * and returns the best distinct hypotheses.
+ *   Lattice pose  (ix, iy, it) = (origin[0] + (float)ix*step[0], origin[1] + (float)iy*step[1], origin[2] + (float)it*step[2]),
+ *                 each multiply and add one f32 rounding, no FMA (an axis with count 1 is its origin, whatever its step).
+ *                 Flat index (it*count[1] + iy)*count[0] + ix.  Poses may lie partly or wholly off the map; headings may lie
+ *                 outside [-pi, pi].
+ *   Distance      exactly what cs_search returns for the same pose passed as an absolute candidate: px = X*Scale + 0.5f,
+ *                 c = cosf(theta)*Scale with the library's libm-identical cosf/sinf, the sum divided by ALL points;
+ *                 INT32_MAX when no point is in bounds.
+ *   Selection     the key of a pose is (distance, flat index).  A pose is reported when its distance is < INT32_MAX and its
+ *                 key is strictly smaller than the key of every other lattice pose within +-window steps on each of the
+ *                 three axes (the box clipped at the lattice edges; theta does not wrap).  window = 0 is a plain top-k.
+ *                 hits receives at most k of them in ascending key order, *n_hits how many.  The result does not depend
+ *                 on the launch shape.  (The window test reads every pose of the box of a minimum: a window as large as
+ *                 the lattice costs as many reads as the lattice has poses, per minimum.)
+ *   State         reads the HoleMap as it stands after everything already queued on the handle and changes nothing else:
+ *                 map, pose, lastOdometryPose, scanCount, the Philox stream position, a candidate sort queued ahead, the
+ *                 glue table and the CS_FLAG_KEEP_DISTANCES buffer stay as they were.  Either map layout.  Uses the
+ *                 handle's own map only, also when it is attached to a candidate-split group.  Waits for its results.
+ *   distances     optional out: count[0]*count[1]*count[2] values in flat order (one device-to-host copy).
+ *   Errors        CS_ERR_INVALID_ARGUMENT: NULL arguments, n_points <= 0, a count < 1, a non-finite origin, a non-finite or
+ *                 non-positive step on an axis with count > 1, window < 0, k outside 1..CS_LATTICE_MAX_HITS.
+ *                 CS_ERR_CAPACITY: n_points > max_points, or more than CS_LATTICE_MAX_POSES poses (split a bigger lattice,
+ *                 e.g. by heading range).  CS_ERR_OUT_OF_MEMORY: the distance volume (4 B per pose, kept by the handle
+ *                 for later calls) could not be allocated.  The handle stays usable after any of these.
+ * To resume tracking: cs_relocalize with a coarse lattice over the map, finer lattices around its hits, then
+ * cs_set_pose(best, odometry of that scan, PositionSearchBeginning) and Update as usual (INTEGRATION.md). */
+#define CS_LATTICE_MAX_POSES (1 << 28) /* poses per call */
+#define CS_LATTICE_MAX_HITS 64
+
+typedef struct cs_lattice {
+  float origin[3];  /* pose of lattice point (0,0,0): x, y (m), theta (rad) */
+  float step[3];    /* spacing along x, y (m), theta (rad) */
+  int32_t count[3]; /* points along x, y, theta; each >= 1 */
+} cs_lattice;
+
+typedef struct cs_lattice_hit {
+  float pose[3];    /* the lattice pose as evaluated (theta NOT normalised) */
+  int32_t distance; /* CalculateDistanceSISD (:226-259) at that pose */
+  int32_t index;    /* flat lattice index */
+} cs_lattice_hit;
+
+cs_status cs_relocalize(cs_processor* h, const float* points, int32_t n_points, const cs_lattice* lattice, int32_t window,
+                        int32_t k, cs_lattice_hit* hits, int32_t* n_hits,
+                        int32_t* distances /* optional: count[0]*count[1]*count[2] values in flat order */);
+
 /* UpdateHoleMap (:496-534) + DrawLaserRayOnHoleMap (:359-443) + ClipRay (:320-345) for an explicit
  * pose; uses the handle's HoleWidth and Quality.  pose_cs: optional host (cos, sin) of pose[2].
  * Asynchronous: returns after enqueueing; visits (optional) forces a wait for the count.            */

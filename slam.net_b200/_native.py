@@ -102,6 +102,25 @@ class Timing(C.Structure):
     ]
 
 
+class Lattice(C.Structure):
+    _fields_ = [
+        ("origin", C.c_float * 3),
+        ("step", C.c_float * 3),
+        ("count", C.c_int32 * 3),
+    ]
+
+
+class LatticeHit(C.Structure):
+    _fields_ = [
+        ("pose", C.c_float * 3),
+        ("distance", C.c_int32),
+        ("index", C.c_int32),
+    ]
+
+
+LATTICE_MAX_POSES = 1 << 28
+LATTICE_MAX_HITS = 64
+
 FLAG_ROW_MAJOR_MAP = 0x1
 FLAG_TIMING = 0x2
 FLAG_KEEP_DISTANCES = 0x4
@@ -140,6 +159,8 @@ SIGNATURES = {
     "cs_obstacle_map_fill": (C.c_int, [_vp, C.c_int32]),
     "cs_get_obstacle_visits": (C.c_int, [_vp, C.POINTER(C.c_int64)]),
     "cs_search": (C.c_int, [_vp, _fp, C.c_int32, _fp, _fp, _fp, C.c_int32, C.c_uint32, C.POINTER(Result), _ip]),
+    "cs_relocalize": (C.c_int, [_vp, _fp, C.c_int32, C.POINTER(Lattice), C.c_int32, C.c_int32, C.POINTER(LatticeHit), _ip,
+                                _ip]),
     "cs_integrate": (C.c_int, [_vp, _fp, C.c_int32, _fp, _fp, C.POINTER(C.c_int64)]),
     "cs_update": (C.c_int, [_vp, _fp, C.c_int32, _fp, _fp, C.POINTER(Result)]),
     "cs_update_segments": (C.c_int, [_vp, _fp, _ip, _fp, C.c_int32, C.c_int32, _fp, C.POINTER(Result)]),

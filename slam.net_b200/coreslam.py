@@ -112,6 +112,15 @@ class SearchResult:
     visits: int
 
 
+@dataclass
+class LatticeHit:
+    """One hypothesis of cs_relocalize: the lattice pose as evaluated (theta not normalised), its distance
+    (CalculateDistanceSISD, CoreSLAMProcessor.cs:226-259) and its flat lattice index."""
+    pose: np.ndarray
+    distance: int
+    index: int
+
+
 def _result(r: N.Result) -> SearchResult:
     return SearchResult(np.array(list(r.pose), dtype=np.float32), int(r.distance), int(r.index), bool(r.searched),
                         int(r.visits))
@@ -251,6 +260,28 @@ class Processor:
         self._ck(N.lib().cs_search(self._h, _ptr(pts), pts.shape[0], _ptr(sp), _ptr(cp), _ptr(cs), n_cand, scan_index,
                                    C.byref(r), None if d is None else d.ctypes.data_as(C.POINTER(C.c_int32))))
         return _result(r), d
+
+    def relocalize(self, points, origin, step, count, window: int = 0, k: int = 1, want_distances=False):
+        """cs_relocalize: the distance of the scan at every pose of the lattice origin + (ix, iy, it) * step, count =
+        (nx, ny, ntheta) poses, and the k best poses that are strict local minima of (distance, flat index) within
+        +-window lattice steps (include/coreslam_b200.h).  Returns (hits, volume): hits is a list of LatticeHit, best
+        first; volume the (ntheta, ny, nx) int32 distances when want_distances, else None.  The handle's state is
+        left as it was."""
+        pts = _f32(points).reshape(-1, 2)
+        lat = N.Lattice()
+        lat.origin = (C.c_float * 3)(*[float(v) for v in origin])
+        lat.step = (C.c_float * 3)(*[float(v) for v in step])
+        lat.count = (C.c_int32 * 3)(*[int(v) for v in count])
+        hits = (N.LatticeHit * N.LATTICE_MAX_HITS)()
+        n = C.c_int32(0)
+        vol = None
+        if want_distances and min(lat.count) >= 1 and lat.count[0] * lat.count[1] * lat.count[2] <= N.LATTICE_MAX_POSES:
+            vol = np.empty((lat.count[2], lat.count[1], lat.count[0]), dtype=np.int32)  # (else the call fails)
+        self._ck(N.lib().cs_relocalize(self._h, _ptr(pts), pts.shape[0], C.byref(lat), int(window), int(k), hits,
+                                       C.byref(n), None if vol is None else vol.ctypes.data_as(C.POINTER(C.c_int32))))
+        out = [LatticeHit(np.array(list(hits[i].pose), dtype=np.float32), int(hits[i].distance), int(hits[i].index))
+               for i in range(n.value)]
+        return out, vol
 
     def integrate(self, points, pose, pose_cs=None, wait=True) -> int:
         pts = _f32(points).reshape(-1, 2)
@@ -712,6 +743,17 @@ class CoreSLAMProcessor:
             raise ValueError("Sequence contains no elements")  # segments.Last() on an empty list (:719)
         self.LastResult = self._proc.update_segments(segments, candidateOffsets)  # :719-752, cloud (:723) included
         self._pose = self.LastResult.pose
+
+    def Relocalize(self, points, origin, step, count, window: int = 0, k: int = 1, want_distances=False):
+        """No reference counterpart: where this scan cloud (ScanCloud.Points) lies on the current HoleMap, searched over
+        a pose lattice (Processor.relocalize).  Changes nothing; adopt a hit with ResumeAt."""
+        return self._proc.relocalize(points, origin, step, count, window, k, want_distances)
+
+    def ResumeAt(self, pose, odometryPose):
+        """Continue tracking from `pose` (e.g. a Relocalize hit): the next Update searches around
+        pose + (odometry - odometryPose), as after PositionSearchBeginning scans."""
+        self._proc.set_pose(pose, odometryPose, self._psb)
+        self._pose = self._proc.get_pose()
 
     def Dispose(self):
         """:757-773"""

@@ -24,11 +24,13 @@
 #include "../../include/coreslam_b200.h"
 #include "cs_kernels.cuh"
 #include "cs_obstacle.cuh"
+#include "cs_lattice.cuh"
 #include "cs_wedge.cuh"
 
 static_assert(sizeof(CsDevResult) == sizeof(cs_result), "cs_result layout");
 static_assert(sizeof(cs_config) == 72, "cs_config layout (ctypes / P/Invoke mirror it)");
 static_assert(sizeof(CsStepHeader) == 48, "CsStepHeader");
+static_assert(sizeof(cs_lattice) == 36 && sizeof(cs_lattice_hit) == 20, "cs_lattice layout (ctypes / P/Invoke mirror it)");
 
 namespace {
 
@@ -68,6 +70,15 @@ template <typename T> cudaError_t alloc(HostBuf<T>& buf, size_t count, unsigned 
   T* p = nullptr;
   const cudaError_t e = cudaHostAlloc(&p, count * sizeof(T), flags);
   buf.reset(p);
+  return e;
+}
+// a scratch block of at least `count` elements (kept when big enough; its contents do not survive a call)
+template <typename T> cudaError_t grow(DevBuf<T>& buf, size_t& cap, size_t count) {
+  if (cap >= count) return cudaSuccess;
+  buf.reset();
+  cap = 0;
+  const cudaError_t e = alloc(buf, count);
+  if (e == cudaSuccess) cap = count;
   return e;
 }
 cudaError_t create(Stream& s) {
@@ -193,6 +204,13 @@ struct cs_processor : CsHost {
   DevBuf<int8_t> d_obst_snap;
 
   DevBuf<float2> d_cloud;  // scan points computed on the device from raw segments (cs_update_segments)
+
+  // cs_relocalize: the scan (allocated on first use), the distance volume and the top-k lists (both grow on demand)
+  DevBuf<float2> d_lat_points;
+  DevBuf<int> d_lat_volume;
+  size_t lat_volume_cap = 0;
+  DevBuf<unsigned long long> d_lat_lists;
+  size_t lat_lists_cap = 0;
 
   // staging: [hdr 64][points][cand][cand_cs]; segments path: [hdr 64][rays][seg_first][seg_poses][cand]
   size_t stage_bytes = 0;
@@ -1427,6 +1445,99 @@ cs_status cs_search(cs_processor* h, const float* points, int32_t n_points, cons
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
   copy_result(best, reinterpret_cast<const CsDevResult*>(h->h_slot.get()));
   best->visits = 0;
+  return CS_OK;
+}
+
+// -----------------------------------------------------------------------------------------------------
+// Relocalisation (no reference counterpart): the distance of every pose of a lattice (cs_lattice_kernel), then the k best
+// window minima (select + merge kernels, see cs_lattice.cuh).  Reads the map as the stream leaves it; writes only its own
+// scratch.
+cs_status cs_relocalize(cs_processor* h, const float* points, int32_t n_points, const cs_lattice* lattice, int32_t window,
+                        int32_t k, cs_lattice_hit* hits, int32_t* n_hits, int32_t* distances) {
+  NvtxRange nvtx_range("cs_relocalize");
+  CS_CHECK_HANDLE(h);
+  if (!points || !lattice || !hits || !n_hits || n_points <= 0)
+    return fail(h, CS_ERR_INVALID_ARGUMENT, "cs_relocalize: bad argument");
+  if (window < 0) return fail(h, CS_ERR_INVALID_ARGUMENT, "cs_relocalize: window %d < 0", window);
+  if (k < 1 || k > CS_LATTICE_MAX_HITS)
+    return fail(h, CS_ERR_INVALID_ARGUMENT, "cs_relocalize: k %d outside 1..%d", k, CS_LATTICE_MAX_HITS);
+  long long total = 1;
+  for (int a = 0; a < 3; a++) {
+    if (lattice->count[a] < 1) return fail(h, CS_ERR_INVALID_ARGUMENT, "cs_relocalize: count[%d] = %d < 1", a, lattice->count[a]);
+    if (!std::isfinite(lattice->origin[a])) return fail(h, CS_ERR_INVALID_ARGUMENT, "cs_relocalize: origin[%d] not finite", a);
+    if (lattice->count[a] > 1 && !(std::isfinite(lattice->step[a]) && lattice->step[a] > 0.f))
+      return fail(h, CS_ERR_INVALID_ARGUMENT, "cs_relocalize: step[%d] must be finite and > 0", a);
+    total *= lattice->count[a];
+    if (total > CS_LATTICE_MAX_POSES) break;
+  }
+  if (n_points > h->max_points) return fail(h, CS_ERR_CAPACITY, "n_points %d > max_points %d", n_points, h->max_points);
+  if (total > CS_LATTICE_MAX_POSES)
+    return fail(h, CS_ERR_CAPACITY, "cs_relocalize: more than CS_LATTICE_MAX_POSES = %d poses", CS_LATTICE_MAX_POSES);
+
+  const int c0 = lattice->count[0], c1 = lattice->count[1], c2 = lattice->count[2];
+  const int sel_blocks = (int)((total + CS_LAT_THREADS * CS_LAT_SEL_PER - 1) / (CS_LAT_THREADS * CS_LAT_SEL_PER));
+  const size_t list_keys = (size_t)sel_blocks * k, list_keys_b = (size_t)((sel_blocks + CS_LAT_MERGE_LISTS - 1) / CS_LAT_MERGE_LISTS) * k;
+  {
+    cudaError_t e = h->d_lat_points ? cudaSuccess : alloc(h->d_lat_points, (size_t)h->max_points);
+    if (e == cudaSuccess) e = grow(h->d_lat_volume, h->lat_volume_cap, (size_t)total);
+    if (e == cudaSuccess) e = grow(h->d_lat_lists, h->lat_lists_cap, list_keys + list_keys_b);
+    if (e != cudaSuccess) {
+      cudaGetLastError();  // (an allocation failure is not sticky: the handle stays usable)
+      return fail(h, CS_ERR_OUT_OF_MEMORY, "cs_relocalize: scratch allocation failed: %s", cudaGetErrorString(e));
+    }
+  }
+  CS_CUDA(h, cudaMemcpyAsync(h->d_lat_points.get(), points, (size_t)n_points * sizeof(float2), cudaMemcpyHostToDevice, h->stream));
+
+  CsLatticeArgs a{};
+  a.map = h->d_map.get();
+  a.size = h->size;
+  a.pitch_tiles = h->pitch_tiles;
+  a.scale = h->scale;
+  a.points = h->d_lat_points.get();
+  a.n_points = n_points;
+  for (int q = 0; q < 3; q++) {
+    a.origin[q] = lattice->origin[q];
+    a.step[q] = lattice->count[q] > 1 ? lattice->step[q] : 0.f;  // (a single point sits at the origin whatever the step)
+    a.count[q] = lattice->count[q];
+  }
+  a.tiles_x = (c0 + CS_LAT_TILE_X - 1) / CS_LAT_TILE_X;
+  a.tiles_y = (c1 + CS_LAT_TILE_Y - 1) / CS_LAT_TILE_Y;
+  a.volume = h->d_lat_volume.get();
+  const unsigned lat_blocks = (unsigned)((long long)a.tiles_x * a.tiles_y * c2);
+  dispatch_layout(h->tiled, [&](auto T) { cs_lattice_kernel<decltype(T)::value><<<lat_blocks, CS_LAT_THREADS, 0, h->stream>>>(a); });
+  h->launches++;
+  CS_CUDA(h, cudaGetLastError());
+
+  unsigned long long* lists = h->d_lat_lists.get();
+  unsigned long long* other = lists + list_keys;
+  const int win = std::min(window, std::max(c0, std::max(c1, c2)));  // (a wider box is the whole lattice; keeps ix + win in range)
+  cs_lattice_select_kernel<<<(unsigned)sel_blocks, CS_LAT_THREADS, 0, h->stream>>>(a.volume, c0, c1, c2, win, k, lists);
+  h->launches++;
+  CS_CUDA(h, cudaGetLastError());
+  for (int n_lists = sel_blocks; n_lists > 1; n_lists = (n_lists + CS_LAT_MERGE_LISTS - 1) / CS_LAT_MERGE_LISTS) {
+    const unsigned blocks = (unsigned)((n_lists + CS_LAT_MERGE_LISTS - 1) / CS_LAT_MERGE_LISTS);
+    cs_lattice_merge_kernel<<<blocks, CS_LAT_THREADS, 0, h->stream>>>(lists, n_lists, k, other);
+    h->launches++;
+    CS_CUDA(h, cudaGetLastError());
+    std::swap(lists, other);
+  }
+
+  unsigned long long keys[CS_LATTICE_MAX_HITS];
+  CS_CUDA(h, cudaMemcpyAsync(keys, lists, (size_t)k * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+  if (distances)
+    CS_CUDA(h, cudaMemcpyAsync(distances, a.volume, (size_t)total * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+  CS_CUDA(h, cudaStreamSynchronize(h->stream));
+  int n = 0;
+  for (; n < k && keys[n] != ~0ull; n++) {
+    const unsigned idx = (unsigned)keys[n];
+    const int ix = (int)(idx % (unsigned)c0), iy = (int)(idx / (unsigned)c0 % (unsigned)c1), it = (int)(idx / ((unsigned)c0 * (unsigned)c1));
+    hits[n].pose[0] = cs_lattice_coord(a.origin[0], a.step[0], ix);
+    hits[n].pose[1] = cs_lattice_coord(a.origin[1], a.step[1], iy);
+    hits[n].pose[2] = cs_lattice_coord(a.origin[2], a.step[2], it);
+    hits[n].distance = (int32_t)(keys[n] >> 32);
+    hits[n].index = (int32_t)idx;
+  }
+  *n_hits = n;
   return CS_OK;
 }
 
