@@ -196,6 +196,26 @@ namespace CoreSLAM.B200
             return hits.Take(n).ToArray();
         }
 
+        /// <summary>Relocalize's hits for the same lattice, window and k, by branch and bound: most poses of a fine lattice over
+        /// the whole map are never evaluated, and a lattice may hold up to 2^31 - 1 poses.  stats: what the search did.
+        /// Changes nothing; adopt a hit with ResumeAt.</summary>
+        public CsLatticeHit[] RelocalizeBounded(Vector2[] points, Vector3 origin, Vector3 step, int countX, int countY, int countTheta,
+                                                int window, int k, out CsRelocalizeStats stats)
+        {
+            var lattice = new CsLattice();
+            lattice.Origin[0] = origin.X; lattice.Origin[1] = origin.Y; lattice.Origin[2] = origin.Z;
+            lattice.Step[0] = step.X; lattice.Step[1] = step.Y; lattice.Step[2] = step.Z;
+            lattice.Count[0] = countX; lattice.Count[1] = countY; lattice.Count[2] = countTheta;
+            var hits = new CsLatticeHit[Native.LatticeMaxHits];
+            int n;
+            CsRelocalizeStats st;
+            fixed (Vector2* p = points)
+            fixed (CsLatticeHit* h = hits)
+                Native.Check(Native.cs_relocalize_bounded(handle, (float*)p, points.Length, ref lattice, window, k, h, out n, &st), handle);
+            stats = st;
+            return hits.Take(n).ToArray();
+        }
+
         /// <summary>Continue tracking from `pose` (e.g. the best Relocalize hit, refined): odometryPose is the odometry of the
         /// scan that pose belongs to.  The next Update searches around pose + (odometry - odometryPose).</summary>
         public void ResumeAt(Vector3 pose, Vector3 odometryPose)

@@ -63,10 +63,24 @@ namespace CoreSLAM.B200
         public int Index;                  // flat lattice index
     }
 
+    [StructLayout(LayoutKind.Sequential)]
+    public struct CsRelocalizeStats        // cs_relocalize_stats, 40 bytes
+    {
+        public long Poses;                 // count[0]*count[1]*count[2]
+        public long Evaluated;             // poses whose exact distance was computed, summed over the passes
+        public long Bounded;               // (node, level) bounds computed, summed over the passes
+        public int Levels;                 // levels of the descent
+        public int Passes;                 // 1, or more when the upper bound had to be raised
+        public int UpperBound;             // U of the last pass
+        public int Reserved;
+    }
+
     internal static unsafe class Native
     {
         public const int LatticeMaxPoses = 1 << 28;   // CS_LATTICE_MAX_POSES
         public const int LatticeMaxHits = 64;         // CS_LATTICE_MAX_HITS
+        public const int LatticeMaxPosesBounded = 2147483647;  // CS_LATTICE_MAX_POSES_BOUNDED
+        public const int LatticeBoundedMaxNodes = 1 << 20;     // CS_LATTICE_BOUNDED_MAX_NODES
 
         private const string Lib = "coreslam_b200";   // libcoreslam_b200.so / coreslam_b200.dll
 
@@ -94,6 +108,10 @@ namespace CoreSLAM.B200
         // pose lattice; distances (optional) receives Count[0]*Count[1]*Count[2] values in flat order
         [DllImport(Lib)] public static extern CsStatus cs_relocalize(IntPtr h, float* pointsXY, int nPoints, ref CsLattice lattice, int window,
                                                                      int k, CsLatticeHit* hits, out int nHits, int* distances);
+        // the same hits by branch and bound, on lattices of up to LatticeMaxPosesBounded poses; stats optional (null)
+        [DllImport(Lib)] public static extern CsStatus cs_relocalize_bounded(IntPtr h, float* pointsXY, int nPoints, ref CsLattice lattice,
+                                                                             int window, int k, CsLatticeHit* hits, out int nHits,
+                                                                             CsRelocalizeStats* stats);
         [DllImport(Lib)] public static extern CsStatus cs_integrate(IntPtr h, float* pointsXY, int nPoints, float* pose3,
                                                                     float* poseCosSin, long* visits);
         [DllImport(Lib)] public static extern CsStatus cs_sync(IntPtr h);

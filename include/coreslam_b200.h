@@ -166,7 +166,7 @@ cs_status cs_search(cs_processor* h, const float* points, int32_t n_points, cons
  *                 CS_ERR_CAPACITY: n_points > max_points, or more than CS_LATTICE_MAX_POSES poses (split a bigger lattice,
  *                 e.g. by heading range).  CS_ERR_OUT_OF_MEMORY: the distance volume (4 B per pose, kept by the handle
  *                 for later calls) could not be allocated.  The handle stays usable after any of these.
- * To resume tracking: cs_relocalize with a coarse lattice over the map, finer lattices around its hits, then
+ * To resume tracking: cs_relocalize_bounded (below) with a fine lattice over the map, then
  * cs_set_pose(best, odometry of that scan, PositionSearchBeginning) and Update as usual (INTEGRATION.md). */
 #define CS_LATTICE_MAX_POSES (1 << 28) /* poses per call */
 #define CS_LATTICE_MAX_HITS 64
@@ -186,6 +186,48 @@ typedef struct cs_lattice_hit {
 cs_status cs_relocalize(cs_processor* h, const float* points, int32_t n_points, const cs_lattice* lattice, int32_t window,
                         int32_t k, cs_lattice_hit* hits, int32_t* n_hits,
                         int32_t* distances /* optional: count[0]*count[1]*count[2] values in flat order */);
+
+/* cs_relocalize_bounded returns exactly the hits of cs_relocalize (poses, distances, indices and order) for the same
+ * lattice, window and k, and accepts lattices of up to CS_LATTICE_MAX_POSES_BOUNDED poses, so a whole room at a fine
+ * step fits one call.  Most poses are never evaluated: it bounds the distance of blocks of poses from below and prunes
+ * the blocks whose bound exceeds an upper bound U on the k-th hit (branch and bound, DESIGN section 4).
+ *   Descent       the lattice is cut, per heading, into nodes of 2^L x 2^L (x, y) poses.  A node's bound is floor(1024 *
+ *                 sum / n_points) over the points of the minimum of the HoleMap over the cells the point can reach from
+ *                 the node's poses (0 for a point that may leave the map); it is <= the distance of every pose of the node.
+ *                 A node whose bound is > U is dropped; the others are split down to 16 x 8 patches, whose poses are
+ *                 evaluated exactly as in cs_relocalize.  A node whose every point lies wholly off the map is dropped at
+ *                 any U: its poses are all int.MaxValue.
+ *   Exactness     U starts as the k-th smallest exact distance of one pose per top-level node.  A pose that passes the
+ *                 window test with distance <= U is a true window minimum.  When fewer than k pass, U is raised and the
+ *                 descent runs again, at the latest with U = INT32_MAX - 1, which prunes only poses of distance int.MaxValue.
+ *   Cost          besides the descent, every call rebuilds min-window grids of the map: up to 11 row-major copies of the
+ *                 HoleMap (2 B per cell each; 11 x 8 MB for a 2048^2 map), kept by the handle like the other scratch.
+ *   State         as cs_relocalize: reads the map as it stands after the queued work and changes nothing else on the handle;
+ *                 either map layout; the handle's own map, also when it is attached to a group.  Waits for its results.
+ *                 There is no distance-volume output: cs_relocalize returns the volume.
+ *   stats         optional out (below).
+ *   Errors        as cs_relocalize, with CS_LATTICE_MAX_POSES_BOUNDED for the pose limit, and CS_ERR_CAPACITY when more
+ *                 than CS_LATTICE_BOUNDED_MAX_NODES nodes survive one level of the descent (at the last level a node is a
+ *                 32 x 32 tile of one heading, so at most 2^30 poses are evaluated; a uniform map prunes nothing), or when
+ *                 the lattice has more than 2^28 such tiles (count[0] and count[1] far below 32 with very many headings),
+ *                 or count[0] or count[1] > 2^30.
+ *                 The handle stays usable after any of these. */
+#define CS_LATTICE_MAX_POSES_BOUNDED 2147483647 /* poses per cs_relocalize_bounded call: the flat index stays an int32 */
+#define CS_LATTICE_BOUNDED_MAX_NODES (1 << 20)  /* nodes that may survive one level of cs_relocalize_bounded's descent */
+
+typedef struct cs_relocalize_stats {
+  int64_t poses;       /* count[0]*count[1]*count[2] */
+  int64_t evaluated;   /* poses whose exact distance was computed, summed over the passes */
+  int64_t bounded;     /* (node, level) bounds computed, summed over the passes */
+  int32_t levels;      /* levels of the descent */
+  int32_t passes;      /* 1, or more when U had to be raised */
+  int32_t upper_bound; /* U of the last pass */
+  int32_t reserved;
+} cs_relocalize_stats;
+
+cs_status cs_relocalize_bounded(cs_processor* h, const float* points, int32_t n_points, const cs_lattice* lattice,
+                                int32_t window, int32_t k, cs_lattice_hit* hits, int32_t* n_hits,
+                                cs_relocalize_stats* stats /* optional */);
 
 /* UpdateHoleMap (:496-534) + DrawLaserRayOnHoleMap (:359-443) + ClipRay (:320-345) for an explicit
  * pose; uses the handle's HoleWidth and Quality.  pose_cs: optional host (cos, sin) of pose[2].

@@ -118,8 +118,22 @@ class LatticeHit(C.Structure):
     ]
 
 
+class RelocalizeStats(C.Structure):
+    _fields_ = [
+        ("poses", C.c_int64),
+        ("evaluated", C.c_int64),
+        ("bounded", C.c_int64),
+        ("levels", C.c_int32),
+        ("passes", C.c_int32),
+        ("upper_bound", C.c_int32),
+        ("reserved", C.c_int32),
+    ]
+
+
 LATTICE_MAX_POSES = 1 << 28
 LATTICE_MAX_HITS = 64
+LATTICE_MAX_POSES_BOUNDED = 2147483647
+LATTICE_BOUNDED_MAX_NODES = 1 << 20
 
 FLAG_ROW_MAJOR_MAP = 0x1
 FLAG_TIMING = 0x2
@@ -161,6 +175,8 @@ SIGNATURES = {
     "cs_search": (C.c_int, [_vp, _fp, C.c_int32, _fp, _fp, _fp, C.c_int32, C.c_uint32, C.POINTER(Result), _ip]),
     "cs_relocalize": (C.c_int, [_vp, _fp, C.c_int32, C.POINTER(Lattice), C.c_int32, C.c_int32, C.POINTER(LatticeHit), _ip,
                                 _ip]),
+    "cs_relocalize_bounded": (C.c_int, [_vp, _fp, C.c_int32, C.POINTER(Lattice), C.c_int32, C.c_int32, C.POINTER(LatticeHit),
+                                        _ip, C.POINTER(RelocalizeStats)]),
     "cs_integrate": (C.c_int, [_vp, _fp, C.c_int32, _fp, _fp, C.POINTER(C.c_int64)]),
     "cs_update": (C.c_int, [_vp, _fp, C.c_int32, _fp, _fp, C.POINTER(Result)]),
     "cs_update_segments": (C.c_int, [_vp, _fp, _ip, _fp, C.c_int32, C.c_int32, _fp, C.POINTER(Result)]),

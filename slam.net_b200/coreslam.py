@@ -261,6 +261,14 @@ class Processor:
                                    C.byref(r), None if d is None else d.ctypes.data_as(C.POINTER(C.c_int32))))
         return _result(r), d
 
+    @staticmethod
+    def _lattice(origin, step, count) -> N.Lattice:
+        lat = N.Lattice()
+        lat.origin = (C.c_float * 3)(*[float(v) for v in origin])
+        lat.step = (C.c_float * 3)(*[float(v) for v in step])
+        lat.count = (C.c_int32 * 3)(*[int(v) for v in count])
+        return lat
+
     def relocalize(self, points, origin, step, count, window: int = 0, k: int = 1, want_distances=False):
         """cs_relocalize: the distance of the scan at every pose of the lattice origin + (ix, iy, it) * step, count =
         (nx, ny, ntheta) poses, and the k best poses that are strict local minima of (distance, flat index) within
@@ -268,10 +276,7 @@ class Processor:
         first; volume the (ntheta, ny, nx) int32 distances when want_distances, else None.  The handle's state is
         left as it was."""
         pts = _f32(points).reshape(-1, 2)
-        lat = N.Lattice()
-        lat.origin = (C.c_float * 3)(*[float(v) for v in origin])
-        lat.step = (C.c_float * 3)(*[float(v) for v in step])
-        lat.count = (C.c_int32 * 3)(*[int(v) for v in count])
+        lat = self._lattice(origin, step, count)
         hits = (N.LatticeHit * N.LATTICE_MAX_HITS)()
         n = C.c_int32(0)
         vol = None
@@ -282,6 +287,22 @@ class Processor:
         out = [LatticeHit(np.array(list(hits[i].pose), dtype=np.float32), int(hits[i].distance), int(hits[i].index))
                for i in range(n.value)]
         return out, vol
+
+    def relocalize_bounded(self, points, origin, step, count, window: int = 0, k: int = 1):
+        """cs_relocalize_bounded: the hits of relocalize for the same lattice, window and k, by branch and bound, on
+        lattices of up to LATTICE_MAX_POSES_BOUNDED poses.  Returns (hits, stats): stats is a dict of
+        cs_relocalize_stats (poses, evaluated, bounded, levels, passes, upper_bound).  The handle's state is left as it
+        was."""
+        pts = _f32(points).reshape(-1, 2)
+        lat = self._lattice(origin, step, count)
+        hits = (N.LatticeHit * N.LATTICE_MAX_HITS)()
+        n = C.c_int32(0)
+        st = N.RelocalizeStats()
+        self._ck(N.lib().cs_relocalize_bounded(self._h, _ptr(pts), pts.shape[0], C.byref(lat), int(window), int(k), hits,
+                                               C.byref(n), C.byref(st)))
+        out = [LatticeHit(np.array(list(hits[i].pose), dtype=np.float32), int(hits[i].distance), int(hits[i].index))
+               for i in range(n.value)]
+        return out, {f: int(getattr(st, f)) for f, _ in N.RelocalizeStats._fields_ if f != "reserved"}
 
     def integrate(self, points, pose, pose_cs=None, wait=True) -> int:
         pts = _f32(points).reshape(-1, 2)
@@ -748,6 +769,11 @@ class CoreSLAMProcessor:
         """No reference counterpart: where this scan cloud (ScanCloud.Points) lies on the current HoleMap, searched over
         a pose lattice (Processor.relocalize).  Changes nothing; adopt a hit with ResumeAt."""
         return self._proc.relocalize(points, origin, step, count, window, k, want_distances)
+
+    def RelocalizeBounded(self, points, origin, step, count, window: int = 0, k: int = 1):
+        """Relocalize's hits by branch and bound (Processor.relocalize_bounded), for fine lattices over a whole map.
+        Returns (hits, stats).  Changes nothing; adopt a hit with ResumeAt."""
+        return self._proc.relocalize_bounded(points, origin, step, count, window, k)
 
     def ResumeAt(self, pose, odometryPose):
         """Continue tracking from `pose` (e.g. a Relocalize hit): the next Update searches around

@@ -25,12 +25,14 @@
 #include "cs_kernels.cuh"
 #include "cs_obstacle.cuh"
 #include "cs_lattice.cuh"
+#include "cs_bnb.cuh"
 #include "cs_wedge.cuh"
 
 static_assert(sizeof(CsDevResult) == sizeof(cs_result), "cs_result layout");
 static_assert(sizeof(cs_config) == 72, "cs_config layout (ctypes / P/Invoke mirror it)");
 static_assert(sizeof(CsStepHeader) == 48, "CsStepHeader");
 static_assert(sizeof(cs_lattice) == 36 && sizeof(cs_lattice_hit) == 20, "cs_lattice layout (ctypes / P/Invoke mirror it)");
+static_assert(sizeof(cs_relocalize_stats) == 40, "cs_relocalize_stats layout (ctypes / P/Invoke mirror it)");
 
 namespace {
 
@@ -211,6 +213,17 @@ struct cs_processor : CsHost {
   size_t lat_volume_cap = 0;
   DevBuf<unsigned long long> d_lat_lists;
   size_t lat_lists_cap = 0;
+  // cs_relocalize_bounded (cs_bnb.cuh): the min-window grids, the top-level seeds, two node lists, the per-tile slot index
+  // and its counters; the distances of the evaluated tiles go to d_lat_volume, the top-k lists to d_lat_lists
+  DevBuf<uint16_t> d_bnb_grids;
+  size_t bnb_grids_cap = 0;
+  DevBuf<int> d_bnb_seeds;
+  size_t bnb_seeds_cap = 0;
+  DevBuf<int4> d_bnb_nodes;
+  size_t bnb_nodes_cap = 0;
+  DevBuf<int> d_bnb_slot;
+  size_t bnb_slot_cap = 0;
+  DevBuf<unsigned long long> d_bnb_counters;
 
   // staging: [hdr 64][points][cand][cand_cs]; segments path: [hdr 64][rays][seg_first][seg_poses][cand]
   size_t stage_bytes = 0;
@@ -1452,42 +1465,33 @@ cs_status cs_search(cs_processor* h, const float* points, int32_t n_points, cons
 // Relocalisation (no reference counterpart): the distance of every pose of a lattice (cs_lattice_kernel), then the k best
 // window minima (select + merge kernels, see cs_lattice.cuh).  Reads the map as the stream leaves it; writes only its own
 // scratch.
-cs_status cs_relocalize(cs_processor* h, const float* points, int32_t n_points, const cs_lattice* lattice, int32_t window,
-                        int32_t k, cs_lattice_hit* hits, int32_t* n_hits, int32_t* distances) {
-  NvtxRange nvtx_range("cs_relocalize");
-  CS_CHECK_HANDLE(h);
-  if (!points || !lattice || !hits || !n_hits || n_points <= 0)
-    return fail(h, CS_ERR_INVALID_ARGUMENT, "cs_relocalize: bad argument");
-  if (window < 0) return fail(h, CS_ERR_INVALID_ARGUMENT, "cs_relocalize: window %d < 0", window);
+
+// The argument checks of cs_relocalize and cs_relocalize_bounded; *total: the poses of the lattice (counting stops past
+// max_poses).
+static cs_status check_relocalize(cs_processor* h, const char* name, const float* points, int32_t n_points, const cs_lattice* lattice,
+                                  int32_t window, int32_t k, const cs_lattice_hit* hits, const int32_t* n_hits, long long max_poses,
+                                  const char* max_name, long long* total) {
+  if (!points || !lattice || !hits || !n_hits || n_points <= 0) return fail(h, CS_ERR_INVALID_ARGUMENT, "%s: bad argument", name);
+  if (window < 0) return fail(h, CS_ERR_INVALID_ARGUMENT, "%s: window %d < 0", name, window);
   if (k < 1 || k > CS_LATTICE_MAX_HITS)
-    return fail(h, CS_ERR_INVALID_ARGUMENT, "cs_relocalize: k %d outside 1..%d", k, CS_LATTICE_MAX_HITS);
-  long long total = 1;
+    return fail(h, CS_ERR_INVALID_ARGUMENT, "%s: k %d outside 1..%d", name, k, CS_LATTICE_MAX_HITS);
+  long long t = 1;
   for (int a = 0; a < 3; a++) {
-    if (lattice->count[a] < 1) return fail(h, CS_ERR_INVALID_ARGUMENT, "cs_relocalize: count[%d] = %d < 1", a, lattice->count[a]);
-    if (!std::isfinite(lattice->origin[a])) return fail(h, CS_ERR_INVALID_ARGUMENT, "cs_relocalize: origin[%d] not finite", a);
+    if (lattice->count[a] < 1) return fail(h, CS_ERR_INVALID_ARGUMENT, "%s: count[%d] = %d < 1", name, a, lattice->count[a]);
+    if (!std::isfinite(lattice->origin[a])) return fail(h, CS_ERR_INVALID_ARGUMENT, "%s: origin[%d] not finite", name, a);
     if (lattice->count[a] > 1 && !(std::isfinite(lattice->step[a]) && lattice->step[a] > 0.f))
-      return fail(h, CS_ERR_INVALID_ARGUMENT, "cs_relocalize: step[%d] must be finite and > 0", a);
-    total *= lattice->count[a];
-    if (total > CS_LATTICE_MAX_POSES) break;
+      return fail(h, CS_ERR_INVALID_ARGUMENT, "%s: step[%d] must be finite and > 0", name, a);
+    t *= lattice->count[a];
+    if (t > max_poses) break;
   }
   if (n_points > h->max_points) return fail(h, CS_ERR_CAPACITY, "n_points %d > max_points %d", n_points, h->max_points);
-  if (total > CS_LATTICE_MAX_POSES)
-    return fail(h, CS_ERR_CAPACITY, "cs_relocalize: more than CS_LATTICE_MAX_POSES = %d poses", CS_LATTICE_MAX_POSES);
+  if (t > max_poses) return fail(h, CS_ERR_CAPACITY, "%s: more than %s = %lld poses", name, max_name, max_poses);
+  *total = t;
+  return CS_OK;
+}
 
-  const int c0 = lattice->count[0], c1 = lattice->count[1], c2 = lattice->count[2];
-  const int sel_blocks = (int)((total + CS_LAT_THREADS * CS_LAT_SEL_PER - 1) / (CS_LAT_THREADS * CS_LAT_SEL_PER));
-  const size_t list_keys = (size_t)sel_blocks * k, list_keys_b = (size_t)((sel_blocks + CS_LAT_MERGE_LISTS - 1) / CS_LAT_MERGE_LISTS) * k;
-  {
-    cudaError_t e = h->d_lat_points ? cudaSuccess : alloc(h->d_lat_points, (size_t)h->max_points);
-    if (e == cudaSuccess) e = grow(h->d_lat_volume, h->lat_volume_cap, (size_t)total);
-    if (e == cudaSuccess) e = grow(h->d_lat_lists, h->lat_lists_cap, list_keys + list_keys_b);
-    if (e != cudaSuccess) {
-      cudaGetLastError();  // (an allocation failure is not sticky: the handle stays usable)
-      return fail(h, CS_ERR_OUT_OF_MEMORY, "cs_relocalize: scratch allocation failed: %s", cudaGetErrorString(e));
-    }
-  }
-  CS_CUDA(h, cudaMemcpyAsync(h->d_lat_points.get(), points, (size_t)n_points * sizeof(float2), cudaMemcpyHostToDevice, h->stream));
-
+// cs_lattice_kernel's arguments for the handle's map, the scan in d_lat_points and the lattice (no output set)
+static CsLatticeArgs lattice_args(const cs_processor* h, const cs_lattice* lattice, int32_t n_points) {
   CsLatticeArgs a{};
   a.map = h->d_map.get();
   a.size = h->size;
@@ -1500,8 +1504,69 @@ cs_status cs_relocalize(cs_processor* h, const float* points, int32_t n_points, 
     a.step[q] = lattice->count[q] > 1 ? lattice->step[q] : 0.f;  // (a single point sits at the origin whatever the step)
     a.count[q] = lattice->count[q];
   }
-  a.tiles_x = (c0 + CS_LAT_TILE_X - 1) / CS_LAT_TILE_X;
-  a.tiles_y = (c1 + CS_LAT_TILE_Y - 1) / CS_LAT_TILE_Y;
+  a.tiles_x = (lattice->count[0] - 1) / CS_LAT_TILE_X + 1;
+  a.tiles_y = (lattice->count[1] - 1) / CS_LAT_TILE_Y + 1;
+  return a;
+}
+
+// n_lists sorted lists of k keys at `lists` -> one, by merge kernels ping-ponging with `other`; `lists` ends at the result
+static cs_status merge_lattice_lists(cs_processor* h, unsigned long long*& lists, unsigned long long* other, int n_lists, int k) {
+  for (; n_lists > 1; n_lists = (n_lists + CS_LAT_MERGE_LISTS - 1) / CS_LAT_MERGE_LISTS) {
+    const unsigned blocks = (unsigned)((n_lists + CS_LAT_MERGE_LISTS - 1) / CS_LAT_MERGE_LISTS);
+    cs_lattice_merge_kernel<<<blocks, CS_LAT_THREADS, 0, h->stream>>>(lists, n_lists, k, other);
+    h->launches++;
+    CS_CUDA(h, cudaGetLastError());
+    std::swap(lists, other);
+  }
+  return CS_OK;
+}
+
+// the keys (distance << 32 | flat index, ~0 = none) of a merged list -> hits; returns how many
+static int lattice_hits(const CsLatticeArgs& a, const unsigned long long* keys, int k, cs_lattice_hit* hits) {
+  int n = 0;
+  for (; n < k && keys[n] != ~0ull; n++) {
+    const unsigned idx = (unsigned)keys[n];
+    const unsigned c0 = (unsigned)a.count[0], c1 = (unsigned)a.count[1];
+    const int ix = (int)(idx % c0), iy = (int)(idx / c0 % c1), it = (int)(idx / (c0 * c1));
+    hits[n].pose[0] = cs_lattice_coord(a.origin[0], a.step[0], ix);
+    hits[n].pose[1] = cs_lattice_coord(a.origin[1], a.step[1], iy);
+    hits[n].pose[2] = cs_lattice_coord(a.origin[2], a.step[2], it);
+    hits[n].distance = (int32_t)(keys[n] >> 32);
+    hits[n].index = (int32_t)idx;
+  }
+  return n;
+}
+
+// select-kernel blocks over n poses, and the keys of their lists plus the merge kernels' first output
+static int lattice_sel_blocks(long long n) { return (int)((n + CS_LAT_THREADS * CS_LAT_SEL_PER - 1) / (CS_LAT_THREADS * CS_LAT_SEL_PER)); }
+static size_t lattice_list_keys(int sel_blocks, int k) {
+  return (size_t)sel_blocks * k + (size_t)((sel_blocks + CS_LAT_MERGE_LISTS - 1) / CS_LAT_MERGE_LISTS) * k;
+}
+
+cs_status cs_relocalize(cs_processor* h, const float* points, int32_t n_points, const cs_lattice* lattice, int32_t window,
+                        int32_t k, cs_lattice_hit* hits, int32_t* n_hits, int32_t* distances) {
+  NvtxRange nvtx_range("cs_relocalize");
+  CS_CHECK_HANDLE(h);
+  long long total = 0;
+  if (cs_status st = check_relocalize(h, "cs_relocalize", points, n_points, lattice, window, k, hits, n_hits, CS_LATTICE_MAX_POSES,
+                                      "CS_LATTICE_MAX_POSES", &total))
+    return st;
+
+  const int c0 = lattice->count[0], c1 = lattice->count[1], c2 = lattice->count[2];
+  const int sel_blocks = lattice_sel_blocks(total);
+  const size_t list_keys = (size_t)sel_blocks * k;
+  {
+    cudaError_t e = h->d_lat_points ? cudaSuccess : alloc(h->d_lat_points, (size_t)h->max_points);
+    if (e == cudaSuccess) e = grow(h->d_lat_volume, h->lat_volume_cap, (size_t)total);
+    if (e == cudaSuccess) e = grow(h->d_lat_lists, h->lat_lists_cap, lattice_list_keys(sel_blocks, k));
+    if (e != cudaSuccess) {
+      cudaGetLastError();  // (an allocation failure is not sticky: the handle stays usable)
+      return fail(h, CS_ERR_OUT_OF_MEMORY, "cs_relocalize: scratch allocation failed: %s", cudaGetErrorString(e));
+    }
+  }
+  CS_CUDA(h, cudaMemcpyAsync(h->d_lat_points.get(), points, (size_t)n_points * sizeof(float2), cudaMemcpyHostToDevice, h->stream));
+
+  CsLatticeArgs a = lattice_args(h, lattice, n_points);
   a.volume = h->d_lat_volume.get();
   const unsigned lat_blocks = (unsigned)((long long)a.tiles_x * a.tiles_y * c2);
   dispatch_layout(h->tiled, [&](auto T) { cs_lattice_kernel<decltype(T)::value><<<lat_blocks, CS_LAT_THREADS, 0, h->stream>>>(a); });
@@ -1509,35 +1574,192 @@ cs_status cs_relocalize(cs_processor* h, const float* points, int32_t n_points, 
   CS_CUDA(h, cudaGetLastError());
 
   unsigned long long* lists = h->d_lat_lists.get();
-  unsigned long long* other = lists + list_keys;
   const int win = std::min(window, std::max(c0, std::max(c1, c2)));  // (a wider box is the whole lattice; keeps ix + win in range)
   cs_lattice_select_kernel<<<(unsigned)sel_blocks, CS_LAT_THREADS, 0, h->stream>>>(a.volume, c0, c1, c2, win, k, lists);
   h->launches++;
   CS_CUDA(h, cudaGetLastError());
-  for (int n_lists = sel_blocks; n_lists > 1; n_lists = (n_lists + CS_LAT_MERGE_LISTS - 1) / CS_LAT_MERGE_LISTS) {
-    const unsigned blocks = (unsigned)((n_lists + CS_LAT_MERGE_LISTS - 1) / CS_LAT_MERGE_LISTS);
-    cs_lattice_merge_kernel<<<blocks, CS_LAT_THREADS, 0, h->stream>>>(lists, n_lists, k, other);
-    h->launches++;
-    CS_CUDA(h, cudaGetLastError());
-    std::swap(lists, other);
-  }
+  if (cs_status st = merge_lattice_lists(h, lists, lists + list_keys, sel_blocks, k)) return st;
 
   unsigned long long keys[CS_LATTICE_MAX_HITS];
   CS_CUDA(h, cudaMemcpyAsync(keys, lists, (size_t)k * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
   if (distances)
     CS_CUDA(h, cudaMemcpyAsync(distances, a.volume, (size_t)total * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
   CS_CUDA(h, cudaStreamSynchronize(h->stream));
-  int n = 0;
-  for (; n < k && keys[n] != ~0ull; n++) {
-    const unsigned idx = (unsigned)keys[n];
-    const int ix = (int)(idx % (unsigned)c0), iy = (int)(idx / (unsigned)c0 % (unsigned)c1), it = (int)(idx / ((unsigned)c0 * (unsigned)c1));
-    hits[n].pose[0] = cs_lattice_coord(a.origin[0], a.step[0], ix);
-    hits[n].pose[1] = cs_lattice_coord(a.origin[1], a.step[1], iy);
-    hits[n].pose[2] = cs_lattice_coord(a.origin[2], a.step[2], it);
-    hits[n].distance = (int32_t)(keys[n] >> 32);
-    hits[n].index = (int32_t)idx;
+  *n_hits = lattice_hits(a, keys, k, hits);
+  return CS_OK;
+}
+
+// Branch and bound over the lattice (cs_bnb.cuh, DESIGN section 4): min-window grids of the map, U from one exact pose
+// per top-level node, then per pass a descent from the top level (nodes of up to 128 x 128 poses) to the 16 x 8 patches
+// of 32 x 32 tiles, the exact distances of the surviving tiles and the window test over them.  The host reads the
+// survivors' count after each level (the next launch's size).
+cs_status cs_relocalize_bounded(cs_processor* h, const float* points, int32_t n_points, const cs_lattice* lattice,
+                                int32_t window, int32_t k, cs_lattice_hit* hits, int32_t* n_hits, cs_relocalize_stats* stats) {
+  NvtxRange nvtx_range("cs_relocalize_bounded");
+  CS_CHECK_HANDLE(h);
+  long long total = 0;
+  if (cs_status st = check_relocalize(h, "cs_relocalize_bounded", points, n_points, lattice, window, k, hits, n_hits,
+                                      CS_LATTICE_MAX_POSES_BOUNDED, "CS_LATTICE_MAX_POSES_BOUNDED", &total))
+    return st;
+
+  const int c0 = lattice->count[0], c1 = lattice->count[1], c2 = lattice->count[2];
+  CsLatticeArgs a = lattice_args(h, lattice, n_points);
+  if (c0 > (1 << 30) || c1 > (1 << 30))  // (the last tile's indices must stay ints)
+    return fail(h, CS_ERR_CAPACITY, "cs_relocalize_bounded: count[0] = %d or count[1] = %d > 2^30", c0, c1);
+  const long long n_tiles = (long long)a.tiles_x * a.tiles_y * c2;
+  if (n_tiles > (1ll << 28))
+    return fail(h, CS_ERR_CAPACITY, "cs_relocalize_bounded: %lld tiles of 32 x 32 poses > 2^28 (count[0], count[1] too small for %d headings)",
+                n_tiles, c2);
+  // top level: the smallest power-of-two node (32 .. 128 poses a side) that covers the lattice's x and y, or 128
+  int top = CS_BNB_LEAF_LEVEL;
+  while (top < 7 && (c0 > (1 << top) || c1 > (1 << top))) top++;
+  const int top_x = ((c0 - 1) >> top) + 1, top_y = ((c1 - 1) >> top) + 1;
+  const long long n_top = (long long)top_x * top_y * c2;
+  // grids G_0 .. G_max_grid: windows as wide as the cell span of the top level's children (wider spans bound by 0)
+  const double span = (double)((1 << (top - 1)) - 1) * std::max(a.step[0], a.step[1]) * h->scale + 2.0;
+  int max_grid = 0;
+  while (max_grid < CS_BNB_MAX_GRID && (double)(1 << max_grid) < span + 1.0) max_grid++;
+  const size_t cells = (size_t)h->size * h->size;
+  const size_t node_cap = (size_t)std::min<long long>(n_tiles, CS_LATTICE_BOUNDED_MAX_NODES);
+  const int seed_blocks = lattice_sel_blocks(n_top);
+  {
+    cudaError_t e = h->d_lat_points ? cudaSuccess : alloc(h->d_lat_points, (size_t)h->max_points);
+    if (e == cudaSuccess && !h->d_bnb_counters) e = alloc(h->d_bnb_counters, 4);
+    if (e == cudaSuccess) e = grow(h->d_bnb_grids, h->bnb_grids_cap, (size_t)(max_grid + 1) * cells);
+    if (e == cudaSuccess) e = grow(h->d_bnb_seeds, h->bnb_seeds_cap, (size_t)n_top);
+    if (e == cudaSuccess) e = grow(h->d_bnb_nodes, h->bnb_nodes_cap, 2 * node_cap);
+    if (e == cudaSuccess) e = grow(h->d_bnb_slot, h->bnb_slot_cap, (size_t)n_tiles);
+    if (e == cudaSuccess) e = grow(h->d_lat_lists, h->lat_lists_cap, lattice_list_keys(seed_blocks, k));
+    if (e != cudaSuccess) {
+      cudaGetLastError();  // (an allocation failure is not sticky: the handle stays usable)
+      return fail(h, CS_ERR_OUT_OF_MEMORY, "cs_relocalize_bounded: scratch allocation failed: %s", cudaGetErrorString(e));
+    }
   }
-  *n_hits = n;
+  a.points = h->d_lat_points.get();  // (allocated above on a handle's first relocalisation)
+  CS_CUDA(h, cudaMemcpyAsync(h->d_lat_points.get(), points, (size_t)n_points * sizeof(float2), cudaMemcpyHostToDevice, h->stream));
+
+  // the grids, rebuilt from the map as the stream leaves it
+  uint16_t* grids = h->d_bnb_grids.get();
+  const unsigned grid_blocks = (unsigned)std::min<size_t>((cells + CS_LAT_THREADS - 1) / CS_LAT_THREADS, 148 * 8);
+  dispatch_layout(h->tiled, [&](auto T) {
+    cs_bnb_grid0_kernel<decltype(T)::value><<<grid_blocks, CS_LAT_THREADS, 0, h->stream>>>(h->d_map.get(), h->size, h->pitch_tiles, grids);
+  });
+  h->launches++;
+  CS_CUDA(h, cudaGetLastError());
+  for (int j = 1; j <= max_grid; j++) {
+    cs_bnb_grid_kernel<<<grid_blocks, CS_LAT_THREADS, 0, h->stream>>>(grids + (j - 1) * cells, h->size, 1 << (j - 1), grids + j * cells);
+    h->launches++;
+    CS_CUDA(h, cudaGetLastError());
+  }
+
+  CsBnbArgs b{};
+  b.grids = grids;
+  b.size = h->size;
+  b.max_grid = max_grid;
+  b.scale = h->scale;
+  b.points = a.points;
+  b.n_points = n_points;
+  for (int q = 0; q < 3; q++) b.origin[q] = a.origin[q], b.step[q] = a.step[q], b.count[q] = a.count[q];
+  b.top_x = top_x;
+  b.top_y = top_y;
+  b.counters = h->d_bnb_counters.get();
+
+  // first U: the k-th smallest exact distance of the top-level nodes' first poses (INT32_MAX - 1 when fewer than k are finite)
+  unsigned long long keys[CS_LATTICE_MAX_HITS];
+  {
+    b.level = top;
+    cs_bnb_seed_kernel<<<(unsigned)n_top, CS_LAT_THREADS, 0, h->stream>>>(b, h->d_bnb_seeds.get());
+    h->launches++;
+    CS_CUDA(h, cudaGetLastError());
+    unsigned long long* lists = h->d_lat_lists.get();
+    cs_lattice_select_kernel<<<(unsigned)seed_blocks, CS_LAT_THREADS, 0, h->stream>>>(h->d_bnb_seeds.get(), (int)n_top, 1, 1, 0, k, lists);
+    h->launches++;
+    CS_CUDA(h, cudaGetLastError());
+    if (cs_status st = merge_lattice_lists(h, lists, lists + (size_t)seed_blocks * k, seed_blocks, k)) return st;
+    CS_CUDA(h, cudaMemcpyAsync(keys, lists, (size_t)k * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+    CS_CUDA(h, cudaStreamSynchronize(h->stream));
+  }
+  const int kMaxU = 2147483646;
+  int upper = keys[k - 1] != ~0ull ? (int)(keys[k - 1] >> 32) : kMaxU;
+
+  const int win = std::min(window, std::max(c0, std::max(c1, c2)));  // (as cs_relocalize)
+  cs_relocalize_stats st{};
+  st.poses = total;
+  st.levels = top - CS_BNB_LEAF_LEVEL + 1;
+  int4* node_buf[2] = {h->d_bnb_nodes.get(), h->d_bnb_nodes.get() + node_cap};
+  unsigned long long counters[4];
+  for (;;) {
+    st.passes++;
+    st.upper_bound = upper;
+    b.upper = upper;
+    // descent: level `top` (every node of the lattice) down to the tiles
+    b.in = nullptr;
+    long long n_in = n_top, n_leaves = 0;
+    for (int level = top, flip = 0; n_in > 0; level--, flip ^= 1) {
+      CS_CUDA(h, cudaMemsetAsync(b.counters, 0, 4 * sizeof(unsigned long long), h->stream));
+      b.level = level;
+      b.out = node_buf[flip];
+      b.out_cap = (int)node_cap;
+      if (level == CS_BNB_LEAF_LEVEL) cs_bnb_bound_kernel<true><<<(unsigned)n_in, CS_LAT_THREADS, 0, h->stream>>>(b);
+      else cs_bnb_bound_kernel<false><<<(unsigned)n_in, CS_LAT_THREADS, 0, h->stream>>>(b);
+      h->launches++;
+      CS_CUDA(h, cudaGetLastError());
+      CS_CUDA(h, cudaMemcpyAsync(counters, b.counters, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+      CS_CUDA(h, cudaStreamSynchronize(h->stream));
+      st.bounded += (int64_t)counters[1];
+      st.evaluated += (int64_t)counters[2];
+      if (counters[0] > node_cap)
+        return fail(h, CS_ERR_CAPACITY, "cs_relocalize_bounded: %llu nodes of %d x %d poses survive, more than CS_LATTICE_BOUNDED_MAX_NODES = %d",
+                    counters[0], 1 << (level - 1), 1 << (level - 1), CS_LATTICE_BOUNDED_MAX_NODES);
+      n_in = (long long)counters[0];
+      b.in = node_buf[flip];
+      if (level == CS_BNB_LEAF_LEVEL) {
+        n_leaves = n_in;
+        break;
+      }
+    }
+
+    // the surviving tiles' exact distances, the window test over them and the k best
+    unsigned long long passed = 0;
+    if (n_leaves == 0) {
+      for (int i = 0; i < k; i++) keys[i] = ~0ull;
+    } else {
+      const int sel_blocks = lattice_sel_blocks(n_leaves * CS_LAT_TILE_X * CS_LAT_TILE_Y);
+      {
+        cudaError_t e = grow(h->d_lat_volume, h->lat_volume_cap, (size_t)n_leaves * CS_LAT_TILE_X * CS_LAT_TILE_Y);
+        if (e == cudaSuccess) e = grow(h->d_lat_lists, h->lat_lists_cap, lattice_list_keys(sel_blocks, k));
+        if (e != cudaSuccess) {
+          cudaGetLastError();
+          return fail(h, CS_ERR_OUT_OF_MEMORY, "cs_relocalize_bounded: scratch allocation failed: %s", cudaGetErrorString(e));
+        }
+      }
+      CS_CUDA(h, cudaMemsetAsync(h->d_bnb_slot.get(), 0xff, (size_t)n_tiles * sizeof(int), h->stream));
+      CS_CUDA(h, cudaMemsetAsync(b.counters, 0, 4 * sizeof(unsigned long long), h->stream));
+      a.volume = h->d_lat_volume.get();
+      a.tiles = b.in;
+      a.tile_slot = h->d_bnb_slot.get();
+      dispatch_layout(h->tiled, [&](auto T) {
+        cs_lattice_kernel<decltype(T)::value, true><<<(unsigned)n_leaves, CS_LAT_THREADS, 0, h->stream>>>(a);
+      });
+      h->launches++;
+      CS_CUDA(h, cudaGetLastError());
+      unsigned long long* lists = h->d_lat_lists.get();
+      cs_lattice_select_tiles_kernel<<<(unsigned)sel_blocks, CS_LAT_THREADS, 0, h->stream>>>(
+          a.volume, a.tiles, a.tile_slot, (int)n_leaves, c0, c1, c2, a.tiles_x, a.tiles_y, win, k, upper, b.counters + 3, lists);
+      h->launches++;
+      CS_CUDA(h, cudaGetLastError());
+      if (cs_status s = merge_lattice_lists(h, lists, lists + (size_t)sel_blocks * k, sel_blocks, k)) return s;
+      CS_CUDA(h, cudaMemcpyAsync(keys, lists, (size_t)k * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+      CS_CUDA(h, cudaMemcpyAsync(&passed, b.counters + 3, sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+      CS_CUDA(h, cudaStreamSynchronize(h->stream));
+    }
+    // k true minima with distance <= U are the k best of the lattice; at U = INT32_MAX - 1 nothing finite was pruned
+    if (passed >= (unsigned long long)k || upper == kMaxU) break;
+    // else the k-th candidate found (distance > U) as the next U, and after three passes the last resort
+    upper = (keys[k - 1] != ~0ull && st.passes < 3) ? std::max(upper + 1, (int)(keys[k - 1] >> 32)) : kMaxU;
+  }
+  *n_hits = lattice_hits(a, keys, k, hits);
+  if (stats) *stats = st;
   return CS_OK;
 }
 

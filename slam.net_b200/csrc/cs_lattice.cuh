@@ -2,8 +2,10 @@
 // (CalculateDistanceSISD, CoreSLAM/CoreSLAMProcessor.cs:226-259) at every pose of a regular (x, y, theta) lattice, then
 // the lattice poses that are strict local minima of (distance, flat index) within a window, best first.
 //
-//   cs_lattice_kernel         distance of every lattice pose -> a volume of int32 (flat index (it*count1 + iy)*count0 + ix)
+//   cs_lattice_kernel         distance of every lattice pose -> a volume of int32 (flat index (it*count1 + iy)*count0 + ix);
+//                             or (LIST) of the poses of listed 32 x 32 tiles -> 1024 values per tile (cs_relocalize_bounded)
 //   cs_lattice_select_kernel  window test of every pose; the k best local minima of each block's poses -> one sorted list
+//   cs_lattice_select_tiles_kernel  the same over the listed tiles only (cs_relocalize_bounded, see cs_bnb.cuh)
 //   cs_lattice_merge_kernel   CS_LAT_MERGE_LISTS sorted lists -> one, until one list remains
 // All are plain stream-ordered launches that poll nothing: the state of the handle (map, pose, step chain) is only read.
 //
@@ -35,6 +37,8 @@ struct CsLatticeArgs {
   int count[3];
   int tiles_x, tiles_y;
   int* volume;
+  const int4* tiles;  // LIST: the tiles to evaluate, {it, tile x, tile y, mask of the warp patches to evaluate}
+  int* tile_slot;     // LIST: dense per-tile index of the lattice ((it*tiles_y + tile y)*tiles_x + tile x) -> list position
 };
 
 // pose coordinate of lattice point i along one axis: origin + (float)i * step, two roundings, no FMA
@@ -47,25 +51,50 @@ __host__ __device__ __forceinline__ float cs_lattice_coord(float origin, float s
 #endif
 }
 
-template <bool TILED>
+// The reference's arithmetic of one lookup (:232-244), shared by every kernel that evaluates or bounds lattice distances:
+// the pose x (or y) in map units, the four per-point products and the (int) cast of the cell coordinates, each operation
+// one rounding.  x is non-decreasing in px and y in py (cs_bnb.cuh relies on it).
+__device__ __forceinline__ float cs_lattice_p(float origin, float step, int i, float scale) {
+  return __fadd_rn(__fmul_rn(cs_lattice_coord(origin, step, i), scale), 0.5f);  // :232-233
+}
+__device__ __forceinline__ float4 cs_lattice_products(float c, float s, float2 p) {
+  return make_float4(__fmul_rn(c, p.x), __fmul_rn(s, p.y), __fmul_rn(s, p.x), __fmul_rn(c, p.y));
+}
+__device__ __forceinline__ int cs_lattice_cell_x(float px, float4 q) { return __float2int_rz(fmaxf(__fsub_rn(__fadd_rn(px, q.x), q.y), -2.0f)); }
+__device__ __forceinline__ int cs_lattice_cell_y(float py, float4 q) { return __float2int_rz(fmaxf(__fadd_rn(__fadd_rn(py, q.z), q.w), -2.0f)); }
+
+// One block takes one 32 x 32 tile of poses of one heading: the tile blockIdx.x of the lattice, or with LIST the tile
+// a.tiles[blockIdx.x], whose warps evaluate only the 16 x 8 patches (warp w: x half w & 1, rows 8 * (w >> 1)) set in its
+// mask and write int.MaxValue for the others.  LIST writes the tile's 1024 poses (row-major, 32 per row) at
+// a.volume + 1024 * blockIdx.x and records the slot in a.tile_slot.
+template <bool TILED, bool LIST = false>
 __global__ void __launch_bounds__(CS_LAT_THREADS) cs_lattice_kernel(CsLatticeArgs a) {
   __shared__ float4 s_prod[CS_LAT_CHUNK];  // (c*X, s*Y, s*X, c*Y) of the chunk's points
-  const int tiles_xy = a.tiles_x * a.tiles_y;
-  const int it = (int)(blockIdx.x / (unsigned)tiles_xy);
-  const int tile = (int)(blockIdx.x % (unsigned)tiles_xy);
+  int it, tile_x, tile_y;
+  unsigned mask = 0xffu;
+  if (LIST) {
+    const int4 e = a.tiles[blockIdx.x];
+    it = e.x, tile_x = e.y, tile_y = e.z, mask = (unsigned)e.w;
+    if (threadIdx.x == 0) a.tile_slot[((size_t)it * a.tiles_y + tile_y) * a.tiles_x + tile_x] = (int)blockIdx.x;
+  } else {
+    const int tiles_xy = a.tiles_x * a.tiles_y;
+    it = (int)(blockIdx.x / (unsigned)tiles_xy);
+    const int tile = (int)(blockIdx.x % (unsigned)tiles_xy);
+    tile_x = tile % a.tiles_x, tile_y = tile / a.tiles_x;
+  }
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int ix = (tile % a.tiles_x) * CS_LAT_TILE_X + (warp & 1) * 16 + (lane & 15);
-  const int iy0 = (tile / a.tiles_x) * CS_LAT_TILE_Y + (warp >> 1) * 8 + (lane >> 4);  // + 2j, j < CS_LAT_PY
+  const int ix = tile_x * CS_LAT_TILE_X + (warp & 1) * 16 + (lane & 15);
+  const int iy0 = tile_y * CS_LAT_TILE_Y + (warp >> 1) * 8 + (lane >> 4);  // + 2j, j < CS_LAT_PY
 
   const float theta = cs_lattice_coord(a.origin[2], a.step[2], it);
   const float c = __fmul_rn(cs_cosf(theta), a.scale);  // :234
   const float s = __fmul_rn(cs_sinf(theta), a.scale);  // :235
-  const float px = __fadd_rn(__fmul_rn(cs_lattice_coord(a.origin[0], a.step[0], ix), a.scale), 0.5f);  // :232
+  const float px = cs_lattice_p(a.origin[0], a.step[0], ix, a.scale);  // :232
   float py[CS_LAT_PY];
 #pragma unroll
-  for (int j = 0; j < CS_LAT_PY; j++)
-    py[j] = __fadd_rn(__fmul_rn(cs_lattice_coord(a.origin[1], a.step[1], iy0 + 2 * j), a.scale), 0.5f);  // :233
-  const bool active = ix < a.count[0] && iy0 < a.count[1];
+  for (int j = 0; j < CS_LAT_PY; j++) py[j] = cs_lattice_p(a.origin[1], a.step[1], iy0 + 2 * j, a.scale);  // :233
+  const bool inside = ix < a.count[0] && iy0 < a.count[1];
+  const bool active = inside && ((mask >> warp) & 1u);
 
   const int size = a.size, pitch_tiles = a.pitch_tiles;
   const uint16_t* __restrict__ map = a.map;
@@ -78,8 +107,7 @@ __global__ void __launch_bounds__(CS_LAT_THREADS) cs_lattice_kernel(CsLatticeArg
     const int n = min(CS_LAT_CHUNK, a.n_points - base);
     __syncthreads();
     for (int i = threadIdx.x; i < n; i += CS_LAT_THREADS) {
-      const float2 p = a.points[base + i];
-      s_prod[i] = make_float4(__fmul_rn(c, p.x), __fmul_rn(s, p.y), __fmul_rn(s, p.x), __fmul_rn(c, p.y));
+      s_prod[i] = cs_lattice_products(c, s, a.points[base + i]);
     }
     __syncthreads();
     if (!active) continue;
@@ -87,11 +115,11 @@ __global__ void __launch_bounds__(CS_LAT_THREADS) cs_lattice_kernel(CsLatticeArg
     for (int i = 0; i < n; i++) {
       const float4 q = s_prod[i];
       // :240-241, left-associative, one rounding per operation; the (int) cast + bounds test of cs_search_kernel (:244)
-      const int x = __float2int_rz(fmaxf(__fsub_rn(__fadd_rn(px, q.x), q.y), -2.0f));
+      const int x = cs_lattice_cell_x(px, q);
       const bool xin = (unsigned)x < (unsigned)size;
 #pragma unroll
       for (int j = 0; j < CS_LAT_PY; j++) {
-        const int y = __float2int_rz(fmaxf(__fadd_rn(__fadd_rn(py[j], q.z), q.w), -2.0f));
+        const int y = cs_lattice_cell_y(py[j], q);
         if (xin && (unsigned)y < (unsigned)size) {
           sum[j] += (unsigned)__ldg(map + cs_cell_offset<TILED>(x, y, size, pitch_tiles));  // :246
           in_any |= 1u << j;
@@ -99,14 +127,17 @@ __global__ void __launch_bounds__(CS_LAT_THREADS) cs_lattice_kernel(CsLatticeArg
       }
     }
   }
-  if (!active) return;
+  if (!inside) return;
   const size_t plane = (size_t)it * a.count[1];
 #pragma unroll
   for (int j = 0; j < CS_LAT_PY; j++) {
     const int iy = iy0 + 2 * j;
     if (iy < a.count[1]) {
       const int d = ((in_any >> j) & 1u) ? (int)(((unsigned long long)sum[j] * 1024ull) / (unsigned)a.n_points) : 2147483647;  // :251-258
-      a.volume[(plane + iy) * a.count[0] + ix] = d;
+      if (LIST)
+        a.volume[(size_t)blockIdx.x * (CS_LAT_TILE_X * CS_LAT_TILE_Y) + (iy - tile_y * CS_LAT_TILE_Y) * CS_LAT_TILE_X + (ix - tile_x * CS_LAT_TILE_X)] = d;
+      else
+        a.volume[(plane + iy) * a.count[0] + ix] = d;
     }
   }
 }
@@ -144,11 +175,31 @@ __device__ __forceinline__ void cs_lattice_block_topk(unsigned long long (&key)[
 __device__ __forceinline__ unsigned long long cs_lattice_key(int d, unsigned idx) { return ((unsigned long long)(unsigned)d << 32) | idx; }
 
 // A pose is a candidate when its distance is < int.MaxValue and its key is below the key of every other pose within
-// +-window steps on each axis (the box clipped at the lattice edges, theta not wrapped).  Block b takes the poses
-// [b * CS_LAT_THREADS * CS_LAT_SEL_PER, ...) and writes its k best candidates to lists[b * k ...].
+// +-window steps on each axis (the box clipped at the lattice edges, theta not wrapped).  dist(n, t, y, x) reads the
+// distance of pose n = (t*c1 + y)*c0 + x.
+template <class Dist>
+__device__ __forceinline__ bool cs_lattice_window_min(const Dist& dist, unsigned long long mine, unsigned idx, int ix, int iy, int it,
+                                                      int c0, int c1, int c2, int window) {
+  const int x0 = max(ix - window, 0), x1 = min(ix + window, c0 - 1);
+  const int y0 = max(iy - window, 0), y1 = min(iy + window, c1 - 1);
+  const int t0 = max(it - window, 0), t1 = min(it + window, c2 - 1);
+  bool best = true;
+  for (int t = t0; t <= t1 && best; t++)
+    for (int y = y0; y <= y1 && best; y++) {
+      const unsigned row = ((unsigned)t * (unsigned)c1 + (unsigned)y) * (unsigned)c0;
+      for (int x = x0; x <= x1; x++) {
+        const unsigned n = row + (unsigned)x;
+        if (n != idx && cs_lattice_key(dist(n, t, y, x), n) < mine) { best = false; break; }
+      }
+    }
+  return best;
+}
+
+// Block b takes the poses [b * CS_LAT_THREADS * CS_LAT_SEL_PER, ...) and writes its k best candidates to lists[b * k ...].
 __global__ void __launch_bounds__(CS_LAT_THREADS)
 cs_lattice_select_kernel(const int* __restrict__ volume, int c0, int c1, int c2, int window, int k, unsigned long long* __restrict__ lists) {
   const unsigned total = (unsigned)c0 * (unsigned)c1 * (unsigned)c2;
+  const auto dist = [&](unsigned n, int, int, int) { return __ldg(volume + n); };
   unsigned long long key[CS_LAT_SEL_PER];
 #pragma unroll
   for (int j = 0; j < CS_LAT_SEL_PER; j++) {
@@ -159,20 +210,45 @@ cs_lattice_select_kernel(const int* __restrict__ volume, int c0, int c1, int c2,
     if (d == 2147483647) continue;
     const unsigned long long mine = cs_lattice_key(d, idx);
     const int ix = (int)(idx % (unsigned)c0), iy = (int)(idx / (unsigned)c0 % (unsigned)c1), it = (int)(idx / ((unsigned)c0 * (unsigned)c1));
-    const int x0 = max(ix - window, 0), x1 = min(ix + window, c0 - 1);
-    const int y0 = max(iy - window, 0), y1 = min(iy + window, c1 - 1);
-    const int t0 = max(it - window, 0), t1 = min(it + window, c2 - 1);
-    bool best = true;
-    for (int t = t0; t <= t1 && best; t++)
-      for (int y = y0; y <= y1 && best; y++) {
-        const unsigned row = ((unsigned)t * (unsigned)c1 + (unsigned)y) * (unsigned)c0;
-        for (int x = x0; x <= x1; x++) {
-          const unsigned n = row + (unsigned)x;
-          if (n != idx && cs_lattice_key(__ldg(volume + n), n) < mine) { best = false; break; }
-        }
-      }
-    if (best) key[j] = mine;
+    if (cs_lattice_window_min(dist, mine, idx, ix, iy, it, c0, c1, c2, window)) key[j] = mine;
   }
+  cs_lattice_block_topk(key, k, lists + (size_t)blockIdx.x * k);
+}
+
+// cs_lattice_select_kernel over the poses of the tiles cs_lattice_kernel<., true> evaluated: tile s of `tiles` holds its
+// 1024 distances at buf + 1024 * s, tile_slot maps a tile of the lattice to s (-1: not evaluated).  A pose of a tile
+// that was not evaluated reads int.MaxValue, so it is larger than any candidate's key and is never one itself.  Also
+// counts into *passed the candidates whose distance is <= upper.
+__global__ void __launch_bounds__(CS_LAT_THREADS)
+cs_lattice_select_tiles_kernel(const int* __restrict__ buf, const int4* __restrict__ tiles, const int* __restrict__ tile_slot, int n_tiles,
+                               int c0, int c1, int c2, int tiles_x, int tiles_y, int window, int k, int upper,
+                               unsigned long long* __restrict__ passed, unsigned long long* __restrict__ lists) {
+  constexpr int TILE = CS_LAT_TILE_X * CS_LAT_TILE_Y;
+  const auto dist = [&](unsigned, int t, int y, int x) {
+    const int s = __ldg(tile_slot + ((size_t)t * tiles_y + y / CS_LAT_TILE_Y) * tiles_x + x / CS_LAT_TILE_X);
+    return s < 0 ? 2147483647 : __ldg(buf + (size_t)s * TILE + (y % CS_LAT_TILE_Y) * CS_LAT_TILE_X + x % CS_LAT_TILE_X);
+  };
+  const unsigned total = (unsigned)n_tiles * TILE;
+  unsigned long long key[CS_LAT_SEL_PER];
+  unsigned n_passed = 0;
+#pragma unroll
+  for (int j = 0; j < CS_LAT_SEL_PER; j++) {
+    key[j] = ~0ull;
+    const unsigned p = (blockIdx.x * CS_LAT_SEL_PER + j) * CS_LAT_THREADS + threadIdx.x;
+    if (p >= total) continue;
+    const int4 e = __ldg(tiles + p / TILE);
+    const int ix = e.y * CS_LAT_TILE_X + (int)(p % CS_LAT_TILE_X), iy = e.z * CS_LAT_TILE_Y + (int)(p % TILE / CS_LAT_TILE_X);
+    if (ix >= c0 || iy >= c1) continue;
+    const int d = __ldg(buf + p);
+    if (d == 2147483647) continue;
+    const unsigned idx = ((unsigned)e.x * (unsigned)c1 + (unsigned)iy) * (unsigned)c0 + (unsigned)ix;
+    const unsigned long long mine = cs_lattice_key(d, idx);
+    if (cs_lattice_window_min(dist, mine, idx, ix, iy, e.x, c0, c1, c2, window)) {
+      key[j] = mine;
+      n_passed += d <= upper;
+    }
+  }
+  if (n_passed) atomicAdd(passed, (unsigned long long)n_passed);
   cs_lattice_block_topk(key, k, lists + (size_t)blockIdx.x * k);
 }
 
