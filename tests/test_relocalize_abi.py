@@ -120,11 +120,11 @@ def test_selection_window_larger_than_the_lattice_and_fewer_than_k():
 
 def test_selection_random_volumes_against_the_definition():
     rng = np.random.default_rng(11)
-    for trial in range(6):
-        shape = tuple(int(v) for v in rng.integers(1, 7, 3))
+    for trial in range(9):
+        shape = tuple(int(v) for v in rng.integers(1, 7 if trial < 6 else 13, 3))
         # many ties, at the magnitudes real distances have (sum * 1024 / P of 16-bit cells: up to 2^26)
         vol = (rng.integers(0, 6, shape) * (1 << 24) + rng.integers(0, 2, shape)).astype(np.int32)
         vol[rng.random(shape) < 0.2] = INT_MAX
-        for window in (0, 1, 2):
+        for window in (0, 1, 2, 3, 5):  # (from 3 on the reference takes the box minimum of the keys)
             for k in (1, 8, 64):
                 _check(vol, window, k)
