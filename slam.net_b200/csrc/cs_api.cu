@@ -462,59 +462,16 @@ double max_range_of(const float* points, int n) {
   return std::sqrt((double)m) * 1.000001;  // float rounding of r^2 (2^-24 relative) stays inside the bound
 }
 
-// What a step is launched on: one processor (n_sessions = 1) or a batch of independent sessions
-// (grid.y = n_sessions; every kernel indexes its session by blockIdx.y).
-// Experiment knobs (environment, read once; tools/README.md lists them), e.g. CS_TUNE_SEARCH_WARPS (2/4/8).
-// Unset = the built-in choice.  They change launch shapes only, never results.
+// The test hooks of the bounded polls (CS_FLAG_DEBUG_BOUNDED_SPIN), read from the environment once per process.
 struct Tune {
-  int search_warps = 0;
-  int search2 = 0, s2_points = 0, s2_threads = 0, s2_min_cand = 0, s2_sort_one_block = 0, copy_stream = 0;
-  int w_general = 0, w_blocks = 0, w_prefetch = 0, w_sub = 0, w_prev = 0, w_carveout = 0, s2_carveout = 0;
-  int spin_ms = 0, fault = 0, w_resident = 0, spec = 0, presort = 0;
+  int spin_ms = 0, fault = 0;
   Tune() {
     auto geti = [](const char* name) { const char* v = getenv(name); return v ? atoi(v) : 0; };
-    search_warps = geti("CS_TUNE_SEARCH_WARPS");
-    search2 = geti("CS_TUNE_SEARCH2");          // -1: never use the slab search, 0: built-in rule
-    s2_points = geti("CS_TUNE_S2_POINTS");      // points per cluster
-    s2_threads = geti("CS_TUNE_S2_THREADS");    // candidates per slab
-    s2_sort_one_block = geti("CS_TUNE_S2_SORT_ONE_BLOCK");  // 1: sort generated candidates with one block whenever they fit
-    copy_stream = geti("CS_TUNE_COPY_STREAM");  // -1: cs_update stages its inputs on the main stream
-    s2_min_cand = geti("CS_TUNE_S2_MIN_CAND");  // fewest candidates the slab search is used for
-    w_general = geti("CS_TUNE_W_GENERAL");      // 1: every task of the wedge kernel takes its general path (tests)
-    w_blocks = geti("CS_TUNE_W_BLOCKS");        // blocks of the wedge kernel per session
-    w_prefetch = geti("CS_TUNE_W_PREFETCH");    // -1: no L2 prefetch of the map around the pose
-    w_carveout = geti("CS_TUNE_W_CARVEOUT");    // shared-memory carve-out (percent) of the wedge kernel
-    s2_carveout = geti("CS_TUNE_S2_CARVEOUT");  // ... of the slab-search and sort kernels
-    w_prev = geti("CS_TUNE_W_PREV");            // -1: every scan builds its task table from its own counts
-    w_resident = geti("CS_TUNE_W_RESIDENT");    // 4: one small scan alone also runs the four-blocks-per-SM instance of the wedge kernel
-    presort = geti("CS_TUNE_PRESORT");          // -1: production mode sorts a scan's candidates in front of its search, never ahead
-    spec = geti("CS_TUNE_SPEC");                // -1: no glue table (the publishing thread always computes the glue itself)
-    w_sub = geti("CS_TUNE_W_SUB");              // most warps a task's rings are split over (1, 2, 4, 8)
-    spin_ms = geti("CS_TUNE_SPIN_MS");          // CS_FLAG_DEBUG_BOUNDED_SPIN: milliseconds a device-side poll lasts (default 2000)
-    fault = geti("CS_TUNE_FAULT");              // tests of the bounded polls: 1 = the draw kernel waits for a pose tag nobody publishes
+    spin_ms = geti("CS_TUNE_SPIN_MS");  // milliseconds a device-side poll lasts (default 2000)
+    fault = geti("CS_TUNE_FAULT");      // 1 = the draw kernel waits for a pose tag nobody publishes
   }
 };
 const Tune& tune() { static Tune t; return t; }
-
-cudaError_t wedge_allow_shared_memory() {
-  // Experiment knobs: the shared-memory carve-out the draw and search kernels ask for (percent of the SM's 228 KB).  A
-  // kernel whose carve-out differs from its predecessor's cannot share an SM with it.
-  cudaError_t e = cudaSuccess;
-  if (tune().w_carveout > 0) {
-    e = cudaFuncSetAttribute(cs_wedge_kernel<true, 4>, cudaFuncAttributePreferredSharedMemoryCarveout, tune().w_carveout);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(cs_wedge_kernel<false, 4>, cudaFuncAttributePreferredSharedMemoryCarveout, tune().w_carveout);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(cs_wedge_kernel<true, 3>, cudaFuncAttributePreferredSharedMemoryCarveout, tune().w_carveout);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(cs_wedge_kernel<false, 3>, cudaFuncAttributePreferredSharedMemoryCarveout, tune().w_carveout);
-  }
-  if (e == cudaSuccess && tune().s2_carveout > 0) {
-    e = cudaFuncSetAttribute(cs_search2_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, tune().s2_carveout);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(cs_search2_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, tune().s2_carveout);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(cs_sort_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, tune().s2_carveout);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(cs_sort_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, tune().s2_carveout);
-  }
-  return e;
-}
-
 
 int device_sm_count(int device) {
   static int cache[64] = {0};
@@ -533,7 +490,6 @@ int device_sm_count(int device) {
 // warps on some SMs against 27.7 on average; 4 warps -> 7 blocks = 28).  Bigger blocks win ties (the scan is
 // staged once per block).
 int cs_search_warps(long long cand_count, int n_sessions, int num_sms) {
-  if (tune().search_warps == 2 || tune().search_warps == 4 || tune().search_warps == 8) return tune().search_warps;
   const long long total = cand_count * (long long)n_sessions;
   if (total > (long long)num_sms * 40) return CS_SEARCH_WARPS;  // more than one wave anyway
   int best = CS_SEARCH_WARPS;
@@ -556,9 +512,8 @@ struct S2Plan {
   int points = 0, threads = 0, clusters = 0, slabs = 0;
 };
 int cs_s2_min_cand(uint32_t flags, int n_sessions = 1) {  // fewest candidates (searchPose included) the slab search is used for; 0 = never
-  if ((flags & CS_FLAG_SEARCH_WARP) || tune().search2 < 0) return 0;
+  if (flags & CS_FLAG_SEARCH_WARP) return 0;
   if (flags & CS_FLAG_SEARCH_SLAB) return 1;
-  if (tune().s2_min_cand > 0) return tune().s2_min_cand;
   // a batch fills the machine with its sessions; what the slabs need is enough candidates to amortise a block's set-up
   return n_sessions > 1 ? kS2MinCandBatch : kS2MinCand;
 }
@@ -582,15 +537,11 @@ bool cs_plan_search2(int n_sessions, int s2_cap, int min_cand, long long cand_co
   constexpr double kSetup = 450.0, kLookup = 26.0, kIpcPerWarp = 0.12, kIpcMax = 3.0;
   int best_points = 0, best_threads = 0;
   double best_cost = 0.0;
-  const int p_lo = tune().s2_points > 0 ? tune().s2_points : CS_S2_BATCH;
-  const int p_hi = tune().s2_points > 0 ? tune().s2_points : CS_S2_MAX_POINTS;
-  const int t_lo = tune().s2_threads > 0 ? (tune().s2_threads + 31) / 32 * 32 : 64;
-  const int t_hi = tune().s2_threads > 0 ? (t_lo < max_threads ? t_lo : max_threads) : max_threads;
-  for (int points = p_lo; points <= p_hi && points <= CS_S2_MAX_POINTS; points += 4) {
+  for (int points = CS_S2_BATCH; points <= CS_S2_MAX_POINTS; points += 4) {
     const long long clusters = (n_points + points - 1) / points;
     if (clusters > CS_S2_MAX_CLUSTERS) continue;
     const int batches = ((int)((n_points + clusters - 1) / clusters) + CS_S2_BATCH - 1) / CS_S2_BATCH;  // of the fullest cluster
-    for (int threads = t_hi; threads >= t_lo; threads -= 32) {  // bigger blocks win ties: one cluster's lines shared by more warps
+    for (int threads = max_threads; threads >= 64; threads -= 32) {  // bigger blocks win ties: one cluster's lines shared by more warps
       const long long slabs = (cand_count + threads - 1) / threads;
       if (slabs > 65535) continue;
       const long long blocks = clusters * slabs * n_sessions;
@@ -616,6 +567,8 @@ bool cs_plan_search2(int n_sessions, int s2_cap, int min_cand, long long cand_co
   return true;
 }
 
+// What a step is launched on: one processor (n_sessions = 1) or a batch of independent sessions
+// (grid.y = n_sessions; every kernel indexes its session by blockIdx.y).
 struct LaunchCtx {
   int s2_cap = 0;            // capacity of the slab-search scratch (0: none)
   int s2_min_cand = 0;       // cs_s2_min_cand of the handle
@@ -686,9 +639,9 @@ cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t s
 // histogram kernel's threads) pull the map within reach of the step into L2 beside the sort.
 cudaError_t launch_sort(const LaunchCtx& c, CsStepArgs& a, bool warm) {
   cudaError_t e = cudaSuccess;
-  warm = warm && c.n_sessions == 1 && c.tiled && tune().w_prefetch >= 0 && tune().w_prefetch != 2;
+  warm = warm && c.n_sessions == 1 && c.tiled;
   const bool one_block = a.cand_count <= CS_SORT_THREADS * CS_SORT_REG &&
-                         (a.cand_mode != CS_CAND_PHILOX || a.cand_count <= CS_SORT_THREADS || c.n_sessions > 1 || tune().s2_sort_one_block > 0);
+                         (a.cand_mode != CS_CAND_PHILOX || a.cand_count <= CS_SORT_THREADS || c.n_sessions > 1);
   if (warm) a.w_prefetch = 1;
   if (one_block) {
     e = launch_pdl(a.cand_mode == CS_CAND_PHILOX ? cs_sort_kernel<true> : cs_sort_kernel<false>,
@@ -719,7 +672,7 @@ cudaError_t launch_step_ctx(const LaunchCtx& c, CsStepArgs a, int n_points, int 
   a.w_prefetch = 0;  // the map around the pose goes to L2 ahead of its use (one session alone; batches hide the latency)
   a.diag = c.diag;
   a.diag_rings = c.diag_rings;
-  a.spec = (tune().spec >= 0 && fused && draws && a.step_mode == CS_STEP_UPDATE) ? c.spec : nullptr;
+  a.spec = (fused && draws && a.step_mode == CS_STEP_UPDATE) ? c.spec : nullptr;
   a.stuck_flag = c.stuck_dev;
   a.spin_ns = c.stuck_dev ? (long long)(tune().spin_ms > 0 ? tune().spin_ms : 2000) * 1000000ll : 0;
   if (phases & CS_PHASE_FINISH) {  // a call that publishes a pose takes the next step id: never 0, alternating parity
@@ -738,7 +691,7 @@ cudaError_t launch_step_ctx(const LaunchCtx& c, CsStepArgs a, int n_points, int 
     a.s2_slot = (c.step->s2_toggle ^= 1);
     a.s2_batch = c.n_sessions > 1 ? 1 : 0;
     // (Measured and dropped: letting the candidate sort — the first kernel of the step, one block — prefetch the map around
-    // the search pose: 65 k prefetches from one SM take 40 us.  CS_TUNE_W_PREFETCH=1 still selects it for experiments.)
+    // the search pose: 65 k prefetches from one SM take 40 us.)
     a.s2_map = c.hs->map;
     a.s2_sorted = c.hs->s2_sorted + (size_t)a.s2_slot * c.hs->s2_cap;
     a.s2_tmp = c.hs->s2_tmp;
@@ -801,9 +754,8 @@ cudaError_t launch_step_ctx(const LaunchCtx& c, CsStepArgs a, int n_points, int 
     a.prep_group = group;
     const int nprep = (n_points + group - 1) / group;
     // (one small scan alone: the 80-register instance, three blocks per SM; see cs_wedge_kernel)
-    const bool latency = c.n_sessions == 1 && n_points <= 2048 && tune().w_resident != 4;
+    const bool latency = c.n_sessions == 1 && n_points <= 2048;
     int blocks = c.n_sessions == 1 ? (latency ? 3 : 4) * c.num_sms : 4;
-    if (tune().w_blocks > 0) blocks = tune().w_blocks;
     if (blocks < nprep) blocks = nprep;
     // A rank of a candidate-split group that shares its device with another rank (several handles of one process on one GPU)
     // must not keep a grid of polling blocks resident while its search kernel waits for the other ranks' keys — the ranks
@@ -815,16 +767,13 @@ cudaError_t launch_step_ctx(const LaunchCtx& c, CsStepArgs a, int n_points, int 
       // The previous scan's counts size this scan's wedges (the table is then ready before the pose) where a scan is a latency
       // chain; a big scan is throughput, its wedges are narrow (a few degrees of heading change between scans would
       // overfill some) and it builds the table from its own counts.
-      a.w_prev = (d > 0 && tune().w_prev >= 0 && n_points <= 2048) ? (d + 2) % 3 : -1;
+      a.w_prev = (d > 0 && n_points <= 2048) ? (d + 2) % 3 : -1;
       a.w_zero = (d + 1) % 3;
       if (c.step->w_slot >= 3000) c.step->w_slot -= 2997;  // (keeps d > 0 and d mod 3)
     }
-    a.w_general = tune().w_general > 0 ? 1 : 0;
-    if (a.w_prefetch == 0 && c.n_sessions == 1 && c.tiled && tune().w_prefetch >= 0) a.w_prefetch = 2;
-    // (Measured and left as an experiment knob, CS_TUNE_W_PREFETCH=3: in batches, the preparing thread of a ray prefetching the
-    // tiles along it — cfg5 2.01 -> 2.08 ms per step: the draw tasks of a batch already keep the memory system busy.)
-    if (c.n_sessions > 1 && c.tiled && tune().w_prefetch == 3) a.w_prefetch = 3;
-    a.w_sub_max = tune().w_sub;
+    if (a.w_prefetch == 0 && c.n_sessions == 1 && c.tiled) a.w_prefetch = 2;
+    // (Measured and dropped: in batches, the preparing thread of a ray prefetching the tiles along it — cfg5 2.01 -> 2.08 ms
+    // per step: the draw tasks of a batch already keep the memory system busy.)
     CsStepArgs draw_args = a;
     if (tune().fault == 1 && c.stuck_dev) draw_args.step_id ^= 0x40000000u;  // (fault injection: a pose tag nobody publishes)
     dispatch_layout(c.tiled, [&](auto T) {
@@ -837,7 +786,7 @@ cudaError_t launch_step_ctx(const LaunchCtx& c, CsStepArgs a, int n_points, int 
   // ---- production mode: the next scan's candidate sort, queued in the shadow of this scan's draw kernel (see Presort).  Not
   // under CS_FLAG_TIMING (the events around the stages would count it to the wrong one).
   const bool ahead_table = a.cand_mode == CS_CAND_OFFSETS && c.next_cand != nullptr && c.log_tag != 0 && !a.cand_cs;
-  if (c.presort && tune().presort >= 0 && used_s2 && fused && draws && (a.cand_mode == CS_CAND_PHILOX || ahead_table) && c.n_sessions == 1 &&
+  if (c.presort && used_s2 && fused && draws && (a.cand_mode == CS_CAND_PHILOX || ahead_table) && c.n_sessions == 1 &&
       !c.ev_done) {
     CsStepArgs b = a;
     if (ahead_table) b.cand = c.next_cand;
@@ -931,7 +880,7 @@ cs_status launch_step(cs_processor* h, CsStepArgs a, int n_points, int rings, bo
     CS_CUDA(h, launch_obstacle_update(c.stream, h->d_sess.get(), h->d_obst.get(), h->ho, a, n_points, 1, c.num_sms, &h->launches));
   }
   if (c.ev_done) cudaEventRecord(h->tm.ev[ev_base + 2].get(), h->stream);
-  if (h->copy_stream) CS_CUDA(h, cudaEventRecord(h->ev_stage_free[h->stage_cur].get(), h->stream));  // this step's readers of its staging buffer are enqueued
+  CS_CUDA(h, cudaEventRecord(h->ev_stage_free[h->stage_cur].get(), h->stream));  // this step's readers of its staging buffer are enqueued
   return CS_OK;
 }
 
@@ -1184,7 +1133,6 @@ cs_status cs_create(const cs_config* cfg, cs_processor** out) {
   const int ray_stride = (max_points + 31) / 32 * 32;
   const int batch_stride = (ray_stride / 32 + 31) / 32 * 32;  // whole 128-byte lines per copy
   CS_CREATE_CUDA(h, alloc_ray_scratch(*h, &s, 1, kRayCopies, ray_stride, batch_stride));
-  CS_CREATE_CUDA(h, wedge_allow_shared_memory());
   CS_CREATE_CUDA(h, alloc(h->d_spec, ((size_t)n_cand + 1) * 8));
   CS_CREATE_CUDA(h, cudaMemset(h->d_spec.get(), 0, ((size_t)n_cand + 1) * 8 * sizeof(unsigned long long)));  // (tag 0 is never a step's)
   CS_CREATE_CUDA(h, alloc(h->d_distances, (size_t)n_cand + 1));
@@ -1204,12 +1152,10 @@ cs_status cs_create(const cs_config* cfg, cs_processor** out) {
   CS_CREATE_CUDA(h, alloc(h->d_cloud, (size_t)max_points));
   CS_CREATE_CUDA(h, alloc(h->h_stage, h->stage_bytes));
   CS_CREATE_CUDA(h, alloc(h->d_stage, h->stage_bytes));
-  if (tune().copy_stream >= 0) {
-    CS_CREATE_CUDA(h, alloc(h->d_stage_b, h->stage_bytes));
-    CS_CREATE_CUDA(h, create(h->copy_stream));
-    CS_CREATE_CUDA(h, create(h->ev_copy));
-    for (Event& e : h->ev_stage_free) CS_CREATE_CUDA(h, create(e));
-  }
+  CS_CREATE_CUDA(h, alloc(h->d_stage_b, h->stage_bytes));
+  CS_CREATE_CUDA(h, create(h->copy_stream));
+  CS_CREATE_CUDA(h, create(h->ev_copy));
+  for (Event& e : h->ev_stage_free) CS_CREATE_CUDA(h, create(e));
   CS_CREATE_CUDA(h, alloc(h->h_slot, 128, cudaHostAllocMapped));
   CS_CREATE_CUDA(h, cudaHostGetDevicePointer((void**)&h->d_slot, h->h_slot.get(), 0));
   memset(h->h_slot.get(), 0, 128);
@@ -1879,20 +1825,14 @@ static cs_status stage_update(cs_processor* h, const float* points, int32_t n_po
   if (with_offsets) memcpy(h->h_stage.get() + sp.off_cand, cand_offsets, (size_t)h->n_cand * 12);
 
   if (timing) cudaEventRecord(h->tm.ev[0].get(), h->stream);
-  uint8_t* d_base = h->d_stage.get();
-  if (h->copy_stream) {
-    // run ahead of the stream: copy into the buffer the scan in flight is not reading, behind nothing but that buffer's
-    // last readers (two scans ago); the main stream picks the copy up through its event
-    h->stage_cur = (h->stage_flip ^= 1);
-    d_base = h->stage_cur ? h->d_stage_b.get() : h->d_stage.get();
-    CS_CUDA(h, cudaStreamWaitEvent(h->copy_stream.get(), h->ev_stage_free[h->stage_cur].get(), 0));
-    CS_CUDA(h, cudaMemcpyAsync(d_base, h->h_stage.get(), sp.total, cudaMemcpyHostToDevice, h->copy_stream.get()));
-    CS_CUDA(h, cudaEventRecord(h->ev_copy.get(), h->copy_stream.get()));
-    CS_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_copy.get(), 0));
-  } else {
-    h->stage_cur = 0;
-    CS_CUDA(h, cudaMemcpyAsync(d_base, h->h_stage.get(), sp.total, cudaMemcpyHostToDevice, h->stream));
-  }
+  // run ahead of the stream: copy into the buffer the scan in flight is not reading, behind nothing but that buffer's
+  // last readers (two scans ago); the main stream picks the copy up through its event
+  h->stage_cur = (h->stage_flip ^= 1);
+  uint8_t* d_base = h->stage_cur ? h->d_stage_b.get() : h->d_stage.get();
+  CS_CUDA(h, cudaStreamWaitEvent(h->copy_stream.get(), h->ev_stage_free[h->stage_cur].get(), 0));
+  CS_CUDA(h, cudaMemcpyAsync(d_base, h->h_stage.get(), sp.total, cudaMemcpyHostToDevice, h->copy_stream.get()));
+  CS_CUDA(h, cudaEventRecord(h->ev_copy.get(), h->copy_stream.get()));
+  CS_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_copy.get(), 0));
   if (seg && n_points > 0) {  // ScanSegmentsToCloud (:723) on the device; the step's first kernel must not start before it is complete
     cs_status cst = launch_cloud(h, d_base + sp.off_points, d_base + off_first, d_base + off_poses, n_points,
                                  seg->n_segments, odometry_pose);
@@ -2358,7 +2298,7 @@ cs_status cs_get_search_plan(cs_processor* h, int32_t n_points, int32_t n_cand, 
   const int sms = device_sm_count(h->device);
   S2Plan s2;
   // (as cs_update launches it: a block carries the glue table's service warp beside the slab's threads)
-  const int cap = (tune().spec >= 0 && h->d_spec) ? CS_S2_MAX_THREADS - 32 : CS_S2_MAX_THREADS;
+  const int cap = h->d_spec ? CS_S2_MAX_THREADS - 32 : CS_S2_MAX_THREADS;
   if (cs_plan_search2(1, h->s2_cap, cs_s2_min_cand(h->cfg.flags), (long long)n_cand + 1, n_points, sms, &s2, cap)) {
     plan[0] = 1; plan[1] = s2.clusters; plan[2] = s2.slabs; plan[3] = s2.threads; plan[4] = s2.points;
   } else {
@@ -2767,7 +2707,6 @@ cs_status cs_batch_create(const cs_config* cfgs, int32_t n_sessions, cs_batch** 
   // (a session of a batch has few blocks: one copy of its rays, nothing to spread)
   CS_CREATE_CUDA(b, alloc_ray_scratch(*b, b->hs.data(), n_sessions, 1, b->max_points, b->max_points / 32 + 1));
   CS_CREATE_CUDA(b, alloc(b->d_checksum, 1));
-  CS_CREATE_CUDA(b, wedge_allow_shared_memory());
   const int min_cand = cs_s2_min_cand(b->flags, n_sessions);
   if (n_sessions > 1 && min_cand > 0 && n_cand + 1 >= min_cand && n_cand + 1 <= CS_SORT_THREADS * CS_SORT_REG) {
     b->s2_cap = n_cand + 1;

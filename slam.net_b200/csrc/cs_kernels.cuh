@@ -195,10 +195,8 @@ struct CsStepArgs {  // by-value kernel argument; session j uses element j of ev
   int w_slot;                    // which third of CsSession::w_top this step counts into (rotates per drawn step)
   int w_prev;                    // the third the previous drawn step counted into (its counts size this step's wedges); -1: none
   int w_zero;                    // the third the next drawn step will count into (zeroed by this step)
-  int w_general;                 // diagnostics: 1 = every task of the wedge integration takes the general path
-  int w_sub_max;                 // most warps the rings of one task are split over (0: 8)
   int w_prefetch;                // the map around the pose is pulled into L2 — 1: by the candidate sort, 2: by the draw kernel's
-                                 // blocks while they wait, 3: (batches) along every ray
+                                 // blocks while they wait
   int empty_cloud;               // 1: the scan has no points and the step searches: no search kernel ran, the arg-min is
                                  // (int.MaxValue, searchPose) by definition (:251-258, :630-648)
   int s2_batch;                  // 1: a batch of sessions (session = blockIdx.z of the search, blockIdx.y of the sort): the values

@@ -81,7 +81,6 @@ struct CsWPrepared {
   float key;
   int dxc;     // -1: the ray draws nothing
   int bm;      // largest dxc of the warp's rays
-  int dyc, flags;  // (of the ray, for cs_w_prefetch_ray)
 };
 __device__ __forceinline__ CsWPrepared cs_w_prepare(CsSession& S, const CsRayFrame& f, const float2 p, int i, bool in_range,
                                                     long long& visits) {
@@ -113,27 +112,7 @@ __device__ __forceinline__ CsWPrepared cs_w_prepare(CsSession& S, const CsRayFra
   }
   CsWPrepared out;
   out.key = key; out.dxc = valid ? r.dxc : -1; out.bm = bm;
-  out.dyc = r.dyc; out.flags = r.flags;
   return out;
-}
-
-// The tiles a ray crosses, to L2 (tiled maps): one prefetch per 8 major steps.  Run by the ray's preparing thread right after the
-// rays are announced, in batches of sessions — there every session's map comes from HBM (the maps of a batch are many times
-// the L2), and the draw tasks, which start a few microseconds later, otherwise pay the DRAM latency once per group of rings.
-__device__ __forceinline__ void cs_w_prefetch_ray(const uint16_t* __restrict__ map, const CsWPrepared& q, int x1, int y1, int size,
-                                                  int pitch_tiles) {
-  if (q.dxc < 1) return;
-  const bool steep = (q.flags & 2) != 0;
-  const int smaj = (q.flags & 4) ? -1 : 1, smin = (q.flags & 8) ? -1 : 1;
-  const float slope = (float)min(q.dyc, q.dxc) / (float)q.dxc;
-  for (int t = 4; t <= q.dxc; t += 8) {
-    const int m = (int)(slope * (float)t + 0.5f);
-    const int x = x1 + (steep ? smin * m : smaj * t), y = y1 + (steep ? smaj * t : smin * m);
-    if ((unsigned)x < (unsigned)size && (unsigned)y < (unsigned)size) {
-      const uint16_t* line = map + ((size_t)(y >> 3) * pitch_tiles + (x >> 3)) * 64;
-      asm volatile("prefetch.global.L2 [%0];" ::"l"(line));
-    }
-  }
 }
 
 // Counts for sizing the wedges: per level the rays that reach it, in all and per key sector.  The lanes of a sector add as
@@ -623,7 +602,7 @@ __device__ void cs_w_fast(const CsSession& S, uint16_t* __restrict__ map, const 
 // price of fetching the rays of the non-candidates of the batches looked at — the latency instance of the kernel does it.
 template <bool TILED, bool PRELOAD>
 __device__ void cs_w_run(const CsSession& S, uint16_t* __restrict__ map, int ka, int kb, unsigned blo, unsigned bhi, int n, int x1,
-                         int y1, int size, int pitch_tiles, int alpha, int force_general, unsigned* s_val, uint32_t* s_cell, int* s_list,
+                         int y1, int size, int pitch_tiles, int alpha, unsigned* s_val, uint32_t* s_cell, int* s_list,
                          unsigned* s_bmap, long long* tl) {
   const unsigned full = 0xffffffffu;
   const int lane = threadIdx.x & 31;
@@ -681,11 +660,11 @@ __device__ void cs_w_run(const CsSession& S, uint16_t* __restrict__ map, int ka,
     if (tl && lane == 0 && tl_pieces == 0) tl[1] = cs_globaltimer();
     tl_pieces++;
     tl_cand = max(tl_cand, ncand);
-    if (ncand > 32 || force_general) tl_mode = 1;
+    if (ncand > 32) tl_mode = 1;
     if (ncand > 0) {
       t.k1 = min(t.k1, kmax);
       __syncwarp();
-      if (ncand <= 32 && !force_general)
+      if (ncand <= 32)
         cs_w_fast<TILED>(S, map, t, ncand, s_list, PRELOAD ? reinterpret_cast<const int4*>(s_cell) : nullptr, x1, y1, size, pitch_tiles, alpha);
       else
         cs_w_general<TILED>(S, map, t, n, x1, y1, size, pitch_tiles, alpha, s_val, s_cell, s_bmap, nw);
@@ -774,9 +753,8 @@ cs_wedge_kernel(CsSession* __restrict__ sessions, CsStepArgs a) {
       // most one sub-task per warp of the grid — a small scan is a latency chain: shorter tasks end it sooner, and equal lengths
       // keep the 64-ring outer levels from ending it; a big scan is throughput: whole levels amortise a task's set-up.
       const int slots = (int)gridDim.x * CS_W_WARPS;
-      const int sub_max = a.w_sub_max > 0 ? a.w_sub_max : 16;
       int rlen = 64;
-      for (int r = 64 / sub_max; r < 64; r *= 2) {
+      for (int r = 4; r < 64; r *= 2) {
         int cnt = 0;
         for (int L0 = 0; L0 < NL; L0 += 32) {
           const int L = L0 + lane;
@@ -860,7 +838,6 @@ cs_wedge_kernel(CsSession* __restrict__ sessions, CsStepArgs a) {
     __threadfence();  // this thread's stores (and counts) are visible device-wide before the block's arrival is counted
     __syncthreads();
     if (tid < copies) atomicAdd(S.prep_words + ((size_t)slot * copies + tid) * 16, 1ull);
-    if (TILED && a.w_prefetch == 3 && my_warp) cs_w_prefetch_ray(map, q, f.x1, f.y1, size, pitch_tiles);
     // off the critical path: the counts that size the next scan's wedges, and the visit count
     if (my_warp && a.w_prev >= 0) cs_w_count(S, q, top);
 #pragma unroll
@@ -999,7 +976,7 @@ cs_wedge_kernel(CsSession* __restrict__ sessions, CsStepArgs a) {
       if (!ok) continue;
       long long* tl = (a.diag && sj == 0 && stask < a.diag_rings) ? a.diag + (size_t)stask * 8 : nullptr;
       if (tl && lane == 0) { tl[0] = cs_globaltimer(); tl[4] = t_start; tl[5] = t_prep; tl[6] = t_sched; tl[7] = cs_smid() | ((long long)blockIdx.x << 16); }
-      cs_w_run<TILED, RESIDENT == 3>(S, map, ka, kb, blo, bhi, n, x1, y1, size, pitch_tiles, alpha, a.w_general, s_val[warp], s_cell[warp],
+      cs_w_run<TILED, RESIDENT == 3>(S, map, ka, kb, blo, bhi, n, x1, y1, size, pitch_tiles, alpha, s_val[warp], s_cell[warp],
                       s_list[warp], s_bmap[warp], tl);
     }
   } else {
@@ -1016,7 +993,7 @@ cs_wedge_kernel(CsSession* __restrict__ sessions, CsStepArgs a) {
       if (!decode(stask, ka, kb, blo, bhi)) continue;
       long long* tl = (a.diag && sj == 0 && stask < a.diag_rings) ? a.diag + (size_t)stask * 8 : nullptr;
       if (tl && lane == 0) { tl[0] = cs_globaltimer(); tl[4] = t_start; tl[5] = t_prep; tl[6] = t_sched; tl[7] = cs_smid() | ((long long)blockIdx.x << 16); }
-      cs_w_run<TILED, RESIDENT == 3>(S, map, ka, kb, blo, bhi, n, x1, y1, size, pitch_tiles, alpha, a.w_general, s_val[warp], s_cell[warp],
+      cs_w_run<TILED, RESIDENT == 3>(S, map, ka, kb, blo, bhi, n, x1, y1, size, pitch_tiles, alpha, s_val[warp], s_cell[warp],
                       s_list[warp], s_bmap[warp], tl);
     }
   }
