@@ -216,6 +216,63 @@ namespace CoreSLAM.B200
             return hits.Take(n).ToArray();
         }
 
+        /// <summary>Relocalize with the last few scans: scans[k] is ScanCloud.Points of scan k (oldest first, at most
+        /// Native.SequenceMaxScans), odometry[k] the odometry pose it came with.  The lattice pose is the pose of the last scan;
+        /// the others are placed by their odometry relative to it, and a pose's distance is the sum of the scans' distances.
+        /// Places one scan cannot tell apart (repeated doors, identical rooms) are told apart.  Adopt a hit with
+        /// ResumeAt(hit pose, odometry[last]).  Changes nothing.</summary>
+        public CsLatticeHit[] RelocalizeSequence(Vector2[][] scans, Vector3[] odometry, Vector3 origin, Vector3 step, int countX, int countY,
+                                                 int countTheta, int window, int k, int[] distances = null)
+        {
+            var lattice = SequenceLattice(scans, odometry, origin, step, countX, countY, countTheta, out var points, out var first, out var odo);
+            if (distances != null && distances.LongLength != (long)countX * countY * countTheta)
+                throw new ArgumentException("distances needs countX*countY*countTheta entries");
+            var hits = new CsLatticeHit[Native.LatticeMaxHits];
+            int n;
+            fixed (Vector2* p = points)
+            fixed (int* f = first)
+            fixed (float* o = odo)
+            fixed (CsLatticeHit* h = hits)
+            fixed (int* d = distances)
+                Native.Check(Native.cs_relocalize_sequence(handle, (float*)p, f, o, scans.Length, ref lattice, window, k, h, out n, d), handle);
+            return hits.Take(n).ToArray();
+        }
+
+        /// <summary>RelocalizeSequence's hits by branch and bound, for fine lattices over the whole map.</summary>
+        public CsLatticeHit[] RelocalizeSequenceBounded(Vector2[][] scans, Vector3[] odometry, Vector3 origin, Vector3 step, int countX,
+                                                        int countY, int countTheta, int window, int k, out CsRelocalizeStats stats)
+        {
+            var lattice = SequenceLattice(scans, odometry, origin, step, countX, countY, countTheta, out var points, out var first, out var odo);
+            var hits = new CsLatticeHit[Native.LatticeMaxHits];
+            int n;
+            CsRelocalizeStats st;
+            fixed (Vector2* p = points)
+            fixed (int* f = first)
+            fixed (float* o = odo)
+            fixed (CsLatticeHit* h = hits)
+                Native.Check(Native.cs_relocalize_sequence_bounded(handle, (float*)p, f, o, scans.Length, ref lattice, window, k, h, out n, &st),
+                             handle);
+            stats = st;
+            return hits.Take(n).ToArray();
+        }
+
+        // the lattice, and the scans back to back with their first points and odometry as cs_relocalize_sequence* take them
+        private static CsLattice SequenceLattice(Vector2[][] scans, Vector3[] odometry, Vector3 origin, Vector3 step, int countX, int countY,
+                                                 int countTheta, out Vector2[] points, out int[] first, out float[] odo)
+        {
+            if (odometry.Length != scans.Length) throw new ArgumentException("odometry needs one pose per scan");
+            first = new int[scans.Length + 1];
+            for (int s = 0; s < scans.Length; s++) first[s + 1] = first[s] + scans[s].Length;
+            points = scans.SelectMany(x => x).ToArray();
+            odo = new float[3 * scans.Length];
+            for (int s = 0; s < scans.Length; s++) { odo[3 * s] = odometry[s].X; odo[3 * s + 1] = odometry[s].Y; odo[3 * s + 2] = odometry[s].Z; }
+            var lattice = new CsLattice();
+            lattice.Origin[0] = origin.X; lattice.Origin[1] = origin.Y; lattice.Origin[2] = origin.Z;
+            lattice.Step[0] = step.X; lattice.Step[1] = step.Y; lattice.Step[2] = step.Z;
+            lattice.Count[0] = countX; lattice.Count[1] = countY; lattice.Count[2] = countTheta;
+            return lattice;
+        }
+
         /// <summary>Continue tracking from `pose` (e.g. the best Relocalize hit, refined): odometryPose is the odometry of the
         /// scan that pose belongs to.  The next Update searches around pose + (odometry - odometryPose).</summary>
         public void ResumeAt(Vector3 pose, Vector3 odometryPose)

@@ -81,6 +81,7 @@ namespace CoreSLAM.B200
         public const int LatticeMaxHits = 64;         // CS_LATTICE_MAX_HITS
         public const int LatticeMaxPosesBounded = 2147483647;  // CS_LATTICE_MAX_POSES_BOUNDED
         public const int LatticeBoundedMaxNodes = 1 << 20;     // CS_LATTICE_BOUNDED_MAX_NODES
+        public const int SequenceMaxScans = 32;                 // CS_SEQUENCE_MAX_SCANS
 
         private const string Lib = "coreslam_b200";   // libcoreslam_b200.so / coreslam_b200.dll
 
@@ -112,6 +113,14 @@ namespace CoreSLAM.B200
         [DllImport(Lib)] public static extern CsStatus cs_relocalize_bounded(IntPtr h, float* pointsXY, int nPoints, ref CsLattice lattice,
                                                                              int window, int k, CsLatticeHit* hits, out int nHits,
                                                                              CsRelocalizeStats* stats);
+        // the same two searches scoring each pose with nScans scans (points back to back, scan k owning
+        // [scanFirst[k], scanFirst[k+1])) placed by their odometry (3 floats each) relative to the last scan's
+        [DllImport(Lib)] public static extern CsStatus cs_relocalize_sequence(IntPtr h, float* pointsXY, int* scanFirst, float* odometry3,
+                                                                              int nScans, ref CsLattice lattice, int window, int k,
+                                                                              CsLatticeHit* hits, out int nHits, int* distances);
+        [DllImport(Lib)] public static extern CsStatus cs_relocalize_sequence_bounded(IntPtr h, float* pointsXY, int* scanFirst, float* odometry3,
+                                                                                      int nScans, ref CsLattice lattice, int window, int k,
+                                                                                      CsLatticeHit* hits, out int nHits, CsRelocalizeStats* stats);
         [DllImport(Lib)] public static extern CsStatus cs_integrate(IntPtr h, float* pointsXY, int nPoints, float* pose3,
                                                                     float* poseCosSin, long* visits);
         [DllImport(Lib)] public static extern CsStatus cs_sync(IntPtr h);

@@ -229,6 +229,46 @@ cs_status cs_relocalize_bounded(cs_processor* h, const float* points, int32_t n_
                                 int32_t window, int32_t k, cs_lattice_hit* hits, int32_t* n_hits,
                                 cs_relocalize_stats* stats /* optional */);
 
+/* cs_relocalize_sequence and cs_relocalize_sequence_bounded score every lattice pose with the last few scans instead of
+ * one: a hypothesis that fits the newest scan but not what the robot saw a little earlier is rejected, which a single
+ * scan cannot do in corridors of repeated doors, rows of shelves or identical rooms.
+ *   Scans         K = n_scans scans, 1 <= K <= CS_SEQUENCE_MAX_SCANS.  points holds them back to back as (x, y) in metres,
+ *                 each in its own lidar frame (ScanCloud.Points); scan k owns points [scan_first[k], scan_first[k+1]),
+ *                 scan_first[0] = 0.  odometry[3k .. 3k+2] is the odometry pose of scan k.
+ *   Anchor        the lattice pose is the pose of the LAST scan, a = odometry[K-1], so a hit is the pose to resume at:
+ *                 cs_set_pose(hit.pose, odometry[K-1], ...).  Relative motion is SE(2) composition (the odometry frame's
+ *                 heading may be unrelated to the map's).  All f32, one rounding per operation in this order, no FMA,
+ *                 cosf/sinf the library's libm-identical ones.  Per scan k, once per call:
+ *                   ca = cosf(a.theta), sa = sinf(a.theta), ex = o_k.x - a.x, ey = o_k.y - a.y,
+ *                   dx_k = ca*ex + sa*ey, dy_k = ca*ey - sa*ex, dtheta_k = o_k.theta - a.theta.
+ *                 At lattice pose (x, y, theta), with c = cosf(theta), s = sinf(theta) unscaled:
+ *                   x_k = x + (c*dx_k - s*dy_k), y_k = y + (s*dx_k + c*dy_k), theta_k = theta + dtheta_k.
+ *   Distance      D = sum over k of d_k, d_k exactly what cs_search returns for scan k at (x_k, y_k, theta_k) as an absolute
+ *                 candidate (the sum divided by scan k's point count); INT32_MAX when some d_k is INT32_MAX.  D <= 32 *
+ *                 1024 * 65535 = 2147450880 < INT32_MAX.
+ *                 At K = 1 every scan sits at the lattice pose: the volume and hits are bit-identical to cs_relocalize's
+ *                 (and the bounded call's hits to cs_relocalize_bounded's), whatever the odometry; such a call runs the
+ *                 single-scan kernels.
+ *   Lattice, window, k, selection, hit order, state, distances and stats
+ *                 as cs_relocalize (cs_relocalize_sequence) and cs_relocalize_bounded (cs_relocalize_sequence_bounded).
+ *                 stats.evaluated counts poses, not (pose, scan) pairs.  The bounded call's node bound is the sum of the
+ *                 scans' bounds; a node where some scan lies wholly off the map at every pose is dropped at any U.
+ *   Errors        as those calls, and CS_ERR_INVALID_ARGUMENT for NULL scan_first or odometry, n_scans outside
+ *                 1..CS_SEQUENCE_MAX_SCANS, scan_first[0] != 0, a scan with fewer than 1 point or a non-finite odometry
+ *                 value; CS_ERR_CAPACITY for a scan with more than max_points points.  The handle stays usable.
+ *   Cost          grows with K: about K times the single-scan call, more when the bounded call needs another pass
+ *                 (DESIGN section 5); the concatenated scans go to device scratch
+ *                 that the handle keeps (8 B per point). */
+#define CS_SEQUENCE_MAX_SCANS 32
+
+cs_status cs_relocalize_sequence(cs_processor* h, const float* points, const int32_t* scan_first, const float* odometry,
+                                 int32_t n_scans, const cs_lattice* lattice, int32_t window, int32_t k,
+                                 cs_lattice_hit* hits, int32_t* n_hits,
+                                 int32_t* distances /* optional: count[0]*count[1]*count[2] values in flat order */);
+cs_status cs_relocalize_sequence_bounded(cs_processor* h, const float* points, const int32_t* scan_first, const float* odometry,
+                                         int32_t n_scans, const cs_lattice* lattice, int32_t window, int32_t k,
+                                         cs_lattice_hit* hits, int32_t* n_hits, cs_relocalize_stats* stats /* optional */);
+
 /* UpdateHoleMap (:496-534) + DrawLaserRayOnHoleMap (:359-443) + ClipRay (:320-345) for an explicit
  * pose; uses the handle's HoleWidth and Quality.  pose_cs: optional host (cos, sin) of pose[2].
  * Asynchronous: returns after enqueueing; visits (optional) forces a wait for the count.            */

@@ -134,6 +134,7 @@ LATTICE_MAX_POSES = 1 << 28
 LATTICE_MAX_HITS = 64
 LATTICE_MAX_POSES_BOUNDED = 2147483647
 LATTICE_BOUNDED_MAX_NODES = 1 << 20
+SEQUENCE_MAX_SCANS = 32
 
 FLAG_ROW_MAJOR_MAP = 0x1
 FLAG_TIMING = 0x2
@@ -177,6 +178,10 @@ SIGNATURES = {
                                 _ip]),
     "cs_relocalize_bounded": (C.c_int, [_vp, _fp, C.c_int32, C.POINTER(Lattice), C.c_int32, C.c_int32, C.POINTER(LatticeHit),
                                         _ip, C.POINTER(RelocalizeStats)]),
+    "cs_relocalize_sequence": (C.c_int, [_vp, _fp, _ip, _fp, C.c_int32, C.POINTER(Lattice), C.c_int32, C.c_int32,
+                                         C.POINTER(LatticeHit), _ip, _ip]),
+    "cs_relocalize_sequence_bounded": (C.c_int, [_vp, _fp, _ip, _fp, C.c_int32, C.POINTER(Lattice), C.c_int32, C.c_int32,
+                                                 C.POINTER(LatticeHit), _ip, C.POINTER(RelocalizeStats)]),
     "cs_integrate": (C.c_int, [_vp, _fp, C.c_int32, _fp, _fp, C.POINTER(C.c_int64)]),
     "cs_update": (C.c_int, [_vp, _fp, C.c_int32, _fp, _fp, C.POINTER(Result)]),
     "cs_update_segments": (C.c_int, [_vp, _fp, _ip, _fp, C.c_int32, C.c_int32, _fp, C.POINTER(Result)]),

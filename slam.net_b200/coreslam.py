@@ -304,6 +304,52 @@ class Processor:
                for i in range(n.value)]
         return out, {f: int(getattr(st, f)) for f, _ in N.RelocalizeStats._fields_ if f != "reserved"}
 
+    @staticmethod
+    def _sequence(scans, odometry):
+        """scans (K arrays of (x, y) points) and odometry (K poses) -> the concatenated points, scan_first and odometry"""
+        pts = [_f32(p).reshape(-1, 2) for p in scans]
+        first = np.zeros(len(pts) + 1, dtype=np.int32)
+        first[1:] = np.cumsum([p.shape[0] for p in pts])
+        cat = np.ascontiguousarray(np.concatenate(pts) if pts else np.zeros((0, 2), np.float32))
+        odo = _f32(odometry).reshape(-1, 3)
+        if odo.shape[0] != len(pts):
+            raise ValueError("odometry needs one pose per scan")
+        return cat, first, odo
+
+    def relocalize_sequence(self, scans, odometry, origin, step, count, window: int = 0, k: int = 1, want_distances=False):
+        """cs_relocalize_sequence: relocalize with the last few scans.  scans: K <= SEQUENCE_MAX_SCANS arrays of points,
+        each in its own lidar frame, oldest first; odometry: their K odometry poses.  The lattice pose is the pose of the
+        last scan; every other scan is placed by its odometry relative to the last, and a pose's distance is the sum of
+        the scans' distances (include/coreslam_b200.h).  Returns (hits, volume) as relocalize."""
+        pts, first, odo = self._sequence(scans, odometry)
+        lat = self._lattice(origin, step, count)
+        hits = (N.LatticeHit * N.LATTICE_MAX_HITS)()
+        n = C.c_int32(0)
+        vol = None
+        if want_distances and min(lat.count) >= 1 and lat.count[0] * lat.count[1] * lat.count[2] <= N.LATTICE_MAX_POSES:
+            vol = np.empty((lat.count[2], lat.count[1], lat.count[0]), dtype=np.int32)  # (else the call fails)
+        self._ck(N.lib().cs_relocalize_sequence(self._h, _ptr(pts), first.ctypes.data_as(C.POINTER(C.c_int32)), _ptr(odo),
+                                                len(first) - 1, C.byref(lat), int(window), int(k), hits, C.byref(n),
+                                                None if vol is None else vol.ctypes.data_as(C.POINTER(C.c_int32))))
+        out = [LatticeHit(np.array(list(hits[i].pose), dtype=np.float32), int(hits[i].distance), int(hits[i].index))
+               for i in range(n.value)]
+        return out, vol
+
+    def relocalize_sequence_bounded(self, scans, odometry, origin, step, count, window: int = 0, k: int = 1):
+        """cs_relocalize_sequence_bounded: the hits of relocalize_sequence by branch and bound, on lattices of up to
+        LATTICE_MAX_POSES_BOUNDED poses.  Returns (hits, stats) as relocalize_bounded."""
+        pts, first, odo = self._sequence(scans, odometry)
+        lat = self._lattice(origin, step, count)
+        hits = (N.LatticeHit * N.LATTICE_MAX_HITS)()
+        n = C.c_int32(0)
+        st = N.RelocalizeStats()
+        self._ck(N.lib().cs_relocalize_sequence_bounded(self._h, _ptr(pts), first.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                        _ptr(odo), len(first) - 1, C.byref(lat), int(window), int(k), hits,
+                                                        C.byref(n), C.byref(st)))
+        out = [LatticeHit(np.array(list(hits[i].pose), dtype=np.float32), int(hits[i].distance), int(hits[i].index))
+               for i in range(n.value)]
+        return out, {f: int(getattr(st, f)) for f, _ in N.RelocalizeStats._fields_ if f != "reserved"}
+
     def integrate(self, points, pose, pose_cs=None, wait=True) -> int:
         pts = _f32(points).reshape(-1, 2)
         v = C.c_int64(-1)
@@ -774,6 +820,16 @@ class CoreSLAMProcessor:
         """Relocalize's hits by branch and bound (Processor.relocalize_bounded), for fine lattices over a whole map.
         Returns (hits, stats).  Changes nothing; adopt a hit with ResumeAt."""
         return self._proc.relocalize_bounded(points, origin, step, count, window, k)
+
+    def RelocalizeSequence(self, scans, odometry, origin, step, count, window: int = 0, k: int = 1, want_distances=False):
+        """Relocalize with the last few scan clouds and the odometry poses they came with (Processor.relocalize_sequence),
+        so that places that look alike to one scan are told apart.  A hit is the pose of the last scan: adopt it with
+        ResumeAt(hit.pose, odometry[-1]).  Changes nothing."""
+        return self._proc.relocalize_sequence(scans, odometry, origin, step, count, window, k, want_distances)
+
+    def RelocalizeSequenceBounded(self, scans, odometry, origin, step, count, window: int = 0, k: int = 1):
+        """RelocalizeSequence's hits by branch and bound (Processor.relocalize_sequence_bounded).  Returns (hits, stats)."""
+        return self._proc.relocalize_sequence_bounded(scans, odometry, origin, step, count, window, k)
 
     def ResumeAt(self, pose, odometryPose):
         """Continue tracking from `pose` (e.g. a Relocalize hit): the next Update searches around

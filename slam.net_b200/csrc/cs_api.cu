@@ -33,6 +33,7 @@ static_assert(sizeof(cs_config) == 72, "cs_config layout (ctypes / P/Invoke mirr
 static_assert(sizeof(CsStepHeader) == 48, "CsStepHeader");
 static_assert(sizeof(cs_lattice) == 36 && sizeof(cs_lattice_hit) == 20, "cs_lattice layout (ctypes / P/Invoke mirror it)");
 static_assert(sizeof(cs_relocalize_stats) == 40, "cs_relocalize_stats layout (ctypes / P/Invoke mirror it)");
+static_assert(CS_LAT_SEQ_MAX == CS_SEQUENCE_MAX_SCANS && CS_SEQUENCE_MAX_SCANS <= CS_LAT_THREADS, "one thread per scan of a sequence");
 
 namespace {
 
@@ -224,6 +225,13 @@ struct cs_processor : CsHost {
   DevBuf<int> d_bnb_slot;
   size_t bnb_slot_cap = 0;
   DevBuf<unsigned long long> d_bnb_counters;
+  // cs_relocalize_sequence*: the concatenated scans (grow on demand), the odometry and scan_first as passed, and the
+  // per-scan records the kernels read (CS_SEQUENCE_MAX_SCANS each, allocated on first use)
+  DevBuf<float2> d_seq_points;
+  size_t seq_points_cap = 0;
+  DevBuf<float> d_seq_odometry;
+  DevBuf<int> d_seq_first;
+  DevBuf<CsSeqScan> d_seq_scans;
 
   // staging: [hdr 64][points][cand][cand_cs]; segments path: [hdr 64][rays][seg_first][seg_poses][cand]
   size_t stage_bytes = 0;
@@ -1412,12 +1420,39 @@ cs_status cs_search(cs_processor* h, const float* points, int32_t n_points, cons
 // window minima (select + merge kernels, see cs_lattice.cuh).  Reads the map as the stream leaves it; writes only its own
 // scratch.
 
-// The argument checks of cs_relocalize and cs_relocalize_bounded; *total: the poses of the lattice (counting stops past
-// max_poses).
-static cs_status check_relocalize(cs_processor* h, const char* name, const float* points, int32_t n_points, const cs_lattice* lattice,
+// The scans of a relocalisation: one scan (cs_relocalize, cs_relocalize_bounded) or a sequence of n_scans whose points
+// are back to back, scan k owning [scan_first[k], scan_first[k+1]), with the odometry pose of each
+// (cs_relocalize_sequence*; n_points is set from scan_first by check_relocalize).
+struct RelocScans {
+  bool seq;
+  const float* points;
+  int32_t n_points;
+  const int32_t* scan_first;
+  const float* odometry;
+  int32_t n_scans;
+};
+
+// The argument checks of the relocalisation calls; *total: the poses of the lattice (counting stops past max_poses).
+static cs_status check_relocalize(cs_processor* h, const char* name, RelocScans& sc, const cs_lattice* lattice,
                                   int32_t window, int32_t k, const cs_lattice_hit* hits, const int32_t* n_hits, long long max_poses,
                                   const char* max_name, long long* total) {
-  if (!points || !lattice || !hits || !n_hits || n_points <= 0) return fail(h, CS_ERR_INVALID_ARGUMENT, "%s: bad argument", name);
+  const bool seq = sc.seq;
+  if (!sc.points || !lattice || !hits || !n_hits || (!seq && sc.n_points <= 0)) return fail(h, CS_ERR_INVALID_ARGUMENT, "%s: bad argument", name);
+  long long most = sc.n_points;  // points of the largest scan
+  if (seq) {
+    if (!sc.scan_first || !sc.odometry) return fail(h, CS_ERR_INVALID_ARGUMENT, "%s: bad argument", name);
+    if (sc.n_scans < 1 || sc.n_scans > CS_SEQUENCE_MAX_SCANS)
+      return fail(h, CS_ERR_INVALID_ARGUMENT, "%s: n_scans %d outside 1..%d", name, sc.n_scans, CS_SEQUENCE_MAX_SCANS);
+    if (sc.scan_first[0] != 0) return fail(h, CS_ERR_INVALID_ARGUMENT, "%s: scan_first[0] = %d != 0", name, sc.scan_first[0]);
+    most = 0;
+    for (int s = 0; s < sc.n_scans; s++) {
+      const long long n = (long long)sc.scan_first[s + 1] - sc.scan_first[s];
+      if (n < 1) return fail(h, CS_ERR_INVALID_ARGUMENT, "%s: scan %d has %lld points", name, s, n);
+      most = std::max(most, n);
+    }
+    for (int i = 0; i < 3 * sc.n_scans; i++)
+      if (!std::isfinite(sc.odometry[i])) return fail(h, CS_ERR_INVALID_ARGUMENT, "%s: odometry[%d][%d] not finite", name, i / 3, i % 3);
+  }
   if (window < 0) return fail(h, CS_ERR_INVALID_ARGUMENT, "%s: window %d < 0", name, window);
   if (k < 1 || k > CS_LATTICE_MAX_HITS)
     return fail(h, CS_ERR_INVALID_ARGUMENT, "%s: k %d outside 1..%d", name, k, CS_LATTICE_MAX_HITS);
@@ -1430,21 +1465,57 @@ static cs_status check_relocalize(cs_processor* h, const char* name, const float
     t *= lattice->count[a];
     if (t > max_poses) break;
   }
-  if (n_points > h->max_points) return fail(h, CS_ERR_CAPACITY, "n_points %d > max_points %d", n_points, h->max_points);
+  if (most > h->max_points) return fail(h, CS_ERR_CAPACITY, "n_points %lld > max_points %d", most, h->max_points);
   if (t > max_poses) return fail(h, CS_ERR_CAPACITY, "%s: more than %s = %lld poses", name, max_name, max_poses);
+  if (seq) sc.n_points = sc.scan_first[sc.n_scans];
+  // one scan sits at the lattice pose itself (its offset is +-0 and its heading change +0, which changes no cell): the
+  // single-scan kernels give the same distances bit for bit, without the sequence's set-up
+  if (seq && sc.n_scans == 1) sc.seq = false;
   *total = t;
   return CS_OK;
 }
 
-// cs_lattice_kernel's arguments for the handle's map, the scan in d_lat_points and the lattice (no output set)
-static CsLatticeArgs lattice_args(const cs_processor* h, const cs_lattice* lattice, int32_t n_points) {
+// The scans to the device: a single scan to d_lat_points, a sequence to d_seq_points with its records in d_seq_scans
+// (cs_seq_offsets_kernel).  Sets the points and sequence fields of *a.
+static cs_status upload_reloc_scans(cs_processor* h, const char* name, const RelocScans& sc, CsLatticeArgs* a) {
+  const bool seq = sc.seq;
+  {
+    cudaError_t e = cudaSuccess;
+    if (!seq && !h->d_lat_points) e = alloc(h->d_lat_points, (size_t)h->max_points);
+    if (seq) {
+      e = grow(h->d_seq_points, h->seq_points_cap, (size_t)sc.n_points);
+      if (e == cudaSuccess && !h->d_seq_scans) e = alloc(h->d_seq_odometry, 3 * CS_SEQUENCE_MAX_SCANS);
+      if (e == cudaSuccess && !h->d_seq_scans) e = alloc(h->d_seq_first, CS_SEQUENCE_MAX_SCANS + 1);
+      if (e == cudaSuccess && !h->d_seq_scans) e = alloc(h->d_seq_scans, CS_SEQUENCE_MAX_SCANS);
+    }
+    if (e != cudaSuccess) {
+      cudaGetLastError();  // (an allocation failure is not sticky: the handle stays usable)
+      return fail(h, CS_ERR_OUT_OF_MEMORY, "%s: scratch allocation failed: %s", name, cudaGetErrorString(e));
+    }
+  }
+  float2* points = seq ? h->d_seq_points.get() : h->d_lat_points.get();
+  CS_CUDA(h, cudaMemcpyAsync(points, sc.points, (size_t)sc.n_points * sizeof(float2), cudaMemcpyHostToDevice, h->stream));
+  a->points = points;
+  a->n_points = sc.n_points;
+  a->seq = CsSeqArgs{nullptr, sc.n_scans};
+  if (seq) {
+    CS_CUDA(h, cudaMemcpyAsync(h->d_seq_odometry.get(), sc.odometry, (size_t)sc.n_scans * 3 * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    CS_CUDA(h, cudaMemcpyAsync(h->d_seq_first.get(), sc.scan_first, (size_t)(sc.n_scans + 1) * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    cs_seq_offsets_kernel<<<1, CS_SEQUENCE_MAX_SCANS, 0, h->stream>>>(h->d_seq_odometry.get(), h->d_seq_first.get(), sc.n_scans, h->d_seq_scans.get());
+    h->launches++;
+    CS_CUDA(h, cudaGetLastError());
+    a->seq.scans = h->d_seq_scans.get();
+  }
+  return CS_OK;
+}
+
+// cs_lattice_kernel's arguments for the handle's map and the lattice (no scans or output set: upload_reloc_scans)
+static CsLatticeArgs lattice_args(const cs_processor* h, const cs_lattice* lattice) {
   CsLatticeArgs a{};
   a.map = h->d_map.get();
   a.size = h->size;
   a.pitch_tiles = h->pitch_tiles;
   a.scale = h->scale;
-  a.points = h->d_lat_points.get();
-  a.n_points = n_points;
   for (int q = 0; q < 3; q++) {
     a.origin[q] = lattice->origin[q];
     a.step[q] = lattice->count[q] > 1 ? lattice->step[q] : 0.f;  // (a single point sits at the origin whatever the step)
@@ -1489,33 +1560,33 @@ static size_t lattice_list_keys(int sel_blocks, int k) {
   return (size_t)sel_blocks * k + (size_t)((sel_blocks + CS_LAT_MERGE_LISTS - 1) / CS_LAT_MERGE_LISTS) * k;
 }
 
-cs_status cs_relocalize(cs_processor* h, const float* points, int32_t n_points, const cs_lattice* lattice, int32_t window,
-                        int32_t k, cs_lattice_hit* hits, int32_t* n_hits, int32_t* distances) {
-  NvtxRange nvtx_range("cs_relocalize");
+// The exhaustive search of cs_relocalize and cs_relocalize_sequence
+static cs_status relocalize(cs_processor* h, const char* name, RelocScans sc, const cs_lattice* lattice, int32_t window, int32_t k,
+                            cs_lattice_hit* hits, int32_t* n_hits, int32_t* distances) {
   CS_CHECK_HANDLE(h);
   long long total = 0;
-  if (cs_status st = check_relocalize(h, "cs_relocalize", points, n_points, lattice, window, k, hits, n_hits, CS_LATTICE_MAX_POSES,
-                                      "CS_LATTICE_MAX_POSES", &total))
+  if (cs_status st = check_relocalize(h, name, sc, lattice, window, k, hits, n_hits, CS_LATTICE_MAX_POSES, "CS_LATTICE_MAX_POSES", &total))
     return st;
 
   const int c0 = lattice->count[0], c1 = lattice->count[1], c2 = lattice->count[2];
   const int sel_blocks = lattice_sel_blocks(total);
   const size_t list_keys = (size_t)sel_blocks * k;
   {
-    cudaError_t e = h->d_lat_points ? cudaSuccess : alloc(h->d_lat_points, (size_t)h->max_points);
-    if (e == cudaSuccess) e = grow(h->d_lat_volume, h->lat_volume_cap, (size_t)total);
+    cudaError_t e = grow(h->d_lat_volume, h->lat_volume_cap, (size_t)total);
     if (e == cudaSuccess) e = grow(h->d_lat_lists, h->lat_lists_cap, lattice_list_keys(sel_blocks, k));
     if (e != cudaSuccess) {
       cudaGetLastError();  // (an allocation failure is not sticky: the handle stays usable)
-      return fail(h, CS_ERR_OUT_OF_MEMORY, "cs_relocalize: scratch allocation failed: %s", cudaGetErrorString(e));
+      return fail(h, CS_ERR_OUT_OF_MEMORY, "%s: scratch allocation failed: %s", name, cudaGetErrorString(e));
     }
   }
-  CS_CUDA(h, cudaMemcpyAsync(h->d_lat_points.get(), points, (size_t)n_points * sizeof(float2), cudaMemcpyHostToDevice, h->stream));
-
-  CsLatticeArgs a = lattice_args(h, lattice, n_points);
+  CsLatticeArgs a = lattice_args(h, lattice);
+  if (cs_status st = upload_reloc_scans(h, name, sc, &a)) return st;
   a.volume = h->d_lat_volume.get();
   const unsigned lat_blocks = (unsigned)((long long)a.tiles_x * a.tiles_y * c2);
-  dispatch_layout(h->tiled, [&](auto T) { cs_lattice_kernel<decltype(T)::value><<<lat_blocks, CS_LAT_THREADS, 0, h->stream>>>(a); });
+  dispatch_layout(h->tiled, [&](auto T) {
+    if (sc.seq) cs_lattice_kernel<decltype(T)::value, false, true><<<lat_blocks, CS_LAT_THREADS, 0, h->stream>>>(a);
+    else cs_lattice_kernel<decltype(T)::value><<<lat_blocks, CS_LAT_THREADS, 0, h->stream>>>(a);
+  });
   h->launches++;
   CS_CUDA(h, cudaGetLastError());
 
@@ -1535,27 +1606,41 @@ cs_status cs_relocalize(cs_processor* h, const float* points, int32_t n_points, 
   return CS_OK;
 }
 
+cs_status cs_relocalize(cs_processor* h, const float* points, int32_t n_points, const cs_lattice* lattice, int32_t window,
+                        int32_t k, cs_lattice_hit* hits, int32_t* n_hits, int32_t* distances) {
+  NvtxRange nvtx_range("cs_relocalize");
+  return relocalize(h, "cs_relocalize", RelocScans{false, points, n_points, nullptr, nullptr, 0}, lattice, window, k, hits, n_hits, distances);
+}
+
+cs_status cs_relocalize_sequence(cs_processor* h, const float* points, const int32_t* scan_first, const float* odometry,
+                                 int32_t n_scans, const cs_lattice* lattice, int32_t window, int32_t k, cs_lattice_hit* hits,
+                                 int32_t* n_hits, int32_t* distances) {
+  NvtxRange nvtx_range("cs_relocalize_sequence");
+  return relocalize(h, "cs_relocalize_sequence", RelocScans{true, points, 0, scan_first, odometry, n_scans}, lattice, window, k, hits, n_hits,
+                    distances);
+}
+
 // Branch and bound over the lattice (cs_bnb.cuh, DESIGN section 4): min-window grids of the map, U from one exact pose
 // per top-level node, then per pass a descent from the top level (nodes of up to 128 x 128 poses) to the 16 x 8 patches
 // of 32 x 32 tiles, the exact distances of the surviving tiles and the window test over them.  The host reads the
-// survivors' count after each level (the next launch's size).
-cs_status cs_relocalize_bounded(cs_processor* h, const float* points, int32_t n_points, const cs_lattice* lattice,
-                                int32_t window, int32_t k, cs_lattice_hit* hits, int32_t* n_hits, cs_relocalize_stats* stats) {
-  NvtxRange nvtx_range("cs_relocalize_bounded");
+// survivors' count after each level (the next launch's size).  Serves cs_relocalize_bounded and
+// cs_relocalize_sequence_bounded.
+static cs_status relocalize_bounded(cs_processor* h, const char* name, RelocScans sc, const cs_lattice* lattice, int32_t window,
+                                    int32_t k, cs_lattice_hit* hits, int32_t* n_hits, cs_relocalize_stats* stats) {
   CS_CHECK_HANDLE(h);
   long long total = 0;
-  if (cs_status st = check_relocalize(h, "cs_relocalize_bounded", points, n_points, lattice, window, k, hits, n_hits,
-                                      CS_LATTICE_MAX_POSES_BOUNDED, "CS_LATTICE_MAX_POSES_BOUNDED", &total))
+  if (cs_status st = check_relocalize(h, name, sc, lattice, window, k, hits, n_hits, CS_LATTICE_MAX_POSES_BOUNDED,
+                                      "CS_LATTICE_MAX_POSES_BOUNDED", &total))
     return st;
 
   const int c0 = lattice->count[0], c1 = lattice->count[1], c2 = lattice->count[2];
-  CsLatticeArgs a = lattice_args(h, lattice, n_points);
+  CsLatticeArgs a = lattice_args(h, lattice);
   if (c0 > (1 << 30) || c1 > (1 << 30))  // (the last tile's indices must stay ints)
-    return fail(h, CS_ERR_CAPACITY, "cs_relocalize_bounded: count[0] = %d or count[1] = %d > 2^30", c0, c1);
+    return fail(h, CS_ERR_CAPACITY, "%s: count[0] = %d or count[1] = %d > 2^30", name, c0, c1);
   const long long n_tiles = (long long)a.tiles_x * a.tiles_y * c2;
   if (n_tiles > (1ll << 28))
-    return fail(h, CS_ERR_CAPACITY, "cs_relocalize_bounded: %lld tiles of 32 x 32 poses > 2^28 (count[0], count[1] too small for %d headings)",
-                n_tiles, c2);
+    return fail(h, CS_ERR_CAPACITY, "%s: %lld tiles of 32 x 32 poses > 2^28 (count[0], count[1] too small for %d headings)",
+                name, n_tiles, c2);
   // top level: the smallest power-of-two node (32 .. 128 poses a side) that covers the lattice's x and y, or 128
   int top = CS_BNB_LEAF_LEVEL;
   while (top < 7 && (c0 > (1 << top) || c1 > (1 << top))) top++;
@@ -1569,8 +1654,7 @@ cs_status cs_relocalize_bounded(cs_processor* h, const float* points, int32_t n_
   const size_t node_cap = (size_t)std::min<long long>(n_tiles, CS_LATTICE_BOUNDED_MAX_NODES);
   const int seed_blocks = lattice_sel_blocks(n_top);
   {
-    cudaError_t e = h->d_lat_points ? cudaSuccess : alloc(h->d_lat_points, (size_t)h->max_points);
-    if (e == cudaSuccess && !h->d_bnb_counters) e = alloc(h->d_bnb_counters, 4);
+    cudaError_t e = h->d_bnb_counters ? cudaSuccess : alloc(h->d_bnb_counters, 4);
     if (e == cudaSuccess) e = grow(h->d_bnb_grids, h->bnb_grids_cap, (size_t)(max_grid + 1) * cells);
     if (e == cudaSuccess) e = grow(h->d_bnb_seeds, h->bnb_seeds_cap, (size_t)n_top);
     if (e == cudaSuccess) e = grow(h->d_bnb_nodes, h->bnb_nodes_cap, 2 * node_cap);
@@ -1578,11 +1662,10 @@ cs_status cs_relocalize_bounded(cs_processor* h, const float* points, int32_t n_
     if (e == cudaSuccess) e = grow(h->d_lat_lists, h->lat_lists_cap, lattice_list_keys(seed_blocks, k));
     if (e != cudaSuccess) {
       cudaGetLastError();  // (an allocation failure is not sticky: the handle stays usable)
-      return fail(h, CS_ERR_OUT_OF_MEMORY, "cs_relocalize_bounded: scratch allocation failed: %s", cudaGetErrorString(e));
+      return fail(h, CS_ERR_OUT_OF_MEMORY, "%s: scratch allocation failed: %s", name, cudaGetErrorString(e));
     }
   }
-  a.points = h->d_lat_points.get();  // (allocated above on a handle's first relocalisation)
-  CS_CUDA(h, cudaMemcpyAsync(h->d_lat_points.get(), points, (size_t)n_points * sizeof(float2), cudaMemcpyHostToDevice, h->stream));
+  if (cs_status st = upload_reloc_scans(h, name, sc, &a)) return st;
 
   // the grids, rebuilt from the map as the stream leaves it
   uint16_t* grids = h->d_bnb_grids.get();
@@ -1604,7 +1687,7 @@ cs_status cs_relocalize_bounded(cs_processor* h, const float* points, int32_t n_
   b.max_grid = max_grid;
   b.scale = h->scale;
   b.points = a.points;
-  b.n_points = n_points;
+  b.n_points = a.n_points;
   for (int q = 0; q < 3; q++) b.origin[q] = a.origin[q], b.step[q] = a.step[q], b.count[q] = a.count[q];
   b.top_x = top_x;
   b.top_y = top_y;
@@ -1614,7 +1697,7 @@ cs_status cs_relocalize_bounded(cs_processor* h, const float* points, int32_t n_
   unsigned long long keys[CS_LATTICE_MAX_HITS];
   {
     b.level = top;
-    cs_bnb_seed_kernel<<<(unsigned)n_top, CS_LAT_THREADS, 0, h->stream>>>(b, h->d_bnb_seeds.get());
+    (sc.seq ? cs_bnb_seed_kernel<true> : cs_bnb_seed_kernel<false>)<<<(unsigned)n_top, CS_LAT_THREADS, 0, h->stream>>>(b, h->d_bnb_seeds.get(), a.seq);
     h->launches++;
     CS_CUDA(h, cudaGetLastError());
     unsigned long long* lists = h->d_lat_lists.get();
@@ -1646,8 +1729,9 @@ cs_status cs_relocalize_bounded(cs_processor* h, const float* points, int32_t n_
       b.level = level;
       b.out = node_buf[flip];
       b.out_cap = (int)node_cap;
-      if (level == CS_BNB_LEAF_LEVEL) cs_bnb_bound_kernel<true><<<(unsigned)n_in, CS_LAT_THREADS, 0, h->stream>>>(b);
-      else cs_bnb_bound_kernel<false><<<(unsigned)n_in, CS_LAT_THREADS, 0, h->stream>>>(b);
+      const bool leaf = level == CS_BNB_LEAF_LEVEL;
+      if (sc.seq) (leaf ? cs_bnb_bound_kernel<true, true> : cs_bnb_bound_kernel<false, true>)<<<(unsigned)n_in, CS_LAT_THREADS, 0, h->stream>>>(b, a.seq);
+      else (leaf ? cs_bnb_bound_kernel<true> : cs_bnb_bound_kernel<false>)<<<(unsigned)n_in, CS_LAT_THREADS, 0, h->stream>>>(b, a.seq);
       h->launches++;
       CS_CUDA(h, cudaGetLastError());
       CS_CUDA(h, cudaMemcpyAsync(counters, b.counters, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
@@ -1655,8 +1739,8 @@ cs_status cs_relocalize_bounded(cs_processor* h, const float* points, int32_t n_
       st.bounded += (int64_t)counters[1];
       st.evaluated += (int64_t)counters[2];
       if (counters[0] > node_cap)
-        return fail(h, CS_ERR_CAPACITY, "cs_relocalize_bounded: %llu nodes of %d x %d poses survive, more than CS_LATTICE_BOUNDED_MAX_NODES = %d",
-                    counters[0], 1 << (level - 1), 1 << (level - 1), CS_LATTICE_BOUNDED_MAX_NODES);
+        return fail(h, CS_ERR_CAPACITY, "%s: %llu nodes of %d x %d poses survive, more than CS_LATTICE_BOUNDED_MAX_NODES = %d",
+                    name, counters[0], 1 << (level - 1), 1 << (level - 1), CS_LATTICE_BOUNDED_MAX_NODES);
       n_in = (long long)counters[0];
       b.in = node_buf[flip];
       if (level == CS_BNB_LEAF_LEVEL) {
@@ -1676,7 +1760,7 @@ cs_status cs_relocalize_bounded(cs_processor* h, const float* points, int32_t n_
         if (e == cudaSuccess) e = grow(h->d_lat_lists, h->lat_lists_cap, lattice_list_keys(sel_blocks, k));
         if (e != cudaSuccess) {
           cudaGetLastError();
-          return fail(h, CS_ERR_OUT_OF_MEMORY, "cs_relocalize_bounded: scratch allocation failed: %s", cudaGetErrorString(e));
+          return fail(h, CS_ERR_OUT_OF_MEMORY, "%s: scratch allocation failed: %s", name, cudaGetErrorString(e));
         }
       }
       CS_CUDA(h, cudaMemsetAsync(h->d_bnb_slot.get(), 0xff, (size_t)n_tiles * sizeof(int), h->stream));
@@ -1685,7 +1769,8 @@ cs_status cs_relocalize_bounded(cs_processor* h, const float* points, int32_t n_
       a.tiles = b.in;
       a.tile_slot = h->d_bnb_slot.get();
       dispatch_layout(h->tiled, [&](auto T) {
-        cs_lattice_kernel<decltype(T)::value, true><<<(unsigned)n_leaves, CS_LAT_THREADS, 0, h->stream>>>(a);
+        if (sc.seq) cs_lattice_kernel<decltype(T)::value, true, true><<<(unsigned)n_leaves, CS_LAT_THREADS, 0, h->stream>>>(a);
+        else cs_lattice_kernel<decltype(T)::value, true><<<(unsigned)n_leaves, CS_LAT_THREADS, 0, h->stream>>>(a);
       });
       h->launches++;
       CS_CUDA(h, cudaGetLastError());
@@ -1707,6 +1792,21 @@ cs_status cs_relocalize_bounded(cs_processor* h, const float* points, int32_t n_
   *n_hits = lattice_hits(a, keys, k, hits);
   if (stats) *stats = st;
   return CS_OK;
+}
+
+cs_status cs_relocalize_bounded(cs_processor* h, const float* points, int32_t n_points, const cs_lattice* lattice,
+                                int32_t window, int32_t k, cs_lattice_hit* hits, int32_t* n_hits, cs_relocalize_stats* stats) {
+  NvtxRange nvtx_range("cs_relocalize_bounded");
+  return relocalize_bounded(h, "cs_relocalize_bounded", RelocScans{false, points, n_points, nullptr, nullptr, 0}, lattice, window, k,
+                            hits, n_hits, stats);
+}
+
+cs_status cs_relocalize_sequence_bounded(cs_processor* h, const float* points, const int32_t* scan_first, const float* odometry,
+                                         int32_t n_scans, const cs_lattice* lattice, int32_t window, int32_t k,
+                                         cs_lattice_hit* hits, int32_t* n_hits, cs_relocalize_stats* stats) {
+  NvtxRange nvtx_range("cs_relocalize_sequence_bounded");
+  return relocalize_bounded(h, "cs_relocalize_sequence_bounded", RelocScans{true, points, 0, scan_first, odometry, n_scans}, lattice,
+                            window, k, hits, n_hits, stats);
 }
 
 cs_status cs_integrate(cs_processor* h, const float* points, int32_t n_points, const float pose[3],

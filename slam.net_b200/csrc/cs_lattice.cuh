@@ -3,7 +3,10 @@
 // the lattice poses that are strict local minima of (distance, flat index) within a window, best first.
 //
 //   cs_lattice_kernel         distance of every lattice pose -> a volume of int32 (flat index (it*count1 + iy)*count0 + ix);
-//                             or (LIST) of the poses of listed 32 x 32 tiles -> 1024 values per tile (cs_relocalize_bounded)
+//                             or (LIST) of the poses of listed 32 x 32 tiles -> 1024 values per tile (cs_relocalize_bounded);
+//                             or (SEQ) the sum over a scan sequence, each scan placed by its odometry relative to the last
+//                             (cs_relocalize_sequence)
+//   cs_seq_offsets_kernel     the odometry of a scan sequence -> each scan's offset from the anchor (the last scan)
 //   cs_lattice_select_kernel  window test of every pose; the k best local minima of each block's poses -> one sorted list
 //   cs_lattice_select_tiles_kernel  the same over the listed tiles only (cs_relocalize_bounded, see cs_bnb.cuh)
 //   cs_lattice_merge_kernel   CS_LAT_MERGE_LISTS sorted lists -> one, until one list remains
@@ -26,6 +29,20 @@
 #define CS_LAT_SEL_PER 16       // poses per thread of the select kernel
 #define CS_LAT_MERGE_LISTS 32   // lists merged by one block of the merge kernel
 #define CS_LAT_MERGE_PER 8      // keys per thread of the merge kernel (CS_LAT_MERGE_LISTS * 64 / CS_LAT_THREADS)
+#define CS_LAT_SEQ_MAX 32       // scans of a sequence (CS_SEQUENCE_MAX_SCANS)
+
+// One scan of a sequence: its points [first, first + count) of the concatenated scans, and its odometry pose relative to
+// the anchor's (the last scan's), in the anchor's frame: with ca, sa = cosf, sinf(anchor theta), e = o - anchor,
+// dx = ca*ex + sa*ey, dy = ca*ey - sa*ex, dtheta = o.theta - anchor.theta (cs_seq_offsets_kernel).
+struct CsSeqScan {
+  int first, count;
+  float dx, dy, dtheta;
+};
+// the scans of a sequence (points index the concatenated scans)
+struct CsSeqArgs {
+  const CsSeqScan* scans;
+  int n_scans;
+};
 
 struct CsLatticeArgs {
   const uint16_t* map;
@@ -39,7 +56,26 @@ struct CsLatticeArgs {
   int* volume;
   const int4* tiles;  // LIST: the tiles to evaluate, {it, tile x, tile y, mask of the warp patches to evaluate}
   int* tile_slot;     // LIST: dense per-tile index of the lattice ((it*tiles_y + tile y)*tiles_x + tile x) -> list position
+  CsSeqArgs seq;      // SEQ: the scans of the sequence
 };
+
+// odometry[3k .. 3k+2] and scan_first[0 .. n_scans] -> out[k]; one thread per scan, one rounding per operation
+__global__ void cs_seq_offsets_kernel(const float* __restrict__ odometry, const int* __restrict__ scan_first, int n_scans,
+                                      CsSeqScan* __restrict__ out) {
+  const int k = threadIdx.x;
+  if (k >= n_scans) return;
+  const float* o = odometry + 3 * k;
+  const float* an = odometry + 3 * (n_scans - 1);
+  const float ca = cs_cosf(an[2]), sa = cs_sinf(an[2]);
+  const float ex = __fsub_rn(o[0], an[0]), ey = __fsub_rn(o[1], an[1]);
+  CsSeqScan q;
+  q.first = scan_first[k];
+  q.count = scan_first[k + 1] - q.first;
+  q.dx = __fadd_rn(__fmul_rn(ca, ex), __fmul_rn(sa, ey));
+  q.dy = __fsub_rn(__fmul_rn(ca, ey), __fmul_rn(sa, ex));
+  q.dtheta = __fsub_rn(o[2], an[2]);
+  out[k] = q;
+}
 
 // pose coordinate of lattice point i along one axis: origin + (float)i * step, two roundings, no FMA
 __host__ __device__ __forceinline__ float cs_lattice_coord(float origin, float step, int i) {
@@ -54,8 +90,9 @@ __host__ __device__ __forceinline__ float cs_lattice_coord(float origin, float s
 // The reference's arithmetic of one lookup (:232-244), shared by every kernel that evaluates or bounds lattice distances:
 // the pose x (or y) in map units, the four per-point products and the (int) cast of the cell coordinates, each operation
 // one rounding.  x is non-decreasing in px and y in py (cs_bnb.cuh relies on it).
+__device__ __forceinline__ float cs_map_p(float coord, float scale) { return __fadd_rn(__fmul_rn(coord, scale), 0.5f); }  // :232-233
 __device__ __forceinline__ float cs_lattice_p(float origin, float step, int i, float scale) {
-  return __fadd_rn(__fmul_rn(cs_lattice_coord(origin, step, i), scale), 0.5f);  // :232-233
+  return cs_map_p(cs_lattice_coord(origin, step, i), scale);
 }
 __device__ __forceinline__ float4 cs_lattice_products(float c, float s, float2 p) {
   return make_float4(__fmul_rn(c, p.x), __fmul_rn(s, p.y), __fmul_rn(s, p.x), __fmul_rn(c, p.y));
@@ -63,51 +100,45 @@ __device__ __forceinline__ float4 cs_lattice_products(float c, float s, float2 p
 __device__ __forceinline__ int cs_lattice_cell_x(float px, float4 q) { return __float2int_rz(fmaxf(__fsub_rn(__fadd_rn(px, q.x), q.y), -2.0f)); }
 __device__ __forceinline__ int cs_lattice_cell_y(float py, float4 q) { return __float2int_rz(fmaxf(__fadd_rn(__fadd_rn(py, q.z), q.w), -2.0f)); }
 
-// One block takes one 32 x 32 tile of poses of one heading: the tile blockIdx.x of the lattice, or with LIST the tile
-// a.tiles[blockIdx.x], whose warps evaluate only the 16 x 8 patches (warp w: x half w & 1, rows 8 * (w >> 1)) set in its
-// mask and write int.MaxValue for the others.  LIST writes the tile's 1024 poses (row-major, 32 per row) at
-// a.volume + 1024 * blockIdx.x and records the slot in a.tile_slot.
-template <bool TILED, bool LIST = false>
-__global__ void __launch_bounds__(CS_LAT_THREADS) cs_lattice_kernel(CsLatticeArgs a) {
-  __shared__ float4 s_prod[CS_LAT_CHUNK];  // (c*X, s*Y, s*X, c*Y) of the chunk's points
-  int it, tile_x, tile_y;
-  unsigned mask = 0xffu;
-  if (LIST) {
-    const int4 e = a.tiles[blockIdx.x];
-    it = e.x, tile_x = e.y, tile_y = e.z, mask = (unsigned)e.w;
-    if (threadIdx.x == 0) a.tile_slot[((size_t)it * a.tiles_y + tile_y) * a.tiles_x + tile_x] = (int)blockIdx.x;
-  } else {
-    const int tiles_xy = a.tiles_x * a.tiles_y;
-    it = (int)(blockIdx.x / (unsigned)tiles_xy);
-    const int tile = (int)(blockIdx.x % (unsigned)tiles_xy);
-    tile_x = tile % a.tiles_x, tile_y = tile / a.tiles_x;
-  }
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int ix = tile_x * CS_LAT_TILE_X + (warp & 1) * 16 + (lane & 15);
-  const int iy0 = tile_y * CS_LAT_TILE_Y + (warp >> 1) * 8 + (lane >> 4);  // + 2j, j < CS_LAT_PY
+// Scan q of a sequence at a lattice pose of heading theta (c0, s0 = cosf, sinf(theta), unscaled): its (c, s) scaled as in
+// :234-235 at theta + dtheta, and the offset (ox, oy) = (c0*dx - s0*dy, s0*dx + c0*dy) its pose adds to the lattice x, y.
+// The offset is the same for every (x, y) pose of the heading, so the cell of a point stays non-decreasing in ix and iy.
+struct CsSeqPose {
+  float c, s, ox, oy;
+};
+__device__ __forceinline__ CsSeqPose cs_seq_pose(float theta, float c0, float s0, float scale, const CsSeqScan& q) {
+  const float t = __fadd_rn(theta, q.dtheta);
+  CsSeqPose p;
+  p.c = __fmul_rn(cs_cosf(t), scale);
+  p.s = __fmul_rn(cs_sinf(t), scale);
+  p.ox = __fsub_rn(__fmul_rn(c0, q.dx), __fmul_rn(s0, q.dy));
+  p.oy = __fadd_rn(__fmul_rn(s0, q.dx), __fmul_rn(c0, q.dy));
+  return p;
+}
 
-  const float theta = cs_lattice_coord(a.origin[2], a.step[2], it);
-  const float c = __fmul_rn(cs_cosf(theta), a.scale);  // :234
-  const float s = __fmul_rn(cs_sinf(theta), a.scale);  // :235
-  const float px = cs_lattice_p(a.origin[0], a.step[0], ix, a.scale);  // :232
-  float py[CS_LAT_PY];
-#pragma unroll
-  for (int j = 0; j < CS_LAT_PY; j++) py[j] = cs_lattice_p(a.origin[1], a.step[1], iy0 + 2 * j, a.scale);  // :233
-  const bool inside = ix < a.count[0] && iy0 < a.count[1];
-  const bool active = inside && ((mask >> warp) & 1u);
+// Every scan's CsSeqPose at lattice heading theta into s_pose, one scan per thread, then a barrier.
+__device__ __forceinline__ void cs_seq_poses(float theta, float scale, const CsSeqArgs& seq, CsSeqPose* s_pose) {
+  if ((int)threadIdx.x < seq.n_scans) s_pose[threadIdx.x] = cs_seq_pose(theta, cs_cosf(theta), cs_sinf(theta), scale, seq.scans[threadIdx.x]);
+  __syncthreads();
+}
 
+// int.MaxValue when no point was in bounds, else floor(1024 * sum / n) (:251-258)
+__device__ __forceinline__ int cs_lattice_distance(bool any, unsigned sum, int n) {
+  return any ? (int)(((unsigned long long)sum * 1024ull) / (unsigned)n) : 2147483647;
+}
+
+// The sums of one scan's points over a thread's CS_LAT_PY poses (one x, the rows py), staged in chunks through s_prod.
+template <bool TILED>
+__device__ __forceinline__ void cs_lattice_sums(const CsLatticeArgs& a, float4* s_prod, const float2* __restrict__ points, int n_points,
+                                                float c, float s, float px, const float (&py)[CS_LAT_PY], bool active,
+                                                unsigned (&sum)[CS_LAT_PY], unsigned& in_any) {
   const int size = a.size, pitch_tiles = a.pitch_tiles;
   const uint16_t* __restrict__ map = a.map;
-  unsigned sum[CS_LAT_PY];  // <= 65535 * 65536 < 2^32 (max_points <= 65536)
-  unsigned in_any = 0;      // bit j: some point of pose j was in bounds
-#pragma unroll
-  for (int j = 0; j < CS_LAT_PY; j++) sum[j] = 0;
-
-  for (int base = 0; base < a.n_points; base += CS_LAT_CHUNK) {
-    const int n = min(CS_LAT_CHUNK, a.n_points - base);
+  for (int base = 0; base < n_points; base += CS_LAT_CHUNK) {
+    const int n = min(CS_LAT_CHUNK, n_points - base);
     __syncthreads();
     for (int i = threadIdx.x; i < n; i += CS_LAT_THREADS) {
-      s_prod[i] = cs_lattice_products(c, s, a.points[base + i]);
+      s_prod[i] = cs_lattice_products(c, s, points[base + i]);
     }
     __syncthreads();
     if (!active) continue;
@@ -127,13 +158,78 @@ __global__ void __launch_bounds__(CS_LAT_THREADS) cs_lattice_kernel(CsLatticeArg
       }
     }
   }
+}
+
+// One block takes one 32 x 32 tile of poses of one heading: the tile blockIdx.x of the lattice, or with LIST the tile
+// a.tiles[blockIdx.x], whose warps evaluate only the 16 x 8 patches (warp w: x half w & 1, rows 8 * (w >> 1)) set in its
+// mask and write int.MaxValue for the others.  LIST writes the tile's 1024 poses (row-major, 32 per row) at
+// a.volume + 1024 * blockIdx.x and records the slot in a.tile_slot.  SEQ: the distance of a pose is the sum over the scans
+// a.seq.scans[0 .. n_scans) of each scan's distance at the pose the scan's offset and heading change give it, int.MaxValue when
+// any scan has no point in bounds (<= 32 * 1024 * 65535 < 2^31 otherwise).
+template <bool TILED, bool LIST = false, bool SEQ = false>
+__global__ void __launch_bounds__(CS_LAT_THREADS) cs_lattice_kernel(CsLatticeArgs a) {
+  __shared__ float4 s_prod[CS_LAT_CHUNK];  // (c*X, s*Y, s*X, c*Y) of the chunk's points
+  int it, tile_x, tile_y;
+  unsigned mask = 0xffu;
+  if (LIST) {
+    const int4 e = a.tiles[blockIdx.x];
+    it = e.x, tile_x = e.y, tile_y = e.z, mask = (unsigned)e.w;
+    if (threadIdx.x == 0) a.tile_slot[((size_t)it * a.tiles_y + tile_y) * a.tiles_x + tile_x] = (int)blockIdx.x;
+  } else {
+    const int tiles_xy = a.tiles_x * a.tiles_y;
+    it = (int)(blockIdx.x / (unsigned)tiles_xy);
+    const int tile = (int)(blockIdx.x % (unsigned)tiles_xy);
+    tile_x = tile % a.tiles_x, tile_y = tile / a.tiles_x;
+  }
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int ix = tile_x * CS_LAT_TILE_X + (warp & 1) * 16 + (lane & 15);
+  const int iy0 = tile_y * CS_LAT_TILE_Y + (warp >> 1) * 8 + (lane >> 4);  // + 2j, j < CS_LAT_PY
+
+  const float theta = cs_lattice_coord(a.origin[2], a.step[2], it);
+  float c = 0.f, s = 0.f, px = 0.f, py[CS_LAT_PY];
+  if (!SEQ) {
+    c = __fmul_rn(cs_cosf(theta), a.scale);  // :234
+    s = __fmul_rn(cs_sinf(theta), a.scale);  // :235
+    px = cs_lattice_p(a.origin[0], a.step[0], ix, a.scale);  // :232
+#pragma unroll
+    for (int j = 0; j < CS_LAT_PY; j++) py[j] = cs_lattice_p(a.origin[1], a.step[1], iy0 + 2 * j, a.scale);  // :233
+  }
+  const bool inside = ix < a.count[0] && iy0 < a.count[1];
+  const bool active = inside && ((mask >> warp) & 1u);
+
+  unsigned sum[CS_LAT_PY];  // <= 65535 * 65536 < 2^32 (max_points <= 65536)
+  unsigned in_any = 0;      // bit j: some point of pose j was in bounds
+#pragma unroll
+  for (int j = 0; j < CS_LAT_PY; j++) sum[j] = 0;
+  unsigned total[CS_LAT_PY];  // SEQ: the sum of the scans' distances (< 2^31), or >= 2^31 once a scan had no point in bounds
+  if (SEQ) {
+    __shared__ CsSeqPose s_pose[CS_LAT_SEQ_MAX];
+    cs_seq_poses(theta, a.scale, a.seq, s_pose);
+    const float x = cs_lattice_coord(a.origin[0], a.step[0], ix);
+    float y[CS_LAT_PY];
+#pragma unroll
+    for (int j = 0; j < CS_LAT_PY; j++) y[j] = cs_lattice_coord(a.origin[1], a.step[1], iy0 + 2 * j), total[j] = 0;
+    for (int k = 0; k < a.seq.n_scans; k++) {
+      const CsSeqScan q = a.seq.scans[k];
+      const CsSeqPose p = s_pose[k];
+      px = cs_map_p(__fadd_rn(x, p.ox), a.scale);
+#pragma unroll
+      for (int j = 0; j < CS_LAT_PY; j++) py[j] = cs_map_p(__fadd_rn(y[j], p.oy), a.scale), sum[j] = 0;
+      in_any = 0;
+      cs_lattice_sums<TILED>(a, s_prod, a.points + q.first, q.count, p.c, p.s, px, py, active, sum, in_any);
+#pragma unroll
+      for (int j = 0; j < CS_LAT_PY; j++) total[j] = (in_any >> j) & 1u ? total[j] + (unsigned)cs_lattice_distance(true, sum[j], q.count) : 0x80000000u;
+    }
+  } else {
+    cs_lattice_sums<TILED>(a, s_prod, a.points, a.n_points, c, s, px, py, active, sum, in_any);
+  }
   if (!inside) return;
   const size_t plane = (size_t)it * a.count[1];
 #pragma unroll
   for (int j = 0; j < CS_LAT_PY; j++) {
     const int iy = iy0 + 2 * j;
     if (iy < a.count[1]) {
-      const int d = ((in_any >> j) & 1u) ? (int)(((unsigned long long)sum[j] * 1024ull) / (unsigned)a.n_points) : 2147483647;  // :251-258
+      const int d = SEQ ? (int)min(total[j], 2147483647u) : cs_lattice_distance((in_any >> j) & 1u, sum[j], a.n_points);
       if (LIST)
         a.volume[(size_t)blockIdx.x * (CS_LAT_TILE_X * CS_LAT_TILE_Y) + (iy - tile_y * CS_LAT_TILE_Y) * CS_LAT_TILE_X + (ix - tile_x * CS_LAT_TILE_X)] = d;
       else
